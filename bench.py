@@ -8,9 +8,14 @@ limb-tokens/sec at 1/2/4/8 B200").
 A "step" is one `Agent.update` (TD3 update, src/agent.py:117-183) on one synthetic replay
 minibatch of the named morphology (default: 3d_humanoid_9_full, N=9 limbs, B=256 — the batch
 start_humanoid.sh really samples, src/configs/default.py:61); even `it` includes the delayed
-actor step + Polyak, so K is rounded up to an even number.  N>1: one process per GPU (torchrun),
+actor step + Polyak.  --steps K timed steps run, exactly K, each from the same seeded initial
+state (restored outside the timed window).  N>1: one process per GPU (torchrun),
 every rank draws its own minibatch (weak scaling) and the flat gradient arena is all-reduced
 over NCCL before the fused clip+Adam pass.  One JSON line is printed by rank 0.
+
+--dump-outputs DIR writes what the last timed step returned and the parameters it left behind as
+DIR/<name>.npy (rank 0).  Inputs and initial weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -51,7 +56,15 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-rollout", action="store_true")
     ap.add_argument("--no-bf16", action="store_true", help="skip the separately reported BF16-input leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the last timed step's loss dict and a fixed sample of the "
+                    "updated parameters as DIR/<name>.npy; with --set and without --packed, every morphology's loss dict, its "
+                    "name as prefix (<morphology>_loss_critic_loss.npy, ...)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
 
 
 def peaks():
@@ -60,6 +73,49 @@ def peaks():
         d = json.load(open(p))
         return {"hbm_gbs": d["hbm_gbs"], "tflops_burst": d["bf16_tflops"], "tflops_sustained": d.get("bf16_tflops_sustained", d["bf16_tflops"]), "src": "measured"}
     return {"hbm_gbs": 6650.0, "tflops_burst": 1590.0, "tflops_sustained": 1400.0, "src": "fallback"}
+
+
+DUMP_SAMPLE = 1 << 21      # parameters kept per network in a dump: 4 nets x 8 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(path, ld, agent):
+    """What a caller of the timed path holds after its last step: the loss dict Agent.update returned (one .npy per key, '/'
+    -> '_', float64) and the parameters of the four networks (<net>_params.npy, float32).  An arena larger than DUMP_SAMPLE
+    floats is sampled at positions drawn from a fixed seed, the same positions in every run."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for k, v in ld.items():
+        np.save(os.path.join(path, k.replace("/", "_") + ".npy"), torch.as_tensor(v).detach().double().cpu().reshape(-1).numpy())
+    for name in ("actor", "critic", "actor_target", "critic_target"):
+        flat = getattr(agent, name).full_arena.detach()
+        if flat.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(1234))[:DUMP_SAMPLE].sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(path, name + "_params.npy"), flat.float().cpu().numpy())
+
+
+def snapshot(agent):
+    """Copies of the state an update carries to the next one: the four networks' arenas and both optimizers' moments and
+    step counts."""
+    opts = (agent.actor_optimizer, agent.critic_optimizer)
+    return ([m.full_arena.detach().clone() for m in (agent.actor, agent.actor_target, agent.critic, agent.critic_target)],
+            [t.clone() for o in opts for t in (o.exp_avg, o.exp_avg_sq, o.step_count)])
+
+
+def restore(agent, snap):
+    """Write a snapshot back in place (the captured graphs keep their pointers) and re-derive the tf32 split of every
+    network that has one, so that the next update finds it fresh and launches nothing extra."""
+    import torch
+    nets, state = snap
+    opts = (agent.actor_optimizer, agent.critic_optimizer)
+    with torch.no_grad():
+        for m, x in zip((agent.actor, agent.actor_target, agent.critic, agent.critic_target), nets):
+            m.full_arena.copy_(x)
+            if m._split is not None:
+                m.refresh_split()
+        for t, x in zip([t for o in opts for t in (o.exp_avg, o.exp_avg_sq, o.step_count)], state):
+            t.copy_(x)
 
 
 class ClockSampler:
@@ -226,8 +282,12 @@ def run_ours(a):
             dist.broadcast(m.full_arena, 0)
     g = G.build_graph(par, device=dev)
     agent.change_morphology(g)
+    # every timed step starts from this seeded state (restored outside the timed window): fp32 atomics make updates differ
+    # from run to run in the last bits, and a trajectory of updates grows that into ~1e-4 (Adam turns the sign of a ~0
+    # gradient into a full step), while one update from a fixed state reproduces to rounding
+    init = snapshot(agent)
     if a.set:
-        return run_set(a, agent, dev, world, rank, local)
+        return run_set(a, agent, dev, world, rank, local, init)
     nbat = 8
     host = [synth.make_batch(B, N, seed=100 + 17 * rank + i) for i in range(nbat)]
     host = [{k: v.pin_memory() for k, v in b.items()} for b in host]
@@ -258,13 +318,18 @@ def run_ours(a):
     l0 = _lib.lib.sgrl_launch_count() + agent.graph_replayed_launches
     barrier()
     for i in range(K):
+        r0 = _lib.lib.sgrl_launch_count()
+        restore(agent, init)
+        l0 += _lib.lib.sgrl_launch_count() - r0          # the split refresh of the restore is not part of the step
         flush.zero_()
         ev[i][0].record()
-        agent.update(devb[it % nbat], it, noise=noise[it % nbat]); it += 1
+        ld = agent.update(devb[it % nbat], it, noise=noise[it % nbat]); it += 1
         ev[i][1].record()
     barrier()
     launches = (_lib.lib.sgrl_launch_count() + agent.graph_replayed_launches - l0) / K
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, ld, agent)
     total_ms = sum(s.elapsed_time(e) for s, e in ev)
     t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -524,7 +589,7 @@ def run_ours(a):
         os._exit(0)
 
 
-def run_set(a, agent, dev, world, rank, local):
+def run_set(a, agent, dev, world, rank, local, init):
     """Multi-morphology step (BASELINE configs "Walker++ multi-morphology update", "cwhh ... sharded across 8 B200"): every
     morphology of the set gets one TD3 update of --batch samples; the set is dealt round-robin over the ranks.  --packed runs a
     rank's morphologies as one packed update; otherwise one update after the other like src/trainer.py:245-250."""
@@ -552,13 +617,15 @@ def run_set(a, agent, dev, world, rank, local):
         if world > 1:
             dist.barrier(); torch.cuda.synchronize()
 
+    per_morph = {}          # one after the other: the loss dict of every morphology's update in the last step
+
     def step(i, batches):
         if packed:
             return agent.update_packed([(graphs[n], batches[n]) for n in mine], i, morph_count=mcount)
         ld = None
         for n in mine:
             agent.change_morphology(graphs[n])
-            ld = agent.update(batches[n], i)
+            ld = per_morph[n] = agent.update(batches[n], i)
         return ld
 
     agent.lazy_stats = True
@@ -568,9 +635,12 @@ def run_set(a, agent, dev, world, rank, local):
     barrier()
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
     for i in range(K):
+        restore(agent, init)
         flush.zero_()
-        ev[i][0].record(); step(it, devb); it += 1; ev[i][1].record()
+        ev[i][0].record(); ld = step(it, devb); it += 1; ev[i][1].record()
     barrier()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, ld if packed else {f"{n}/{k}": v for n, d in per_morph.items() for k, v in d.items()}, agent)
     t = torch.tensor([sum(s.elapsed_time(e) for s, e in ev)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -91,7 +91,7 @@ def test_modules_build_on_cpu_with_reference_state_dict_keys():
     a.load_state_dict(sd)
     k = "actor.transformer_encoder.layers.2.linear4.weight"
     p = dict(a.named_parameters())[k]
-    assert p.data_ptr() >= a.full_arena.data_ptr() and torch.equal(p.data, sd[k])
+    assert p.data_ptr() >= a.full_arena.data_ptr() and torch.equal(p.data, sd[k].to(p.device))     # the arena is on cuda:0 when there is one
     assert abs(a.live_arena.double().sum().item() - sum(v.double().sum().item() for n, v in sd.items() if not O.is_dead(n))) < 1e-3
     a2 = a.double().float()      # _apply must restore the aliasing
     assert all(q.data_ptr() == a2.full_arena.data_ptr() + 4 * off for q, off, _ in a2._slots)

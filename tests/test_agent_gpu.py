@@ -154,29 +154,42 @@ def test_replayed_graph_gradients_equal_eager_gradients(B):
     run-to-run freedom in the backward is the order of the split-K atomics (~1e-7), so the raw gradients of both must
     agree far below the parity bar; a forked weight-gradient GEMM reading a half-written dY would not.
 
+    The actor gradient of a step is taken through the critic as that step's own Adam update left it, and the two agents'
+    critics differ there by the atomics order of their critic gradients (~1e-10).  That is enough to put a relu unit of the
+    actor step's critic forward on the other side of its kink now and then, which moves the actor gradient by a share of one
+    sample (2e-5 at B=256).  So the eager actor gradient it is compared with comes from a third agent, eager as well, that
+    starts the step from the same state but with the replaying agent's updated critic and a critic learning rate of 0: both
+    actor gradients then go through bit-identical forward passes.
+
     (Comparing LATER steps tensor by tensor against an fp64 oracle is not meaningful: of the ~6 M relu evaluations of a
     step a handful have |pre-activation| < 1e-6 of their row scale, and their sign - hence a gradient contribution of up
     to 1e-2 of one sample - is decided by fp32 summation order; tools/debug_relu_masks.py lists them.  Fresh-weight
     gradients are checked against the oracle in tests/test_backward_gpu.py.)"""
     ag, _, _ = make_agent()
     eg, _, _ = make_agent()
-    eg.use_graphs = False
+    xg, _, _ = make_agent()
+    eg.use_graphs = xg.use_graphs = False
     par = M.ALL["3d_humanoid_9_full"]
     g = G.build_graph(par, device="cuda")
-    ag.change_morphology(g); eg.change_morphology(g)
+    ag.change_morphology(g); eg.change_morphology(g); xg.change_morphology(g)
     for it in range(8):
         # both start every step from bit-identical state (the atomics-order noise of the previous step would otherwise grow,
         # through a relu kink, into a 1e-4 difference within a few steps)
-        eg.load_state_dict(ag.state_dict())
-        eg.critic_optimizer.load_state_dict(ag.critic_optimizer.state_dict())
-        eg.actor_optimizer.load_state_dict(ag.actor_optimizer.state_dict())
+        for other in (eg, xg):
+            other.load_state_dict(ag.state_dict())
+            other.critic_optimizer.load_state_dict(ag.critic_optimizer.state_dict())
+            other.actor_optimizer.load_state_dict(ag.actor_optimizer.state_dict())
         b = {k: v.cuda() for k, v in synth.make_batch(B, len(par), seed=50 + it).items()}
         noise = torch.randn(B, 27, generator=torch.Generator().manual_seed(100 + it)).cuda() * 0.2
         la, le = ag.update(b, it, noise=noise), eg.update(b, it, noise=noise)
         assert abs(la["loss/critic_loss"].item() - le["loss/critic_loss"].item()) <= 1e-6 * abs(le["loss/critic_loss"].item()), it
         assert parity.rel_err(ag.critic.grad_arena(), eg.critic.grad_arena()) < 1e-5, it
         if it % 2 == 0:
-            assert parity.rel_err(ag.actor.grad_arena(), eg.actor.grad_arena()) < 1e-5, it
+            xg.critic.load_state_dict(ag.critic.state_dict())
+            xg.critic_optimizer.lr = 0.0
+            xg.update(b, it, noise=noise)
+            assert torch.equal(xg.critic.full_arena, ag.critic.full_arena), it
+            assert parity.rel_err(ag.actor.grad_arena(), xg.actor.grad_arena()) < 1e-5, it
         for ma, me in ((ag.critic, eg.critic), (ag.actor, eg.actor), (ag.critic_target, eg.critic_target)):
             assert parity.rel_err(ma.full_arena, me.full_arena) < 1e-5, it     # one Adam sign flip of a ~0 gradient entry moves this by ~2e-6
     plan = next(iter(ag._plans.values()))

@@ -1,5 +1,6 @@
 """Device-resident replay buffer (sgrl_b200/buffer.py, csrc/replay.cuh) vs the numpy restatement of
 src/common/buffer.py (oracle/replay_oracle.py) and, when present, the unmodified reference class."""
+import os
 import random
 import sys
 import types
@@ -65,6 +66,18 @@ def test_oracle_against_reference_buffer():
     got = orc.get_batch([0, 5, 36, 5])
     for k in want:
         np.testing.assert_array_equal(got[k], want[k])
+
+
+def test_oracle_against_pins():
+    """The oracle's storage, seeded samples and get_batch vs tests/golden/pins.npz.  Those were recorded from the oracle
+    itself (tests/golden/make_pins.py), not from the reference class: where the reference is not available they still
+    catch any change to the behaviour the device buffer is checked against."""
+    from golden.make_pins import AD as PAD, CAP, OD as POD, buffer_draws
+    pins = np.load(os.path.join(os.path.dirname(parity.GOLDEN), "pins.npz"))
+    got = buffer_draws(ReplayOracle(POD, PAD, CAP))
+    assert sorted(got) == sorted(k for k in pins.files if k.startswith("buffer/"))
+    for k, v in got.items():
+        np.testing.assert_array_equal(v, pins[k], err_msg=k)
 
 
 # ---------------------------------------------------------------------------- host logic (no GPU needed)

@@ -1,4 +1,6 @@
 """Host graph tables vs the reference's getGraphDict (when present) and vs goldens."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -28,6 +30,18 @@ def test_relation_against_golden():
         np.testing.assert_array_equal(torch.stack(g["traversals"]).numpy(), gold[name + "/traversals"])
         np.testing.assert_allclose(g["relation"].numpy(), gold[name + "/relation"], rtol=0, atol=2e-6)
         assert g["relation"].shape == (len(M.ALL[name]),) * 2 + (3,)
+
+
+def test_graph_tables_against_pins():
+    """Every morphology's tables vs tests/golden/pins.npz.  Those were recorded from build_graph itself
+    (tests/golden/make_pins.py), not from the reference: they pin the 22 morphologies set_golden.npz does not hold, and the
+    single-limb case, where the reference is not available to compare with."""
+    pins = np.load(os.path.join(os.path.dirname(parity.GOLDEN), "pins.npz"))
+    for name, par in M.ALL.items():
+        g = G.build_graph(par)
+        np.testing.assert_array_equal(torch.stack(g["traversals"]).numpy(), pins[f"graph/{name}/traversals"], err_msg=name)
+        np.testing.assert_allclose(g["relation"].numpy(), pins[f"graph/{name}/relation"], rtol=0, atol=2e-6, err_msg=name)
+    assert G.build_graph([-1]) == {"parents": [-1]}
 
 
 @pytest.mark.skipif(ref_loader.find_reference() is None, reason="reference not on this machine")
