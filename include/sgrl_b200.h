@@ -100,20 +100,6 @@ int sgrl_set_forward(const SgrlNetCall* call, const float* obs, int64_t obs_stri
 int sgrl_set_backward(const SgrlNetCall* call, const float* dout, int64_t dout_stride, int need_wgrad,
                       float* dact, int64_t dact_stride, sgrl_stream_t stream);
 
-/* Data-parallel variant of sgrl_set_backward (need_wgrad = 1): the parameter gradients become final stage by stage — heads
- * and final norm (stage n_layers), then encoder layers n_layers-1 .. 1; layer 0 and the embeddings when the call's work is
- * done — and an event is recorded per stage on an internal stream without delaying the data-gradient chain.
- * sgrl_stream_wait_stage(waiter, owner, stage) makes `waiter` wait for stage `stage` (1..n_layers) of the staged backward
- * last enqueued on `owner`, so the all-reduce of that stage's gradient range (sgrl_param_range) overlaps the backward of
- * the stages below.  Replaces the single flat all-reduce after loss.backward() that a DistributedDataParallel wrapper
- * around the reference's modules would bucket the same way (src/agent.py:151-156, 171-176). */
-int sgrl_set_backward_staged(const SgrlNetCall* call, const float* dout, int64_t dout_stride, float* dact,
-                             int64_t dact_stride, sgrl_stream_t stream);
-int sgrl_stream_wait_stage(sgrl_stream_t waiter, sgrl_stream_t owner, int stage);
-/* float range [offset, offset + floats) inside one net's live arena: which = 0..n_layers-1: encoder layer; n_layers: the
- * embedding-side globals (pos_encoder .. encoder.bias); n_layers + 1: the heads (gg_proj .. end of the live arena) */
-int sgrl_param_range(int kind, int n_layers, int which, int64_t* offset, int64_t* floats);
-
 /* ---- single kernels (unit tests, profiling) ---------------------------------------------- */
 /* K1: Z=[X P^T | gd], G=Z^T Z, F=||G||+1 (subequivariant_attentions.py:90-96; SEActor.py:93-100,
  * 256-262).  X (T,3,128); v0 (T,3,8) or NULL (head variant, C=136); P1,P2 (30,C) (P2/Z2 NULL for
@@ -154,17 +140,10 @@ int sgrl_gemm_presplit(const float* A, int lda, int trans_a, const float* B_hi, 
  *  sgrl_gemm_gd: Z (T3,32) = [A W^T | gd]: the invariant projections g_proj / g_proj2 / g_proj3 (W (30,K) inside a matrix of
  *    row stride ldw whose two following rows are readable) with columns 30,31 of row 3t+r taken from gd (T,3,2)
  *    (subequivariant_attentions.py:91-92, SEActor.py:94-95, 109-110).
- *  sgrl_gemm_ln: N = 128.  x0 = (A W^T + b) [/ rowdiv];  x = x0 + res;  y = LayerNorm(x; gamma, beta) (eps 1e-5);
- *    optionally y2 = LayerNorm(y; gamma2, beta2): ng_out + norm1, linear2 + norm2 (+ the encoder's final norm)
- *    (SEActor.py:89-91, 121-123, 164-165).  x, x0 (T,128), stats, stats2 (T,2: mean, rstd) nullable.
  *  sgrl_gemm_pair: two independent projections C_i = A_i W_i^T + b_i [relu] in ONE grouped launch. */
 int sgrl_gemm_gram(const float* Z, const float* W_hi, const float* W_lo, const float* bias, float* C, int ldc, float* F, float* G,
                    int T, int N, int relu, sgrl_stream_t stream);
 int sgrl_gemm_gd(const float* A, int lda, const float* W_hi, const float* W_lo, int ldw, const float* gd, float* Z, int T3, int K,
-                 sgrl_stream_t stream);
-int sgrl_gemm_ln(const float* A, int lda, const float* W_hi, const float* W_lo, const float* bias, const float* rowdiv,
-                 const float* res, int ldres, const float* gamma, const float* beta, const float* gamma2, const float* beta2,
-                 float* y, int ldy, float* x, float* x0, float* stats, float* y2, int ldy2, float* stats2, int T, int K,
                  sgrl_stream_t stream);
 int sgrl_gemm_pair(const float* A0, int lda0, const float* W0_hi, const float* W0_lo, const float* b0, float* C0, int ldc0, int M0, int N0,
                    int K0, const float* A1, int lda1, const float* W1_hi, const float* W1_lo, const float* b1, float* C1, int ldc1, int M1,

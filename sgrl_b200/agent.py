@@ -132,11 +132,6 @@ class _UpdatePlan:
         self.ws = f(max(cr.ws_floats(T, 2), ac.ws_floats(T, 1)))
         self.s1, self.s2, self.s3, self.s_cap = agent._streams(dev)
         self.ev_start, self.ev_a, self.ev_b, self.ev_c = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
-        # SGRL_TWIN_SPLIT (bit 0: target critics, bit 1: critic forward, bit 2: critic backward): run the twin critics as two
-        # one-net chains on two streams instead of one nb = 2 chain (decided per plan: the captured graphs bake it in)
-        self.twin = int(os.environ.get("SGRL_TWIN_SPLIT", "0"))
-        self.s4, self.s5 = agent._twin_streams(dev)
-        self.ev_a0, self.ev_a4, self.ev_b5, self.ev_l = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
         # the fused Adam / Polyak passes of this plan also rewrite the tf32 split (decided once per plan: the captured graphs
         # bake the pointers in).  Plans too small for the tcgen05 path leave the split stale; _run_update then marks it so.
         self.keep_split = all(m.use_tc and T >= m.SPLIT_MIN_TOKENS for m in (agent.actor, agent.critic, agent.actor_target, agent.critic_target))
@@ -329,26 +324,13 @@ class Agent(nn.Module):
         return dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
 
     def _streams(self, dev):
-        """The step's forward streams, shared by every plan of the agent: s1 carries the critical chain (actor-target ->
-        twin critic-target, src/agent.py:127-139) and the capture stream the loss / backward / optimizer chain — both at
-        raised priority; s2 (actor forward of the delayed step) and s3 (critic forward) only have to be ready by the time
-        the critical chain arrives and run at plain priority, like the library's weight-gradient lanes (csrc/net.cuh Side).
-        SGRL_PRIO=1 turns the priorities on; the default is plain priority everywhere: measured on B200 the raised
-        priorities made the B=256 update 2 % slower (5.13 vs 5.03 ms, profiles/r02z_ab_knobs.txt) — the step is bound by
-        SM-time, not by the order in which waiting CTAs are placed."""
+        """The step's streams, shared by every plan of the agent: s1 carries the critical chain (actor-target ->
+        twin critic-target, src/agent.py:127-139), s2 the actor forward of the delayed step, s3 the critic forward, and the
+        capture stream the loss / backward / optimizer chain."""
         st = getattr(self, "_stream_set", None)
         if st is None or st[0] != dev:
-            hi = -1 if os.environ.get("SGRL_PRIO", "0") == "1" else 0
-            st = (dev, torch.cuda.Stream(device=dev, priority=hi), torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev),
-                  torch.cuda.Stream(device=dev, priority=hi))
+            st = (dev,) + tuple(torch.cuda.Stream(device=dev) for _ in range(4))
             self._stream_set = st
-        return st[1:]
-
-    def _twin_streams(self, dev):
-        st = getattr(self, "_twin_stream_set", None)
-        if st is None or st[0] != dev:
-            st = (dev, torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev))
-            self._twin_stream_set = st
         return st[1:]
 
     def _allreduce(self, g: torch.Tensor, world: int):
@@ -361,33 +343,11 @@ class Agent(nn.Module):
             dist.all_reduce(g, op=dist.ReduceOp.SUM)
 
     def _backward_allreduce(self, module, tb, stash, dout, nb, ws, world):
-        """loss.backward() + the data-parallel gradient sum (src/agent.py:151, 171; a DistributedDataParallel wrapper around
-        the reference would bucket it the same way).  world > 1: the backward records an event per stage
-        (sgrl_set_backward_staged) and the NCCL all-reduce of a stage's gradient range runs on a communication stream while the
-        backward of the stages below continues; only layer 0 + the embedding-side parameters are reduced after the backward.
-        Off by default: measured on 2 and 8 B200s the staged form is ~1 % SLOWER than one flat all-reduce after the backward
-        (5.66 vs 5.60 ms per update at N = 8, profiles/r04n_*: eight small NCCL launches whose kernels compete with the backward for
-        SMs cost more than the 0.2 ms of exposed transfer they hide).  SGRL_AR_BUCKETS=1 enables it."""
+        """loss.backward() + the data-parallel gradient sum (src/agent.py:151, 171): one flat all-reduce of the gradient arena
+        after the backward."""
         g = module.grad_arena()
-        if world <= 1 or os.environ.get("SGRL_AR_BUCKETS", "0") == "0" or not g.is_cuda:
-            module.backward_raw(tb, stash, dout, nb, g, False, trusted_split=True, ws=ws)
-            self._allreduce(g, world)
-            return
-        import torch.distributed as dist
-        main = torch.cuda.current_stream()
-        comm = self._streams(g.device)[2]            # s3: idle during the backward (it carried the critic forward)
-        module.backward_raw(tb, stash, dout, nb, g, False, trusted_split=True, ws=ws, staged=True)
-        for stage, ranges in module.grad_buckets(nb):
-            if stage == 0:
-                check(lib.sgrl_stream_fence(stream()))    # eager runs only (no-op under capture), see _allreduce
-                for off, n in ranges:
-                    dist.all_reduce(g[off:off + n], op=dist.ReduceOp.SUM)
-                continue
-            check(lib.sgrl_stream_wait_stage(comm.cuda_stream, main.cuda_stream, stage), "sgrl_stream_wait_stage")
-            with torch.cuda.stream(comm):
-                for off, n in ranges:
-                    dist.all_reduce(g[off:off + n], op=dist.ReduceOp.SUM)
-        main.wait_stream(comm)
+        module.backward_raw(tb, stash, dout, nb, g, False, trusted_split=True, ws=ws)
+        self._allreduce(g, world)
 
     def _plan(self, tb) -> "_UpdatePlan":
         key = id(tb)
@@ -499,7 +459,6 @@ class Agent(nn.Module):
         tb, T, st = p.tb, p.tb.T, stream()
         world = self._world()
         main = torch.cuda.current_stream()
-        twin = p.twin
         p.scal.zero_()
         p.ev_start.record(main)
         # ---- chain A (stream s1): y = r + (1-d) * gamma * min_i Q_i'(s', clip(pi'(s') + clip(eps)))        agent.py:127-139
@@ -513,18 +472,7 @@ class Agent(nn.Module):
             else:
                 check(lib.sgrl_td3_smooth_action(ptr(p.a_t), ptr(p.noise), ptr(p.next_action), float(a.noise_clip), float(a.max_action), T * 3,
                                                  stream()))
-            if twin & 1:      # the twin target critics as two one-net chains (s1, s4) instead of one nb = 2 chain
-                check(lib.sgrl_stream_fence(stream()))
-                p.ev_a0.record(p.s1)
-                with torch.cuda.stream(p.s4):
-                    p.s4.wait_event(p.ev_a0)
-                    self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2, trusted_split=True, out=p.tq, stash=p.stash_ct, z=1)
-                    check(lib.sgrl_stream_fence(stream()))
-                    p.ev_a4.record(p.s4)
-                self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2, trusted_split=True, out=p.tq, stash=p.stash_ct, z=0)
-                p.s1.wait_event(p.ev_a4)
-            else:
-                self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2, trusted_split=True, out=p.tq, stash=p.stash_ct)
+            self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2, trusted_split=True, out=p.tq, stash=p.stash_ct)
             check(lib.sgrl_stream_fence(stream()))       # eager runs only (no-op under capture): see csrc/net.cuh stream_fence
             p.ev_a.record(p.s1)
         # ---- chain C (stream s2, delayed actor step only): pi(s) — independent of the critic step           agent.py:167
@@ -535,40 +483,18 @@ class Agent(nn.Module):
                 check(lib.sgrl_stream_fence(stream()))
                 p.ev_c.record(p.s2)
         # ---- chain B (stream s3, then main): critic step                                                    agent.py:142-156
-        if twin & 2:
-            with torch.cuda.stream(p.s5):
-                p.s5.wait_event(p.ev_start)
-                self.critic.forward_raw(tb, p.obs, p.act, keep=True, nb=2, trusted_split=True, out=p.q, stash=p.stash_c, z=1)
-                check(lib.sgrl_stream_fence(stream()))
-                p.ev_b5.record(p.s5)
         with torch.cuda.stream(p.s3):
             p.s3.wait_event(p.ev_start)
-            self.critic.forward_raw(tb, p.obs, p.act, keep=True, nb=2, trusted_split=True, out=p.q, stash=p.stash_c, z=0 if twin & 2 else None)
+            self.critic.forward_raw(tb, p.obs, p.act, keep=True, nb=2, trusted_split=True, out=p.q, stash=p.stash_c)
             check(lib.sgrl_stream_fence(stream()))
             p.ev_b.record(p.s3)
         main.wait_event(p.ev_b)
-        if twin & 2:
-            main.wait_event(p.ev_b5)
         main.wait_event(p.ev_a)
         check(lib.sgrl_td3_critic_loss(ptr(p.q[0]), ptr(p.q[1]), ptr(p.tq[0]), ptr(p.tq[1]), ptr(p.rew), ptr(p.done), ptr(tb.tok_graph),
                                        ptr(tb.tok_weight), ptr(p.target), ptr(p.dq[0]), ptr(p.dq[1]), ptr(p.scal), float(a.discount), float(self.reward_scale), T,
                                        ptr(p.rstats), tb.G, st))
         self.critic_optimizer.zero_grad()
-        if twin & 4 and not (world > 1 and os.environ.get("SGRL_AR_BUCKETS", "0") != "0"):
-            # the twin critics' backward passes as two one-net chains (main, s5); their gradient ranges, stashes and workspaces are disjoint
-            g = self.critic.grad_arena()
-            check(lib.sgrl_stream_fence(stream()))
-            p.ev_l.record(main)
-            with torch.cuda.stream(p.s5):
-                p.s5.wait_event(p.ev_l)
-                self.critic.backward_raw(tb, p.stash_c, p.dq, 2, g, False, trusted_split=True, ws=p.ws, z=1)
-                check(lib.sgrl_stream_fence(stream()))
-                p.ev_b5.record(p.s5)
-            self.critic.backward_raw(tb, p.stash_c, p.dq, 2, g, False, trusted_split=True, ws=p.ws, z=0)
-            main.wait_event(p.ev_b5)
-            self._allreduce(g, world)
-        else:
-            self._backward_allreduce(self.critic, tb, p.stash_c, p.dq, 2, p.ws, world)
+        self._backward_allreduce(self.critic, tb, p.stash_c, p.dq, 2, p.ws, world)
         self.critic_optimizer.step(max_norm=float(a.grad_clipping_value), world_size=world, keep_split=p.keep_split)
         # ---- delayed actor step + Polyak                                                                    agent.py:165-180
         if actor_step:

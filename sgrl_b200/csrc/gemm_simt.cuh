@@ -32,11 +32,9 @@ struct GemmP {
   int vecA, vecB;                           // set by the launcher: operand rows may be fetched as float4
   const float* Bhi; const float* Blo;       // tcgen05 path only, optional: B pre-split into tf32 hi/lo parts (same layout/strides as B)
   int vecE;                                 // set by the tcgen05 launcher: C/mask/res rows allow float4 access
-  int sched;                                // tcgen05 MMA issue order experiment knob (SGRL_TC_SCHED)
   int pdl_late;                             // tcgen05 path: griddepcontrol.launch_dependents when the accumulators are complete instead of at entry (SGRL_PDL_LATE)
   int csk;                                  // tcgen05 path, set by the launcher: K is split over a (1, splitk, 1) cluster, rank 0 reduces through DSMEM
   int lat;                                  // tcgen05 path: launch sits on the step's critical chain (target-network forwards, data gradients): tile model may use its own wave
-  int shal;                                 // tcgen05 path: latency-regime launch (few thousand token rows): shallow operand ring, see TcCfg SHAL
   int sm2_ok;                               // tcgen05 path: the single-accumulator two-CTAs-per-SM variant may be used (inference passes only)
   long long* dbg;                           // optional (tools/gemm_trace.py): SM-clock timestamps of one CTA's pipeline phases
   int dbg_cta;                              // which CTA (blockIdx.x) writes them (SGRL_TRACE_CTA, default 0)
@@ -54,13 +52,6 @@ struct GemmP {
   float* gramG;                             // out (nullable): the generated rows (T, GP_K), kept for the weight-gradient GEMM (z-stride zsGramZ)
   // epilogue: columns 30, 31 of row m (= 3 t + r) are REPLACED by gd[t][r][0..1] (gdcols (T, 3, 2)): Z = [X P^T | gd] with N = 32
   const float* gdcols; long long zsGd;
-  // epilogue: residual + LayerNorm over the 128 columns of a row (N == 128, one tile per row; SEActor.py:90-91, 122-123, 164-165):
-  //   x = epi(acc) (+ res1);  C = LN(x; ln_gamma, ln_beta);  ln_x (nullable, ld 128) = x;  ln_stats (T, 2) = (mean, rstd)
-  //   optional second norm (the encoder's final LayerNorm after the last layer): ln2_y (ld ln2_ldy) = LN(C; ln2_gamma, ln2_beta), ln2_stats
-  // gamma/beta use zsBias as their z-stride, ln_x / ln_stats / ln2_y / ln2_stats use zsC.
-  const float* ln_gamma; const float* ln_beta; float* ln_x; float* ln_stats;
-  float* ln_x0;                             // nullable, ld 128: epi(acc) before the residual is added (linear2(..)/F, needed by the backward of the division)
-  const float* ln2_gamma; const float* ln2_beta; float* ln2_y; int ln2_ldy; float* ln2_stats;
   float* rowsum; long long zsRowsum;        // optional: rowsum[m] += alpha * sum_k A(m,k)  (bias gradient of a weight-gradient GEMM, A = dY^T); tcgen05 path
                                             // fuses it into the operand conversion, elsewhere a column-sum kernel follows the GEMM (run_gemm, net.cuh)
 };

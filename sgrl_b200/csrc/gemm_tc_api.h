@@ -1,5 +1,5 @@
 // Entry points of the tcgen05 GEMM translation unit (gemm_tc.cu: gemm_tc.cuh + gemm_tc_persist.cuh).
-// The tensor-core kernels are compiled on their own: their code generation (30-odd instantiations of ~260 KB each) must not
+// The tensor-core kernels are compiled on their own: their code generation (22 instantiations of 160–260 KB each) must not
 // move when an unrelated kernel of the library changes.  Measured: built in ONE translation unit with nvcc -split-compile, the
 // same gemm_tc.cuh came out as 260 KB or 298 KB per kernel depending on what else was in the module, and the B=256 update ran
 // 4.41 or 4.96 ms (profiles/r05p_ln_rowdiv.txt, r05q_timeline_ln.txt: every GEMM launch ~15 % slower, nothing else changed;

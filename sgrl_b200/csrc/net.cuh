@@ -62,16 +62,12 @@ inline int stream_fence(cudaStream_t st) {
 struct SideSet {
   static constexpr int N = 4;              // lane 0: independent branch of the dependency chain; lanes 1..3: dW / bias-gradient work
   cudaStream_t s[N]; cudaEvent_t fork_ev; cudaEvent_t join_ev[N];
-  cudaStream_t s0_low;                     // low-priority twin of the branch lane: swapped in when the owning stream has no raised priority
-  // staged backward (data-parallel gradient buckets): s_mark collects "everything of stage k has been enqueued and finished"
-  // without making the data-gradient chain wait for it; stage_ev[k] is what a communication stream waits on
-  cudaStream_t s_mark; cudaEvent_t mark_ev[N]; cudaEvent_t mark_main; cudaEvent_t stage_ev[MAX_LAYERS + 1]; bool marked;
   bool used[N]; int rr; cudaStream_t owner;
 };
 struct Side {
   static constexpr int NSETS = 8;          // one set per distinct main stream seen (main, the agent's two forward streams, a capture stream, ...)
   SideSet set[NSETS];
-  bool made = false; int enabled = -1; int nowners = 0; int fork_fence = 0; int pr_least = 0;
+  bool made = false; int enabled = -1; int nowners = 0; int fork_fence = 0;
   int dev = -1;                            // device the lanes were created on: one process drives one GPU (DESIGN.md §6)
   int init() {
     if (enabled < 0) { const char* e = getenv("SGRL_SIDE"); enabled = e ? atoi(e) : 1; }
@@ -82,26 +78,12 @@ struct Side {
       SGRL_CHECK(cur == dev, "the library's side streams belong to another CUDA device: one process per GPU (set the device before the first call)");
     }
     if (!made && enabled) {              // everything is created up front: nothing but event record/wait happens later (capture-safe)
-      // Stream priorities (SGRL_PRIO=1 enables; measured 2 % SLOWER on the B=256 update, profiles/r02z_ab_knobs.txt): the branch lane carries work of the dependency chain and inherits the
-      // priority class of the stream it forks from (the agent raises the priority of the step's critical chains); the
-      // weight-gradient lanes only have to finish before the optimizer step and fill the SMs the chain leaves idle (lowest
-      // priority) instead of delaying the chain's next kernel.
-      int pr_greatest = 0;
-      SGRL_CUDA(cudaDeviceGetStreamPriorityRange(&pr_least, &pr_greatest));
-      { const char* e = getenv("SGRL_PRIO"); if (!e || atoi(e) == 0) pr_greatest = pr_least; }      // off by default, see Agent._streams
-      const int pr_hi = pr_greatest < pr_least ? (pr_least - 1 < pr_greatest ? pr_greatest : pr_least - 1) : pr_least;
       for (int k = 0; k < NSETS; ++k) {
         for (int i = 0; i < SideSet::N; ++i) {
-          SGRL_CUDA(cudaStreamCreateWithPriority(&set[k].s[i], cudaStreamNonBlocking, i == 0 ? pr_hi : pr_least));
+          SGRL_CUDA(cudaStreamCreateWithFlags(&set[k].s[i], cudaStreamNonBlocking));
           SGRL_CUDA(cudaEventCreateWithFlags(&set[k].join_ev[i], cudaEventDisableTiming));
           set[k].used[i] = false;
         }
-        SGRL_CUDA(cudaStreamCreateWithPriority(&set[k].s0_low, cudaStreamNonBlocking, pr_least));
-        SGRL_CUDA(cudaStreamCreateWithFlags(&set[k].s_mark, cudaStreamNonBlocking));
-        for (int i = 0; i < SideSet::N; ++i) SGRL_CUDA(cudaEventCreateWithFlags(&set[k].mark_ev[i], cudaEventDisableTiming));
-        SGRL_CUDA(cudaEventCreateWithFlags(&set[k].mark_main, cudaEventDisableTiming));
-        for (int i = 0; i <= MAX_LAYERS; ++i) SGRL_CUDA(cudaEventCreateWithFlags(&set[k].stage_ev[i], cudaEventDisableTiming));
-        set[k].marked = false;
         SGRL_CUDA(cudaEventCreateWithFlags(&set[k].fork_ev, cudaEventDisableTiming));
         set[k].rr = 0; set[k].owner = nullptr;
       }
@@ -119,9 +101,6 @@ struct Side {
     if (nowners < NSETS) {
       SideSet& ss = set[nowners++];
       ss.owner = main;
-      int pr = pr_least;
-      if (cudaStreamGetPriority(main, &pr) != cudaSuccess) { cudaGetLastError(); pr = pr_least; }
-      if (pr >= pr_least) { cudaStream_t t = ss.s[0]; ss.s[0] = ss.s0_low; ss.s0_low = t; }   // plain-priority owner: plain-priority branch lane
       return ss;
     }
     return set[(reinterpret_cast<uintptr_t>(main) >> 6) % NSETS];      // more mains than sets: share (only costs overlap)
@@ -143,7 +122,6 @@ struct NetCtx {
   AttnGraphs gr; const int* rank3;
   float max_action;
   int bwd = 0;                            // set by net_backward (tile-model hint: data-gradient chain)
-  int staged = 0;                         // backward: record a stage event when the parameter gradients of a stage are final (sgrl_set_backward_staged)
   int use_tc;                             // 0: fp32 SIMT; 1: eligible GEMMs on the tcgen05 kernel (3xTF32, fp32 parity); 2: tcgen05 in BF16-input mode
   cudaStream_t stream;
 
@@ -156,19 +134,12 @@ struct NetCtx {
   int ks() const { return D + ng(); }
 };
 
-// latency regime: so few token rows that every projection is at most one tile per SM; the GEMMs then use the shallow operand ring
-// (gemm_tc.cuh TcCfg SHAL) so that other streams' kernels fit next to them.  SGRL_TC_SHALLOW_MAXT: most token rows x nets.
-inline int shallow_regime(const NetCtx& c) {
-  static const long long maxt = getenv("SGRL_TC_SHALLOW_MAXT") ? atoll(getenv("SGRL_TC_SHALLOW_MAXT")) : 6144;
-  return (long long)c.T * c.nb <= maxt ? 1 : 0;
-}
 inline int run_gemm(const NetCtx& c, const GemmP& g, cudaStream_t st = nullptr) {
   if (!st) st = c.stream;
   if (c.use_tc && gemm_tc_eligible(g)) {
     GemmP gi = g;
     gi.sm2_ok = c.keep ? 0 : 1;
     gi.lat = (!c.keep || c.bwd) ? 1 : 0;
-    gi.shal = shallow_regime(c);
     gi.prec = c.use_tc == 2 ? 1 : 0;      // use_tc 2: BF16-input mode (reported separately, never the default)
     return gemm_tc(gi, st);
   }
@@ -192,7 +163,7 @@ inline int run_group(const NetCtx& c, const GemmP* gs, int n, cudaStream_t st = 
   for (int i = 0; i < n && all_tc; ++i) all_tc = gemm_tc_eligible(gs[i]);
   if (all_tc) {
     GemmP gp[TC_MAXG];
-    for (int i = 0; i < n; ++i) { gp[i] = gs[i]; gp[i].prec = c.use_tc == 2 ? 1 : 0; gp[i].lat = (!c.keep || c.bwd) ? 1 : 0; gp[i].shal = shallow_regime(c); }
+    for (int i = 0; i < n; ++i) { gp[i] = gs[i]; gp[i].prec = c.use_tc == 2 ? 1 : 0; gp[i].lat = (!c.keep || c.bwd) ? 1 : 0; }
     return gemm_tc_group(gp, n, st);
   }
   for (int i = 0; i < n; ++i) SGRL_TRY(run_gemm(c, gs[i], st));
@@ -364,45 +335,9 @@ inline int zero_df_frames(const NetCtx& c) {
   return 0;
 }
 
-// vec(G) consumers whose gradients become final with backward stage `stage` (L = heads, l = encoder layer l)
-inline FoldDesc fold_desc_stage(const NetCtx& c, int stage) {
-  FoldDesc d; d.n = 0;
-  if (stage == c.L) { d.src[0] = c.lay.gp[G_H1G_W]; d.dst[0] = fold_offset(c.L, c.L, 0); d.rows[0] = D; d.n = 1; return d; }
-  for (int w = 0; w < 2; ++w) { d.src[d.n] = c.lay.lp[stage][w ? L_FG1_W : L_G1_W]; d.dst[d.n] = fold_offset(c.L, stage, w); d.rows[d.n] = HID; ++d.n; }
-  return d;
-}
 inline int unfold_grads(const NetCtx& c, const FoldDesc& d, cudaStream_t st) {
   launch_k(unfold_sym_kernel, dim3(64, d.n, c.nb), 256, 0, st, c.ws + c.wl.gf, c.zsW, c.grads, c.zsG, d);
   SGRL_LAUNCH_OK();
-  return 0;
-}
-// Staged backward: every weight-gradient launch of stage `stage` has been enqueued (side lanes, branch lane, main stream).
-// The mark stream waits for all of them, unfolds the stage's vec(G) gradients and records stage_ev[stage]; neither the
-// data-gradient chain nor the lanes wait for anything.  A communication stream that waits on the event
-// (sgrl_stream_wait_stage) may all-reduce the stage's gradient range while the backward of the stages below runs.
-inline int stage_mark(const NetCtx& c, int stage) {
-  Side& sd = g_side;
-  if (side_off(sd)) {          // no side streams: everything is on the main stream
-    SGRL_TRY(unfold_grads(c, fold_desc_stage(c, stage), c.stream));
-    SideSet& ss0 = sd.of(c.stream);
-    SGRL_TRY(stream_fence(c.stream));
-    SGRL_CUDA(cudaEventRecord(ss0.stage_ev[stage], c.stream));
-    return 0;
-  }
-  SideSet& ss = sd.of(c.stream);
-  if (sd.fork_fence) SGRL_TRY(stream_fence(c.stream));
-  SGRL_CUDA(cudaEventRecord(ss.mark_main, c.stream));
-  SGRL_CUDA(cudaStreamWaitEvent(ss.s_mark, ss.mark_main, 0));
-  for (int i = 0; i < SideSet::N; ++i) {
-    if (!ss.used[i]) continue;
-    if (sd.fork_fence) SGRL_TRY(stream_fence(ss.s[i]));
-    SGRL_CUDA(cudaEventRecord(ss.mark_ev[i], ss.s[i]));
-    SGRL_CUDA(cudaStreamWaitEvent(ss.s_mark, ss.mark_ev[i], 0));
-  }
-  SGRL_TRY(unfold_grads(c, fold_desc_stage(c, stage), ss.s_mark));
-  if (sd.fork_fence) SGRL_TRY(stream_fence(ss.s_mark));
-  SGRL_CUDA(cudaEventRecord(ss.stage_ev[stage], ss.s_mark));
-  ss.marked = true;
   return 0;
 }
 
@@ -437,9 +372,6 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
     SGRL_LAUNCH_OK();
   }
   if (fused && !fold_pending) SGRL_TRY(fold_weights(c, st));
-  // residual + LayerNorm inside the N = 128 GEMMs' epilogue (gemm_tc.cuh) — measured slower than GEMM + layernorm kernel on
-  // the branch lane at 2 304 tokens (23.2 vs 11.0 + 3.5 us, tools/fused_bench.py), so off by default
-  static const int ln_epi = getenv("SGRL_LN_EPI") ? atoi(getenv("SGRL_LN_EPI")) : 0;
   for (int l = 0; l < c.L; ++l) {
     const long long* lp = Y.lp[l];
     float* Vg = c.SL(l, S_VGIN);
@@ -450,18 +382,18 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
     float* h_next = last ? c.S(T_HL) : c.SL(l + 1, S_UA) + 128;
     const int ld_hn = last ? 128 : 256;
     if (fused) {
-      // ---- fused schedule (tcgen05 path): 12 launches per layer on ONE stream, no forks (SURVEY.md Appendix G) ----
+      // ---- fused schedule (tcgen05 path): 12 launches per layer on the main stream, the LayerNorms on the branch lane (SURVEY.md Appendix G) ----
       //  Z1 = [Vg g_proj^T | gd]                                  projection on the tensor pipe, gd columns in the epilogue
       //  a1 = relu(linear_g1(tri(Z1^T Z1)))  (+ F1, + G1 if kept)  Gram rows generated inside the GEMM as its A operand
       //  [ u[:, :128] = linear_g2(a1)  ||  vg = vg_proj(Vg) ]      grouped launch
       //  q|k|v = (W u + b)/F1                                      one N = 768 GEMM
       //  attention core
-      //  [ h1 = LN1(h + ng_out(o))  ||  dV = g_out(og) ]           grouped, residual + LayerNorm in the epilogue
+      //  [ x1 = ng_out(o)  ||  dV = g_out(og) ]                   grouped; h1 = LN1(h + x1) on the branch lane
       //  [ Z2 = [dV g_proj2^T | gd]  ||  Z3 = [dV g_proj3^T | gd] ] grouped
       //  a2 = relu(linear_g1'(tri(Z2^T Z2)))  (+ F2, + G2)
       //  u'[:, :128] = linear_g2'(a2)
       //  t31 = relu([linear3 | linear1](u'))
-      //  [ h' = LN2(h1 + linear2(t1)/F2) (+ final norm)  ||  M = linear4(t3)/F2 ]   grouped
+      //  [ f = linear2(t1)/F2  ||  M = linear4(t3)/F2 ]           grouped; h' = LN2(h1 + f) (+ final norm) on the branch lane
       //  Vg' = Vg + dV + linear5(Z3 . M)                           matrix apply + linear5 + residuals
       GemmP gz = lin(c, Vg, 128, zS, lp[L_GPROJ], -1, c.SL(l, S_Z1), 32, zS, T3, 32, 128);
       gz.gdcols = c.S(T_GD); gz.zsGd = zS;
@@ -479,19 +411,12 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
       SGRL_TRY(run_gemm(c, g));
       SGRL_TRY(attention_fwd(c.SL(l, S_QKV), c.SL(l, S_VGP), c.S(T_GD), c.SL(l, S_O), c.SL(l, S_OG), c.keep ? c.SL(l, S_P) : nullptr, zS,
                              l == 0 ? c.P(Y.gp[G_REL_W]) : nullptr, l == 0 ? c.P(Y.gp[G_REL_B]) : nullptr, c.zsP, c.gr, c.nb, st));
-      if (ln_epi) {
-        pr[0] = lin(c, c.SL(l, S_O), 256, zS, lp[L_NGO_W], lp[L_NGO_B], ub + 128, 256, zS, T, 128, 256);
-        pr[0].res1 = ua + 128; pr[0].zsR1 = zS; pr[0].ldr1 = 256;
-        pr[0].ln_gamma = c.P(lp[L_N1_W]); pr[0].ln_beta = c.P(lp[L_N1_B]); pr[0].ln_x = c.SL(l, S_X1); pr[0].ln_stats = c.SL(l, S_ST1);
-      } else {
-        pr[0] = lin(c, c.SL(l, S_O), 256, zS, lp[L_NGO_W], lp[L_NGO_B], c.SL(l, S_X1), 128, zS, T, 128, 256);
-      }
+      pr[0] = lin(c, c.SL(l, S_O), 256, zS, lp[L_NGO_W], lp[L_NGO_B], c.SL(l, S_X1), 128, zS, T, 128, 256);
       pr[1] = lin(c, c.SL(l, S_OG), 256, zS, lp[L_GO_W], -1, c.SL(l, S_DV), 128, zS, T3, 128, 256);
       SGRL_TRY(run_group(c, pr, 2));
-      if (!ln_epi) {     // h1 = LN1(h + ng_out(o)) on the branch lane: first needed by [linear3 | linear1]
-        SGRL_TRY(side_fork(c, &sb, 0));
-        SGRL_TRY(layernorm_fwd(c, ua + 128, 256, c.SL(l, S_X1), 128, lp[L_N1_W], lp[L_N1_B], c.SL(l, S_X1), ub + 128, 256, c.SL(l, S_ST1), sb));
-      }
+      // h1 = LN1(h + ng_out(o)) on the branch lane: first needed by [linear3 | linear1]
+      SGRL_TRY(side_fork(c, &sb, 0));
+      SGRL_TRY(layernorm_fwd(c, ua + 128, 256, c.SL(l, S_X1), 128, lp[L_N1_W], lp[L_N1_B], c.SL(l, S_X1), ub + 128, 256, c.SL(l, S_ST1), sb));
       pr[0] = lin(c, c.SL(l, S_DV), 128, zS, lp[L_GP2], -1, c.SL(l, S_Z2), 32, zS, T3, 32, 128);
       pr[0].gdcols = c.S(T_GD); pr[0].zsGd = zS;
       pr[1] = lin(c, c.SL(l, S_DV), 128, zS, lp[L_GP3], -1, c.SL(l, S_Z3), 32, zS, T3, 32, 128);
@@ -502,34 +427,22 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
       SGRL_TRY(run_gemm(c, g1));
       g = lin(c, c.SL(l, S_A2), 256, zS, lp[L_FG2_W], lp[L_FG2_B], ub, 256, zS, T, 128, 256);
       SGRL_TRY(run_gemm(c, g));
-      if (!ln_epi) SGRL_TRY(side_join(c, 0));
+      SGRL_TRY(side_join(c, 0));
       g = lin(c, ub, 256, zS, lp[L_L3_W], lp[L_L3_B], c.SL(l, S_T31), 512, zS, T, 512, 256); g.relu = 1;   // [linear3 | linear1]
       SGRL_TRY(run_gemm(c, g));
-      if (ln_epi) {
-        pr[0] = lin(c, c.SL(l, S_T31) + 256, 512, zS, lp[L_L2_W], lp[L_L2_B], h_next, ld_hn, zS, T, 128, 256);
-        pr[0].res1 = ub + 128; pr[0].zsR1 = zS; pr[0].ldr1 = 256;
-        pr[0].ln_gamma = c.P(lp[L_N2_W]); pr[0].ln_beta = c.P(lp[L_N2_B]); pr[0].ln_x = c.SL(l, S_X2); pr[0].ln_stats = c.SL(l, S_ST2);
-        pr[0].ln_x0 = c.SL(l, S_FF);
-        if (last) {        // the encoder's final LayerNorm rides on the last layer's norm2: h_final -> right part of SH = [s0 | h]
-          pr[0].ln2_gamma = c.P(Y.gp[G_NORM_W]); pr[0].ln2_beta = c.P(Y.gp[G_NORM_B]);
-          pr[0].ln2_y = c.S(T_SH) + ng; pr[0].ln2_ldy = KS; pr[0].ln2_stats = c.S(T_STF);
-        }
-      } else {
-        pr[0] = lin(c, c.SL(l, S_T31) + 256, 512, zS, lp[L_L2_W], lp[L_L2_B], c.SL(l, S_FF), 128, zS, T, 128, 256);
-      }
+      pr[0] = lin(c, c.SL(l, S_T31) + 256, 512, zS, lp[L_L2_W], lp[L_L2_B], c.SL(l, S_FF), 128, zS, T, 128, 256);
       pr[0].rowdiv = c.SL(l, S_F2); pr[0].zsRow = zS;
       pr[1] = lin(c, c.SL(l, S_T31), 512, zS, lp[L_L4_W], lp[L_L4_B], c.SL(l, S_MM), 1024, zS, T, 1024, 256);
       pr[1].rowdiv = c.SL(l, S_F2); pr[1].zsRow = zS;
       SGRL_TRY(run_group(c, pr, 2));
-      if (!ln_epi) {     // h' = LN2(h1 + linear2(..)/F2) (+ the encoder's final norm) on the branch lane, next to the matrix apply
-        SGRL_TRY(side_fork(c, &sb, 0));
-        SGRL_TRY(layernorm_fwd(c, ub + 128, 256, c.SL(l, S_FF), 128, lp[L_N2_W], lp[L_N2_B], c.SL(l, S_X2), h_next, ld_hn, c.SL(l, S_ST2), sb));
-        if (last) SGRL_TRY(layernorm_fwd(c, c.S(T_HL), 128, nullptr, 0, Y.gp[G_NORM_W], Y.gp[G_NORM_B], nullptr, c.S(T_SH) + ng, KS, c.S(T_STF), sb));
-      }
+      // h' = LN2(h1 + linear2(..)/F2) (+ the encoder's final norm) on the branch lane, next to the matrix apply
+      SGRL_TRY(side_fork(c, &sb, 0));
+      SGRL_TRY(layernorm_fwd(c, ub + 128, 256, c.SL(l, S_FF), 128, lp[L_N2_W], lp[L_N2_B], c.SL(l, S_X2), h_next, ld_hn, c.SL(l, S_ST2), sb));
+      if (last) SGRL_TRY(layernorm_fwd(c, c.S(T_HL), 128, nullptr, 0, Y.gp[G_NORM_W], Y.gp[G_NORM_B], nullptr, c.S(T_SH) + ng, KS, c.S(T_STF), sb));
       launch_k(matapply_l5_fwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, c.SL(l, S_Z3), c.SL(l, S_MM), c.P(lp[L_L5_W]), c.zsP, Vg, c.SL(l, S_DV),
                c.keep ? c.SL(l, S_R) : nullptr, Vg_next, zS, T);
       SGRL_LAUNCH_OK();
-      if (!ln_epi) SGRL_TRY(side_join(c, 0));
+      SGRL_TRY(side_join(c, 0));
       continue;
     }
     // -- attention block: invariant features of Vg -> u = [g-mlp | h]
@@ -738,8 +651,6 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
   }
   if (head_side) SGRL_TRY(side_join(c, 0));
 
-  const bool staged = wg && c.staged;
-  if (staged) SGRL_TRY(stage_mark(c, c.L));
   // ---------------------------------------------------------------- encoder layers (frame l reads frame l+1)
   for (int l = c.L - 1; l >= 0; --l) {
     fin = l + 1; f = l;
@@ -839,7 +750,6 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     SGRL_TRY(run_gemm(c, g));
     // dh(in) = dx1 + du[:, 128:]: materialised only for the embedding stage (three readers); the layer below sums the two itself
     if (l == 0) SGRL_TRY(block_copy(c, W(W_DH), 128, zW, W(W_DH1), 128, zW, T, 128, 0, W(W_DUA) + 128, 256, zW));
-    if (staged && l > 0) SGRL_TRY(stage_mark(c, l));
   }
   // ---------------------------------------------------------------- embedding (reads frame 0)
   f = 0; fin = 0;
@@ -858,17 +768,8 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     SGRL_TRY(run_gemm(c, g));
   }
   SGRL_TRY(side_join(c));
-  if (wg) {      // gradients of the folded weights -> (rows,1024) gradient tensors (staged: only layer 0 is left)
-    SGRL_TRY(unfold_grads(c, staged ? fold_desc_stage(c, 0) : fold_desc(c), st));
-  }
-  if (staged && !side_off(g_side)) {      // the mark stream rejoins the main stream (capture: every forked stream must)
-    SideSet& ss = g_side.of(c.stream);
-    if (ss.marked) {
-      if (g_side.fork_fence) SGRL_TRY(stream_fence(ss.s_mark));
-      SGRL_CUDA(cudaEventRecord(ss.mark_main, ss.s_mark));
-      SGRL_CUDA(cudaStreamWaitEvent(c.stream, ss.mark_main, 0));
-      ss.marked = false;
-    }
+  if (wg) {      // gradients of the folded weights -> (rows,1024) gradient tensors
+    SGRL_TRY(unfold_grads(c, fold_desc(c), st));
   }
   return 0;
 }

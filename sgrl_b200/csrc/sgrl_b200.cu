@@ -128,36 +128,6 @@ int sgrl_set_backward(const SgrlNetCall* call, const float* dout, int64_t dout_s
   return net_backward(c, dout, dout_stride, need_wgrad, dact, dact_stride);
 }
 
-int sgrl_set_backward_staged(const SgrlNetCall* call, const float* dout, int64_t dout_stride, float* dact, int64_t dact_stride,
-                             sgrl_stream_t stream) {
-  NetCtx c;
-  SGRL_TRY(make_ctx(call, ST(stream), c));
-  SGRL_CHECK(call->keep == 1, "backward needs a forward that ran with keep=1");
-  SGRL_CHECK(call->ws != nullptr && call->ws_stride >= c.wl.total, "workspace missing or smaller than sgrl_ws_floats()");
-  SGRL_CHECK(dout != nullptr && call->grads != nullptr, "null dout / gradient arena");
-  c.staged = 1;
-  return net_backward(c, dout, dout_stride, 1, dact, dact_stride);
-}
-
-int sgrl_stream_wait_stage(sgrl_stream_t waiter, sgrl_stream_t owner, int stage) {
-  SGRL_CHECK(stage >= 1 && stage <= MAX_LAYERS, "stage out of range");
-  SGRL_TRY(g_side.init());
-  SideSet& ss = g_side.of(ST(owner));
-  SGRL_CUDA(cudaStreamWaitEvent(ST(waiter), ss.stage_ev[stage], 0));
-  return 0;
-}
-
-int sgrl_param_range(int kind, int n_layers, int which, int64_t* offset, int64_t* floats) {
-  SGRL_CHECK(n_layers >= 1 && n_layers <= MAX_LAYERS && which >= 0 && which <= n_layers + 1 && offset && floats, "bad arguments");
-  const NetLayout L = make_layout(kind, n_layers);
-  long long b, e;
-  if (which < n_layers) { b = L.lp[which][0]; e = which + 1 < n_layers ? L.lp[which + 1][0] : L.gp[G_POS0]; }
-  else if (which == n_layers) { b = L.gp[G_POS0]; e = L.gp[G_GG_W]; }
-  else { b = L.gp[G_GG_W]; e = L.live_floats; }
-  *offset = b; *floats = e - b;
-  return 0;
-}
-
 int sgrl_inv_feature_fwd(const float* X, const float* v0, const float* gd, const float* P1, const float* P2, float* Z, float* Z2,
                          float* G, float* F, int T, sgrl_stream_t stream) {
   SGRL_CHECK(X && gd && P1 && Z && G && F, "null pointer");
@@ -234,20 +204,6 @@ int sgrl_gemm_gd(const float* A, int lda, const float* W_hi, const float* W_lo, 
   GemmP g = gemm_defaults();
   g.A = A; g.lda = lda; g.B = W_hi; g.Bhi = W_hi; g.Blo = W_lo; g.ldb = ldw; g.C = Z; g.ldc = 32;
   g.M = T3; g.N = 32; g.K = K; g.gdcols = gd;
-  SGRL_CHECK(gemm_tc_eligible(g), "shape not eligible for the tcgen05 path");
-  return gemm_tc(g, ST(stream));
-}
-
-int sgrl_gemm_ln(const float* A, int lda, const float* W_hi, const float* W_lo, const float* bias, const float* rowdiv,
-                 const float* res, int ldres, const float* gamma, const float* beta, const float* gamma2, const float* beta2,
-                 float* y, int ldy, float* x, float* x0, float* stats, float* y2, int ldy2, float* stats2, int T, int K,
-                 sgrl_stream_t stream) {
-  SGRL_CHECK(A && W_hi && W_lo && gamma && beta && y, "null pointer");
-  GemmP g = gemm_defaults();
-  g.A = A; g.lda = lda; g.B = W_hi; g.Bhi = W_hi; g.Blo = W_lo; g.ldb = K; g.C = y; g.ldc = ldy;
-  g.M = T; g.N = 128; g.K = K; g.bias = bias; g.rowdiv = rowdiv; g.res1 = res; g.ldr1 = ldres;
-  g.ln_gamma = gamma; g.ln_beta = beta; g.ln_x = x; g.ln_x0 = x0; g.ln_stats = stats;
-  g.ln2_gamma = gamma2; g.ln2_beta = beta2; g.ln2_y = y2; g.ln2_ldy = ldy2; g.ln2_stats = stats2;
   SGRL_CHECK(gemm_tc_eligible(g), "shape not eligible for the tcgen05 path");
   return gemm_tc(g, ST(stream));
 }

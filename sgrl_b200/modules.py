@@ -310,9 +310,7 @@ class SetNetModule(nn.Module):
         return t
 
     # ------------------------------------------------------------------ raw kernel passes
-    def _call(self, tb: GraphTables, nb: int, keep: int, stash, grads=None, ws=None, split=(None, None), z: Optional[int] = None) -> NetCall:
-        """z: run ONLY net instance z of buffers laid out for nb instances, as a one-net call (the twin critics as two
-        independent chains on two streams, Agent._update_impl); every per-instance pointer is advanced to instance z."""
+    def _call(self, tb: GraphTables, nb: int, keep: int, stash, grads=None, ws=None, split=(None, None)) -> NetCall:
         k = NetCall()
         k.kind, k.n_layers, k.nb, k.T, k.G = self._kind, self._n_layers, nb, tb.T, tb.G
         k.keep, k.use_tc, k.max_limbs = keep, int(self.use_tc), int(tb.nmax)
@@ -324,18 +322,6 @@ class SetNetModule(nn.Module):
         if ws is not None:
             k.ws = ptr(ws)
             k.ws_stride = ws.numel() // nb
-        if z is not None:
-            zb = 4 * z * self._live
-            k.nb = 1
-            k.params += zb
-            if split[0] is not None:
-                k.params_hi += zb
-                k.params_lo += zb
-            if grads is not None:
-                k.grads += zb
-            k.stash += 4 * z * k.stash_stride
-            if ws is not None:
-                k.ws += 4 * z * k.ws_stride
         k.cu_limbs, k.rel_off, k.relation, k.rank3 = ptr(tb.cu_limbs), ptr(tb.rel_off), ptr(tb.relation), ptr(tb.rank3)
         k.max_action = self._max_action
         return k
@@ -347,11 +333,9 @@ class SetNetModule(nn.Module):
         return nb * lib.sgrl_ws_floats(self._n_layers, T)
 
     def forward_raw(self, tb: GraphTables, obs: torch.Tensor, act: Optional[torch.Tensor], keep: bool, nb: Optional[int] = None,
-                    out: Optional[torch.Tensor] = None, trusted_split: bool = False, stash: Optional[torch.Tensor] = None,
-                    z: Optional[int] = None):
+                    out: Optional[torch.Tensor] = None, trusted_split: bool = False, stash: Optional[torch.Tensor] = None):
         """Run nb nets on tokens obs (T,41) [act (T,3)].  Returns (out (nb,T,od), stash).  `out` / `stash` may be
-        caller-owned buffers (Agent.update's static plan); otherwise they are allocated here.  z: only instance z of the nb
-        (out[z] and stash slice z are written; `out` and `stash` must be the caller's nb-instance buffers)."""
+        caller-owned buffers (Agent.update's static plan); otherwise they are allocated here."""
         nb = self._nb if nb is None else nb
         od = 3 if self._kind == ACTOR else 1
         dev = self._arena.device
@@ -361,54 +345,23 @@ class SetNetModule(nn.Module):
             stash = torch.empty(self.stash_floats(tb.T, keep, nb), dtype=torch.float32, device=dev)
         if out is None:
             out = torch.empty(nb, tb.T, od, dtype=torch.float32, device=dev)
-        k = self._call(tb, nb, int(keep), stash, split=self._split_for(tb.T, trusted_split), z=z)
-        check(lib.sgrl_set_forward(C.byref(k), ptr(obs), 0, ptr(act), 0, ptr(out) + (0 if z is None else 4 * z * tb.T * od), tb.T * od, stream()),
-              "sgrl_set_forward")
+        k = self._call(tb, nb, int(keep), stash, split=self._split_for(tb.T, trusted_split))
+        check(lib.sgrl_set_forward(C.byref(k), ptr(obs), 0, ptr(act), 0, ptr(out), tb.T * od, stream()), "sgrl_set_forward")
         return out, stash
 
     def backward_raw(self, tb: GraphTables, stash: torch.Tensor, dout: torch.Tensor, nb: int, grads: Optional[torch.Tensor],
-                     want_dact: bool, trusted_split: bool = False, ws: Optional[torch.Tensor] = None, dact: Optional[torch.Tensor] = None,
-                     staged: bool = False, z: Optional[int] = None):
-        """dout (nb,T,od).  Accumulates parameter gradients into `grads` (None: data-only).  staged: record the per-stage
-        events of sgrl_set_backward_staged (data-parallel gradient buckets, Agent._backward_allreduce).  z: only instance z
-        (see forward_raw; dout, ws, grads and stash are the nb-instance buffers)."""
+                     want_dact: bool, trusted_split: bool = False, ws: Optional[torch.Tensor] = None, dact: Optional[torch.Tensor] = None):
+        """dout (nb,T,od).  Accumulates parameter gradients into `grads` (None: data-only)."""
         dev = self._arena.device
         if ws is None:
             ws = torch.empty(self.ws_floats(tb.T, nb), dtype=torch.float32, device=dev)
         if want_dact and dact is None:
             dact = torch.empty(nb, tb.T, 3, dtype=torch.float32, device=dev)
         od = 3 if self._kind == ACTOR else 1
-        k = self._call(tb, nb, 1, stash, grads=grads, ws=ws, split=self._split_for(tb.T, trusted_split), z=z)
-        if z is not None:
-            if staged or want_dact:
-                raise _lib.SgrlError("backward_raw(z=..): one-instance slices support neither the staged form nor d/d(action)")
-            check(lib.sgrl_set_backward(C.byref(k), ptr(dout) + 4 * z * tb.T * od, tb.T * od, 1 if grads is not None else 0, None, tb.T * 3, stream()),
-                  "sgrl_set_backward")
-            return None
-        if staged and grads is not None:
-            check(lib.sgrl_set_backward_staged(C.byref(k), ptr(dout), tb.T * od, ptr(dact), tb.T * 3, stream()), "sgrl_set_backward_staged")
-            return dact
+        k = self._call(tb, nb, 1, stash, grads=grads, ws=ws, split=self._split_for(tb.T, trusted_split))
         check(lib.sgrl_set_backward(C.byref(k), ptr(dout), tb.T * od, 1 if grads is not None else 0, ptr(dact), tb.T * 3, stream()),
               "sgrl_set_backward")
         return dact
-
-    def grad_buckets(self, nb: int):
-        """Gradient-arena ranges in the order the staged backward completes them: [(stage, [(offset, floats), ...]), ...] with
-        stage = n_layers (heads), then 1 (encoder layers n_layers-1 .. 1, contiguous in the arena), then 0 (layer 0 and the
-        embedding-side globals: final only when the backward has finished).  One range per net instance."""
-        L, live = self._n_layers, self._live
-
-        def rng(which):
-            off, n = C.c_int64(), C.c_int64()
-            check(lib.sgrl_param_range(self._kind, L, which, C.byref(off), C.byref(n)), "sgrl_param_range")
-            return off.value, n.value
-        heads, emb, l0 = rng(L + 1), rng(L), rng(0)
-        out = [(L, [(z * live + heads[0], heads[1]) for z in range(nb)])]
-        if L > 1:
-            b, e = rng(1)[0], rng(L - 1)[0] + rng(L - 1)[1]
-            out.append((1, [(z * live + b, e - b) for z in range(nb)]))
-        out.append((0, [(z * live + l0[0], l0[1]) for z in range(nb)] + [(z * live + emb[0], emb[1]) for z in range(nb)]))
-        return out
 
     # ------------------------------------------------------------------ autograd bridge
     def _run(self, state: torch.Tensor, action: Optional[torch.Tensor], nb: int) -> torch.Tensor:

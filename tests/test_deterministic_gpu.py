@@ -63,15 +63,3 @@ def test_mode_switch_is_reported():
     lib.sgrl_deterministic(prev)
     assert lib.sgrl_deterministic(-1) == prev
 
-
-def test_twin_split_chains_match_the_batched_twin(monkeypatch):
-    """SGRL_TWIN_SPLIT=7: the twin critics (target forward, forward, backward) as two one-net calls on two streams through
-    forward_raw / backward_raw(z=...) instead of one nb = 2 call: same parameters after 4 updates up to summation order."""
-    ref, gref, lref = run_updates(False, "3d_humanoid_9_full", 64, 4)
-    monkeypatch.setenv("SGRL_TWIN_SPLIT", "7")
-    got, ggot, lgot = run_updates(False, "3d_humanoid_9_full", 64, 4)
-    for x, y in zip(ref, got):
-        assert parity.rel_err(x, y) < 1e-5
-    for x, y in zip(gref, ggot):
-        assert parity.rel_err(x, y) < 1e-4
-    assert parity.rel_err(lref, lgot) < 1e-5

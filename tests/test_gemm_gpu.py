@@ -134,12 +134,12 @@ def test_persistent_projection_kernel(monkeypatch, M, N, K, rowdiv, relu):
 
 
 @pytest.mark.parametrize("N", [64, 128, 512])
-def test_shallow_ring_is_bit_identical_to_deep_ring(monkeypatch, N):
-    """The shallow operand ring (csrc/gemm_tc.cuh TcCfg SHAL: 2 stages, used for latency-regime launches so that other streams'
-    kernels fit next to a GEMM CTA) performs the same arithmetic in the same order as the deep ring: forward projection against
-    pre-split weights, data gradient (B read MN-major), weight gradient (both operands MN-major, split on the fly) and the
-    Gram-generating projection must agree BIT FOR BIT.  SGRL_TC_SHALLOW=2 forces it, 0 forbids it (read per launch plan)."""
+def test_update_shapes_against_fp64(N):
+    """The tcgen05 kernel at the 2 304-row shapes of a B=256 humanoid update, against fp64 torch: forward projection against
+    pre-split weights, data gradient (pre-split B read MN-major), weight gradient (both operands MN-major, split on the fly)
+    and the Gram-generating projection."""
     from sgrl_b200._lib import lib, ptr, stream, check
+    from sgrl_b200.packing import pack_indices
     g = torch.Generator(device="cuda").manual_seed(N)
     M, K = 2304, 256
     X = torch.randn(M, K, device="cuda", generator=g)
@@ -153,26 +153,23 @@ def test_shallow_ring_is_bit_identical_to_deep_ring(monkeypatch, N):
     Wf = torch.randn(N, 544, device="cuda", generator=g) / 23.0
     fhi, flo = torch.empty_like(Wf), torch.empty_like(Wf)
     check(lib.sgrl_split_tf32(ptr(Wf), ptr(fhi), ptr(flo), Wf.numel(), stream()))
-    outs = {}
-    for mode in ("2", "0"):
-        monkeypatch.setenv("SGRL_TC_SHALLOW", mode)
-        Y = torch.zeros(M, N, device="cuda")
-        check(lib.sgrl_gemm_presplit(ptr(X), K, 0, ptr(hi), ptr(lo), K, 0, ptr(Y), N, M, N, K, 1.0, ptr(b), ptr(F), 1, 0, 1, stream()))
-        dX = torch.zeros(M, K, device="cuda")        # dX = dY W: B = W (N,K) read "transposed"
-        check(lib.sgrl_gemm_presplit(ptr(dY), N, 0, ptr(hi), ptr(lo), K, 1, ptr(dX), K, M, K, N, 1.0, None, None, 0, 0, 1, stream()))
-        dW = torch.zeros(N, K, device="cuda")        # dW = dY^T X: both operands read "transposed", no split over K
-        check(lib.sgrl_gemm(ptr(dY), N, 1, ptr(X), K, 1, ptr(dW), K, N, K, M, 1.0, None, None, 0, 1, 2, 1, stream()))   # splitk > 1: "may be split" (no cluster split-K)
-        C = torch.zeros(M, N, device="cuda")
-        Fo = torch.zeros(M, device="cuda")
-        check(lib.sgrl_gemm_gram(ptr(Z), ptr(fhi), ptr(flo), ptr(b), ptr(C), N, ptr(Fo), None, M, N, 1, stream()))
-        torch.cuda.synchronize()
-        outs[mode] = (Y, dX, dW, C, Fo)
-    ref = torch.relu(X.double() @ W.double().T + b.double()) / F.double()[:, None]
-    assert rel(outs["2"][0], ref) < TOL[1]
-    assert rel(outs["2"][1], dY.double() @ W.double()) < TOL[1]
-    assert rel(outs["2"][2], dY.double().T @ X.double()) < TOL[1]
-    for i, (a, c) in enumerate(zip(outs["2"], outs["0"])):
-        if i == 2 and N < 512:      # small weight gradients are split over K with fp32 atomics: equal up to summation order
-            assert rel(a, c) < 1e-6
-        else:
-            assert torch.equal(a, c)
+    Y = torch.zeros(M, N, device="cuda")
+    check(lib.sgrl_gemm_presplit(ptr(X), K, 0, ptr(hi), ptr(lo), K, 0, ptr(Y), N, M, N, K, 1.0, ptr(b), ptr(F), 1, 0, 1, stream()))
+    dX = torch.zeros(M, K, device="cuda")        # dX = dY W: B = W (N,K) read "transposed"
+    check(lib.sgrl_gemm_presplit(ptr(dY), N, 0, ptr(hi), ptr(lo), K, 1, ptr(dX), K, M, K, N, 1.0, None, None, 0, 0, 1, stream()))
+    dW = torch.zeros(N, K, device="cuda")        # dW = dY^T X: both operands read "transposed"
+    check(lib.sgrl_gemm(ptr(dY), N, 1, ptr(X), K, 1, ptr(dW), K, N, K, M, 1.0, None, None, 0, 1, 2, 1, stream()))   # splitk > 1: "may be split" (no cluster split-K)
+    C = torch.zeros(M, N, device="cuda")
+    Fo = torch.zeros(M, device="cuda")
+    check(lib.sgrl_gemm_gram(ptr(Z), ptr(fhi), ptr(flo), ptr(b), ptr(C), N, ptr(Fo), None, M, N, 1, stream()))
+    torch.cuda.synchronize()
+    assert rel(Y, torch.relu(X.double() @ W.double().T + b.double()) / F.double()[:, None]) < TOL[1]
+    assert rel(dX, dY.double() @ W.double()) < TOL[1]
+    assert rel(dW, dY.double().T @ X.double()) < TOL[1]
+    Zd = Z.double()
+    G = Zd.transpose(1, 2) @ Zd                  # (M,32,32); the kernel generates its packed upper triangle (csrc/layout.h)
+    slots, ri, ci = pack_indices()
+    Gp = torch.zeros(M, 544, dtype=torch.float64, device="cuda")
+    Gp[:, slots] = G[:, ri, ci]
+    assert rel(C, torch.relu(Gp @ Wf.double().T + b.double())) < TOL[1]
+    assert rel(Fo, G.reshape(M, -1).norm(dim=1) + 1.0) < 1e-6

@@ -1,6 +1,6 @@
 #!/bin/bash
 # A/B runs of the B=256 humanoid-9 update under environment knobs: bash tools/ab_update.sh "NAME=VAL ..." "..." (one quoted group per run)
-# prints ms/step (device-timed) and end-to-end samples/s per run.  usage (GPU box): bash tools/ab_update.sh "" "SGRL_PRIO=0" ...
+# prints ms/step (device-timed) and end-to-end samples/s per run.  usage (GPU box): bash tools/ab_update.sh "" "SGRL_PDL_LATE=0" ...
 cd "$(dirname "$0")/.."
 for envs in "$@"; do
   out=$(env $envs timeout 300 python bench.py --steps ${AB_STEPS:-60} --warmup 6 --no-cpu-baseline --no-rollout --no-bf16 2>/dev/null | tail -1)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Prints the SM-clock timeline of CTA 0 of one tcgen05 GEMM launch (sgrl_gemm_trace): prologue, TMA issue,
 operand landing, split done, MMA issue, accumulator ready, epilogue done.  usage: gemm_trace.py M N K [pre] [tb] [mode]
-mode: gram (A generated from Z, K = 544) | ln (N = 128 with the LayerNorm epilogue)"""
+mode: gram (A generated from Z, K = 544)"""
 import os
 import sys
 
@@ -23,14 +23,10 @@ def main():
 
     mode = sys.argv[6] if len(sys.argv) > 6 else ""
     Z, F = torch.randn(M, 96, device="cuda"), torch.zeros(M, device="cuda")
-    res, gam, st = torch.randn(M, N, device="cuda"), torch.randn(N, device="cuda"), torch.zeros(M, 2, device="cuda")
 
     def run():
         if mode == "gram":
             check(lib.sgrl_gemm_gram(ptr(Z), ptr(hi), ptr(lo), None, ptr(Y), N, ptr(F), None, M, N, 0, stream()))
-        elif mode == "ln":
-            check(lib.sgrl_gemm_ln(ptr(X), K, ptr(hi), ptr(lo), ptr(gam), None, ptr(res), N, ptr(gam), ptr(gam), None, None,
-                                   ptr(Y), N, None, None, ptr(st), None, 0, None, M, K, stream()))
         elif pre:
             check(lib.sgrl_gemm_presplit(ptr(X), K, 0, ptr(hi), ptr(lo), W.shape[1], tb, ptr(Y), N, M, N, K, 1.0, None, None, 0, 0, 1, stream()))
         else:

@@ -7,7 +7,7 @@ mkdir -p gpurun_out
 timeout 600 $RUN bench.py --gpus $N --steps 60 --warmup 6 --no-cpu-baseline --no-bf16 --check-replicas --rollout-sweep 1024,4096,16384,65536 \
   > gpurun_out/${TAG}_n${N}.json 2> gpurun_out/${TAG}_n${N}.err; tail -c 300 gpurun_out/${TAG}_n${N}.json; echo
 if [ "$AB" = "ab" ]; then
-  SGRL_AR_BUCKETS=0 timeout 600 $RUN bench.py --gpus $N --steps 60 --warmup 6 --no-cpu-baseline --no-bf16 --no-rollout \
+  timeout 600 $RUN bench.py --gpus $N --steps 60 --warmup 6 --no-cpu-baseline --no-bf16 --no-rollout \
     > gpurun_out/${TAG}_n${N}_flat.json 2> gpurun_out/${TAG}_n${N}_flat.err; tail -c 200 gpurun_out/${TAG}_n${N}_flat.json; echo
 fi
 timeout 600 $RUN bench.py --gpus $N --set 3d_cwhh --packed --batch 100 --steps 30 --warmup 4 \
