@@ -7,7 +7,8 @@
  * the stub a reference maintainer would add.
  *
  * Conventions: every pointer is a DEVICE pointer to contiguous row-major fp32 (int32 for
- * indices) owned by the caller; the library allocates nothing, never synchronises and never
+ * indices) owned by the caller (one exception: the HOST descriptor array of
+ * sgrl_replay_gather_packed); the library allocates nothing, never synchronises and never
  * throws.  Every call enqueues work on the given cudaStream_t (pass
  * torch.cuda.current_stream().cuda_stream) and returns 0, or a negative code with a
  * thread-local message in sgrl_last_error().  Calls are re-entrant per stream.
@@ -212,6 +213,21 @@ int sgrl_replay_gather(const float* rows, int64_t row_floats, int64_t capacity, 
                        float* obs, float* action, float* next_obs, float* reward, float* done, sgrl_stream_t stream);
 int sgrl_replay_scatter(float* rows, int64_t row_floats, int64_t capacity, const int64_t* dst, const float* staged, int n,
                         sgrl_stream_t stream);
+
+/* One gather over up to 64 replay buffers (one per morphology of a packed multi-morphology update, src/trainer.py:239-253).
+ * `parts` is a HOST array (the one exception to the device-pointer convention), read while the call enqueues the launch and
+ * free to reuse when it returns.  Part i contributes parts[i].batch rows; idx (device, sum of batch) holds the row numbers of
+ * all parts one after the other (negative ones wrap like numpy's).  The outputs are the parts' batches concatenated: sample b
+ * of part i goes to obs / next_obs + (O_i + b*obs_dim_i), action + (A_i + b*act_dim_i) and reward / done [R_i + b], where O_i,
+ * A_i and R_i sum obs_dim*batch, act_dim*batch and batch over the parts before i.  With obs_dim = 41*n and act_dim = 3*n this is
+ * the packed token layout of Agent.update_packed.  Each part's geometry is checked like sgrl_replay_gather's. */
+typedef struct {
+  const float* rows;   /* the part's buffer: capacity rows of row_floats = 2*obs_dim + act_dim + 2 */
+  int64_t row_floats, capacity;
+  int32_t obs_dim, act_dim, batch, pad_;
+} SgrlReplayPart;
+int sgrl_replay_gather_packed(const SgrlReplayPart* parts, int n_parts, const int64_t* idx, float* obs, float* action,
+                              float* next_obs, float* reward, float* done, sgrl_stream_t stream);
 
 #ifdef __cplusplus
 }

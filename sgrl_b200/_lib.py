@@ -45,6 +45,13 @@ class NetCall(C.Structure):
     ]
 
 
+class ReplayPart(C.Structure):
+    _fields_ = [
+        ("rows", c_f), ("row_floats", c_i64), ("capacity", c_i64),
+        ("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("batch", C.c_int32), ("pad_", C.c_int32),
+    ]
+
+
 _PROTOS = {
     "sgrl_version": (c_int, []),
     "sgrl_last_error": (C.c_char_p, []),
@@ -85,6 +92,7 @@ _PROTOS = {
     "sgrl_deterministic": (c_int, [c_int]),
     "sgrl_replay_gather": (c_int, [c_f, c_i64, c_i64, c_f, c_int, c_int, c_int, c_f, c_f, c_f, c_f, c_f, c_f]),
     "sgrl_replay_scatter": (c_int, [c_f, c_i64, c_i64, c_f, c_f, c_int, c_f]),
+    "sgrl_replay_gather_packed": (c_int, [C.POINTER(ReplayPart), c_int, c_f, c_f, c_f, c_f, c_f, c_f, c_f]),
 }
 EXPORTS = tuple(_PROTOS)
 

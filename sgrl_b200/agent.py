@@ -138,6 +138,7 @@ class _UpdatePlan:
         self.graphs = {}
         self.graph_launches = {}      # (actor_step, rng) -> kernels of this library inside the captured graph
         self.eager_runs = {}
+        self.i_dev = None             # row numbers of a packed buffer gather (stage_indices), allocated on first use
 
     def load(self, batches, noises):
         """Stage the replay batch of every morphology of the plan (host numpy / CPU or device tensors) into the static
@@ -175,13 +176,38 @@ class _UpdatePlan:
         if on_host:
             self.inbuf.copy_(self.h_in[k], non_blocking=True)
             self.h_ev[k].record()
+        return self.load_noise(noises)
+
+    def load_noise(self, noises):
+        """Target-policy noise of every morphology of the plan (or None: drawn in the smoothing kernel).  Returns True when
+        noise was injected."""
         if noises is None or all(nz is None for nz in noises):
             return False
-        for (t0, t1, g0, g1, n), nz in zip(parts, noises):
+        for (t0, t1, g0, g1, n), nz in zip(self.tb.parts, noises):
             if nz is None:
                 raise ValueError("target-policy noise must be given for every morphology of the plan or for none")
             self.noise[t0:t1].view(g1 - g0, n * 3).copy_(_as_tensor(nz).reshape(g1 - g0, n * 3), non_blocking=True)
         return True
+
+    def stage_indices(self, indices):
+        """Row numbers of a packed buffer gather (indices[i]: the rows drawn for morphology i) -> self.i_dev, as ONE H2D copy
+        out of a pinned, double-buffered block (the pattern of load).  Returns per morphology its slice of the host block."""
+        if self.i_dev is None:
+            G = self.tb.G
+            self.i_host = [torch.empty(G, dtype=torch.int64, pin_memory=True) for _ in range(2)]
+            self.i_np = [h.numpy() for h in self.i_host]
+            self.i_ev = [torch.cuda.Event(), torch.cuda.Event()]
+            self.i_turn = 0
+            self.i_dev = torch.empty(G, dtype=torch.int64, device=self.inbuf.device)
+        k = self.i_turn
+        self.i_turn ^= 1
+        self.i_ev[k].synchronize()                        # the copy that last read this block has finished
+        h = self.i_np[k]
+        for (_, _, g0, g1, _), idx in zip(self.tb.parts, indices):
+            h[g0:g1] = idx
+        self.i_dev.copy_(self.i_host[k], non_blocking=True)
+        self.i_ev[k].record()
+        return [h[g0:g1] for (_, _, g0, g1, _) in self.tb.parts]
 
     def replay(self, actor_step: bool, rng: bool):
         key = (actor_step, rng)
@@ -381,15 +407,50 @@ class Agent(nn.Module):
         parameters; the limb-tokens of all morphologies go through every kernel together (SURVEY.md §8f rank 1).
         morph_count: data-parallel ranks holding different numbers of morphologies pass (total morphologies / world) so the
         all-reduced gradient is the mean over all morphologies (modules.make_packed_tables)."""
+        tb = self._packed_tables_for([(g, int(b["obs"].shape[0])) for g, b in batches], morph_count)
+        return self._run_update(tb, [b for _, b in batches], it, noises)
+
+    def _packed_tables_for(self, specs, morph_count):
+        """Packed tables of specs = [(graph_dict, batch size), ...], cached per (graphs, batch sizes, morph_count).
+        update_packed and update_packed_from_buffers share the cache, so equal shapes share one plan and its graphs."""
         from .modules import make_packed_tables
-        key = tuple((id(g.get("relation")), tuple(g["parents"]), int(b["obs"].shape[0])) for g, b in batches) + (morph_count,)
+        key = tuple((id(g.get("relation")), tuple(g["parents"]), B) for g, B in specs) + (morph_count,)
         tb = self._packed_tables.get(key)
         if tb is None:
             while len(self._packed_tables) >= self.max_plans:
                 self._packed_tables.pop(next(iter(self._packed_tables)))
-            tb = make_packed_tables([(g, int(b["obs"].shape[0])) for g, b in batches], self.actor.full_arena.device, morph_count)
+            tb = make_packed_tables(specs, self.actor.full_arena.device, morph_count)
             self._packed_tables[key] = tb
-        return self._run_update(tb, [b for _, b in batches], it, noises)
+        return tb
+
+    def update_packed_from_buffers(self, parts, batch_size: int, it: int, noises=None, morph_count: Optional[float] = None,
+                                   sequential: bool = False, allow_duplicate: bool = False):
+        """``update_packed([(g, buffer.sample(batch_size)) for g, buffer in parts], it, noises, morph_count)`` without
+        materialising the batches: parts = [(graph_dict, sgrl_b200.buffer.ReplayBuffer), ...], one device buffer per morphology
+        like the reference keeps them (src/main.py:141-155, src/trainer.py:239-253).  The indices are drawn buffer by buffer in
+        list order, exactly as the reference draws them (equal seeds give equal batches; a buffer holding fewer than batch_size
+        rows gives a smaller batch), sent as ONE H2D copy, and ONE gather launch writes the rows of all buffers into the static
+        inputs of the packed update's plan, which update_packed shares.  Per step: one copy and one launch outside the graph."""
+        from .buffer import check_packed_buffers, gather_packed_into
+        dev = self.actor.full_arena.device
+        buffers = [buf for _, buf in parts]
+        check_packed_buffers(buffers, dev)
+        for i, (g, buf) in enumerate(parts):
+            n = len(g["parents"])
+            if buf.obs_dim != 41 * n or buf.action_dim != 3 * n:
+                raise ValueError(f"buffer {i} rows ({buf.obs_dim} obs, {buf.action_dim} action floats) do not match its "
+                                 f"morphology ({n} limbs)")
+            if buf.max_sample_size == 0:
+                raise ValueError(f"buffer {i} is empty")
+        idx = [buf.draw_indices(batch_size, sequential, allow_duplicate) for buf in buffers]
+        tb = self._packed_tables_for([(g, len(ix)) for (g, _), ix in zip(parts, idx)], morph_count)
+
+        def load(plan):
+            rows = plan.stage_indices(idx)
+            gather_packed_into(buffers, rows, plan.obs, plan.act, plan.nobs, plan.rew, plan.done, idx_dev=plan.i_dev)
+            return plan.load_noise(noises)
+
+        return self._run_update(tb, None, it, None, loader=load)
 
     def update_from_buffer(self, buffer, batch_size: int, it: int, noise: Optional[torch.Tensor] = None,
                            sequential: bool = False, allow_duplicate: bool = False):

@@ -16,6 +16,9 @@ fp32 row in HBM, ``[obs | action | next_obs | reward | done]``:
 * ``gather_into`` gathers straight into caller-owned buffers: ``Agent.update_from_buffer``
   uses it to fill the static inputs of its captured CUDA graph, so a training step is
   index draw -> 2 KB H2D -> gather -> graph replay, with no host synchronisation.
+* ``gather_packed_into`` does the same for several buffers at once (one per morphology) in
+  one launch, writing the packed layout of a mixed-morphology update
+  (``Agent.update_packed_from_buffers``).
 
 Same constructor, attributes (``curr``, ``max_sample_size``, ``max_buffer_size``, the five
 ``*_buffer`` arrays as numpy properties for the trainer's snapshot code,
@@ -31,7 +34,9 @@ from typing import Dict, Optional
 import numpy as np
 import torch
 
-from ._lib import check, lib, ptr, stream
+from ._lib import ReplayPart, check, lib, ptr, stream
+
+MAX_PACKED_PARTS = 64          # SGRL_REPLAY_MAX_PARTS: buffers one packed gather reads (csrc/replay.cuh)
 
 
 def _dim(space) -> int:
@@ -42,6 +47,64 @@ def _dim(space) -> int:
         raise NotImplementedError("sgrl_b200.ReplayBuffer stores continuous (Box) observations/actions only; "
                                   "the SET hot path has no discrete-action variant (buffer.py:42-45)")
     return int(shape[0])
+
+
+def _check_indices(idx: np.ndarray, capacity) -> None:
+    """numpy's error for obs_buffer[indices] (the reference fancy-indexes its arrays, buffer.py:103-120) when an index lies
+    outside [-capacity, capacity).  capacity: the buffer's row count, or one per index (a gather over several buffers)."""
+    bad = (idx >= capacity) | (idx < -capacity)
+    if bad.any():
+        cap = capacity if np.ndim(capacity) == 0 else capacity[int(np.argmax(bad))]
+        raise IndexError(f"index out of bounds for a buffer of {int(cap)} rows")
+
+
+def check_packed_buffers(buffers, device) -> None:
+    """What a packed gather needs of its buffers: 1..MAX_PACKED_PARTS of them, all with their rows on `device`."""
+    if not 1 <= len(buffers) <= MAX_PACKED_PARTS:
+        raise ValueError(f"a packed gather reads 1 to {MAX_PACKED_PARTS} buffers, got {len(buffers)}")
+    for i, buf in enumerate(buffers):
+        if buf.rows.device != torch.device(device):
+            raise ValueError(f"buffer {i} keeps its rows on {buf.rows.device}, the batch goes to {device}")
+
+
+def gather_packed_into(buffers, indices, obs, action, next_obs, reward, done, idx_dev=None) -> int:
+    """rows of several buffers -> one packed batch, in ONE gather launch (``sgrl_replay_gather_packed``).  indices[i] are the
+    row numbers drawn from buffers[i]; the outputs are contiguous fp32 device buffers holding the parts' batches one after the
+    other: obs / next_obs sum(B_i * obs_dim_i) floats, action sum(B_i * action_dim_i), reward / done sum(B_i).  With
+    obs_dim = 41 N and action_dim = 3 N that is the packed token layout of ``Agent.update_packed``.  idx_dev: a device int64
+    tensor that already holds the concatenated indices (a caller with its own upload); otherwise they are sent from pinned
+    memory here.  Returns the number of rows gathered."""
+    check_packed_buffers(buffers, obs.device)
+    if len(indices) != len(buffers):
+        raise ValueError(f"{len(buffers)} buffers, {len(indices)} index lists")
+    for buf in buffers:
+        buf.flush()
+    flat = [np.asarray(ix, dtype=np.int64).reshape(-1) for ix in indices]
+    counts = [x.size for x in flat]
+    flat = np.concatenate(flat)
+    _check_indices(flat, np.repeat(np.array([b.max_buffer_size for b in buffers], dtype=np.int64), counts))
+    G = flat.size
+    need = ((obs, sum(c * b.obs_dim for c, b in zip(counts, buffers))), (action, sum(c * b.action_dim for c, b in zip(counts, buffers))),
+            (next_obs, sum(c * b.obs_dim for c, b in zip(counts, buffers))), (reward, G), (done, G))
+    for t, n in need:
+        if t.numel() != n or not t.is_contiguous() or t.dtype != torch.float32:
+            raise ValueError(f"gather_packed_into: expected a contiguous fp32 buffer of {n} floats, got {tuple(t.shape)}")
+    if idx_dev is None:
+        idx_dev = torch.from_numpy(flat)
+        if obs.device.type == "cuda":
+            idx_dev = idx_dev.pin_memory()          # torch's caching host allocator, as in ReplayBuffer._indices_to_device
+        idx_dev = idx_dev.to(obs.device, non_blocking=True)
+    elif idx_dev.numel() != G or idx_dev.dtype != torch.int64 or idx_dev.device != obs.device or not idx_dev.is_contiguous():
+        raise ValueError(f"idx_dev: expected {G} contiguous int64 indices on {obs.device}")
+    if G == 0:
+        return 0
+    desc = (ReplayPart * len(buffers))()
+    for d, b, c in zip(desc, buffers, counts):
+        d.rows, d.row_floats, d.capacity = ptr(b.rows), b.row_floats, b.max_buffer_size
+        d.obs_dim, d.act_dim, d.batch = b.obs_dim, b.action_dim, c
+    check(lib.sgrl_replay_gather_packed(desc, len(buffers), ptr(idx_dev), ptr(obs), ptr(action), ptr(next_obs), ptr(reward), ptr(done),
+                                        stream()), "sgrl_replay_gather_packed")
+    return G
 
 
 class ReplayBuffer(object):
@@ -153,8 +216,7 @@ class ReplayBuffer(object):
         if torch.is_tensor(indices) and indices.device == self.device and indices.dtype == torch.int64:
             return indices.contiguous()
         idx = torch.as_tensor(np.asarray(indices), dtype=torch.int64).reshape(-1)
-        if idx.numel() and (int(idx.max()) >= self.max_buffer_size or int(idx.min()) < -self.max_buffer_size):
-            raise IndexError(f"index out of bounds for a buffer of {self.max_buffer_size} rows")       # numpy's error for obs_buffer[indices]
+        _check_indices(idx.numpy(), self.max_buffer_size)
         if self.device.type == "cuda":
             idx = idx.pin_memory()          # torch's caching host allocator: no cudaHostAlloc per call, reuse is stream-safe
         return idx.to(self.device, non_blocking=True)

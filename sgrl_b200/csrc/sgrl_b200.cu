@@ -22,7 +22,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 2; }
+int sgrl_version(void) { return 3; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -331,12 +331,37 @@ int sgrl_deterministic(int enable) {
   return prev;
 }
 
+static int replay_part(ReplayPart& q, const float* rows, int64_t row_floats, int64_t capacity, int obs_dim, int act_dim, int batch) {
+  SGRL_CHECK(rows != nullptr, "null pointer");
+  SGRL_CHECK(obs_dim > 0 && act_dim > 0 && row_floats == 2LL * obs_dim + act_dim + 2 && capacity > 0 && batch >= 0, "bad replay row geometry");
+  q.rows = rows; q.rw = row_floats; q.cap = capacity; q.od = obs_dim; q.ad = act_dim;
+  return 0;
+}
+
 int sgrl_replay_gather(const float* rows, int64_t row_floats, int64_t capacity, const int64_t* idx, int batch, int obs_dim, int act_dim,
                        float* obs, float* action, float* next_obs, float* reward, float* done, sgrl_stream_t stream) {
-  SGRL_CHECK(rows && idx && obs && action && next_obs && reward && done, "null pointer");
-  SGRL_CHECK(obs_dim > 0 && act_dim > 0 && row_floats == 2LL * obs_dim + act_dim + 2 && capacity > 0 && batch >= 0, "bad replay row geometry");
+  SGRL_CHECK(idx && obs && action && next_obs && reward && done, "null pointer");
+  ReplayParts P;
+  P.n = 1;
+  SGRL_TRY(replay_part(P.p[0], rows, row_floats, capacity, obs_dim, act_dim, batch));
   ReplayOut o{obs, action, next_obs, reward, done};
-  return replay_gather(rows, row_floats, reinterpret_cast<const long long*>(idx), batch, obs_dim, act_dim, capacity, o, ST(stream));
+  return replay_gather(P, &batch, reinterpret_cast<const long long*>(idx), o, ST(stream));
+}
+
+int sgrl_replay_gather_packed(const SgrlReplayPart* parts, int n_parts, const int64_t* idx, float* obs, float* action, float* next_obs,
+                              float* reward, float* done, sgrl_stream_t stream) {
+  SGRL_CHECK(parts && idx && obs && action && next_obs && reward && done, "null pointer");
+  SGRL_CHECK(n_parts >= 1 && n_parts <= SGRL_REPLAY_MAX_PARTS, "n_parts must be 1..64");
+  ReplayParts P;
+  P.n = n_parts;
+  int B[SGRL_REPLAY_MAX_PARTS];
+  for (int i = 0; i < n_parts; ++i) {
+    const SgrlReplayPart& s = parts[i];
+    SGRL_TRY(replay_part(P.p[i], s.rows, s.row_floats, s.capacity, s.obs_dim, s.act_dim, s.batch));
+    B[i] = s.batch;
+  }
+  ReplayOut o{obs, action, next_obs, reward, done};
+  return replay_gather(P, B, reinterpret_cast<const long long*>(idx), o, ST(stream));
 }
 
 int sgrl_replay_scatter(float* rows, int64_t row_floats, int64_t capacity, const int64_t* dst, const float* staged, int n, sgrl_stream_t stream) {
