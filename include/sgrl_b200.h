@@ -97,9 +97,16 @@ int sgrl_set_forward(const SgrlNetCall* call, const float* obs, int64_t obs_stri
 
 /* loss.backward() through the same modules (agent.py:151,171).  dout: nb x (T x 3|1) gradient
  * w.r.t. `out`.  need_wgrad=1 accumulates parameter gradients into call->grads (zero it first);
- * dact (critics, nullable): nb x (T x 3) gradient w.r.t. the action input (agent.py:167). */
+ * dact (critics, nullable): nb x (T x 3) gradient w.r.t. the action input (agent.py:167).
+ * sgrl_set_backward is sgrl_set_backward_dobs with dobs = NULL. */
 int sgrl_set_backward(const SgrlNetCall* call, const float* dout, int64_t dout_stride, int need_wgrad,
                       float* dact, int64_t dact_stride, sgrl_stream_t stream);
+/* The same pass, plus (dobs non-NULL) the gradient w.r.t. the observation input: nb x (T x 41), dobs_stride floats
+ * between the nets' blocks (>= 41 * T when nb > 1), overwritten.  Works with need_wgrad = 0 too.  It costs one extra
+ * launch at the end of the pass, which reads the finished backward workspace and the forward stash; with dobs = NULL
+ * the pass launches and computes exactly what sgrl_set_backward does.  Deterministic (no atomics). */
+int sgrl_set_backward_dobs(const SgrlNetCall* call, const float* dout, int64_t dout_stride, int need_wgrad,
+                           float* dact, int64_t dact_stride, float* dobs, int64_t dobs_stride, sgrl_stream_t stream);
 
 /* ---- single kernels (unit tests, profiling) ---------------------------------------------- */
 /* K1: Z=[X P^T | gd], G=Z^T Z, F=||G||+1 (subequivariant_attentions.py:90-96; SEActor.py:93-100,

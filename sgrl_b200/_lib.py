@@ -67,6 +67,7 @@ _PROTOS = {
     "sgrl_stash_info": (c_int, [c_int, c_int, c_i64, c_int, C.c_char_p, c_int, C.POINTER(c_i64), C.POINTER(c_int)]),
     "sgrl_set_forward": (c_int, [C.POINTER(NetCall), c_f, c_i64, c_f, c_i64, c_f, c_i64, c_f]),
     "sgrl_set_backward": (c_int, [C.POINTER(NetCall), c_f, c_i64, c_int, c_f, c_i64, c_f]),
+    "sgrl_set_backward_dobs": (c_int, [C.POINTER(NetCall), c_f, c_i64, c_int, c_f, c_i64, c_f, c_i64, c_f]),
     "sgrl_inv_feature_fwd": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_int, c_f]),
     "sgrl_inv_feature_bwd": (c_int, [c_f, c_f, c_f, c_f, c_f, c_int, c_f]),
     "sgrl_attention_fwd": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_int, c_int, c_f, c_f, c_f, c_f]),

@@ -71,6 +71,154 @@ __global__ void __launch_bounds__(128) embed_fwd_kernel(
   }
 }
 
+// =====================================================================================
+// Gradient w.r.t. the observation input, d obs (T,41), gathered at the end of the backward from what the data-gradient
+// chain has already produced (oracle/set_oracle.py::transformer_model).  With x = obs[t], V0[r][j] = x[3j+r], s0 = x[24:41]:
+//   d V0[r][j] += sqrt(128) * sum_c dVg0[r][c] Wg[c][j]                       g_encoder          (frame 0 dVg)
+//   d s0[k]    += sqrt(128) * sum_c dh0[c] We[c][k]                           encoder            (frame 0 dh)
+//   d V0[r][j] += sum_{p<30} dZh[r][p] gg_proj[p][j]   (+ dZh2 . g_proj, actor) head invariants (head frame dZ1 | dZ3)
+//   d s0[k]    += dSH[k]                                                      linear1_ng([s0 | h]) (head frame dSH)
+//   d V0[r][5+i] += dy_i w_r, dy_i = dOut_i max_action (1 - tanh^2)          actor output axes
+// and gd = V0[..., 1:3] (obs vectors 1, 2) enters as columns 30, 31 of every Z (each layer's Z1, Z2, Z3 and the head's) and as
+// channels 126, 127 of the attention values of both heads:
+//   d gd_j[r][k] += sum_Z dZ[r][30+k] + sum_l sum_h sum_{i in graph(j)} P_l[i][h][j] dOG_l[i][r][128h + 126 + k].
+// One warp per token: every lane accumulates its share of the 41 outputs (embedding terms: lane = channel c + 32q; Z terms:
+// lane = Z column p; attention terms: lane = (query i, head h)), then 41 butterfly sums.  No atomics, no order that depends
+// on timing: bit-identical across runs.  The token's graph comes from a binary search over cu_limbs (ragged packed tables).
+// =====================================================================================
+struct InGradP {
+  const float* dvg0; const float* dh0;             // frame 0: dVg (T,3,128), dh (T,128)                     z-stride zsW
+  const float* dzh; const float* dzh2;             // head frame: dZ1 (T,3,32); actor: dZ3 (T,3,32), else nullptr
+  const float* dsh; int ldsh;                      // head frame: d[s0 | (act) | h] (T,ldsh)
+  const float* dz[3 * MAX_LAYERS];                 // layer frames: dZ1, dZ2, dZ3 of layer l at 3l..3l+2 (only columns 30, 31 read)
+  const float* dog[MAX_LAYERS];                    // layer frames: d og (T,3,256)
+  const float* P[MAX_LAYERS];                      // stash: attention probabilities (T,2,16)                  z-stride zsS
+  const float* Wg; const float* We; const float* gg; const float* gph;   // parameters (gph: actor only)  z-stride zsP
+  int ng;                                          // columns of encoder.weight (17 actor | 20 critic)
+  const float* dout; long long zsDo;               // actor only: dOut (T,3), out (T,3), w (T,3)
+  const float* out; const float* w3; float max_action;
+  float* dobs; long long zsDobs;
+  const int* cu_limbs; int G, T, L;
+  long long zsW, zsS, zsP;
+};
+
+__global__ void __launch_bounds__(256) input_grad_kernel(InGradP p) {
+  SGRL_PDL_ENTER();
+  __shared__ float sWg[GN][128];           // sqrt(128) * g_encoder.weight, transposed
+  __shared__ float sWe[17][128];           // sqrt(128) * encoder.weight[:, :17], transposed
+  __shared__ float sZh[2][GN][32];         // [gg_proj | g_proj][:, :8] transposed; columns 30, 31 route to V0 vectors 1, 2
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, z = blockIdx.y;
+  const bool actor = p.dzh2 != nullptr;
+  const float s128 = 11.313708498984761f;
+  {
+    const float* Wg = p.Wg + z * p.zsP; const float* We = p.We + z * p.zsP; const float* gg = p.gg + z * p.zsP;
+    const float* gph = actor ? p.gph + z * p.zsP : nullptr;
+    for (int i = threadIdx.x; i < GN * 128; i += 256) { const int j = i >> 7, c = i & 127; sWg[j][c] = s128 * __ldg(Wg + c * GN + j); }
+    for (int i = threadIdx.x; i < 17 * 128; i += 256) { const int k = i >> 7, c = i & 127; sWe[k][c] = s128 * __ldg(We + c * p.ng + k); }
+    for (int i = threadIdx.x; i < 2 * GN * 32; i += 256) {
+      const int m = i / (GN * 32), j = (i >> 5) % GN, q = i & 31;
+      const float* W = m ? gph : gg;
+      sZh[m][j][q] = q < NPJ ? (W ? __ldg(W + q * (D + GN) + j) : 0.f) : (q - NPJ + 1 == j ? 1.f : 0.f);
+    }
+  }
+  __syncthreads();
+  const float e1 = lane == 30 ? 1.f : 0.f, e2 = lane == 31 ? 1.f : 0.f;
+  const long long zW = z * p.zsW, zS = z * p.zsS;
+  for (int t = blockIdx.x * 8 + warp; t < p.T; t += gridDim.x * 8) {
+    float pv[3][GN], ps[17];
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+      for (int j = 0; j < GN; ++j) pv[r][j] = 0.f;
+#pragma unroll
+    for (int k = 0; k < 17; ++k) ps[k] = 0.f;
+    // ---- embedding: Vg0 = sqrt(128) V0 Wg^T, h0 = sqrt(128) (We s0 + be) + pos
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int c = lane + 32 * q;
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const float d = __ldg(p.dvg0 + zW + ((long long)t * 3 + r) * 128 + c);
+#pragma unroll
+        for (int j = 0; j < GN; ++j) pv[r][j] = fmaf(d, sWg[j][c], pv[r][j]);
+      }
+      const float dh = __ldg(p.dh0 + zW + (long long)t * 128 + c);
+#pragma unroll
+      for (int k = 0; k < 17; ++k) ps[k] = fmaf(dh, sWe[k][c], ps[k]);
+    }
+    // ---- head invariants: Zh = [[V0 | Vg] gg_proj^T | gd] (actor: also Zh2 with g_proj), lane = column of Z
+#pragma unroll
+    for (int m = 0; m < 2; ++m) {
+      const float* dz = m ? p.dzh2 : p.dzh;
+      if (!dz) continue;
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const float d = __ldg(dz + zW + ((long long)t * 3 + r) * 32 + lane);
+#pragma unroll
+        for (int j = 0; j < GN; ++j) pv[r][j] = fmaf(d, sZh[m][j][lane], pv[r][j]);
+      }
+    }
+    // ---- gd columns 30, 31 of every encoder layer's Z1, Z2, Z3
+    for (int s = 0; s < 3 * p.L; ++s) {
+      if (lane < NPJ) continue;
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const float d = __ldg(p.dz[s] + zW + ((long long)t * 3 + r) * 32 + lane);
+        pv[r][1] = fmaf(d, e1, pv[r][1]);
+        pv[r][2] = fmaf(d, e2, pv[r][2]);
+      }
+    }
+    // ---- attention values: gd rides in channels 126, 127 of every (r, head); lane = (query i, head h) of the token's graph
+    {
+      int lo = 0, hi = p.G;                   // cu_limbs[lo] <= t < cu_limbs[hi]
+      while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (__ldg(p.cu_limbs + mid) <= t) lo = mid; else hi = mid; }
+      const int t0 = __ldg(p.cu_limbs + lo), n = __ldg(p.cu_limbs + lo + 1) - t0;
+      const int i = lane >> 1, h = lane & 1;
+      if (i < n) {
+        const long long ti = t0 + i;
+        for (int l = 0; l < p.L; ++l) {
+          const float pr = __ldg(p.P[l] + zS + ti * 32 + h * 16 + (t - t0));
+          const float* dog = p.dog[l] + zW + ti * 768 + h * 128 + 126;
+#pragma unroll
+          for (int r = 0; r < 3; ++r) {
+            const float2 v = __ldg(reinterpret_cast<const float2*>(dog + r * 256));
+            pv[r][1] = fmaf(pr, v.x, pv[r][1]);
+            pv[r][2] = fmaf(pr, v.y, pv[r][2]);
+          }
+        }
+      }
+    }
+    // ---- reduce over the warp; lane o (and 32 + o) owns obs column o
+    float v0 = 0.f, v1 = 0.f;
+#pragma unroll
+    for (int j = 0; j < GN; ++j)
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const float s = warp_sum(pv[r][j]);
+        if (lane == 3 * j + r) v0 = s;
+      }
+#pragma unroll
+    for (int k = 0; k < 17; ++k) {
+      const float s = warp_sum(ps[k]);
+      if (24 + k < 32) { if (lane == 24 + k) v0 = s; }
+      else if (lane == 24 + k - 32) v1 = s;
+    }
+    // head scalar branch [s0 | h] -> linear1_ng: columns 0..16 of dSH
+    if (lane >= 24) v0 += __ldg(p.dsh + zW + (long long)t * p.ldsh + (lane - 24));
+    if (lane < 9) v1 += __ldg(p.dsh + zW + (long long)t * p.ldsh + (lane + 8));
+    // actor output: out_i = max_action tanh(sum_r V0[r][5+i] w_r)  ->  d V0[r][5+i] += dy_i w_r  (obs columns 15..23)
+    if (actor && lane >= 15 && lane < 24) {
+      const int i = lane / 3 - 5, r = lane % 3;
+      const float a = __ldg(p.out + zS + (long long)t * 3 + i) / p.max_action;
+      const float dy = __ldg(p.dout + z * p.zsDo + (long long)t * 3 + i) * p.max_action * (1.f - a * a);
+      v0 = fmaf(dy, __ldg(p.w3 + zS + (long long)t * 3 + r), v0);
+    }
+    float* o = p.dobs + z * p.zsDobs + (long long)t * 41;
+    o[lane] = v0;
+    if (lane < 9) o[32 + lane] = v1;
+  }
+}
+
 // scatter-add of dh0 into the three positional tables
 __global__ void __launch_bounds__(128) pos_embed_bwd_kernel(
     const float* __restrict__ dH, int ldh, long long zsW, const int* __restrict__ rank3,

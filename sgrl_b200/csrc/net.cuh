@@ -548,8 +548,37 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
 // receives d/d(action) (T x 3), overwritten.
 // The data-gradient chain runs on c.stream; every dW GEMM / bias column sum forks to a side
 // stream (side_fork) right after the dY it consumes has been produced.
+// dobs (nullable): receives d/d(obs) (T x 41), overwritten, per instance stride zsDobs — one extra launch at the very end,
+// once every frame it reads is complete (input_grad below); nullptr leaves the pass exactly as it is without it.
 // ======================================================================================
-inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, int need_wgrad, float* dact, long long zsDact) {
+// d/d(obs) from the stash, the finished workspace frames and the parameters (misc.cuh input_grad_kernel); main stream, after
+// the final join.  Algorithmic bytes per token: see tools/obs_grad_bench.py.
+inline int input_grad(const NetCtx& c, const float* dOut, long long zsDo, float* dobs, long long zsDobs) {
+  const NetLayout& Y = c.lay;
+  InGradP p{};
+  p.dvg0 = c.W(0, W_DVG); p.dh0 = c.W(0, W_DH);
+  p.dzh = c.W(c.L, W_DZ1); p.dzh2 = c.kind == ACTOR ? c.W(c.L, W_DZ3) : nullptr;
+  p.dsh = c.W(c.L, W_DSH); p.ldsh = c.ks();
+  for (int l = 0; l < c.L; ++l) {
+    p.dz[3 * l] = c.W(l, W_DZ1); p.dz[3 * l + 1] = c.W(l, W_DZ2); p.dz[3 * l + 2] = c.W(l, W_DZ3);
+    p.dog[l] = c.W(l, W_DOG); p.P[l] = c.SL(l, S_P);
+  }
+  p.Wg = c.P(Y.gp[G_GENC_W]); p.We = c.P(Y.gp[G_ENC_W]); p.gg = c.P(Y.gp[G_GG_W]);
+  p.gph = c.kind == ACTOR ? c.P(Y.gp[G_GPH_W]) : nullptr;
+  p.ng = c.ng();
+  if (c.kind == ACTOR) { p.dout = dOut; p.zsDo = zsDo; p.out = c.S(T_OUT); p.w3 = c.S(T_W3); }
+  p.max_action = c.max_action;
+  p.dobs = dobs; p.zsDobs = zsDobs;
+  p.cu_limbs = c.gr.cu_limbs; p.G = c.gr.G; p.T = c.T; p.L = c.L;
+  p.zsW = c.zsW; p.zsS = c.zsS; p.zsP = c.zsP;
+  int gx = grid_for_warps(c.T); if (gx > 2 * NUM_SMS) gx = 2 * NUM_SMS;
+  launch_k(input_grad_kernel, dim3(gx, c.nb), 256, 0, c.stream, p);
+  SGRL_LAUNCH_OK();
+  return 0;
+}
+
+inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, int need_wgrad, float* dact, long long zsDact,
+                        float* dobs = nullptr, long long zsDobs = 0) {
   NetCtx c = c_in; c.bwd = 1;
   const int T = c.T, T3 = 3 * c.T, ng = c.ng(), KS = c.ks();
   const NetLayout& Y = c.lay;
@@ -771,6 +800,7 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
   if (wg) {      // gradients of the folded weights -> (rows,1024) gradient tensors
     SGRL_TRY(unfold_grads(c, fold_desc(c), st));
   }
+  if (dobs) SGRL_TRY(input_grad(c, dOut, zsDo, dobs, zsDobs));
   return 0;
 }
 

@@ -22,7 +22,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 3; }
+int sgrl_version(void) { return 4; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -118,14 +118,20 @@ int sgrl_set_forward(const SgrlNetCall* call, const float* obs, int64_t obs_stri
   return net_forward(c, obs, obs_stride, act, act_stride, out, out_stride);
 }
 
-int sgrl_set_backward(const SgrlNetCall* call, const float* dout, int64_t dout_stride, int need_wgrad, float* dact,
-                      int64_t dact_stride, sgrl_stream_t stream) {
+int sgrl_set_backward_dobs(const SgrlNetCall* call, const float* dout, int64_t dout_stride, int need_wgrad, float* dact,
+                           int64_t dact_stride, float* dobs, int64_t dobs_stride, sgrl_stream_t stream) {
   NetCtx c;
   SGRL_TRY(make_ctx(call, ST(stream), c));
   SGRL_CHECK(call->keep == 1, "backward needs a forward that ran with keep=1");
   SGRL_CHECK(call->ws != nullptr && call->ws_stride >= c.wl.total, "workspace missing or smaller than sgrl_ws_floats()");
   SGRL_CHECK(dout != nullptr, "null dout");
-  return net_backward(c, dout, dout_stride, need_wgrad, dact, dact_stride);
+  SGRL_CHECK(dobs == nullptr || c.nb == 1 || dobs_stride >= 41LL * c.T, "dobs_stride smaller than 41 * T: the nets' d/d(obs) would overlap");
+  return net_backward(c, dout, dout_stride, need_wgrad, dact, dact_stride, dobs, dobs_stride);
+}
+
+int sgrl_set_backward(const SgrlNetCall* call, const float* dout, int64_t dout_stride, int need_wgrad, float* dact,
+                      int64_t dact_stride, sgrl_stream_t stream) {
+  return sgrl_set_backward_dobs(call, dout, dout_stride, need_wgrad, dact, dact_stride, nullptr, 0, stream);
 }
 
 int sgrl_inv_feature_fwd(const float* X, const float* v0, const float* gd, const float* P1, const float* P2, float* Z, float* Z2,

@@ -350,17 +350,21 @@ class SetNetModule(nn.Module):
         return out, stash
 
     def backward_raw(self, tb: GraphTables, stash: torch.Tensor, dout: torch.Tensor, nb: int, grads: Optional[torch.Tensor],
-                     want_dact: bool, trusted_split: bool = False, ws: Optional[torch.Tensor] = None, dact: Optional[torch.Tensor] = None):
-        """dout (nb,T,od).  Accumulates parameter gradients into `grads` (None: data-only)."""
+                     want_dact: bool, trusted_split: bool = False, ws: Optional[torch.Tensor] = None, dact: Optional[torch.Tensor] = None,
+                     dobs: Optional[torch.Tensor] = None):
+        """dout (nb,T,od).  Accumulates parameter gradients into `grads` (None: data-only).  `dobs`: optional caller-owned
+        contiguous (nb,T,41) fp32 CUDA tensor that receives the gradient w.r.t. the observation input (overwritten)."""
         dev = self._arena.device
         if ws is None:
             ws = torch.empty(self.ws_floats(tb.T, nb), dtype=torch.float32, device=dev)
         if want_dact and dact is None:
             dact = torch.empty(nb, tb.T, 3, dtype=torch.float32, device=dev)
+        if dobs is not None and (dobs.dtype != torch.float32 or not dobs.is_contiguous() or tuple(dobs.shape) != (nb, tb.T, LIMB_OBS)):
+            raise ValueError(f"dobs must be a contiguous float32 ({nb}, {tb.T}, {LIMB_OBS}) tensor, got {dobs.dtype} {tuple(dobs.shape)}")
         od = 3 if self._kind == ACTOR else 1
         k = self._call(tb, nb, 1, stash, grads=grads, ws=ws, split=self._split_for(tb.T, trusted_split))
-        check(lib.sgrl_set_backward(C.byref(k), ptr(dout), tb.T * od, 1 if grads is not None else 0, ptr(dact), tb.T * 3, stream()),
-              "sgrl_set_backward")
+        check(lib.sgrl_set_backward_dobs(C.byref(k), ptr(dout), tb.T * od, 1 if grads is not None else 0, ptr(dact), tb.T * 3,
+                                         ptr(dobs), tb.T * LIMB_OBS, stream()), "sgrl_set_backward_dobs")
         return dact
 
     # ------------------------------------------------------------------ autograd bridge
@@ -369,20 +373,24 @@ class SetNetModule(nn.Module):
         tb = self._tables(B)
         obs = state.detach().to(torch.float32).contiguous()
         act = action.detach().to(torch.float32).contiguous() if action is not None else None
-        needs = torch.is_grad_enabled() and (any(p.requires_grad for p, _, _ in self._slots) or (action is not None and action.requires_grad))
+        state_grad = state.requires_grad
+        needs = torch.is_grad_enabled() and (any(p.requires_grad for p, _, _ in self._slots) or (action is not None and action.requires_grad)
+                                             or state_grad)
         if not needs:
             out, _ = self.forward_raw(tb, obs, act, keep=False, nb=nb)
             return out
-        return _SetNetFn.apply(self, tb, nb, self._anchor, obs, action if action is not None and action.requires_grad else None, act)
+        return _SetNetFn.apply(self, tb, nb, self._anchor, obs, action if action is not None and action.requires_grad else None, act,
+                               state if state_grad else None)
 
 
 class _SetNetFn(torch.autograd.Function):
     """loss.backward() support for the drop-in modules.  Parameter gradients are produced by
     the backward kernels into a scratch arena and then added to each ``p.grad`` (torch
-    semantics: accumulate until zero_grad)."""
+    semantics: accumulate until zero_grad).  Gradients w.r.t. the action (critics) and the
+    state come back through autograd like any torch input gradient."""
 
     @staticmethod
-    def forward(ctx, mod: SetNetModule, tb, nb, anchor, obs, action_in, act):
+    def forward(ctx, mod: SetNetModule, tb, nb, anchor, obs, action_in, act, state_in=None):
         out, stash = mod.forward_raw(tb, obs, act, keep=True, nb=nb)
         ctx.mod, ctx.tb, ctx.nb, ctx.stash = mod, tb, nb, stash
         ctx.want_dact = action_in is not None
@@ -392,8 +400,10 @@ class _SetNetFn(torch.autograd.Function):
     def backward(ctx, dout):
         mod, nb = ctx.mod, ctx.nb
         want_w = any(p.requires_grad for p, _, _ in mod._slots)
+        want_dobs = ctx.needs_input_grad[7]
         scratch = torch.zeros(mod._nb * mod._live, dtype=torch.float32, device=dout.device) if want_w else None
-        dact = mod.backward_raw(ctx.tb, ctx.stash, dout.contiguous().to(torch.float32), nb, scratch, ctx.want_dact)
+        dobs = torch.empty(nb, ctx.tb.T, LIMB_OBS, dtype=torch.float32, device=dout.device) if want_dobs else None
+        dact = mod.backward_raw(ctx.tb, ctx.stash, dout.contiguous().to(torch.float32), nb, scratch, ctx.want_dact, dobs=dobs)
         if want_w:
             for p, a, n in mod._slots:
                 if not p.requires_grad or a >= nb * mod._live:
@@ -407,7 +417,8 @@ class _SetNetFn(torch.autograd.Function):
         d_action = None
         if ctx.want_dact:
             d_action = dact.sum(0).view(ctx.tb.G, -1)
-        return None, None, None, None, None, d_action, None
+        d_state = dobs.sum(0).view(ctx.tb.G, -1) if want_dobs else None      # twin critics: sum over both nets, like d_action
+        return None, None, None, None, None, d_action, None, d_state
 
 
 class SEPolicy(SetNetModule):
