@@ -61,7 +61,7 @@ int sgrl_stash_info(int kind, int n_layers, int64_t T, int keep, const char* nam
 typedef struct {
   int32_t kind;        /* SGRL_ACTOR: TransformerModel(41 -> 3), SGRL_CRITIC: (44 -> 1) */
   int32_t n_layers;    /* attention_layers (3) */
-  int32_t nb;          /* nets evaluated together on the same input (2 = twin critics) */
+  int32_t nb;          /* nets evaluated together, 1..16 (2 = twin critics; 2K = the twin critics of K seeds) */
   int32_t T;           /* limb-tokens in the packed batch */
   int32_t G;           /* graphs (samples) in the batch */
   int32_t keep;        /* 1: keep every layer's activations for backward */
@@ -79,7 +79,8 @@ typedef struct {
   const float* relation;   /* packed relation tables, utils.py:476-481 */
   const int32_t* rank3;    /* (T,3) traversal ranks of each token's limb, utils.py:368-409 */
   float max_action;
-  float pad_;
+  int32_t in_nets;     /* net z reads its obs / act at obs + (z % in_nets) * obs_stride (act likewise); 0 = nb.  Seed-batched
+                        * twin critics (nets [critic1 of seeds 0..K-1 | critic2 of seeds 0..K-1]) use nb = 2K, in_nets = K */
   /* optional (both or neither): tf32 hi/lo split of `params` (same layout; sgrl_split_tf32, or kept fresh by
    * sgrl_adam_clip / sgrl_polyak) so the tcgen05 projections stream pre-split weights by TMA */
   const float* params_hi;
@@ -90,7 +91,7 @@ typedef struct {
  * TransformerModel.forward (SEActor.py:237-287), MyTransformerEncoderLayer.forward (:82-125)
  * and multi_head_attention_forward (subequivariant_attentions.py:82-154).
  * obs (T,41); act (T,3) for critics (NULL for actors); obs_stride/act_stride = floats between
- * the inputs of consecutive nets (0: shared).  out: nb x (T x 3) tanh-squashed actions scaled by
+ * consecutive input blocks (0: shared), net z reading block z % in_nets.  out: nb x (T x 3) tanh-squashed actions scaled by
  * max_action, or nb x (T x 1) per-limb Q. */
 int sgrl_set_forward(const SgrlNetCall* call, const float* obs, int64_t obs_stride, const float* act,
                      int64_t act_stride, float* out, int64_t out_stride, sgrl_stream_t stream);
@@ -181,6 +182,14 @@ int sgrl_td3_critic_loss(const float* q1, const float* q2, const float* tq1, con
                          double* reward_stats /*nullable: {sum, sum of squares} of reward*reward_scale over the G graphs, agent.py:158-161*/,
                          int G, sgrl_stream_t stream);
 int sgrl_td3_actor_loss(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, sgrl_stream_t stream);
+/* The same for K = 1..8 independent seeds sharing the tables (agent.py:136-148, 167 once per seed; sgrl_td3_critic_loss /
+ * sgrl_td3_actor_loss are the K = 1 case).  Nets in the seed-batched order: q, tq, dq (2K, T) = [critic1 of seeds 0..K-1 |
+ * critic2 of seeds 0..K-1]; reward, done (K, G); target (K, T); loss (K, accumulates); reward_stats (K, 2) or NULL.
+ * Actor: q1, dq1 (K, T) (critic1 of each seed), loss (K, accumulates).  One launch each. */
+int sgrl_td3_critic_loss_seeds(const float* q, const float* tq, const float* reward, const float* done, const int32_t* tok_graph,
+                               const float* tok_weight, float* target, float* dq, float* loss, float discount, float reward_scale, int T,
+                               double* reward_stats, int G, int K, sgrl_stream_t stream);
+int sgrl_td3_actor_loss_seeds(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, int K, sgrl_stream_t stream);
 
 /* ---- K6: optimizer (agent.py:150-156,170-178; common/functional.py:7-10) -------------------- */
 int sgrl_sumsq(const float* g, int64_t n, float* out /*accumulates*/, sgrl_stream_t stream);
@@ -191,6 +200,14 @@ int sgrl_sumsq(const float* g, int64_t n, float* out /*accumulates*/, sgrl_strea
 int sgrl_adam_clip(float* p, const float* g, float* m, float* v, int64_t n, const float* sumsq, const int32_t* step,
                    double lr, double beta1, double beta2, double eps, float max_norm, float grad_scale,
                    float* p_hi /*nullable: refreshed tf32 split of p*/, float* p_lo, sgrl_stream_t stream);
+/* Per-seed clip_grad_norm_ + Adam over an arena of `nets` nets of n_net floats each (agent.py:150-156,170-178 once per seed).
+ * sgrl_sumsq_nets writes (accumulates) one sum of squares per net into out[nets]; sgrl_adam_clip_groups clips net z by the norm
+ * over its group {z' : z' % groups == z % groups} (seed-batched twin critics: nets k and K + k, groups = K).  One launch each
+ * (sumsq: two); sgrl_sumsq / sgrl_adam_clip are the one-net, one-group case. */
+int sgrl_sumsq_nets(const float* g, int64_t n_net, int nets, float* out, sgrl_stream_t stream);
+int sgrl_adam_clip_groups(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
+                          const int32_t* step, double lr, double beta1, double beta2, double eps, float max_norm, float grad_scale,
+                          float* p_hi, float* p_lo, sgrl_stream_t stream);
 int sgrl_bump_step(int32_t* step, sgrl_stream_t stream);
 int sgrl_polyak(float* target, const float* source, int64_t n, float tau,
                 float* t_hi /*nullable: refreshed tf32 split of target[0:n_split]*/, float* t_lo, int64_t n_split, sgrl_stream_t stream);

@@ -40,7 +40,7 @@ class NetCall(C.Structure):
         ("params", c_f), ("grads", c_f), ("stash", c_f), ("stash_stride", c_i64),
         ("ws", c_f), ("ws_stride", c_i64),
         ("cu_limbs", c_f), ("rel_off", c_f), ("relation", c_f), ("rank3", c_f),
-        ("max_action", C.c_float), ("pad_", C.c_float),
+        ("max_action", C.c_float), ("in_nets", C.c_int32),
         ("params_hi", c_f), ("params_lo", c_f),
     ]
 
@@ -85,7 +85,12 @@ _PROTOS = {
     "sgrl_td3_smooth_action_rng": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, C.c_float, c_i64, C.c_uint64, c_f, c_f]),
     "sgrl_td3_critic_loss": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, C.c_float, C.c_float, c_int, c_f, c_int, c_f]),
     "sgrl_td3_actor_loss": (c_int, [c_f, c_f, c_f, c_f, c_int, c_f]),
+    "sgrl_td3_critic_loss_seeds": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, C.c_float, C.c_float, c_int, c_f, c_int, c_int, c_f]),
+    "sgrl_td3_actor_loss_seeds": (c_int, [c_f, c_f, c_f, c_f, c_int, c_int, c_f]),
     "sgrl_sumsq": (c_int, [c_f, c_i64, c_f, c_f]),
+    "sgrl_sumsq_nets": (c_int, [c_f, c_i64, c_int, c_f, c_f]),
+    "sgrl_adam_clip_groups": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_int, c_int, c_f, c_f, C.c_double, C.c_double, C.c_double, C.c_double,
+                                      C.c_float, C.c_float, c_f, c_f, c_f]),
     "sgrl_adam_clip": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_f, c_f, C.c_double, C.c_double, C.c_double, C.c_double, C.c_float, C.c_float, c_f, c_f, c_f]),
     "sgrl_bump_step": (c_int, [c_f, c_f]),
     "sgrl_polyak": (c_int, [c_f, c_f, c_i64, C.c_float, c_f, c_f, c_i64, c_f]),

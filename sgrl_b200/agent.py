@@ -27,11 +27,13 @@ from .modules import SECritic, SEPolicy, SetNetModule
 
 class FusedAdam:
     """torch.optim.Adam(lr, betas=(0.9,0.999), eps=1e-8) + clip_grad_norm_ over a module's flat
-    live arena in one kernel pass (src/agent.py:104-105,152-156,172-176)."""
+    live arena in one kernel pass (src/agent.py:104-105,152-156,172-176).  groups = K > 1: the module's nets are K independent
+    optimizers' parameters (seed-batched agents), net z clipped by the norm over the nets z' with z' % K == z % K."""
 
-    def __init__(self, module: SetNetModule, lr: float, betas=(0.9, 0.999), eps: float = 1e-8):
+    def __init__(self, module: SetNetModule, lr: float, betas=(0.9, 0.999), eps: float = 1e-8, groups: int = 1):
         self.module = module
         self.lr, self.betas, self.eps = float(lr), (float(betas[0]), float(betas[1])), float(eps)
+        self.groups = int(groups)
         self._alloc()
 
     def _alloc(self):
@@ -39,7 +41,7 @@ class FusedAdam:
         self.exp_avg = torch.zeros_like(live)
         self.exp_avg_sq = torch.zeros_like(live)
         self.step_count = torch.zeros(1, dtype=torch.int32, device=live.device)
-        self.sumsq = torch.zeros(1, dtype=torch.float32, device=live.device)
+        self.sumsq = torch.zeros(self.module._nb if self.groups > 1 else 1, dtype=torch.float32, device=live.device)   # per net
         self._arena_ptr = live.data_ptr()
 
     def _sync_device(self):
@@ -59,18 +61,19 @@ class FusedAdam:
         self._sync_device()
         m = self.module
         g, p = m.grad_arena(), m.live_arena
-        n, st = p.numel(), stream()
+        nets, st = self.sumsq.numel(), stream()
+        n_net = p.numel() // nets
         self.sumsq.zero_()
         if max_norm > 0:
-            check(lib.sgrl_sumsq(ptr(g), n, ptr(self.sumsq), st), "sgrl_sumsq")
+            check(lib.sgrl_sumsq_nets(ptr(g), n_net, nets, ptr(self.sumsq), st), "sgrl_sumsq_nets")
         check(lib.sgrl_bump_step(ptr(self.step_count), st), "sgrl_bump_step")
         fresh = m.split_is_fresh() if keep_split is None else (keep_split and m._split is not None)
         if not fresh:
             m.invalidate_split()
         hi, lo = (m._split[0], m._split[1]) if fresh else (None, None)     # keep a valid tf32 split valid (else it is rebuilt lazily)
-        check(lib.sgrl_adam_clip(ptr(p), ptr(g), ptr(self.exp_avg), ptr(self.exp_avg_sq), n, ptr(self.sumsq), ptr(self.step_count),
-                                 self.lr, self.betas[0], self.betas[1], self.eps, float(max_norm), 1.0 / world_size, ptr(hi), ptr(lo), st),
-              "sgrl_adam_clip")
+        check(lib.sgrl_adam_clip_groups(ptr(p), ptr(g), ptr(self.exp_avg), ptr(self.exp_avg_sq), n_net, nets, self.groups, ptr(self.sumsq),
+                                        ptr(self.step_count), self.lr, self.betas[0], self.betas[1], self.eps, float(max_norm), 1.0 / world_size,
+                                        ptr(hi), ptr(lo), st), "sgrl_adam_clip_groups")
 
     def state_dict(self):
         return {"step": self.step_count.clone(), "exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone(),
@@ -97,17 +100,22 @@ def soft_update_network(source: SetNetModule, target: SetNetModule, tau: float, 
 
 class _UpdatePlan:
     """Static device state of Agent.update for one (morphology tables, batch size): input staging buffers, activation
-    stashes, backward workspace, small result buffers, the three forward streams and the two captured graphs."""
+    stashes, backward workspace, small result buffers, the three forward streams and the two captured graphs.
+    With K = agent.n_seeds seeds every input and result holds K blocks, seed k's at k*T tokens / k*G graphs; the actor
+    modules run K nets, the critics 2K = [critic1 of every seed | critic2 of every seed]."""
 
     def __init__(self, agent: "Agent", tb):
         dev = agent.actor.full_arena.device
+        K = agent.n_seeds
         T, G = tb.T, tb.G
         f = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=dev)
         self.tb, self.agent = tb, agent
+        # (token0, token1, graph0, graph1, limbs) of every (seed, morphology), seed-major: where load() puts each batch
+        self.spans = [(k * T + t0, k * T + t1, k * G + g0, k * G + g1, n) for k in range(K) for (t0, t1, g0, g1, n) in tb.parts]
         # inputs as packed tokens: (T,41) observations / (T,3) actions are exactly the reference's (B, N*41) / (B, N*3) rows.
         # One contiguous block [obs | next_obs | action | reward | done] so that a host batch arrives as ONE H2D copy out of a
         # pinned, double-buffered staging block (the reference issues five pageable copies, src/agent.py:119-125)
-        sizes = (T * 41, T * 41, T * 3, G, G)
+        sizes = (K * T * 41, K * T * 41, K * T * 3, K * G, K * G)
         self.inbuf = f(sum(sizes))
         self.obs, self.nobs, self.act, self.rew, self.done = (v.view(-1, w) if w else v for v, w in
                                                               zip(torch.split(self.inbuf, sizes), (41, 41, 3, 0, 0)))
@@ -115,21 +123,22 @@ class _UpdatePlan:
         self.h_np = [tuple(x.numpy() for x in torch.split(h, sizes)) for h in self.h_in]
         self.h_ev = [torch.cuda.Event(), torch.cuda.Event()]
         self.h_turn = 0
-        self.noise = f(T, 3)
+        self.noise = f(K * T, 3)
         # target-policy noise drawn inside the smoothing kernel (Philox keyed by seed, counter = draw): graph-replay safe
         self.draw = torch.zeros(1, dtype=torch.int32, device=dev)
         self.seed = (torch.initial_seed() + 0x9E3779B97F4A7C15 * (len(agent._plans) + 1)) & 0xFFFFFFFFFFFFFFFF
-        self.rstats = torch.zeros(2, dtype=torch.float64, device=dev)     # {sum, sum of squares} of the scaled rewards
-        self.a_t, self.next_action, self.pi = f(1, T, 3), f(T, 3), f(1, T, 3)
-        self.tq, self.q, self.q1 = f(2, T, 1), f(2, T, 1), f(1, T, 1)
-        self.dq, self.dq1, self.dact = f(2, T, 1), f(1, T, 1), f(1, T, 3)
-        self.target, self.scal = f(T), torch.zeros(2, dtype=torch.float32, device=dev)
+        self.rstats = torch.zeros(K, 2, dtype=torch.float64, device=dev)  # per seed {sum, sum of squares} of the scaled rewards
+        self.a_t, self.next_action, self.pi = f(K, T, 3), f(K * T, 3), f(K, T, 3)
+        self.tq, self.q, self.q1 = f(2 * K, T, 1), f(2 * K, T, 1), f(K, T, 1)
+        self.dq, self.dq1, self.dact = f(2 * K, T, 1), f(K, T, 1), f(K, T, 3)
+        self.target = f(K * T)
+        self.scal = torch.zeros(2 * K, dtype=torch.float32, device=dev)      # critic losses of the seeds, then their actor losses
         ac, cr = agent.actor, agent.critic
-        self.stash_at = f(ac.stash_floats(T, False, 1))
-        self.stash_ct = f(cr.stash_floats(T, False, 2))
-        self.stash_c = f(cr.stash_floats(T, True, 2))
-        self.stash_a = f(ac.stash_floats(T, True, 1))
-        self.ws = f(max(cr.ws_floats(T, 2), ac.ws_floats(T, 1)))
+        self.stash_at = f(ac.stash_floats(T, False, K))
+        self.stash_ct = f(cr.stash_floats(T, False, 2 * K))
+        self.stash_c = f(cr.stash_floats(T, True, 2 * K))
+        self.stash_a = f(ac.stash_floats(T, True, K))
+        self.ws = f(max(cr.ws_floats(T, 2 * K), ac.ws_floats(T, K)))
         self.s1, self.s2, self.s3, self.s_cap = agent._streams(dev)
         self.ev_start, self.ev_a, self.ev_b, self.ev_c = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
         # the fused Adam / Polyak passes of this plan also rewrite the tf32 split (decided once per plan: the captured graphs
@@ -142,10 +151,11 @@ class _UpdatePlan:
 
     def load(self, batches, noises):
         """Stage the replay batch of every morphology of the plan (host numpy / CPU or device tensors) into the static
-        input buffers.  batches[i]: dict obs (B_i, 41 N_i), action (B_i, 3 N_i), next_obs, reward (B_i,1), done (B_i,1).
+        input buffers.  batches[i]: dict obs (B_i, 41 N_i), action (B_i, 3 N_i), next_obs, reward (B_i,1), done (B_i,1);
+        seed-major when the agent has several seeds (self.spans).
         Host batches are packed into a pinned staging block and sent as one copy; device batches are copied in place.
         Returns True when noise was injected (False: the smoothing kernel draws it)."""
-        parts = self.tb.parts
+        parts = self.spans
         if len(batches) != len(parts):
             raise ValueError(f"plan holds {len(parts)} morphologies, got {len(batches)} batches")
         keys = (("obs", 41), ("next_obs", 41), ("action", 3))
@@ -183,7 +193,9 @@ class _UpdatePlan:
         noise was injected."""
         if noises is None or all(nz is None for nz in noises):
             return False
-        for (t0, t1, g0, g1, n), nz in zip(self.tb.parts, noises):
+        if len(noises) != len(self.spans):
+            raise ValueError(f"plan holds {len(self.spans)} batches, got {len(noises)} noise tensors")
+        for (t0, t1, g0, g1, n), nz in zip(self.spans, noises):
             if nz is None:
                 raise ValueError("target-policy noise must be given for every morphology of the plan or for none")
             self.noise[t0:t1].view(g1 - g0, n * 3).copy_(_as_tensor(nz).reshape(g1 - g0, n * 3), non_blocking=True)
@@ -193,7 +205,7 @@ class _UpdatePlan:
         """Row numbers of a packed buffer gather (indices[i]: the rows drawn for morphology i) -> self.i_dev, as ONE H2D copy
         out of a pinned, double-buffered block (the pattern of load).  Returns per morphology its slice of the host block."""
         if self.i_dev is None:
-            G = self.tb.G
+            G = self.tb.G * self.agent.n_seeds
             self.i_host = [torch.empty(G, dtype=torch.int64, pin_memory=True) for _ in range(2)]
             self.i_np = [h.numpy() for h in self.i_host]
             self.i_ev = [torch.cuda.Event(), torch.cuda.Event()]
@@ -203,11 +215,11 @@ class _UpdatePlan:
         self.i_turn ^= 1
         self.i_ev[k].synchronize()                        # the copy that last read this block has finished
         h = self.i_np[k]
-        for (_, _, g0, g1, _), idx in zip(self.tb.parts, indices):
+        for (_, _, g0, g1, _), idx in zip(self.spans, indices):
             h[g0:g1] = idx
         self.i_dev.copy_(self.i_host[k], non_blocking=True)
         self.i_ev[k].record()
-        return [h[g0:g1] for (_, _, g0, g1, _) in self.tb.parts]
+        return [h[g0:g1] for (_, _, g0, g1, _) in self.spans]
 
     def replay(self, actor_step: bool, rng: bool):
         key = (actor_step, rng)
@@ -240,28 +252,31 @@ class _UpdatePlan:
 
 class _RolloutPlan:
     """Static state of the actor's rollout forward for one packed table set: pinned host staging for observations and
-    actions, their device twins, the activation scratch, and the captured graph."""
+    actions, their device twins, the activation scratch, and the captured graph.  K = agent.n_seeds actors act at once,
+    seed k on the k-th block of T tokens."""
 
     def __init__(self, agent: "Agent", tb):
         ac = agent.actor
         dev = ac.full_arena.device
         self.tb, self.agent = tb, agent
-        T = tb.T
-        self.h_obs = torch.zeros(T, 41, dtype=torch.float32, pin_memory=True)
-        self.h_out = torch.zeros(T, 3, dtype=torch.float32, pin_memory=True)
+        K, T = agent.n_seeds, tb.T
+        self.spans = [(k * T + t0, k * T + t1, g0, g1, n) for k in range(K) for (t0, t1, g0, g1, n) in tb.parts]
+        self.h_obs = torch.zeros(K * T, 41, dtype=torch.float32, pin_memory=True)
+        self.h_out = torch.zeros(K * T, 3, dtype=torch.float32, pin_memory=True)
         self.h_obs_np, self.h_out_np = self.h_obs.numpy().reshape(-1), self.h_out.numpy().reshape(-1)
-        self.obs = torch.zeros(T, 41, dtype=torch.float32, device=dev)
-        self.out = torch.zeros(1, T, 3, dtype=torch.float32, device=dev)
-        self.stash = torch.empty(ac.stash_floats(T, False, 1), dtype=torch.float32, device=dev)
+        self.obs = torch.zeros(K * T, 41, dtype=torch.float32, device=dev)
+        self.out = torch.zeros(K, T, 3, dtype=torch.float32, device=dev)
+        self.stash = torch.empty(ac.stash_floats(T, False, K), dtype=torch.float32, device=dev)
         self.graph, self.graph_launches, self.eager_runs = None, 0, 0
 
     def _forward(self):
-        self.agent.actor.forward_raw(self.tb, self.obs, None, keep=False, nb=1, trusted_split=True, out=self.out, stash=self.stash)
+        K = self.agent.n_seeds
+        self.agent.actor.forward_raw(self.tb, self.obs, None, keep=False, nb=K, in_nets=K, trusted_split=True, out=self.out, stash=self.stash)
 
     def run(self, obs_list):
-        """obs_list: one array per part of the table set (env, or the (B,41N) batch of a single-morphology plan).
-        Returns per part a numpy view (valid until the next run) of its actions."""
-        ag, parts = self.agent, self.tb.parts
+        """obs_list: one array per part of the table set (env, or the (B,41N) batch of a single-morphology plan), seed-major
+        when the agent has several seeds.  Returns per part a numpy view (valid until the next run) of its actions."""
+        ag, parts = self.agent, self.spans
         if len(obs_list) != len(parts):
             raise ValueError(f"plan holds {len(parts)} parts, got {len(obs_list)} observations")
         for (t0, t1, _, _, n), o in zip(parts, obs_list):
@@ -295,7 +310,7 @@ class _RolloutPlan:
             if self.graph is not None:
                 self.graph.replay()
                 ag.graph_replayed_launches += self.graph_launches
-        self.h_out.copy_(self.out[0], non_blocking=True)
+        self.h_out.copy_(self.out.view(-1, 3), non_blocking=True)
         torch.cuda.current_stream().synchronize()
         return [self.h_out_np[t0 * 3:t1 * 3] for (t0, t1, _, _, _) in parts]
 
@@ -323,6 +338,11 @@ class Agent(nn.Module):
             self.critic_target.full_arena.copy_(self.critic.full_arena)
         self.actor_optimizer = FusedAdam(self.actor, lr=args.lr)
         self.critic_optimizer = FusedAdam(self.critic, lr=args.lr)
+        self.n_seeds = 1
+        self._init_runtime(args)
+
+    def _init_runtime(self, args):
+        """Step state shared by Agent and SeedBatchedAgent: counters, switches and the caches of plans and graphs."""
         self.models2eval()
         self.tot_update_count = 0
         self.target_smoothing_tau = args.agent.target_smoothing_tau
@@ -398,7 +418,7 @@ class Agent(nn.Module):
         `self.use_graphs = False` runs the same sequence eagerly."""
         B = int(data_batch["obs"].shape[0])
         tb = self.actor._tables(B)
-        return self._run_update(tb, [data_batch], it, None if noise is None else [noise])
+        return self._run_update(tb, [data_batch], it, None if noise is None else [noise])[0]
 
     def update_packed(self, batches, it: int, noises=None, morph_count: Optional[float] = None):
         """One TD3 update on a PACKED batch of several morphologies: batches = [(graph_dict, data_batch), ...].  The loss is
@@ -408,7 +428,7 @@ class Agent(nn.Module):
         morph_count: data-parallel ranks holding different numbers of morphologies pass (total morphologies / world) so the
         all-reduced gradient is the mean over all morphologies (modules.make_packed_tables)."""
         tb = self._packed_tables_for([(g, int(b["obs"].shape[0])) for g, b in batches], morph_count)
-        return self._run_update(tb, [b for _, b in batches], it, noises)
+        return self._run_update(tb, [b for _, b in batches], it, noises)[0]
 
     def _packed_tables_for(self, specs, morph_count):
         """Packed tables of specs = [(graph_dict, batch size), ...], cached per (graphs, batch sizes, morph_count).
@@ -450,7 +470,7 @@ class Agent(nn.Module):
             gather_packed_into(buffers, rows, plan.obs, plan.act, plan.nobs, plan.rew, plan.done, idx_dev=plan.i_dev)
             return plan.load_noise(noises)
 
-        return self._run_update(tb, None, it, None, loader=load)
+        return self._run_update(tb, None, it, None, loader=load)[0]
 
     def update_from_buffer(self, buffer, batch_size: int, it: int, noise: Optional[torch.Tensor] = None,
                            sequential: bool = False, allow_duplicate: bool = False):
@@ -472,9 +492,10 @@ class Agent(nn.Module):
             plan.noise.view(B, n * 3).copy_(torch.as_tensor(noise, dtype=torch.float32).reshape(B, n * 3), non_blocking=True)
             return True
 
-        return self._run_update(tb, None, it, None, loader=load)
+        return self._run_update(tb, None, it, None, loader=load)[0]
 
     def _run_update(self, tb, batches, it: int, noises, loader=None):
+        """The step of every seed; returns one loss dict per seed."""
         a = self.args
         dev = self.actor.full_arena.device
         if dev.type != "cuda":
@@ -504,20 +525,26 @@ class Agent(nn.Module):
         else:
             for m in (self.critic,) + ((self.actor, self.critic_target, self.actor_target) if actor_step else ()):
                 m.invalidate_split()
+        K, P = self.n_seeds, len(tb.parts)
         scal = plan.scal.clone()
-        loss_dict = {"loss/critic_loss": scal[0]}
-        loss_dict.update(self._reward_stats([b["reward"] for b in batches] if batches is not None else [plan.rew], plan))
-        if actor_step:
-            loss_dict["loss/actor_loss"] = scal[1]
+        rewards = [[b["reward"] for b in batches[k * P:(k + 1) * P]] for k in range(K)] if batches is not None else [[plan.rew]] * K
+        loss_dicts = []
+        for k, stats in enumerate(self._reward_stats(rewards, plan)):
+            loss_dict = {"loss/critic_loss": scal[k]}
+            loss_dict.update(stats)
+            if actor_step:
+                loss_dict["loss/actor_loss"] = scal[K + k]
+            loss_dicts.append(loss_dict)
         self.tot_update_count += 1
         self._last_target = plan.target
-        return loss_dict
+        return loss_dicts
 
     def _update_impl(self, p: "_UpdatePlan", actor_step: bool, rng: bool = False):
         """Enqueue one update on the current stream (+ p.s1, p.s2 and the library's side streams).  Capture-safe:
         no allocation, no host synchronisation."""
         a = self.args
         tb, T, st = p.tb, p.tb.T, stream()
+        K = self.n_seeds          # actor modules: K nets; critics: 2K, net z reading seed z % K's batch
         world = self._world()
         main = torch.cuda.current_stream()
         p.scal.zero_()
@@ -525,66 +552,75 @@ class Agent(nn.Module):
         # ---- chain A (stream s1): y = r + (1-d) * gamma * min_i Q_i'(s', clip(pi'(s') + clip(eps)))        agent.py:127-139
         with torch.cuda.stream(p.s1):
             p.s1.wait_event(p.ev_start)
-            self.actor_target.forward_raw(tb, p.nobs, None, keep=False, trusted_split=True, out=p.a_t, stash=p.stash_at)
-            if rng:       # eps ~ N(0, policy_noise^2) drawn in the kernel; p.noise receives it (tests, logging)
+            self.actor_target.forward_raw(tb, p.nobs, None, keep=False, nb=K, in_nets=K, trusted_split=True, out=p.a_t, stash=p.stash_at)
+            if rng:       # eps ~ N(0, policy_noise^2) drawn in the kernel (each seed its own draws); p.noise receives it (tests, logging)
                 check(lib.sgrl_bump_step(ptr(p.draw), stream()))
                 check(lib.sgrl_td3_smooth_action_rng(ptr(p.a_t), ptr(p.next_action), ptr(p.noise), float(a.policy_noise), float(a.noise_clip),
-                                                     float(a.max_action), T * 3, p.seed, ptr(p.draw), stream()))
+                                                     float(a.max_action), K * T * 3, p.seed, ptr(p.draw), stream()))
             else:
-                check(lib.sgrl_td3_smooth_action(ptr(p.a_t), ptr(p.noise), ptr(p.next_action), float(a.noise_clip), float(a.max_action), T * 3,
+                check(lib.sgrl_td3_smooth_action(ptr(p.a_t), ptr(p.noise), ptr(p.next_action), float(a.noise_clip), float(a.max_action), K * T * 3,
                                                  stream()))
-            self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2, trusted_split=True, out=p.tq, stash=p.stash_ct)
+            self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2 * K, in_nets=K, trusted_split=True, out=p.tq,
+                                           stash=p.stash_ct)
             check(lib.sgrl_stream_fence(stream()))       # eager runs only (no-op under capture): see csrc/net.cuh stream_fence
             p.ev_a.record(p.s1)
         # ---- chain C (stream s2, delayed actor step only): pi(s) — independent of the critic step           agent.py:167
         if actor_step:
             with torch.cuda.stream(p.s2):
                 p.s2.wait_event(p.ev_start)
-                self.actor.forward_raw(tb, p.obs, None, keep=True, trusted_split=True, out=p.pi, stash=p.stash_a)
+                self.actor.forward_raw(tb, p.obs, None, keep=True, nb=K, in_nets=K, trusted_split=True, out=p.pi, stash=p.stash_a)
                 check(lib.sgrl_stream_fence(stream()))
                 p.ev_c.record(p.s2)
         # ---- chain B (stream s3, then main): critic step                                                    agent.py:142-156
         with torch.cuda.stream(p.s3):
             p.s3.wait_event(p.ev_start)
-            self.critic.forward_raw(tb, p.obs, p.act, keep=True, nb=2, trusted_split=True, out=p.q, stash=p.stash_c)
+            self.critic.forward_raw(tb, p.obs, p.act, keep=True, nb=2 * K, in_nets=K, trusted_split=True, out=p.q, stash=p.stash_c)
             check(lib.sgrl_stream_fence(stream()))
             p.ev_b.record(p.s3)
         main.wait_event(p.ev_b)
         main.wait_event(p.ev_a)
-        check(lib.sgrl_td3_critic_loss(ptr(p.q[0]), ptr(p.q[1]), ptr(p.tq[0]), ptr(p.tq[1]), ptr(p.rew), ptr(p.done), ptr(tb.tok_graph),
-                                       ptr(tb.tok_weight), ptr(p.target), ptr(p.dq[0]), ptr(p.dq[1]), ptr(p.scal), float(a.discount), float(self.reward_scale), T,
-                                       ptr(p.rstats), tb.G, st))
+        check(lib.sgrl_td3_critic_loss_seeds(ptr(p.q), ptr(p.tq), ptr(p.rew), ptr(p.done), ptr(tb.tok_graph), ptr(tb.tok_weight), ptr(p.target),
+                                             ptr(p.dq), ptr(p.scal), float(a.discount), float(self.reward_scale), T, ptr(p.rstats), tb.G, K, st))
         self.critic_optimizer.zero_grad()
-        self._backward_allreduce(self.critic, tb, p.stash_c, p.dq, 2, p.ws, world)
+        self._backward_allreduce(self.critic, tb, p.stash_c, p.dq, 2 * K, p.ws, world)
         self.critic_optimizer.step(max_norm=float(a.grad_clipping_value), world_size=world, keep_split=p.keep_split)
         # ---- delayed actor step + Polyak                                                                    agent.py:165-180
         if actor_step:
             main.wait_event(p.ev_c)
-            self.critic.forward_raw(tb, p.obs, p.pi[0], keep=True, nb=1, trusted_split=True, out=p.q1, stash=p.stash_c)
-            check(lib.sgrl_td3_actor_loss(ptr(p.q1), ptr(tb.tok_weight), ptr(p.dq1), ptr(p.scal[1:]), T, st))
-            self.critic.backward_raw(tb, p.stash_c, p.dq1, 1, None, True, trusted_split=True, ws=p.ws, dact=p.dact)   # only d/d(action)
+            # critic1 of every seed = the first K nets of the critic arena
+            self.critic.forward_raw(tb, p.obs, p.pi, keep=True, nb=K, in_nets=K, trusted_split=True, out=p.q1, stash=p.stash_c)
+            check(lib.sgrl_td3_actor_loss_seeds(ptr(p.q1), ptr(tb.tok_weight), ptr(p.dq1), ptr(p.scal[K:]), T, K, st))
+            self.critic.backward_raw(tb, p.stash_c, p.dq1, K, None, True, trusted_split=True, ws=p.ws, dact=p.dact)   # only d/d(action)
             self.actor_optimizer.zero_grad()
-            self._backward_allreduce(self.actor, tb, p.stash_a, p.dact, 1, p.ws, world)
+            self._backward_allreduce(self.actor, tb, p.stash_a, p.dact, K, p.ws, world)
             self.actor_optimizer.step(max_norm=float(a.grad_clipping_value), world_size=world, keep_split=p.keep_split)
             self.try_update_target_network(keep_split=p.keep_split)
 
     train_step = update   # BASELINE.json calls the TD3 step "train()"; the reference name is update (agent.py:117)
 
-    def _reward_stats(self, rewards_in, plan):
+    def _reward_stats(self, rewards_per_seed, plan):
         """agent.py:158-162 returns Python floats (two device syncs in the reference).  When the batch arrived from host
         memory the statistics are computed there and nothing synchronises; otherwise they come from the sum / sum of
-        squares the critic-loss kernel accumulated in fp64 (one 16-byte read; `lazy_stats`: left on the device)."""
+        squares the critic-loss kernel accumulated in fp64 (one 16-byte read per seed, one sync for all of them;
+        `lazy_stats`: left on the device).  rewards_per_seed[k]: the reward arrays of seed k; returns one dict per seed."""
         s = self.reward_scale
-        if all(isinstance(r, np.ndarray) or (torch.is_tensor(r) and not r.is_cuda) for r in rewards_in):
-            r = torch.cat([torch.as_tensor(x, dtype=torch.float32).reshape(-1) for x in rewards_in]) * s
-            return {"misc/train_reward_mean": r.mean().item(), "misc/train_reward_var": r.var().item() if r.numel() > 1 else float("nan")}
+        if all(isinstance(r, np.ndarray) or (torch.is_tensor(r) and not r.is_cuda) for rs in rewards_per_seed for r in rs):
+            out = []
+            for rewards_in in rewards_per_seed:
+                r = torch.cat([torch.as_tensor(x, dtype=torch.float32).reshape(-1) for x in rewards_in]) * s
+                out.append({"misc/train_reward_mean": r.mean().item(), "misc/train_reward_var": r.var().item() if r.numel() > 1 else float("nan")})
+            return out
         n = plan.tb.G
-        st = plan.rstats.clone() if self.lazy_stats else plan.rstats.cpu()
-        mean = st[0] / n
-        var = (st[1] - st[0] * st[0] / n) / (n - 1) if n > 1 else st[0] * float("nan")
-        if self.lazy_stats:
-            return {"misc/train_reward_mean": mean, "misc/train_reward_var": var}
-        return {"misc/train_reward_mean": float(mean), "misc/train_reward_var": float(var)}
+        sts = plan.rstats.clone() if self.lazy_stats else plan.rstats.cpu()
+        out = []
+        for st in sts:
+            mean = st[0] / n
+            var = (st[1] - st[0] * st[0] / n) / (n - 1) if n > 1 else st[0] * float("nan")
+            if self.lazy_stats:
+                out.append({"misc/train_reward_mean": mean, "misc/train_reward_var": var})
+            else:
+                out.append({"misc/train_reward_mean": float(mean), "misc/train_reward_var": float(var)})
+        return out
 
     def try_update_target_network(self, keep_split: Optional[bool] = None):
         soft_update_network(self.critic, self.critic_target, self.target_smoothing_tau, keep_split)
@@ -629,9 +665,14 @@ class Agent(nn.Module):
         (mixed morphologies) are packed into one ragged batch: obs_list[i] is env i's un-padded (41*N_i,) observation,
         graphs[i] its graph dict; returns [ (1, 3*N_i) numpy action ] in env order.  One pinned H2D copy, one replayed
         CUDA graph of the packed actor forward, one D2H copy.  Exploration noise / zero-padding stay with the caller."""
-        from .modules import make_packed_tables
         if len(obs_list) != len(graphs) or not obs_list:
             raise ValueError("select_actions needs one graph per observation")
+        out = self._rollout_plan(self._rollout_tables_for(graphs)).run(obs_list)
+        return [o.reshape(1, -1).copy() for o in out]
+
+    def _rollout_tables_for(self, graphs):
+        """Packed tables of one env per graph, cached per list of graphs."""
+        from .modules import make_packed_tables
         key = tuple((id(g.get("relation")), tuple(g["parents"])) for g in graphs)
         tb = self._rollout_tables.get(key)
         if tb is None:
@@ -639,8 +680,7 @@ class Agent(nn.Module):
                 self._rollout_tables.pop(next(iter(self._rollout_tables)))
             tb = make_packed_tables([(g, 1) for g in graphs], self.actor.full_arena.device)
             self._rollout_tables[key] = tb
-        out = self._rollout_plan(tb).run(obs_list)
-        return [o.reshape(1, -1).copy() for o in out]
+        return tb
 
     def change_morphology(self, graph):
         self.actor.change_morphology(graph)

@@ -21,6 +21,9 @@ extern long long g_launches;   // kernels launched by this library (bench.py's g
 #define SGRL_TRY(call) do { int r__ = (call); if (r__ != 0) return r__; } while (0)
 
 constexpr int NUM_SMS = 148;  // B200
+// nets of one module call (SgrlNetCall.nb) and of one grouped optimizer pass: K seeds of twin critics are 2K nets.  Nothing
+// else bounds nb: grids put it on gridDim.y / gridDim.z and the GEMM cost model, split-K and tensor maps take it as a count.
+constexpr int MAX_NETS = 16;
 
 // ---- launches: every kernel of the library is launched with programmatic dependent launch (PDL) allowed, and begins
 // with SGRL_PDL_ENTER(): "my dependents may start launching" + "wait until the kernel before me has completed and its

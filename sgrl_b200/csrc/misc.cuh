@@ -21,12 +21,12 @@ __global__ void __launch_bounds__(128) embed_fwd_kernel(
     const float* __restrict__ Wg, const float* __restrict__ We, const float* __restrict__ be,
     const float* __restrict__ E0, const float* __restrict__ E1, const float* __restrict__ E2, long long zsP,
     float* __restrict__ V0, float* __restrict__ GD, float* __restrict__ SH, int ldsh,
-    float* __restrict__ VG, float* __restrict__ H, int ldh, long long zsS, int T, int ng) {
+    float* __restrict__ VG, float* __restrict__ H, int ldh, long long zsS, int T, int ng, int in_nets) {
   SGRL_PDL_ENTER();
   __shared__ float xs[E_TOK][48];
   __shared__ int rk[E_TOK][3];
   const int c = threadIdx.x, z = blockIdx.y;
-  obs += z * zsObs; if (act) act += z * zsAct;
+  obs += (z % in_nets) * zsObs; if (act) act += (z % in_nets) * zsAct;     // nets z, z + in_nets, ... share one input block
   Wg += z * zsP; We += z * zsP; be += z * zsP; E0 += z * zsP; E1 += z * zsP; E2 += z * zsP;
   V0 += z * zsS; GD += z * zsS; SH += z * zsS; VG += z * zsS; H += z * zsS;
   float wg[GN], we[20];

@@ -1,6 +1,7 @@
 // SET network executor: sequences the kernels of one forward / backward pass of nb
-// identical-shape networks (nb=2: twin critics sharing their input, SECritic.py:86-87)
-// over a packed batch of limb graphs.  Host C++ only; every launch goes to ctx.stream.
+// identical-shape networks (nb=2: twin critics sharing their input, SECritic.py:86-87;
+// nb=2K: the twin critics of K seeds, net z reading seed z % K's batch) over a packed batch
+// of limb graphs.  Host C++ only; every launch goes to ctx.stream.
 //
 // Forward follows TransformerModel.forward (SEActor.py:237-287) / SURVEY.md Appendix A/G;
 // backward follows SURVEY.md Appendix H.  Activations needed by the backward live in the
@@ -112,6 +113,7 @@ inline bool side_off(const Side& sd) { return !sd.enabled || g_prof.on || det_en
 
 struct NetCtx {
   int kind, L, nb, T;
+  int in_nets;                            // net z reads input block z % in_nets (1..nb; only the embedding reads the inputs)
   int keep;                               // 0: inference pass (nothing kept for a backward)
   NetLayout lay;
   const float* params; long long zsP;     // live arena; z-stride = lay.live_floats
@@ -368,7 +370,7 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
     int gx = ceil_div(T, E_TOK); if (gx > 4 * NUM_SMS) gx = 4 * NUM_SMS;
     launch_k(embed_fwd_kernel, dim3(gx, c.nb), 128, 0, st, obs, zsObs, c.kind == CRITIC ? act : nullptr, zsAct, c.rank3,
         c.P(Y.gp[G_GENC_W]), c.P(Y.gp[G_ENC_W]), c.P(Y.gp[G_ENC_B]), c.P(Y.gp[G_POS0]), c.P(Y.gp[G_POS1]), c.P(Y.gp[G_POS2]), c.zsP,
-        c.S(T_V0), c.S(T_GD), c.S(T_SH), KS, c.SL(0, S_VGIN), c.SL(0, S_UA) + 128, 256, zS, T, ng);
+        c.S(T_V0), c.S(T_GD), c.S(T_SH), KS, c.SL(0, S_VGIN), c.SL(0, S_UA) + 128, 256, zS, T, ng, c.in_nets);
     SGRL_LAUNCH_OK();
   }
   if (fused && !fold_pending) SGRL_TRY(fold_weights(c, st));

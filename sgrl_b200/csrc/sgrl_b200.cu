@@ -22,7 +22,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 4; }
+int sgrl_version(void) { return 5; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -91,10 +91,12 @@ static int make_ctx(const SgrlNetCall* k, cudaStream_t st, NetCtx& c) {
   SGRL_CHECK(k != nullptr, "null call");
   SGRL_CHECK(k->kind == ACTOR || k->kind == CRITIC, "kind must be SGRL_ACTOR or SGRL_CRITIC");
   SGRL_CHECK(k->n_layers >= 1 && k->n_layers <= MAX_LAYERS, "n_layers out of range");
-  SGRL_CHECK(k->nb >= 1 && k->nb <= 4, "nb out of range");
+  SGRL_CHECK(k->nb >= 1 && k->nb <= MAX_NETS, "nb out of range (1..16)");
+  SGRL_CHECK(k->in_nets >= 0 && k->in_nets <= k->nb, "in_nets out of range (0..nb)");
   SGRL_CHECK(k->T >= 1 && k->G >= 1, "empty batch");
   SGRL_CHECK(k->params && k->stash && k->cu_limbs && k->relation && k->rank3, "null device pointer");
   c.kind = k->kind; c.L = k->n_layers; c.nb = k->nb; c.T = k->T; c.keep = k->keep;
+  c.in_nets = k->in_nets ? k->in_nets : k->nb;
   c.lay = make_layout(k->kind, k->n_layers);
   c.params = k->params; c.zsP = c.lay.live_floats;
   SGRL_CHECK((k->params_hi == nullptr) == (k->params_lo == nullptr), "params_hi and params_lo go together");
@@ -246,29 +248,59 @@ int sgrl_td3_smooth_action_rng(const float* pi_target, float* next_action, float
   return 0;
 }
 
+// grid.y = seed: the kernels offset every per-seed operand by blockIdx.y (td3.cuh); one seed is the single-agent entry point
+static int critic_loss(const float* q1, const float* q2, const float* tq1, const float* tq2, const float* reward, const float* done,
+                       const int32_t* tok_graph, const float* tok_weight, float* target, float* dq1, float* dq2, float* loss, float discount,
+                       float reward_scale, int T, double* reward_stats, int G, int K, cudaStream_t st) {
+  SGRL_CHECK(q1 && q2 && tq1 && tq2 && reward && done && tok_graph && target && dq1 && dq2 && loss, "null pointer");
+  SGRL_CHECK(K >= 1 && K <= MAX_NETS / 2 && T >= 1 && G >= 1, "bad seed count or batch");
+  int gx = ceil_div(T, 256); if (gx > NUM_SMS) gx = NUM_SMS;
+  if (det_enabled()) gx = 1;      // the loss scalar: one add
+  launch_k(td3_critic_loss_kernel, dim3(gx, K), 256, 0, st, q1, q2, tq1, tq2, reward, done, tok_graph, tok_weight, target, dq1, dq2, loss, discount, reward_scale, T, reward_stats, G);
+  SGRL_LAUNCH_OK();
+  return 0;
+}
+
+static int actor_loss(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, int K, cudaStream_t st) {
+  SGRL_CHECK(q1 && dq1 && loss, "null pointer");
+  SGRL_CHECK(K >= 1 && K <= MAX_NETS && T >= 1, "bad seed count or batch");
+  int gx = ceil_div(T, 256); if (gx > NUM_SMS) gx = NUM_SMS;
+  if (det_enabled()) gx = 1;      // the loss scalar: one add
+  launch_k(td3_actor_loss_kernel, dim3(gx, K), 256, 0, st, q1, tok_weight, dq1, loss, T);
+  SGRL_LAUNCH_OK();
+  return 0;
+}
+
 int sgrl_td3_critic_loss(const float* q1, const float* q2, const float* tq1, const float* tq2, const float* reward, const float* done,
                          const int32_t* tok_graph, const float* tok_weight, float* target, float* dq1, float* dq2, float* loss, float discount,
                          float reward_scale, int T, double* reward_stats, int G, sgrl_stream_t stream) {
-  SGRL_CHECK(q1 && q2 && tq1 && tq2 && reward && done && tok_graph && target && dq1 && dq2 && loss, "null pointer");
-  int gx = ceil_div(T, 256); if (gx > NUM_SMS) gx = NUM_SMS;
-  if (det_enabled()) gx = 1;      // the loss scalar: one add
-  launch_k(td3_critic_loss_kernel, gx, 256, 0, ST(stream), q1, q2, tq1, tq2, reward, done, tok_graph, tok_weight, target, dq1, dq2, loss, discount, reward_scale, T, reward_stats, G);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return critic_loss(q1, q2, tq1, tq2, reward, done, tok_graph, tok_weight, target, dq1, dq2, loss, discount, reward_scale, T, reward_stats,
+                     G, 1, ST(stream));
+}
+
+int sgrl_td3_critic_loss_seeds(const float* q, const float* tq, const float* reward, const float* done, const int32_t* tok_graph,
+                               const float* tok_weight, float* target, float* dq, float* loss, float discount, float reward_scale, int T,
+                               double* reward_stats, int G, int K, sgrl_stream_t stream) {
+  SGRL_CHECK(q && tq && dq, "null pointer");
+  const long long h = (long long)K * T;      // critic2 of seed k is net K + k
+  return critic_loss(q, q + h, tq, tq + h, reward, done, tok_graph, tok_weight, target, dq, dq + h, loss, discount, reward_scale, T,
+                     reward_stats, G, K, ST(stream));
 }
 
 int sgrl_td3_actor_loss(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, sgrl_stream_t stream) {
-  SGRL_CHECK(q1 && dq1 && loss, "null pointer");
-  int gx = ceil_div(T, 256); if (gx > NUM_SMS) gx = NUM_SMS;
-  if (det_enabled()) gx = 1;      // the loss scalar: one add
-  launch_k(td3_actor_loss_kernel, gx, 256, 0, ST(stream), q1, tok_weight, dq1, loss, T);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return actor_loss(q1, tok_weight, dq1, loss, T, 1, ST(stream));
 }
 
-int sgrl_sumsq(const float* g, int64_t n, float* out, sgrl_stream_t stream) {
+int sgrl_td3_actor_loss_seeds(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, int K, sgrl_stream_t stream) {
+  return actor_loss(q1, tok_weight, dq1, loss, T, K, ST(stream));
+}
+
+int sgrl_sumsq(const float* g, int64_t n, float* out, sgrl_stream_t stream) { return sgrl_sumsq_nets(g, n, 1, out, stream); }
+
+int sgrl_sumsq_nets(const float* g, int64_t n, int nets, float* out, sgrl_stream_t stream) {
   SGRL_CHECK(g && out, "null pointer");
   SGRL_CHECK(aligned16(g), "gradient arena must be 16-byte aligned");
+  SGRL_CHECK(nets >= 1 && nets <= MAX_NETS && (nets == 1 || (n & 3) == 0), "nets must be 1..16, n % 4 == 0 for several nets");
   // scratch for the per-block partial sums: one slot per destination scalar (hashed), so the optimizers of different modules
   // never share one; allocated on first use (an eager call: Agent.update runs each plan eagerly before capturing it)
   constexpr int SLOTS = 16;
@@ -283,10 +315,10 @@ int sgrl_sumsq(const float* g, int64_t n, float* out, sgrl_stream_t stream) {
     SGRL_CUDA(cudaMalloc(&scratch[dev], sizeof(float) * SLOTS * SUMSQ_MAX_BLOCKS));
   }
   float* part = scratch[dev] + ((reinterpret_cast<uintptr_t>(out) >> 2) * 2654435761u % SLOTS) * SUMSQ_MAX_BLOCKS;
-  int nb = grid_for_flat(n); if (nb > SUMSQ_MAX_BLOCKS) nb = SUMSQ_MAX_BLOCKS;
-  launch_k(sumsq_partial_kernel, nb, 256, 0, ST(stream), g, (long long)n, part);
+  int nb = grid_for_flat(n); if (nb > SUMSQ_MAX_BLOCKS / nets) nb = SUMSQ_MAX_BLOCKS / nets;      // blocks per net
+  launch_k(sumsq_partial_kernel, dim3(nb, nets), 256, 0, ST(stream), g, (long long)n, part);
   SGRL_LAUNCH_OK();
-  launch_k(sumsq_final_kernel, 1, 256, 0, ST(stream), (const float*)part, nb, out);
+  launch_k(sumsq_final_kernel, nets, 256, 0, ST(stream), (const float*)part, nb, out);
   SGRL_LAUNCH_OK();
   return 0;
 }
@@ -302,11 +334,19 @@ int sgrl_split_tf32(const float* w, float* hi, float* lo, int64_t n, sgrl_stream
 int sgrl_adam_clip(float* p, const float* g, float* m, float* v, int64_t n, const float* sumsq, const int32_t* step, double lr,
                    double beta1, double beta2, double eps, float max_norm, float grad_scale, float* p_hi, float* p_lo,
                    sgrl_stream_t stream) {
+  return sgrl_adam_clip_groups(p, g, m, v, n, 1, 1, sumsq, step, lr, beta1, beta2, eps, max_norm, grad_scale, p_hi, p_lo, stream);
+}
+
+int sgrl_adam_clip_groups(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
+                          const int32_t* step, double lr, double beta1, double beta2, double eps, float max_norm, float grad_scale,
+                          float* p_hi, float* p_lo, sgrl_stream_t stream) {
   SGRL_CHECK(p && g && m && v && sumsq && step, "null pointer");
+  SGRL_CHECK(nets >= 1 && nets <= MAX_NETS && groups >= 1 && groups <= nets && nets % groups == 0, "nets must be 1..16, a multiple of groups");
   SGRL_CHECK((p_hi == nullptr) == (p_lo == nullptr) && (!p_hi || (aligned16(p_hi) && aligned16(p_lo))), "p_hi/p_lo go together, 16-byte aligned");
-  SGRL_CHECK((n & 3) == 0 && aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v), "arenas must be 16-byte aligned, n % 4 == 0");
+  SGRL_CHECK((n_net & 3) == 0 && aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v), "arenas must be 16-byte aligned, n % 4 == 0");
+  const int64_t n = n_net * nets;
   AdamCfg c{lr, beta1, beta2, (float)beta1, (float)beta2, (float)(1.0 - beta1), (float)(1.0 - beta2), (float)eps, max_norm, grad_scale};
-  launch_k(adam_clip_kernel, grid_for_flat(n), 256, 0, ST(stream), p, g, m, v, n, sumsq, step, c, p_hi, p_lo);
+  launch_k(adam_clip_kernel, grid_for_flat(n), 256, 0, ST(stream), p, g, m, v, (long long)n, sumsq, step, c, p_hi, p_lo, (long long)n_net, nets, groups);
   SGRL_LAUNCH_OK();
   return 0;
 }

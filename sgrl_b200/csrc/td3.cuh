@@ -66,6 +66,12 @@ __global__ void __launch_bounds__(256) td3_critic_loss_kernel(
     float discount, float reward_scale, int T, double* __restrict__ rstats, int G) {
   SGRL_PDL_ENTER();
   __shared__ float red[8];
+  {      // seed k = blockIdx.y (sgrl_td3_critic_loss_seeds): its own (T) outputs, (G) rewards, loss and reward statistics
+    const long long k = blockIdx.y;
+    q1 += k * T; q2 += k * T; tq1 += k * T; tq2 += k * T; target += k * T; dq1 += k * T; dq2 += k * T;
+    reward += k * G; done += k * G; loss += k;
+    if (rstats) rstats += 2 * k;
+  }
   if (rstats && blockIdx.x == 0 && threadIdx.x < 32) {
     // sum and sum of squares of the scaled rewards (agent.py:158-161 logs their mean / variance): fp64, one warp
     double s1 = 0.0, s2 = 0.0;
@@ -103,6 +109,7 @@ __global__ void __launch_bounds__(256) td3_actor_loss_kernel(const float* __rest
                                                              float* __restrict__ loss, int T) {
   SGRL_PDL_ENTER();
   __shared__ float red[8];
+  q1 += (long long)blockIdx.y * T; dq += (long long)blockIdx.y * T; loss += blockIdx.y;      // seed blockIdx.y
   float acc = 0.f;
   const float invT = 1.f / (float)T;
   for (int t = blockIdx.x * 256 + threadIdx.x; t < T; t += gridDim.x * 256) {
@@ -121,12 +128,14 @@ __global__ void __launch_bounds__(256) td3_actor_loss_kernel(const float* __rest
 }
 
 // sum of squares of a flat gradient buffer                                                  clip_grad_norm_, agent.py:152-155
-// Deterministic (no atomics): every block leaves its partial sum in a scratch slot, a second one-block launch adds the
-// partials in index order.  The norm feeds the clip coefficient of every data-parallel replica: with an atomic reduction the
-// ranks disagreed in its last bit and the replicas drifted apart after ~40 steps (tools/dp_debug.py, bench.py --check-replicas).
+// Deterministic (no atomics): every block leaves its partial sum in a scratch slot, a second launch adds the partials in
+// index order.  The norm feeds the clip coefficient of every data-parallel replica: with an atomic reduction the ranks
+// disagreed in its last bit and the replicas drifted apart after ~40 steps (tools/dp_debug.py, bench.py --check-replicas).
+// blockIdx.y / the final kernel's blockIdx.x = net: one sum per net of n floats (sgrl_sumsq_nets; one net = sgrl_sumsq).
 constexpr int SUMSQ_MAX_BLOCKS = 2048;
 __global__ void __launch_bounds__(256) sumsq_partial_kernel(const float* __restrict__ g, long long n, float* __restrict__ partial) {
   SGRL_PDL_ENTER();
+  g += blockIdx.y * n; partial += blockIdx.y * gridDim.x;
   __shared__ float red[8];
   float acc = 0.f;
   const long long n4 = n >> 2;
@@ -147,6 +156,7 @@ __global__ void __launch_bounds__(256) sumsq_partial_kernel(const float* __restr
 }
 __global__ void __launch_bounds__(256) sumsq_final_kernel(const float* __restrict__ partial, int nb, float* __restrict__ out) {
   SGRL_PDL_ENTER();
+  partial += blockIdx.x * nb; out += blockIdx.x;
   __shared__ double red[8];
   double acc = 0.0;
   for (int i = threadIdx.x; i < nb; i += 256) acc += (double)partial[i];
@@ -171,6 +181,8 @@ struct AdamCfg { double lr, beta1d, beta2d; float beta1, beta2, omb1, omb2, eps,
 //   coef = min(1, max_norm / (||g|| + 1e-6))     (torch.nn.utils.clip_grad_norm_)
 //   m = m + (1-b1)(g - m);  v = b2 v + (1-b2) g^2;  p -= lr/(1-b1^t) * m / (sqrt(v)/sqrt(1-b2^t) + eps)
 // grad_scale pre-multiplies g (1/world_size after a sum all-reduce).
+// Per-group clipping (sgrl_adam_clip_groups): the arena holds `nets` nets of n_net floats and sumsq one sum per net; net z is
+// clipped by the norm over its group {z' : z' % groups == z % groups}.  One net, one group: the single global norm.
 // hi/lo (nullable): the refreshed tf32 split of the parameters for the tcgen05 projections (csrc/gemm_tc.cuh).
 __device__ __forceinline__ void split_store4(float4 pv, float* hi, float* lo, long long i4) {
   float4 h, l;
@@ -192,22 +204,28 @@ __global__ void __launch_bounds__(256) split_tf32_kernel(const float* __restrict
 
 __global__ void __launch_bounds__(256) adam_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                         float* __restrict__ v, long long n, const float* __restrict__ sumsq,
-                                                        const int* __restrict__ step, AdamCfg c, float* __restrict__ hi, float* __restrict__ lo) {
+                                                        const int* __restrict__ step, AdamCfg c, float* __restrict__ hi, float* __restrict__ lo,
+                                                        long long n_net, int nets, int groups) {
   SGRL_PDL_ENTER();
-  __shared__ float sh[3];
-  if (threadIdx.x == 0) {
-    const float nrm = sqrtf(*sumsq) * c.grad_scale;
+  __shared__ float sh[2 + MAX_NETS];      // step size, sqrt of the second bias correction, per group: clip coef * grad_scale
+  if (threadIdx.x < groups) {
+    float s = sumsq[threadIdx.x];
+    for (int z = threadIdx.x + groups; z < nets; z += groups) s += sumsq[z];
+    const float nrm = sqrtf(s) * c.grad_scale;
     float coef = 1.f;
     if (c.max_norm > 0.f) { coef = c.max_norm / (nrm + 1e-6f); coef = coef > 1.f ? 1.f : coef; }
+    sh[2 + threadIdx.x] = coef * c.grad_scale;
+  }
+  if (threadIdx.x == 0) {
     const double t = (double)(*step);
-    sh[0] = coef * c.grad_scale;
-    sh[1] = (float)(c.lr / (1.0 - pow(c.beta1d, t)));
-    sh[2] = (float)sqrt(1.0 - pow(c.beta2d, t));
+    sh[0] = (float)(c.lr / (1.0 - pow(c.beta1d, t)));
+    sh[1] = (float)sqrt(1.0 - pow(c.beta2d, t));
   }
   __syncthreads();
-  const float gs = sh[0], step_size = sh[1], bc2s = sh[2];
+  const float step_size = sh[0], bc2s = sh[1];
   const long long n4 = n >> 2;
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n4; i += gridDim.x * 256LL) {
+    const float gs = groups == 1 ? sh[2] : sh[2 + (int)((i * 4) / n_net) % groups];
     float4 pv = *reinterpret_cast<float4*>(p + i * 4);
     const float4 gv = ldg4(g + i * 4);
     float4 mv = *reinterpret_cast<float4*>(m + i * 4), vv = *reinterpret_cast<float4*>(v + i * 4);

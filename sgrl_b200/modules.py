@@ -310,9 +310,9 @@ class SetNetModule(nn.Module):
         return t
 
     # ------------------------------------------------------------------ raw kernel passes
-    def _call(self, tb: GraphTables, nb: int, keep: int, stash, grads=None, ws=None, split=(None, None)) -> NetCall:
+    def _call(self, tb: GraphTables, nb: int, keep: int, stash, grads=None, ws=None, split=(None, None), in_nets: int = 0) -> NetCall:
         k = NetCall()
-        k.kind, k.n_layers, k.nb, k.T, k.G = self._kind, self._n_layers, nb, tb.T, tb.G
+        k.kind, k.n_layers, k.nb, k.T, k.G, k.in_nets = self._kind, self._n_layers, nb, tb.T, tb.G, in_nets
         k.keep, k.use_tc, k.max_limbs = keep, int(self.use_tc), int(tb.nmax)
         k.params = ptr(self.live_arena)
         k.params_hi, k.params_lo = ptr(split[0]), ptr(split[1])
@@ -333,9 +333,11 @@ class SetNetModule(nn.Module):
         return nb * lib.sgrl_ws_floats(self._n_layers, T)
 
     def forward_raw(self, tb: GraphTables, obs: torch.Tensor, act: Optional[torch.Tensor], keep: bool, nb: Optional[int] = None,
-                    out: Optional[torch.Tensor] = None, trusted_split: bool = False, stash: Optional[torch.Tensor] = None):
+                    out: Optional[torch.Tensor] = None, trusted_split: bool = False, stash: Optional[torch.Tensor] = None,
+                    in_nets: int = 0):
         """Run nb nets on tokens obs (T,41) [act (T,3)].  Returns (out (nb,T,od), stash).  `out` / `stash` may be
-        caller-owned buffers (Agent.update's static plan); otherwise they are allocated here."""
+        caller-owned buffers (Agent.update's static plan); otherwise they are allocated here.  in_nets = 0: every net reads
+        the same obs / act; in_nets = K: obs (K*T,41) [act (K*T,3)] hold K input blocks and net z reads block z % K."""
         nb = self._nb if nb is None else nb
         od = 3 if self._kind == ACTOR else 1
         dev = self._arena.device
@@ -345,8 +347,10 @@ class SetNetModule(nn.Module):
             stash = torch.empty(self.stash_floats(tb.T, keep, nb), dtype=torch.float32, device=dev)
         if out is None:
             out = torch.empty(nb, tb.T, od, dtype=torch.float32, device=dev)
-        k = self._call(tb, nb, int(keep), stash, split=self._split_for(tb.T, trusted_split))
-        check(lib.sgrl_set_forward(C.byref(k), ptr(obs), 0, ptr(act), 0, ptr(out), tb.T * od, stream()), "sgrl_set_forward")
+        k = self._call(tb, nb, int(keep), stash, split=self._split_for(tb.T, trusted_split), in_nets=in_nets)
+        blk = tb.T if in_nets else 0
+        check(lib.sgrl_set_forward(C.byref(k), ptr(obs), blk * LIMB_OBS, ptr(act), blk * LIMB_ACT, ptr(out), tb.T * od, stream()),
+              "sgrl_set_forward")
         return out, stash
 
     def backward_raw(self, tb: GraphTables, stash: torch.Tensor, dout: torch.Tensor, nb: int, grads: Optional[torch.Tensor],

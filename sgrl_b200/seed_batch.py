@@ -1,0 +1,222 @@
+"""Seed-batched TD3: K independent SET agents trained in one captured update per step.
+
+RL results are reported over seeds (the reference's configs run B = 100 and B = 256).  At those batch sizes one agent's step
+is bound by the latency of its kernel chain, not by work, so K agents stepped one after the other cost about K steps.
+``SeedBatchedAgent`` stacks the seeds on the executor's net axis instead: the actor modules hold K nets, the critic modules
+2K nets ordered [critic1 of seeds 0..K-1 | critic2 of seeds 0..K-1], and every kernel of the step runs once for all seeds,
+net z reading seed z % K's batch.  The update sequence is ``Agent._update_impl`` itself (it takes the seed count from
+``n_seeds``); clipping and Adam are per seed (one grouped launch each), Polyak and the all-reduce cover the whole arena.
+
+Each seed has its own initial weights (those of ``torch.manual_seed(seed); Agent(args)``), Adam state, target networks,
+replay data and target-policy noise; all seeds share the hyper-parameters and, at each step, the morphology.
+"""
+from __future__ import annotations
+
+import contextlib
+from typing import List, Sequence
+
+import torch
+
+from ._lib import ACTOR, CRITIC
+from .agent import Agent, FusedAdam
+from .modules import SetNetModule
+
+MAX_SEEDS = 8
+
+
+@contextlib.contextmanager
+def _rng_kept():
+    """Runs its body without changing the caller's CPU / current-CUDA-device random streams."""
+    devices = [torch.cuda.current_device()] if torch.cuda.is_available() else []
+    with torch.random.fork_rng(devices=devices):
+        yield
+
+
+def _seed_nets(K: int, k: int, per_agent: int):
+    """(net z of the seed-batched module, net j of seed k's own module): net j of every seed, then net j + 1."""
+    return [(j * K + k, j) for j in range(per_agent)]
+
+
+def _copy_seed(b: SetNetModule, one: SetNetModule, K: int, k: int, to_batched: bool):
+    """Seed k's parameters (live and dead) between a seed-batched module and the seed's own module."""
+    L, D = b._live, b._dead
+    with torch.no_grad():
+        for z, j in _seed_nets(K, k, one._nb):
+            for bz, oj in ((b._arena[z * L:(z + 1) * L], one._arena[j * L:(j + 1) * L]),
+                           (b._arena[b._nb * L + z * D:b._nb * L + (z + 1) * D], one._arena[one._nb * L + j * D:one._nb * L + (j + 1) * D])):
+                (bz if to_batched else oj).copy_(oj if to_batched else bz)
+
+
+def _copy_seed_adam(b: FusedAdam, one: FusedAdam, K: int, k: int, to_batched: bool):
+    """Seed k's Adam moments (live arena only) between a seed-batched optimizer and the seed's own."""
+    L = b.module._live
+    with torch.no_grad():
+        for z, j in _seed_nets(K, k, one.module._nb):
+            for bt, ot in ((b.exp_avg, one.exp_avg), (b.exp_avg_sq, one.exp_avg_sq)):
+                bz, oj = bt[z * L:(z + 1) * L], ot[j * L:(j + 1) * L]
+                (bz if to_batched else oj).copy_(oj if to_batched else bz)
+
+
+class SeedBatchedAgent(Agent):
+    """K = len(seeds) (1..8) independent TD3 agents over the SET modules, stepped together.
+
+    ``update(batches, it)`` performs one TD3 step (src/agent.py:117-183) for every seed as ONE captured CUDA graph and returns
+    one loss dict per seed, with the keys ``Agent.update`` returns.  ``agent(k)`` gives seed k as a standalone ``Agent`` (its
+    ``state_dict`` has the reference's 818 keys); ``from_agents`` builds a seed-batched agent from existing ones."""
+
+    def __init__(self, args, seeds: Sequence[int]):
+        seeds = list(seeds)
+        _check_count(len(seeds))
+        agents = []
+        with _rng_kept():
+            for sd in seeds:
+                torch.manual_seed(sd)
+                agents.append(Agent(args))
+        self._init_from(agents)
+
+    @classmethod
+    def from_agents(cls, agents: Sequence[Agent]) -> "SeedBatchedAgent":
+        """A seed-batched copy of existing agents: parameters, target networks, Adam moments and step counts.  The agents
+        must have taken the same number of optimizer steps (the seeds share one step counter)."""
+        agents = list(agents)
+        _check_count(len(agents))
+        for name in ("actor_optimizer", "critic_optimizer"):
+            steps = {int(getattr(a, name).step_count.item()) for a in agents}
+            if len(steps) != 1:
+                raise ValueError(f"the agents' {name} step counts differ ({sorted(steps)}): seed-batched agents step together")
+        self = cls.__new__(cls)
+        self._init_from(agents)
+        return self
+
+    def _init_from(self, agents: List[Agent]):
+        nn_init = super(Agent, self).__init__          # nn.Module.__init__: the modules are built here, not by Agent.__init__
+        nn_init()
+        a0 = agents[0]
+        args = a0.args
+        K = len(agents)
+        dev = a0.actor.full_arena.device
+        self.args, self.n_seeds = args, K
+        with _rng_kept():                               # the arenas are overwritten below: their own init draws nothing visible
+            self.actor = SetNetModule(ACTOR, [f"actor_{k}" for k in range(K)], args, max_action=args.max_action, device=dev)
+            self.actor_target = SetNetModule(ACTOR, [f"actor_{k}" for k in range(K)], args, max_action=args.max_action, device=dev)
+            names = [f"critic{j + 1}_{k}" for j in range(2) for k in range(K)]
+            self.critic = SetNetModule(CRITIC, names, args, device=dev)
+            self.critic_target = SetNetModule(CRITIC, names, args, device=dev)
+        for m in ("actor", "actor_target", "critic", "critic_target"):
+            for k, a in enumerate(agents):
+                _copy_seed(getattr(self, m), getattr(a, m), K, k, True)
+            getattr(self, m).use_tc = getattr(a0, m).use_tc
+        self.actor_optimizer = FusedAdam(self.actor, lr=a0.actor_optimizer.lr, betas=a0.actor_optimizer.betas, eps=a0.actor_optimizer.eps,
+                                         groups=K)
+        self.critic_optimizer = FusedAdam(self.critic, lr=a0.critic_optimizer.lr, betas=a0.critic_optimizer.betas,
+                                          eps=a0.critic_optimizer.eps, groups=K)
+        for name in ("actor_optimizer", "critic_optimizer"):
+            opt = getattr(self, name)
+            for k, a in enumerate(agents):
+                _copy_seed_adam(opt, getattr(a, name), K, k, True)
+            opt.step_count.copy_(getattr(a0, name).step_count)
+        self._init_runtime(args)
+        self.tot_update_count = a0.tot_update_count
+        self.target_smoothing_tau, self.reward_scale = a0.target_smoothing_tau, a0.reward_scale
+        if hasattr(a0.actor, "graph"):
+            self.change_morphology(a0.actor.graph)
+
+    def agent(self, k: int) -> Agent:
+        """Seed k as a standalone ``Agent`` (a copy): parameters, target networks, Adam state and update count."""
+        if not 0 <= k < self.n_seeds:
+            raise ValueError(f"seed index {k} outside 0..{self.n_seeds - 1}")
+        dev = self.actor.full_arena.device
+        with _rng_kept():
+            a = Agent(self.args)
+        a.to(dev)
+        for m in ("actor", "actor_target", "critic", "critic_target"):
+            _copy_seed(getattr(self, m), getattr(a, m), self.n_seeds, k, False)
+            getattr(a, m).use_tc = getattr(self, m).use_tc
+        for name in ("actor_optimizer", "critic_optimizer"):
+            mine, one = getattr(self, name), getattr(a, name)
+            one._sync_device()
+            _copy_seed_adam(mine, one, self.n_seeds, k, False)
+            one.step_count.copy_(mine.step_count)
+            one.lr, one.betas, one.eps = mine.lr, mine.betas, mine.eps
+        a.tot_update_count = self.tot_update_count
+        a.target_smoothing_tau, a.reward_scale = self.target_smoothing_tau, self.reward_scale
+        a.data_parallel, a.lazy_stats, a.use_graphs = self.data_parallel, self.lazy_stats, self.use_graphs
+        if hasattr(self.actor, "graph"):
+            a.change_morphology(self.actor.graph)
+        return a
+
+    # ------------------------------------------------------------------ TD3 step
+    def update(self, batches, it: int, noises=None):
+        """One TD3 step of every seed on the current morphology.  batches[k]: seed k's batch as ``Agent.update`` takes it
+        (obs (B,41N), action (B,3N), next_obs, reward (B,1), done (B,1)), the same B for every seed.  noises: None (drawn on
+        the device, each seed its own draws) or K tensors (B,3N).  Returns K loss dicts; the reward statistics cost one host
+        synchronisation for all seeds (none for host batches or with ``lazy_stats``)."""
+        self._check_list(batches, "batches")
+        if noises is not None:
+            self._check_list(noises, "noises")
+        sizes = {int(b["obs"].shape[0]) for b in batches}
+        if len(sizes) != 1:
+            raise ValueError(f"every seed's batch must hold the same number of samples, got {sorted(sizes)}")
+        tb = self.actor._tables(sizes.pop())
+        return self._run_update(tb, list(batches), it, None if noises is None else list(noises))
+
+    train_step = update
+
+    def update_from_buffers(self, buffers, batch_size: int, it: int, noises=None, sequential: bool = False, allow_duplicate: bool = False):
+        """``update([buf.sample(batch_size) for buf in buffers], it, noises)`` without materialising the batches: buffers[k] is
+        seed k's device ``sgrl_b200.buffer.ReplayBuffer`` holding transitions of the current morphology.  The indices are drawn
+        buffer by buffer with ``buf.draw_indices``, sent as ONE H2D copy, and ONE gather launch writes every seed's rows into
+        its block of the step's static inputs."""
+        from .buffer import check_packed_buffers, gather_packed_into
+        self._check_list(buffers, "buffers")
+        if noises is not None:
+            self._check_list(noises, "noises")
+        check_packed_buffers(buffers, self.actor.full_arena.device)
+        n = self.actor.num_limbs
+        for k, buf in enumerate(buffers):
+            if buf.obs_dim != 41 * n or buf.action_dim != 3 * n:
+                raise ValueError(f"buffer {k} rows ({buf.obs_dim} obs, {buf.action_dim} action floats) do not match the current "
+                                 f"morphology ({n} limbs)")
+            if buf.max_sample_size == 0:
+                raise ValueError(f"buffer {k} is empty")
+        idx = [buf.draw_indices(batch_size, sequential, allow_duplicate) for buf in buffers]
+        sizes = sorted({len(ix) for ix in idx})
+        if len(sizes) != 1:
+            raise ValueError(f"the buffers gave batches of {sizes} rows: every seed needs the same batch size")
+        tb = self.actor._tables(sizes[0])
+
+        def load(plan):
+            rows = plan.stage_indices(idx)
+            gather_packed_into(buffers, rows, plan.obs, plan.act, plan.nobs, plan.rew, plan.done, idx_dev=plan.i_dev)
+            return plan.load_noise(noises)
+
+        return self._run_update(tb, None, it, None, loader=load)
+
+    # ------------------------------------------------------------------ acting
+    @torch.no_grad()
+    def select_actions(self, obs_per_seed, graphs, deterministic=False):
+        """``Agent.select_actions`` for every seed in ONE replayed actor forward: obs_per_seed[k][i] is env i of seed k (its
+        un-padded (41*N_i,) observation), graphs[i] env i's graph dict, the same list for every seed.  Returns per seed the
+        list of (1, 3*N_i) numpy actions in env order."""
+        self._check_list(obs_per_seed, "obs_per_seed")
+        n = len(graphs)
+        if n == 0 or any(len(o) != n for o in obs_per_seed):
+            raise ValueError("select_actions needs, for every seed, one observation per graph")
+        out = self._rollout_plan(self._rollout_tables_for(graphs)).run([o for seed in obs_per_seed for o in seed])
+        return [[o.reshape(1, -1).copy() for o in out[k * n:(k + 1) * n]] for k in range(self.n_seeds)]
+
+    def _check_list(self, xs, what: str):
+        if len(xs) != self.n_seeds:
+            raise ValueError(f"{what}: expected one per seed ({self.n_seeds}), got {len(xs)}")
+
+    # single-agent entry points that have no seed-batched meaning here
+    def _single(self, *a, **kw):
+        raise NotImplementedError("SeedBatchedAgent steps every seed at once: use update / update_from_buffers / select_actions, "
+                                  "or agent(k) for one seed")
+
+    update_packed = update_packed_from_buffers = update_from_buffer = select_action = _single
+
+
+def _check_count(K: int):
+    if not 1 <= K <= MAX_SEEDS:
+        raise ValueError(f"a seed-batched agent trains 1 to {MAX_SEEDS} seeds, got {K}")

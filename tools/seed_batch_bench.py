@@ -1,0 +1,113 @@
+#!/usr/bin/env python
+"""K seeds of TD3 on one GPU: one seed-batched update against K single-agent updates, one process.
+
+  python tools/seed_batch_bench.py [--steps 200] [--rounds 2] [--batches 100,256] [--seeds 1,2,4,8]
+
+Workload: 3d_humanoid_9_full at the reference configs' batch sizes (B = 100; B = 256 as in start_humanoid.sh), K seeds each
+with its own device batch (synthetic, fixed across steps).  Arms, alternated A/B/A/B:
+
+  A  agents[k].update(batches[k], it) for k = 0..K-1, back to back         K replayed graphs per step
+  B  SeedBatchedAgent.update(batches, it)                                  one replayed graph per step
+
+Per arm and round: device ms per step between CUDA events around --steps steps (followed by a synchronise), the ratio
+B / A (A is K times the single-agent step), library kernels executed per step (through graph replays and outside them) and
+the card's name and power limit, read in the same run.  Prints one JSON line; writes nothing.
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import statistics
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+
+from tools.packed_replay_bench import card  # noqa: E402
+
+MORPH = "3d_humanoid_9_full"
+
+
+def run_case(B, K, steps, rounds, warmup, dev):
+    import torch
+    from sgrl_b200 import graph as G, morphologies as M, synth
+    from sgrl_b200._lib import lib
+    from sgrl_b200.agent import Agent
+    from sgrl_b200.config import default_args
+    from sgrl_b200.seed_batch import SeedBatchedAgent
+    par = M.ALL[MORPH]
+    g = G.build_graph(par, device=dev)
+    seeds = list(range(K))
+    singles = []
+    for s in seeds:
+        torch.manual_seed(s)
+        singles.append(Agent(default_args()))
+    sb = SeedBatchedAgent(default_args(), seeds)
+    for ag in singles + [sb]:
+        ag.lazy_stats = True
+        ag.change_morphology(g)
+    batches = [{k: v.to(dev) for k, v in synth.make_batch(B, len(par), seed=100 + s).items()} for s in seeds]
+    it = [0]
+
+    def arm_a():
+        for ag, b in zip(singles, batches):
+            ag.update(b, it[0])
+
+    def arm_b():
+        sb.update(batches, it[0])
+
+    arms = {"A_k_agents": (arm_a, singles), "B_seed_batched": (arm_b, [sb])}
+    for fn, _ in arms.values():              # eager run + capture of both step kinds
+        for _ in range(max(warmup, 4)):
+            fn(); it[0] += 1
+    torch.cuda.synchronize()
+    res = {k: {"device_ms": [], "kernels_per_step": []} for k in arms}
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(rounds):
+        for name, (fn, ags) in arms.items():
+            torch.cuda.synchronize()
+            l0 = lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags)
+            ev0.record()
+            for _ in range(steps):
+                fn(); it[0] += 1
+            ev1.record()
+            torch.cuda.synchronize()
+            r = res[name]
+            r["device_ms"].append(round(ev0.elapsed_time(ev1) / steps, 4))
+            r["kernels_per_step"].append((lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags) - l0) / steps)
+    for r in res.values():
+        r["device_ms_median"] = statistics.median(r["device_ms"])
+    a, b = res["A_k_agents"]["device_ms_median"], res["B_seed_batched"]["device_ms_median"]
+    return {"batch": B, "seeds": K, "limb_tokens_per_seed": B * len(par), "arms": res, "ratio_B_over_A": round(b / a, 4),
+            "seed_batched_faster": b < a}
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps per arm and round (>= 200 for a reported number)")
+    ap.add_argument("--rounds", type=int, default=2, help="A/B rounds")
+    ap.add_argument("--warmup", type=int, default=6, help="untimed steps per arm before the first round (at least 4)")
+    ap.add_argument("--batches", default="100,256")
+    ap.add_argument("--seeds", default="1,2,4,8")
+    a = ap.parse_args()
+    Bs = [int(x) for x in a.batches.split(",") if x]
+    Ks = [int(x) for x in a.seeds.split(",") if x]
+    if a.steps < 1 or a.rounds < 1 or not Bs or not all(1 <= k <= 8 for k in Ks):
+        ap.error("--steps and --rounds must be >= 1, --seeds within 1..8")
+    import torch
+    if not torch.cuda.is_available():
+        raise SystemExit("seed_batch_bench needs a CUDA device")
+    torch.cuda.set_device(0)
+    dev = torch.device("cuda", 0)
+    out = {"metric": "seed_batched_td3_update", "morphology": MORPH, "steps": a.steps, "rounds": a.rounds, **card(0), "cases": []}
+    for B in Bs:
+        for K in Ks:
+            out["cases"].append(run_case(B, K, a.steps, a.rounds, a.warmup, dev))
+            torch.cuda.empty_cache()
+    print(json.dumps(out))
+
+
+if __name__ == "__main__":
+    main()
