@@ -121,7 +121,8 @@ int sgrl_inv_feature_bwd(const float* dG, const float* dF, const float* Z, const
                          sgrl_stream_t stream);
 /* K2: attention core (subequivariant_attentions.py:109-151) on packed graphs.  qkv (T,768) holds
  * the already /F-divided and scaled q|k|v; vgp (T,3,252); gd (T,3,2); rel_w (2,3), rel_b (2) or NULL.
- * Outputs o (T,256), og (T,3,256), p (T,2,16). */
+ * Outputs o (T,256), og (T,3,256), p (T,2,16) (p[t, h, j] = 0 for j >= the graph's limbs); p NULL: inference pass, no
+ * probability store.  The backward's drel_w (2,3) needs relation (the tables the forward's bias was formed from). */
 int sgrl_attention_fwd(const float* qkv, const float* vgp, const float* gd, const float* rel_w, const float* rel_b,
                        const int32_t* cu_limbs, const int32_t* rel_off, const float* relation, int G,
                        int max_limbs /* largest graph (2..16), 0 = unknown: sizes the shared-memory staging */,

@@ -153,7 +153,7 @@ int sgrl_inv_feature_bwd(const float* dG, const float* dF, const float* Z, const
 int sgrl_attention_fwd(const float* qkv, const float* vgp, const float* gd, const float* rel_w, const float* rel_b,
                        const int32_t* cu_limbs, const int32_t* rel_off, const float* relation, int G, int max_limbs, float* o, float* og,
                        float* p, sgrl_stream_t stream) {
-  SGRL_CHECK(qkv && vgp && gd && cu_limbs && o && og && p, "null pointer");
+  SGRL_CHECK(qkv && vgp && gd && cu_limbs && o && og, "null pointer");      // p == NULL: inference pass, no probability store
   SGRL_CHECK((rel_w == nullptr) || (rel_b && relation), "bias needs rel_b and relation");
   AttnGraphs gr{cu_limbs, rel_off, relation, G, 0, max_limbs};
   return attention_fwd(qkv, vgp, gd, o, og, p, 0, rel_w, rel_b, 0, gr, 1, ST(stream));
@@ -163,6 +163,7 @@ int sgrl_attention_bwd(const float* qkv, const float* vgp, const float* gd, cons
                        const int32_t* cu_limbs, const int32_t* rel_off, const float* relation, int G, int max_limbs, float* dqkv,
                        float* dvgp, float* drel_w, sgrl_stream_t stream) {
   SGRL_CHECK(qkv && vgp && gd && p && d_o && d_og && cu_limbs && dqkv && dvgp, "null pointer");
+  SGRL_CHECK((drel_w == nullptr) || relation, "drel_w needs relation");
   AttnGraphs gr{cu_limbs, rel_off, relation, G, 0, max_limbs};
   return attention_bwd(qkv, vgp, gd, p, 0, d_o, d_og, dqkv, dvgp, 0, drel_w, 0, gr, 1, ST(stream));
 }

@@ -64,6 +64,15 @@ def test_error_reporting_without_gpu():
     assert _lib.lib.sgrl_ws_floats(3, 900) > 0
 
 
+def test_attention_bwd_rejects_drel_w_without_relation():
+    """The backward forms d rel_encoder.weight from the relation tables: drel_w without relation is refused before any
+    launch (G = 0: even without the check nothing would be enqueued, so the call cannot touch memory)."""
+    from sgrl_b200 import _lib
+    lib, fake = _lib.lib, 256
+    rc = lib.sgrl_attention_bwd(fake, fake, fake, fake, fake, fake, fake, None, None, 0, 0, fake, fake, fake, None)
+    assert rc < 0 and b"drel_w needs relation" in lib.sgrl_last_error()
+
+
 def test_deterministic_mode_switch_without_gpu():
     """sgrl_deterministic(enable): 1 / 0 switch the mode, -1 only queries; each call returns the previous state (no GPU work)."""
     from sgrl_b200 import _lib
