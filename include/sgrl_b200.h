@@ -7,8 +7,8 @@
  * the stub a reference maintainer would add.
  *
  * Conventions: every pointer is a DEVICE pointer to contiguous row-major fp32 (int32 for
- * indices) owned by the caller (one exception: the HOST descriptor array of
- * sgrl_replay_gather_packed); the library allocates nothing, never synchronises and never
+ * indices) owned by the caller (two exceptions: the HOST descriptor arrays of
+ * sgrl_replay_gather_packed and sgrl_replay_gather_seeds); the library allocates nothing, never synchronises and never
  * throws.  Every call enqueues work on the given cudaStream_t (pass
  * torch.cuda.current_stream().cuda_stream) and returns 0, or a negative code with a
  * thread-local message in sgrl_last_error().  Calls are re-entrant per stream.
@@ -253,6 +253,14 @@ typedef struct {
 } SgrlReplayPart;
 int sgrl_replay_gather_packed(const SgrlReplayPart* parts, int n_parts, const int64_t* idx, float* obs, float* action,
                               float* next_obs, float* reward, float* done, sgrl_stream_t stream);
+
+/* The packed gather of n_seeds independent agents (a seed-batched packed update): `parts` (HOST, as above) holds n_seeds x M
+ * descriptors seed-major, M = n_parts / n_seeds parts (one per morphology) per seed; n_seeds 1..8, M 1..64.  Part i of every
+ * seed must have the obs_dim, act_dim and batch of seed 0's part i (the seeds share the morphologies; their buffers, capacities
+ * and indices are their own), anything else is refused.  The layout is sgrl_replay_gather_packed's over all n_parts parts, so
+ * seed k's rows start at k x the per-seed totals: the block of seed k in a seed-batched update's inputs. */
+int sgrl_replay_gather_seeds(const SgrlReplayPart* parts, int n_parts, int n_seeds, const int64_t* idx, float* obs, float* action,
+                             float* next_obs, float* reward, float* done, sgrl_stream_t stream);
 
 #ifdef __cplusplus
 }

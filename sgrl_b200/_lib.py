@@ -99,6 +99,7 @@ _PROTOS = {
     "sgrl_replay_gather": (c_int, [c_f, c_i64, c_i64, c_f, c_int, c_int, c_int, c_f, c_f, c_f, c_f, c_f, c_f]),
     "sgrl_replay_scatter": (c_int, [c_f, c_i64, c_i64, c_f, c_f, c_int, c_f]),
     "sgrl_replay_gather_packed": (c_int, [C.POINTER(ReplayPart), c_int, c_f, c_f, c_f, c_f, c_f, c_f, c_f]),
+    "sgrl_replay_gather_seeds": (c_int, [C.POINTER(ReplayPart), c_int, c_int, c_f, c_f, c_f, c_f, c_f, c_f, c_f]),
 }
 EXPORTS = tuple(_PROTOS)
 

@@ -18,7 +18,8 @@ fp32 row in HBM, ``[obs | action | next_obs | reward | done]``:
   index draw -> 2 KB H2D -> gather -> graph replay, with no host synchronisation.
 * ``gather_packed_into`` does the same for several buffers at once (one per morphology) in
   one launch, writing the packed layout of a mixed-morphology update
-  (``Agent.update_packed_from_buffers``).
+  (``Agent.update_packed_from_buffers``); ``gather_seeds_into`` does it for K seeds' buffers
+  (``SeedBatchedAgent.update_packed_from_buffers_per_seed``).
 
 Same constructor, attributes (``curr``, ``max_sample_size``, ``max_buffer_size``, the five
 ``*_buffer`` arrays as numpy properties for the trainer's snapshot code,
@@ -37,6 +38,7 @@ import torch
 from ._lib import ReplayPart, check, lib, ptr, stream
 
 MAX_PACKED_PARTS = 64          # SGRL_REPLAY_MAX_PARTS: buffers one packed gather reads (csrc/replay.cuh)
+MAX_SEEDS = 8                  # SGRL_REPLAY_MAX_SEEDS: seeds one seed-batched gather reads, MAX_PACKED_PARTS buffers each
 
 
 def _dim(space) -> int:
@@ -58,23 +60,37 @@ def _check_indices(idx: np.ndarray, capacity) -> None:
         raise IndexError(f"index out of bounds for a buffer of {int(cap)} rows")
 
 
-def check_packed_buffers(buffers, device) -> None:
-    """What a packed gather needs of its buffers: 1..MAX_PACKED_PARTS of them, all with their rows on `device`."""
+def check_packed_buffers(buffers, device, owner: str = "") -> None:
+    """What a packed gather needs of its buffers: 1..MAX_PACKED_PARTS of them, all with their rows on `device`.  owner: prefix
+    of the messages (the seed the buffers belong to)."""
     if not 1 <= len(buffers) <= MAX_PACKED_PARTS:
         raise ValueError(f"a packed gather reads 1 to {MAX_PACKED_PARTS} buffers, got {len(buffers)}")
     for i, buf in enumerate(buffers):
         if buf.rows.device != torch.device(device):
-            raise ValueError(f"buffer {i} keeps its rows on {buf.rows.device}, the batch goes to {device}")
+            raise ValueError(f"{owner}buffer {i} keeps its rows on {buf.rows.device}, the batch goes to {device}")
 
 
-def gather_packed_into(buffers, indices, obs, action, next_obs, reward, done, idx_dev=None) -> int:
-    """rows of several buffers -> one packed batch, in ONE gather launch (``sgrl_replay_gather_packed``).  indices[i] are the
-    row numbers drawn from buffers[i]; the outputs are contiguous fp32 device buffers holding the parts' batches one after the
-    other: obs / next_obs sum(B_i * obs_dim_i) floats, action sum(B_i * action_dim_i), reward / done sum(B_i).  With
-    obs_dim = 41 N and action_dim = 3 N that is the packed token layout of ``Agent.update_packed``.  idx_dev: a device int64
-    tensor that already holds the concatenated indices (a caller with its own upload); otherwise they are sent from pinned
-    memory here.  Returns the number of rows gathered."""
-    check_packed_buffers(buffers, obs.device)
+def check_seed_buffers(buffers_per_seed, device) -> None:
+    """What a seed-batched packed gather needs: 1..MAX_SEEDS seeds, each with the same number (1..MAX_PACKED_PARTS) of buffers
+    on `device`, buffer i of every seed holding rows of the geometry of seed 0's buffer i."""
+    K = len(buffers_per_seed)
+    if not 1 <= K <= MAX_SEEDS:
+        raise ValueError(f"a seed-batched gather reads 1 to {MAX_SEEDS} seeds, got {K}")
+    first = buffers_per_seed[0]
+    for k, bufs in enumerate(buffers_per_seed):
+        check_packed_buffers(bufs, device, f"seed {k} ")
+        if len(bufs) != len(first):
+            raise ValueError(f"seed {k} has {len(bufs)} buffers, seed 0 has {len(first)}: every seed reads one per morphology")
+        for i, (b, b0) in enumerate(zip(bufs, first)):
+            if (b.obs_dim, b.action_dim) != (b0.obs_dim, b0.action_dim):
+                raise ValueError(f"seed {k} buffer {i} holds rows of {b.obs_dim} obs / {b.action_dim} action floats, seed 0's "
+                                 f"buffer {i} rows of {b0.obs_dim} / {b0.action_dim}")
+
+
+def _gather_parts(what, launch, buffers, indices, obs, action, next_obs, reward, done, idx_dev) -> int:
+    """What every packed gather shares: flush the buffers, check indices[i] against buffers[i]'s own capacity and the outputs'
+    sizes, send the concatenated indices (unless idx_dev already holds them), fill one descriptor per buffer and
+    launch(desc, idx_dev).  Returns the number of rows gathered."""
     if len(indices) != len(buffers):
         raise ValueError(f"{len(buffers)} buffers, {len(indices)} index lists")
     for buf in buffers:
@@ -88,7 +104,7 @@ def gather_packed_into(buffers, indices, obs, action, next_obs, reward, done, id
             (next_obs, sum(c * b.obs_dim for c, b in zip(counts, buffers))), (reward, G), (done, G))
     for t, n in need:
         if t.numel() != n or not t.is_contiguous() or t.dtype != torch.float32:
-            raise ValueError(f"gather_packed_into: expected a contiguous fp32 buffer of {n} floats, got {tuple(t.shape)}")
+            raise ValueError(f"{what}: expected a contiguous fp32 buffer of {n} floats, got {tuple(t.shape)}")
     if idx_dev is None:
         idx_dev = torch.from_numpy(flat)
         if obs.device.type == "cuda":
@@ -102,9 +118,50 @@ def gather_packed_into(buffers, indices, obs, action, next_obs, reward, done, id
     for d, b, c in zip(desc, buffers, counts):
         d.rows, d.row_floats, d.capacity = ptr(b.rows), b.row_floats, b.max_buffer_size
         d.obs_dim, d.act_dim, d.batch = b.obs_dim, b.action_dim, c
-    check(lib.sgrl_replay_gather_packed(desc, len(buffers), ptr(idx_dev), ptr(obs), ptr(action), ptr(next_obs), ptr(reward), ptr(done),
-                                        stream()), "sgrl_replay_gather_packed")
+    launch(desc, idx_dev)
     return G
+
+
+def gather_packed_into(buffers, indices, obs, action, next_obs, reward, done, idx_dev=None) -> int:
+    """rows of several buffers -> one packed batch, in ONE gather launch (``sgrl_replay_gather_packed``).  indices[i] are the
+    row numbers drawn from buffers[i]; the outputs are contiguous fp32 device buffers holding the parts' batches one after the
+    other: obs / next_obs sum(B_i * obs_dim_i) floats, action sum(B_i * action_dim_i), reward / done sum(B_i).  With
+    obs_dim = 41 N and action_dim = 3 N that is the packed token layout of ``Agent.update_packed``.  idx_dev: a device int64
+    tensor that already holds the concatenated indices (a caller with its own upload); otherwise they are sent from pinned
+    memory here.  Returns the number of rows gathered."""
+    check_packed_buffers(buffers, obs.device)
+    outs = (obs, action, next_obs, reward, done)
+
+    def launch(desc, idx):
+        check(lib.sgrl_replay_gather_packed(desc, len(buffers), ptr(idx), *(ptr(t) for t in outs), stream()), "sgrl_replay_gather_packed")
+
+    return _gather_parts("gather_packed_into", launch, buffers, indices, *outs, idx_dev)
+
+
+def gather_seeds_into(buffers_per_seed, indices_per_seed, obs, action, next_obs, reward, done, idx_dev=None) -> int:
+    """``gather_packed_into`` of K seeds' buffers in ONE launch (``sgrl_replay_gather_seeds``): buffers_per_seed[k][i] is seed
+    k's buffer of morphology i and indices_per_seed[k][i] the rows drawn from it.  Every seed reads the same number of rows
+    from its buffer i, of the same geometry, so the outputs hold seed after seed one packed batch each, seed k's at k times
+    the per-seed totals: the input layout of ``SeedBatchedAgent.update_packed_per_seed``.  idx_dev as in gather_packed_into
+    (all seeds' indices, seed-major).  Returns the number of rows gathered."""
+    check_seed_buffers(buffers_per_seed, obs.device)
+    K, P = len(buffers_per_seed), len(buffers_per_seed[0])
+    if len(indices_per_seed) != K:
+        raise ValueError(f"{K} seeds of buffers, {len(indices_per_seed)} seeds of index lists")
+    for k, ixs in enumerate(indices_per_seed):
+        if len(ixs) != P:
+            raise ValueError(f"seed {k}: {P} buffers, {len(ixs)} index lists")
+        for i, ix in enumerate(ixs):
+            if np.size(ix) != np.size(indices_per_seed[0][i]):
+                raise ValueError(f"seed {k} draws {np.size(ix)} rows from buffer {i}, seed 0 {np.size(indices_per_seed[0][i])}: every "
+                                 f"seed needs the same batch size per morphology")
+    buffers = [b for bufs in buffers_per_seed for b in bufs]
+    outs = (obs, action, next_obs, reward, done)
+
+    def launch(desc, idx):
+        check(lib.sgrl_replay_gather_seeds(desc, len(buffers), K, ptr(idx), *(ptr(t) for t in outs), stream()), "sgrl_replay_gather_seeds")
+
+    return _gather_parts("gather_seeds_into", launch, buffers, [ix for ixs in indices_per_seed for ix in ixs], *outs, idx_dev)
 
 
 class ReplayBuffer(object):

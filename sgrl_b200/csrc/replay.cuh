@@ -16,23 +16,29 @@ struct ReplayOut {
   float* obs; float* act; float* nobs; float* rew; float* done;
 };
 
-// Up to SGRL_REPLAY_MAX_PARTS buffers gathered by one launch (Agent.update_packed_from_buffers: one buffer per morphology).
-// Part p owns the batch rows [g0, g0 + B_p) of the launch; its samples are written contiguously from float obs0 of obs /
-// next_obs and act0 of action, so part after part the outputs are the packed token layout of a mixed-morphology update
-// (obs0 = 41 * first token of the part).  The descriptors travel by value as a kernel parameter (64 x 56 B).
+// Up to CAP buffers gathered by one launch (Agent.update_packed_from_buffers: one buffer per morphology; the seed-batched
+// packed update: one per seed and morphology, seed-major).  Part p owns the batch rows [g0, g0 + B_p) of the launch; its
+// samples are written contiguously from float obs0 of obs / next_obs and act0 of action, so part after part the outputs are
+// the packed token layout of a mixed-morphology update (obs0 = 41 * first token of the part).  The descriptors travel by
+// value as a kernel parameter: 64 x 56 B for the one-agent gather, 512 x 56 B (28.7 KB, within the 32 764-byte kernel
+// parameter limit of CUDA >= 12.1) for the seed-batched one.
 #define SGRL_REPLAY_MAX_PARTS 64
+#define SGRL_REPLAY_MAX_SEEDS 8
+#define SGRL_REPLAY_MAX_SEED_PARTS (SGRL_REPLAY_MAX_SEEDS * SGRL_REPLAY_MAX_PARTS)
 struct ReplayPart {
   const float* rows; long long rw, cap, obs0, act0;
   int od, ad, g0, pad_;
 };
+template <int CAP>
 struct ReplayParts {
-  ReplayPart p[SGRL_REPLAY_MAX_PARTS];
+  ReplayPart p[CAP];
   int n, G;        // parts, batch rows of all parts
 };
 
 // idx (G) int64 row numbers, part after part.  Rows are 4-byte aligned only (rw is odd for most morphologies), so the copy is
 // scalar but fully coalesced: lane k reads float k, k+32, ...
-__global__ void __launch_bounds__(256) replay_gather_kernel(const __grid_constant__ ReplayParts P, const long long* __restrict__ idx,
+template <int CAP>
+__global__ void __launch_bounds__(256) replay_gather_kernel(const __grid_constant__ ReplayParts<CAP> P, const long long* __restrict__ idx,
                                                             ReplayOut o) {
   SGRL_PDL_ENTER();
   const int lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
@@ -80,7 +86,8 @@ __global__ void __launch_bounds__(256) replay_scatter_kernel(float* __restrict__
 }
 
 // P.p[i].g0 / obs0 / act0 and P.G are filled in here from the parts' batch sizes (B[i]) in order.
-inline int replay_gather(ReplayParts& P, const int* B, const long long* idx, const ReplayOut& o, cudaStream_t st) {
+template <int CAP>
+inline int replay_gather(ReplayParts<CAP>& P, const int* B, const long long* idx, const ReplayOut& o, cudaStream_t st) {
   long long obs0 = 0, act0 = 0, G = 0;
   double bytes = 0;
   for (int i = 0; i < P.n; ++i) {
@@ -94,7 +101,7 @@ inline int replay_gather(ReplayParts& P, const int* B, const long long* idx, con
   if (G == 0) return 0;
   int gx = ceil_div(P.G, 8); if (gx > 8 * NUM_SMS) gx = 8 * NUM_SMS;
   prof_begin(PC_OTHER, bytes, st);
-  launch_k(replay_gather_kernel, gx, 256, 0, st, P, idx, o);
+  launch_k(replay_gather_kernel<CAP>, gx, 256, 0, st, P, idx, o);
   prof_end(st);
   SGRL_LAUNCH_OK();
   return 0;

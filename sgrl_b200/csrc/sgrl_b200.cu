@@ -22,7 +22,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 5; }
+int sgrl_version(void) { return 6; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -388,27 +388,56 @@ static int replay_part(ReplayPart& q, const float* rows, int64_t row_floats, int
 int sgrl_replay_gather(const float* rows, int64_t row_floats, int64_t capacity, const int64_t* idx, int batch, int obs_dim, int act_dim,
                        float* obs, float* action, float* next_obs, float* reward, float* done, sgrl_stream_t stream) {
   SGRL_CHECK(idx && obs && action && next_obs && reward && done, "null pointer");
-  ReplayParts P;
+  ReplayParts<SGRL_REPLAY_MAX_PARTS> P;
   P.n = 1;
   SGRL_TRY(replay_part(P.p[0], rows, row_floats, capacity, obs_dim, act_dim, batch));
   ReplayOut o{obs, action, next_obs, reward, done};
   return replay_gather(P, &batch, reinterpret_cast<const long long*>(idx), o, ST(stream));
 }
 
-int sgrl_replay_gather_packed(const SgrlReplayPart* parts, int n_parts, const int64_t* idx, float* obs, float* action, float* next_obs,
-                              float* reward, float* done, sgrl_stream_t stream) {
-  SGRL_CHECK(parts && idx && obs && action && next_obs && reward && done, "null pointer");
-  SGRL_CHECK(n_parts >= 1 && n_parts <= SGRL_REPLAY_MAX_PARTS, "n_parts must be 1..64");
-  ReplayParts P;
-  P.n = n_parts;
-  int B[SGRL_REPLAY_MAX_PARTS];
-  for (int i = 0; i < n_parts; ++i) {
+// parts[0..n) (n <= CAP, checked by the caller) -> one gather launch with CAP descriptors in its parameter bank
+extern "C++" {
+template <int CAP>
+static int replay_gather_parts(const SgrlReplayPart* parts, int n, const int64_t* idx, float* obs, float* action, float* next_obs,
+                               float* reward, float* done, cudaStream_t st) {
+  ReplayParts<CAP> P;
+  P.n = n;
+  int B[CAP];
+  for (int i = 0; i < n; ++i) {
     const SgrlReplayPart& s = parts[i];
     SGRL_TRY(replay_part(P.p[i], s.rows, s.row_floats, s.capacity, s.obs_dim, s.act_dim, s.batch));
     B[i] = s.batch;
   }
   ReplayOut o{obs, action, next_obs, reward, done};
-  return replay_gather(P, B, reinterpret_cast<const long long*>(idx), o, ST(stream));
+  return replay_gather(P, B, reinterpret_cast<const long long*>(idx), o, st);
+}
+}  // extern "C++"
+
+int sgrl_replay_gather_packed(const SgrlReplayPart* parts, int n_parts, const int64_t* idx, float* obs, float* action, float* next_obs,
+                              float* reward, float* done, sgrl_stream_t stream) {
+  SGRL_CHECK(parts && idx && obs && action && next_obs && reward && done, "null pointer");
+  SGRL_CHECK(n_parts >= 1 && n_parts <= SGRL_REPLAY_MAX_PARTS, "n_parts must be 1..64");
+  return replay_gather_parts<SGRL_REPLAY_MAX_PARTS>(parts, n_parts, idx, obs, action, next_obs, reward, done, ST(stream));
+}
+
+int sgrl_replay_gather_seeds(const SgrlReplayPart* parts, int n_parts, int n_seeds, const int64_t* idx, float* obs, float* action,
+                             float* next_obs, float* reward, float* done, sgrl_stream_t stream) {
+  SGRL_CHECK(parts && idx && obs && action && next_obs && reward && done, "null pointer");
+  SGRL_CHECK(n_seeds >= 1 && n_seeds <= SGRL_REPLAY_MAX_SEEDS, "n_seeds must be 1..8");
+  SGRL_CHECK(n_parts >= n_seeds && n_parts % n_seeds == 0 && n_parts / n_seeds <= SGRL_REPLAY_MAX_PARTS,
+             "n_parts must be n_seeds x (1..64 parts per seed)");
+  const int M = n_parts / n_seeds;
+  for (int k = 1; k < n_seeds; ++k)        // every seed's part i has seed 0's geometry: seed k's rows land at k x the per-seed totals
+    for (int i = 0; i < M; ++i) {
+      const SgrlReplayPart &a = parts[i], &b = parts[k * M + i];
+      if (b.obs_dim != a.obs_dim || b.act_dim != a.act_dim || b.batch != a.batch) {
+        char m[200];
+        snprintf(m, sizeof(m), "seed %d part %d: obs_dim, act_dim, batch (%d, %d, %d) differ from seed 0's (%d, %d, %d)", k, i,
+                 (int)b.obs_dim, (int)b.act_dim, (int)b.batch, (int)a.obs_dim, (int)a.act_dim, (int)a.batch);
+        return fail(-2, m, __FILE__, __LINE__);
+      }
+    }
+  return replay_gather_parts<SGRL_REPLAY_MAX_SEED_PARTS>(parts, n_parts, idx, obs, action, next_obs, reward, done, ST(stream));
 }
 
 int sgrl_replay_scatter(float* rows, int64_t row_floats, int64_t capacity, const int64_t* dst, const float* staged, int n, sgrl_stream_t stream) {

@@ -13,15 +13,14 @@ replay data and target-policy noise; all seeds share the hyper-parameters and, a
 from __future__ import annotations
 
 import contextlib
-from typing import List, Sequence
+from typing import List, Optional, Sequence
 
 import torch
 
 from ._lib import ACTOR, CRITIC
 from .agent import Agent, FusedAdam
+from .buffer import MAX_SEEDS
 from .modules import SetNetModule
-
-MAX_SEEDS = 8
 
 
 @contextlib.contextmanager
@@ -61,7 +60,8 @@ class SeedBatchedAgent(Agent):
     """K = len(seeds) (1..8) independent TD3 agents over the SET modules, stepped together.
 
     ``update(batches, it)`` performs one TD3 step (src/agent.py:117-183) for every seed as ONE captured CUDA graph and returns
-    one loss dict per seed, with the keys ``Agent.update`` returns.  ``agent(k)`` gives seed k as a standalone ``Agent`` (its
+    one loss dict per seed, with the keys ``Agent.update`` returns; ``update_packed_per_seed`` does the same for packed
+    multi-morphology batches (``Agent.update_packed`` per seed).  ``agent(k)`` gives seed k as a standalone ``Agent`` (its
     ``state_dict`` has the reference's 818 keys); ``from_agents`` builds a seed-batched agent from existing ones."""
 
     def __init__(self, args, seeds: Sequence[int]):
@@ -192,6 +192,89 @@ class SeedBatchedAgent(Agent):
 
         return self._run_update(tb, None, it, None, loader=load)
 
+    def update_packed_per_seed(self, batches_per_seed, it: int, noises=None, morph_count: Optional[float] = None):
+        """``Agent.update_packed`` of every seed in ONE captured step: batches_per_seed[k] is what seed k's own agent would pass
+        to update_packed, [(graph_dict, data_batch), ...].  The seeds share the morphologies (the same parents in the same
+        order) and the batch size of each; seed 0's graph dicts build the packed tables.  noises: None or K lists of one
+        (B_i, 3 N_i) tensor per morphology.  Returns K loss dicts; seed k's loss is the mean over its morphologies, as in
+        update_packed.  morph_count: as in ``Agent.update_packed`` (data parallelism)."""
+        graphs = self._check_seed_morphologies(batches_per_seed, "batches_per_seed")
+        specs = [(g, int(b["obs"].shape[0])) for g, b in batches_per_seed[0]]
+        for k, parts in enumerate(batches_per_seed):
+            for i, ((_, b), (_, B)) in enumerate(zip(parts, specs)):
+                if int(b["obs"].shape[0]) != B:
+                    raise ValueError(f"seed {k} morphology {i}: a batch of {int(b['obs'].shape[0])} samples, seed 0's holds {B}: "
+                                     f"every seed needs the same batch size per morphology")
+        flat_noises = self._seed_noises(noises, len(graphs))
+        tb = self._packed_tables_for(specs, morph_count)
+        return self._run_update(tb, [b for parts in batches_per_seed for _, b in parts], it, flat_noises)
+
+    def update_packed_from_buffers_per_seed(self, parts_per_seed, batch_size: int, it: int, noises=None,
+                                            morph_count: Optional[float] = None, sequential: bool = False, allow_duplicate: bool = False):
+        """``update_packed_per_seed([[(g, buf.sample(batch_size)) for g, buf in parts] for parts in parts_per_seed], ...)``
+        without materialising the batches: parts_per_seed[k] = [(graph_dict, ReplayBuffer), ...] is seed k's device buffer of
+        each morphology.  The indices are drawn with ``buf.draw_indices`` seed after seed, buffer after buffer (the draws of K
+        agents calling ``update_packed_from_buffers`` in seed order), sent as ONE H2D copy, and ONE gather launch
+        (``gather_seeds_into``) writes every seed's rows into its block of the step's static inputs.  Per step: one copy and
+        one library launch outside the graph.  The plan is update_packed_per_seed's."""
+        from .buffer import check_seed_buffers, gather_seeds_into
+        graphs = self._check_seed_morphologies(parts_per_seed, "parts_per_seed")
+        flat_noises = self._seed_noises(noises, len(graphs))
+        for k, parts in enumerate(parts_per_seed):
+            for i, (g, buf) in enumerate(parts):
+                n = len(g["parents"])
+                if buf.obs_dim != 41 * n or buf.action_dim != 3 * n:
+                    raise ValueError(f"seed {k} buffer {i} rows ({buf.obs_dim} obs, {buf.action_dim} action floats) do not match its "
+                                     f"morphology ({n} limbs)")
+                if buf.max_sample_size == 0:
+                    raise ValueError(f"seed {k} buffer {i} is empty")
+        buffers = [[buf for _, buf in parts] for parts in parts_per_seed]
+        check_seed_buffers(buffers, self.actor.full_arena.device)
+        idx = [[buf.draw_indices(batch_size, sequential, allow_duplicate) for buf in bufs] for bufs in buffers]
+        for k in range(1, self.n_seeds):
+            for i, (a, b) in enumerate(zip(idx[k], idx[0])):
+                if len(a) != len(b):
+                    raise ValueError(f"seed {k} buffer {i} gave a batch of {len(a)} rows, seed 0's {len(b)}: every seed needs the "
+                                     f"same batch size per morphology")
+        tb = self._packed_tables_for([(g, len(ix)) for g, ix in zip(graphs, idx[0])], morph_count)
+        P = len(graphs)
+
+        def load(plan):
+            rows = plan.stage_indices([ix for seed in idx for ix in seed])
+            gather_seeds_into(buffers, [rows[k * P:(k + 1) * P] for k in range(self.n_seeds)], plan.obs, plan.act, plan.nobs,
+                              plan.rew, plan.done, idx_dev=plan.i_dev)
+            return plan.load_noise(flat_noises)
+
+        return self._run_update(tb, None, it, None, loader=load)
+
+    def _check_seed_morphologies(self, parts_per_seed, what: str):
+        """One list of (graph_dict, data) per seed, 1..MAX_PACKED_PARTS of them, the same morphologies in the same order for
+        every seed.  Returns seed 0's graph dicts, which build the packed tables."""
+        from .buffer import MAX_PACKED_PARTS
+        self._check_list(parts_per_seed, what)
+        first = parts_per_seed[0]
+        if not 1 <= len(first) <= MAX_PACKED_PARTS:
+            raise ValueError(f"{what}: a packed update holds 1 to {MAX_PACKED_PARTS} morphologies per seed, got {len(first)}")
+        shape = [tuple(int(x) for x in g["parents"]) for g, _ in first]
+        for k, parts in enumerate(parts_per_seed):
+            if len(parts) != len(first):
+                raise ValueError(f"{what}: seed {k} has {len(parts)} morphologies, seed 0 has {len(first)}")
+            for i, (g, _) in enumerate(parts):
+                if tuple(int(x) for x in g["parents"]) != shape[i]:
+                    raise ValueError(f"{what}: seed {k} morphology {i} has other parents than seed 0's morphology {i}: every seed "
+                                     f"needs the same morphologies in the same order")
+        return [g for g, _ in first]
+
+    def _seed_noises(self, noises, P: int):
+        """None, or K lists of P noise tensors -> the seed-major flat list a packed plan takes."""
+        if noises is None:
+            return None
+        self._check_list(noises, "noises")
+        for k, nz in enumerate(noises):
+            if len(nz) != P:
+                raise ValueError(f"noises: seed {k} has {len(nz)} tensors for {P} morphologies")
+        return [n for nz in noises for n in nz]
+
     # ------------------------------------------------------------------ acting
     @torch.no_grad()
     def select_actions(self, obs_per_seed, graphs, deterministic=False):
@@ -211,8 +294,8 @@ class SeedBatchedAgent(Agent):
 
     # single-agent entry points that have no seed-batched meaning here
     def _single(self, *a, **kw):
-        raise NotImplementedError("SeedBatchedAgent steps every seed at once: use update / update_from_buffers / select_actions, "
-                                  "or agent(k) for one seed")
+        raise NotImplementedError("SeedBatchedAgent steps every seed at once: use update / update_from_buffers / "
+                                  "update_packed_per_seed / update_packed_from_buffers_per_seed / select_actions, or agent(k) for one seed")
 
     update_packed = update_packed_from_buffers = update_from_buffer = select_action = _single
 

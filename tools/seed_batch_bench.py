@@ -30,10 +30,37 @@ from tools.packed_replay_bench import card  # noqa: E402
 MORPH = "3d_humanoid_9_full"
 
 
+def time_arms(arms, steps, rounds, it, before_window=None):
+    """The alternated A/B timing of the seed benchmarks: arms = {name: (fn, agents)}, fn() one step of the arm (reading it[0],
+    which is bumped after every step).  Per arm and round: device ms per step between CUDA events around `steps` steps followed
+    by a synchronise, and the library kernels executed per step (through graph replays and outside them).  before_window(name),
+    if given, runs untimed before each window.  Returns {name: {"device_ms", "kernels_per_step", "device_ms_median"}}."""
+    import torch
+    from sgrl_b200._lib import lib
+    res = {k: {"device_ms": [], "kernels_per_step": []} for k in arms}
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(rounds):
+        for name, (fn, ags) in arms.items():
+            if before_window is not None:
+                before_window(name)
+            torch.cuda.synchronize()
+            l0 = lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags)
+            ev0.record()
+            for _ in range(steps):
+                fn(); it[0] += 1
+            ev1.record()
+            torch.cuda.synchronize()
+            r = res[name]
+            r["device_ms"].append(round(ev0.elapsed_time(ev1) / steps, 4))
+            r["kernels_per_step"].append((lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags) - l0) / steps)
+    for r in res.values():
+        r["device_ms_median"] = statistics.median(r["device_ms"])
+    return res
+
+
 def run_case(B, K, steps, rounds, warmup, dev):
     import torch
     from sgrl_b200 import graph as G, morphologies as M, synth
-    from sgrl_b200._lib import lib
     from sgrl_b200.agent import Agent
     from sgrl_b200.config import default_args
     from sgrl_b200.seed_batch import SeedBatchedAgent
@@ -63,22 +90,7 @@ def run_case(B, K, steps, rounds, warmup, dev):
         for _ in range(max(warmup, 4)):
             fn(); it[0] += 1
     torch.cuda.synchronize()
-    res = {k: {"device_ms": [], "kernels_per_step": []} for k in arms}
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for _ in range(rounds):
-        for name, (fn, ags) in arms.items():
-            torch.cuda.synchronize()
-            l0 = lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags)
-            ev0.record()
-            for _ in range(steps):
-                fn(); it[0] += 1
-            ev1.record()
-            torch.cuda.synchronize()
-            r = res[name]
-            r["device_ms"].append(round(ev0.elapsed_time(ev1) / steps, 4))
-            r["kernels_per_step"].append((lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags) - l0) / steps)
-    for r in res.values():
-        r["device_ms_median"] = statistics.median(r["device_ms"])
+    res = time_arms(arms, steps, rounds, it)
     a, b = res["A_k_agents"]["device_ms_median"], res["B_seed_batched"]["device_ms_median"]
     return {"batch": B, "seeds": K, "limb_tokens_per_seed": B * len(par), "arms": res, "ratio_B_over_A": round(b / a, 4),
             "seed_batched_faster": b < a}
