@@ -163,6 +163,17 @@ int sgrl_gemm_pair(const float* A0, int lda0, const float* W0_hi, const float* W
 int sgrl_split_tf32(const float* w, float* hi, float* lo, int64_t n, sgrl_stream_t stream);
 
 /* ---- K5: TD3 glue (agent.py:127-148,167) -------------------------------------------------- */
+/* The per-step TD3 scalars of one seed.  The _hp entry points below take a DEVICE table of such rows, one per seed (seed k =
+ * row k), and their kernels read it when they run: a captured CUDA graph applies the values the table holds at replay, so a
+ * caller changes hyper-parameters between updates by rewriting the table in stream order, without recapturing.  Adam's betas
+ * and eps, max_action, policy_freq and grad_scale stay by-value arguments shared by all seeds. */
+typedef struct {
+  double actor_lr, critic_lr;      /* Adam learning rates (doubles, like the Python floats torch.optim.Adam forms its step from) */
+  float discount, reward_scale;    /* critic target r * reward_scale + (1 - done) * discount * min(Q1', Q2') */
+  float policy_noise, noise_clip;  /* target-policy smoothing: eps ~ N(0, policy_noise^2) clipped to +-noise_clip */
+  float tau, one_minus_tau;        /* Polyak; one_minus_tau = (float)(1.0 - (double)tau), as sgrl_polyak forms it */
+  float max_norm, pad_;            /* clip_grad_norm_ threshold, <= 0: no clipping */
+} SgrlTd3Hparams;                  /* 48 bytes */
 int sgrl_td3_smooth_action(const float* pi_target, const float* noise, float* next_action, float noise_clip,
                            float max_action, int64_t n, sgrl_stream_t stream);
 /* The same with the target-policy noise drawn inside the kernel: eps ~ N(0, policy_noise^2) (agent.py:128,
@@ -172,6 +183,14 @@ int sgrl_td3_smooth_action(const float* pi_target, const float* noise, float* ne
 int sgrl_td3_smooth_action_rng(const float* pi_target, float* next_action, float* noise_out, float policy_noise,
                                float noise_clip, float max_action, int64_t n, uint64_t seed, const int32_t* draw,
                                sgrl_stream_t stream);
+/* Both smoothing kernels with per-seed scalars: n = K * per_seed elements, element i belongs to seed i / per_seed (3T for K
+ * seeds of T tokens) and takes row i / per_seed's noise_clip (and policy_noise).  The Philox counter and key are those of
+ * sgrl_td3_smooth_action_rng, so one seed with the same seed and draw gives the same noise. */
+int sgrl_td3_smooth_action_hp(const float* pi_target, const float* noise, float* next_action, const SgrlTd3Hparams* hp,
+                              int64_t per_seed, float max_action, int64_t n, sgrl_stream_t stream);
+int sgrl_td3_smooth_action_rng_hp(const float* pi_target, float* next_action, float* noise_out, const SgrlTd3Hparams* hp,
+                                  int64_t per_seed, float max_action, int64_t n, uint64_t seed, const int32_t* draw,
+                                  sgrl_stream_t stream);
 /* target = r*scale + (1-done)*discount*min(tq1,tq2) broadcast over limbs; loss (1 float, accumulates)
  * = mse(q1,target)+mse(q2,target); dq1,dq2 = dloss/dq. tok_graph (T) maps token -> sample.
  * tok_weight (T, nullable): weight of each token in the loss for packed mixed-morphology batches
@@ -191,6 +210,10 @@ int sgrl_td3_critic_loss_seeds(const float* q, const float* tq, const float* rew
                                const float* tok_weight, float* target, float* dq, float* loss, float discount, float reward_scale, int T,
                                double* reward_stats, int G, int K, sgrl_stream_t stream);
 int sgrl_td3_actor_loss_seeds(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, int K, sgrl_stream_t stream);
+/* sgrl_td3_critic_loss_seeds with seed k's discount and reward_scale from hp[k] (K rows), the reward statistics included. */
+int sgrl_td3_critic_loss_seeds_hp(const float* q, const float* tq, const float* reward, const float* done, const int32_t* tok_graph,
+                                  const float* tok_weight, float* target, float* dq, float* loss, const SgrlTd3Hparams* hp, int T,
+                                  double* reward_stats, int G, int K, sgrl_stream_t stream);
 
 /* ---- K6: optimizer (agent.py:150-156,170-178; common/functional.py:7-10) -------------------- */
 int sgrl_sumsq(const float* g, int64_t n, float* out /*accumulates*/, sgrl_stream_t stream);
@@ -209,9 +232,20 @@ int sgrl_sumsq_nets(const float* g, int64_t n_net, int nets, float* out, sgrl_st
 int sgrl_adam_clip_groups(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
                           const int32_t* step, double lr, double beta1, double beta2, double eps, float max_norm, float grad_scale,
                           float* p_hi, float* p_lo, sgrl_stream_t stream);
+/* sgrl_adam_clip_groups with group g's learning rate and clip threshold from hp[g] (`groups` rows): actor_lr when
+ * lr_of = SGRL_ACTOR, critic_lr when SGRL_CRITIC, and max_norm (<= 0: group g is not clipped).  sumsq must hold every net's
+ * sum of squares, whatever the thresholds. */
+int sgrl_adam_clip_groups_hp(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
+                             const int32_t* step, const SgrlTd3Hparams* hp, int lr_of, double beta1, double beta2, double eps,
+                             float grad_scale, float* p_hi, float* p_lo, sgrl_stream_t stream);
 int sgrl_bump_step(int32_t* step, sgrl_stream_t stream);
 int sgrl_polyak(float* target, const float* source, int64_t n, float tau,
                 float* t_hi /*nullable: refreshed tf32 split of target[0:n_split]*/, float* t_lo, int64_t n_split, sgrl_stream_t stream);
+/* sgrl_polyak over a module arena of `nets` nets ([live nets | dead nets], live_net and dead_net floats per net, multiples of
+ * 64: sgrl_arena_floats) with net z, live or dead, updated by the tau / one_minus_tau of seed z % K (hp: K rows, nets % K == 0).
+ * t_hi / t_lo (nullable) cover the live nets. */
+int sgrl_polyak_hp(float* target, const float* source, int nets, int64_t live_net, int64_t dead_net, const SgrlTd3Hparams* hp, int K,
+                   float* t_hi, float* t_lo, sgrl_stream_t stream);
 
 /* Call before recording an event on `stream` that another stream will wait on when the last work on `stream` was a
  * kernel of this library and the stream is not being captured: enqueues an empty non-programmatic launch (see

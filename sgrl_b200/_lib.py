@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import numpy as np
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -52,6 +53,12 @@ class ReplayPart(C.Structure):
     ]
 
 
+# One row of the per-seed TD3 table (SgrlTd3Hparams): the layout of the C struct, 48 bytes
+TD3_HPARAMS = np.dtype([("actor_lr", "<f8"), ("critic_lr", "<f8"), ("discount", "<f4"), ("reward_scale", "<f4"),
+                        ("policy_noise", "<f4"), ("noise_clip", "<f4"), ("tau", "<f4"), ("one_minus_tau", "<f4"),
+                        ("max_norm", "<f4"), ("pad_", "<f4")])
+assert TD3_HPARAMS.itemsize == 48
+
 _PROTOS = {
     "sgrl_version": (c_int, []),
     "sgrl_last_error": (C.c_char_p, []),
@@ -83,17 +90,23 @@ _PROTOS = {
     "sgrl_split_tf32": (c_int, [c_f, c_f, c_f, c_i64, c_f]),
     "sgrl_td3_smooth_action": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, c_i64, c_f]),
     "sgrl_td3_smooth_action_rng": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, C.c_float, c_i64, C.c_uint64, c_f, c_f]),
+    "sgrl_td3_smooth_action_hp": (c_int, [c_f, c_f, c_f, c_f, c_i64, C.c_float, c_i64, c_f]),
+    "sgrl_td3_smooth_action_rng_hp": (c_int, [c_f, c_f, c_f, c_f, c_i64, C.c_float, c_i64, C.c_uint64, c_f, c_f]),
     "sgrl_td3_critic_loss": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, C.c_float, C.c_float, c_int, c_f, c_int, c_f]),
     "sgrl_td3_actor_loss": (c_int, [c_f, c_f, c_f, c_f, c_int, c_f]),
     "sgrl_td3_critic_loss_seeds": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, C.c_float, C.c_float, c_int, c_f, c_int, c_int, c_f]),
     "sgrl_td3_actor_loss_seeds": (c_int, [c_f, c_f, c_f, c_f, c_int, c_int, c_f]),
+    "sgrl_td3_critic_loss_seeds_hp": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_int, c_f, c_int, c_int, c_f]),
     "sgrl_sumsq": (c_int, [c_f, c_i64, c_f, c_f]),
     "sgrl_sumsq_nets": (c_int, [c_f, c_i64, c_int, c_f, c_f]),
     "sgrl_adam_clip_groups": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_int, c_int, c_f, c_f, C.c_double, C.c_double, C.c_double, C.c_double,
                                       C.c_float, C.c_float, c_f, c_f, c_f]),
     "sgrl_adam_clip": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_f, c_f, C.c_double, C.c_double, C.c_double, C.c_double, C.c_float, C.c_float, c_f, c_f, c_f]),
+    "sgrl_adam_clip_groups_hp": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_int, c_int, c_f, c_f, c_f, c_int, C.c_double, C.c_double, C.c_double,
+                                         C.c_float, c_f, c_f, c_f]),
     "sgrl_bump_step": (c_int, [c_f, c_f]),
     "sgrl_polyak": (c_int, [c_f, c_f, c_i64, C.c_float, c_f, c_f, c_i64, c_f]),
+    "sgrl_polyak_hp": (c_int, [c_f, c_f, c_int, c_i64, c_i64, c_f, c_int, c_f, c_f, c_f]),
     "sgrl_stream_fence": (c_int, [c_f]),
     "sgrl_deterministic": (c_int, [c_int]),
     "sgrl_replay_gather": (c_int, [c_f, c_i64, c_i64, c_f, c_int, c_int, c_int, c_f, c_f, c_f, c_f, c_f, c_f]),

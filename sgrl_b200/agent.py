@@ -15,14 +15,27 @@ from __future__ import annotations
 import ctypes as C
 import os
 import warnings
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import numpy as np
 import torch
 import torch.nn as nn
 
-from ._lib import check, lib, ptr, stream
+from ._lib import TD3_HPARAMS, check, lib, ptr, stream
 from .modules import SECritic, SEPolicy, SetNetModule
+
+
+def hparam_table(seeds: List[Dict[str, float]]) -> np.ndarray:
+    """The rows of the per-seed TD3 table (SgrlTd3Hparams, include/sgrl_b200.h) for seeds[k] = {actor_lr, critic_lr, discount,
+    policy_noise, noise_clip, grad_clipping_value, target_smoothing_tau, reward_scale}.  The fp32 fields are rounded exactly
+    as the by-value float arguments were, and one_minus_tau = (float)(1.0 - (double)tau) as sgrl_polyak forms it."""
+    rows = np.zeros(len(seeds), dtype=TD3_HPARAMS)
+    for field, key in (("actor_lr", "actor_lr"), ("critic_lr", "critic_lr"), ("discount", "discount"), ("reward_scale", "reward_scale"),
+                       ("policy_noise", "policy_noise"), ("noise_clip", "noise_clip"), ("tau", "target_smoothing_tau"),
+                       ("max_norm", "grad_clipping_value")):
+        rows[field] = [float(h[key]) for h in seeds]
+    rows["one_minus_tau"] = 1.0 - rows["tau"].astype(np.float64)
+    return rows
 
 
 class FusedAdam:
@@ -54,23 +67,34 @@ class FusedAdam:
         self._sync_device()
         self.module.grad_arena().zero_()
 
-    def step(self, max_norm: float = 0.0, world_size: int = 1, keep_split: Optional[bool] = None):
+    def step(self, max_norm: float = 0.0, world_size: int = 1, keep_split: Optional[bool] = None,
+             hparams: Optional[torch.Tensor] = None):
         """Clip (if max_norm > 0) and apply one Adam step from module.grad_arena().  keep_split: also rewrite the tf32
         hi/lo split of the parameters (None: if it is fresh now).  A caller that captures this call into a CUDA graph
-        passes the decision explicitly and invalidates the split itself when it is False (Agent._run_update)."""
+        passes the decision explicitly and invalidates the split itself when it is False (Agent._run_update).
+        hparams: the device table of per-seed TD3 scalars (one SgrlTd3Hparams row per group, Agent._sync_hparams).  Group g's
+        learning rate (the actor or critic one, after the module's kind) and clip threshold are then read from row g when the
+        kernel runs, in place of self.lr and max_norm, and the gradient norms are always computed."""
         self._sync_device()
         m = self.module
         g, p = m.grad_arena(), m.live_arena
         nets, st = self.sumsq.numel(), stream()
         n_net = p.numel() // nets
+        if hparams is not None and hparams.numel() != self.groups * TD3_HPARAMS.itemsize:
+            raise ValueError(f"hparams holds {hparams.numel() // TD3_HPARAMS.itemsize} rows for {self.groups} optimizer groups")
         self.sumsq.zero_()
-        if max_norm > 0:
+        if max_norm > 0 or hparams is not None:
             check(lib.sgrl_sumsq_nets(ptr(g), n_net, nets, ptr(self.sumsq), st), "sgrl_sumsq_nets")
         check(lib.sgrl_bump_step(ptr(self.step_count), st), "sgrl_bump_step")
         fresh = m.split_is_fresh() if keep_split is None else (keep_split and m._split is not None)
         if not fresh:
             m.invalidate_split()
         hi, lo = (m._split[0], m._split[1]) if fresh else (None, None)     # keep a valid tf32 split valid (else it is rebuilt lazily)
+        if hparams is not None:
+            check(lib.sgrl_adam_clip_groups_hp(ptr(p), ptr(g), ptr(self.exp_avg), ptr(self.exp_avg_sq), n_net, nets, self.groups,
+                                               ptr(self.sumsq), ptr(self.step_count), ptr(hparams), m._kind, self.betas[0], self.betas[1],
+                                               self.eps, 1.0 / world_size, ptr(hi), ptr(lo), st), "sgrl_adam_clip_groups_hp")
+            return
         check(lib.sgrl_adam_clip_groups(ptr(p), ptr(g), ptr(self.exp_avg), ptr(self.exp_avg_sq), n_net, nets, self.groups, ptr(self.sumsq),
                                         ptr(self.step_count), self.lr, self.betas[0], self.betas[1], self.eps, float(max_norm), 1.0 / world_size,
                                         ptr(hi), ptr(lo), st), "sgrl_adam_clip_groups")
@@ -85,9 +109,12 @@ class FusedAdam:
         self.lr, self.betas, self.eps = sd["lr"], tuple(sd["betas"]), sd["eps"]
 
 
-def soft_update_network(source: SetNetModule, target: SetNetModule, tau: float, keep_split: Optional[bool] = None):
+def soft_update_network(source: SetNetModule, target: SetNetModule, tau: float, keep_split: Optional[bool] = None,
+                        hparams: Optional[torch.Tensor] = None):
     """theta_t <- tau*theta + (1-tau)*theta_t over ALL parameters incl. the dead ones
-    (src/common/functional.py:7-10) as one pass over the flat arenas.  keep_split: see FusedAdam.step."""
+    (src/common/functional.py:7-10) as one pass over the flat arenas.  keep_split: see FusedAdam.step.
+    hparams: the device table of per-seed TD3 scalars (K rows); net z of the modules, live or dead, then takes seed z % K's
+    tau from it when the kernel runs, and `tau` is not used."""
     s, t = source.full_arena, target.full_arena
     if s.device.type != "cuda":
         raise RuntimeError("sgrl_b200.soft_update_network needs the modules on a CUDA device (no CPU fallback)")
@@ -95,6 +122,10 @@ def soft_update_network(source: SetNetModule, target: SetNetModule, tau: float, 
     if not fresh:
         target.invalidate_split()
     hi, lo = (target._split[0], target._split[1]) if fresh else (None, None)
+    if hparams is not None:
+        check(lib.sgrl_polyak_hp(ptr(t), ptr(s), target._nb, target._live, target._dead, ptr(hparams), hparams.numel() // TD3_HPARAMS.itemsize,
+                                 ptr(hi), ptr(lo), stream()), "sgrl_polyak_hp")
+        return
     check(lib.sgrl_polyak(ptr(t), ptr(s), s.numel(), float(tau), ptr(hi), ptr(lo), target.live_arena.numel(), stream()), "sgrl_polyak")
 
 
@@ -361,6 +392,8 @@ class Agent(nn.Module):
         self._rollout_tables: Dict = {}
         self._rollout_sig = None
         self._loss = None
+        self._hp = None              # device table of the per-seed TD3 scalars (_sync_hparams), and the rows it holds
+        self._hp_rows = None
 
     # ------------------------------------------------------------------ TD3 step
     def _world(self):
@@ -394,6 +427,28 @@ class Agent(nn.Module):
         g = module.grad_arena()
         module.backward_raw(tb, stash, dout, nb, g, False, trusted_split=True, ws=ws)
         self._allreduce(g, world)
+
+    def _seed_hparams(self) -> List[Dict[str, float]]:
+        """The per-step TD3 scalars of every seed, read before each update.  An Agent takes them from its attributes, so a
+        change made between updates applies to a replayed CUDA graph as it does eagerly."""
+        a = self.args
+        return [dict(actor_lr=self.actor_optimizer.lr, critic_lr=self.critic_optimizer.lr, discount=a.discount, policy_noise=a.policy_noise,
+                     noise_clip=a.noise_clip, grad_clipping_value=a.grad_clipping_value, target_smoothing_tau=self.target_smoothing_tau,
+                     reward_scale=self.reward_scale)]
+
+    def _sync_hparams(self, dev) -> torch.Tensor:
+        """The device table the step's kernels read the TD3 scalars from (one SgrlTd3Hparams row per seed, allocated once per
+        device).  The rows of _seed_hparams() are copied in stream order when they differ from the rows last copied: in steady
+        state nothing is copied."""
+        rows = hparam_table(self._seed_hparams()).tobytes()
+        if self._hp is None or self._hp.device != dev:
+            self._hp = torch.zeros(len(rows), dtype=torch.uint8, device=dev)
+            self._hp_rows = None
+        if rows != self._hp_rows:
+            # pageable source: the copy has staged it when copy_ returns, so a later change cannot race the transfer
+            self._hp.copy_(torch.frombuffer(bytearray(rows), dtype=torch.uint8), non_blocking=True)
+            self._hp_rows = rows
+        return self._hp
 
     def _plan(self, tb) -> "_UpdatePlan":
         key = id(tb)
@@ -506,7 +561,8 @@ class Agent(nn.Module):
         # load_state_dict are detected (SetNetModule._write_stamp), writes through p.data need module.invalidate_split()
         for m in mods:
             m._split_for(tb.T, True)
-        sig = tuple((m._arena.data_ptr(), int(m.use_tc), 0 if m._split is None else m._split.data_ptr()) for m in mods)
+        hp = self._sync_hparams(dev)
+        sig = tuple((m._arena.data_ptr(), int(m.use_tc), 0 if m._split is None else m._split.data_ptr()) for m in mods) + (hp.data_ptr(),)
         if sig != self._plan_sig:
             self._plans.clear()
             self._plan_sig = sig
@@ -541,8 +597,10 @@ class Agent(nn.Module):
 
     def _update_impl(self, p: "_UpdatePlan", actor_step: bool, rng: bool = False):
         """Enqueue one update on the current stream (+ p.s1, p.s2 and the library's side streams).  Capture-safe:
-        no allocation, no host synchronisation."""
+        no allocation, no host synchronisation.  The per-seed TD3 scalars are read from the table self._hp when the kernels
+        run (_run_update fills it); only max_action and policy_freq are baked in."""
         a = self.args
+        hp = self._hp
         tb, T, st = p.tb, p.tb.T, stream()
         K = self.n_seeds          # actor modules: K nets; critics: 2K, net z reading seed z % K's batch
         world = self._world()
@@ -555,11 +613,11 @@ class Agent(nn.Module):
             self.actor_target.forward_raw(tb, p.nobs, None, keep=False, nb=K, in_nets=K, trusted_split=True, out=p.a_t, stash=p.stash_at)
             if rng:       # eps ~ N(0, policy_noise^2) drawn in the kernel (each seed its own draws); p.noise receives it (tests, logging)
                 check(lib.sgrl_bump_step(ptr(p.draw), stream()))
-                check(lib.sgrl_td3_smooth_action_rng(ptr(p.a_t), ptr(p.next_action), ptr(p.noise), float(a.policy_noise), float(a.noise_clip),
-                                                     float(a.max_action), K * T * 3, p.seed, ptr(p.draw), stream()))
+                check(lib.sgrl_td3_smooth_action_rng_hp(ptr(p.a_t), ptr(p.next_action), ptr(p.noise), ptr(hp), T * 3, float(a.max_action),
+                                                        K * T * 3, p.seed, ptr(p.draw), stream()))
             else:
-                check(lib.sgrl_td3_smooth_action(ptr(p.a_t), ptr(p.noise), ptr(p.next_action), float(a.noise_clip), float(a.max_action), K * T * 3,
-                                                 stream()))
+                check(lib.sgrl_td3_smooth_action_hp(ptr(p.a_t), ptr(p.noise), ptr(p.next_action), ptr(hp), T * 3, float(a.max_action), K * T * 3,
+                                                    stream()))
             self.critic_target.forward_raw(tb, p.nobs, p.next_action, keep=False, nb=2 * K, in_nets=K, trusted_split=True, out=p.tq,
                                            stash=p.stash_ct)
             check(lib.sgrl_stream_fence(stream()))       # eager runs only (no-op under capture): see csrc/net.cuh stream_fence
@@ -579,11 +637,11 @@ class Agent(nn.Module):
             p.ev_b.record(p.s3)
         main.wait_event(p.ev_b)
         main.wait_event(p.ev_a)
-        check(lib.sgrl_td3_critic_loss_seeds(ptr(p.q), ptr(p.tq), ptr(p.rew), ptr(p.done), ptr(tb.tok_graph), ptr(tb.tok_weight), ptr(p.target),
-                                             ptr(p.dq), ptr(p.scal), float(a.discount), float(self.reward_scale), T, ptr(p.rstats), tb.G, K, st))
+        check(lib.sgrl_td3_critic_loss_seeds_hp(ptr(p.q), ptr(p.tq), ptr(p.rew), ptr(p.done), ptr(tb.tok_graph), ptr(tb.tok_weight),
+                                                ptr(p.target), ptr(p.dq), ptr(p.scal), ptr(hp), T, ptr(p.rstats), tb.G, K, st))
         self.critic_optimizer.zero_grad()
         self._backward_allreduce(self.critic, tb, p.stash_c, p.dq, 2 * K, p.ws, world)
-        self.critic_optimizer.step(max_norm=float(a.grad_clipping_value), world_size=world, keep_split=p.keep_split)
+        self.critic_optimizer.step(world_size=world, keep_split=p.keep_split, hparams=hp)
         # ---- delayed actor step + Polyak                                                                    agent.py:165-180
         if actor_step:
             main.wait_event(p.ev_c)
@@ -593,8 +651,8 @@ class Agent(nn.Module):
             self.critic.backward_raw(tb, p.stash_c, p.dq1, K, None, True, trusted_split=True, ws=p.ws, dact=p.dact)   # only d/d(action)
             self.actor_optimizer.zero_grad()
             self._backward_allreduce(self.actor, tb, p.stash_a, p.dact, K, p.ws, world)
-            self.actor_optimizer.step(max_norm=float(a.grad_clipping_value), world_size=world, keep_split=p.keep_split)
-            self.try_update_target_network(keep_split=p.keep_split)
+            self.actor_optimizer.step(world_size=world, keep_split=p.keep_split, hparams=hp)
+            self.try_update_target_network(keep_split=p.keep_split, hparams=hp)
 
     train_step = update   # BASELINE.json calls the TD3 step "train()"; the reference name is update (agent.py:117)
 
@@ -602,11 +660,12 @@ class Agent(nn.Module):
         """agent.py:158-162 returns Python floats (two device syncs in the reference).  When the batch arrived from host
         memory the statistics are computed there and nothing synchronises; otherwise they come from the sum / sum of
         squares the critic-loss kernel accumulated in fp64 (one 16-byte read per seed, one sync for all of them;
-        `lazy_stats`: left on the device).  rewards_per_seed[k]: the reward arrays of seed k; returns one dict per seed."""
-        s = self.reward_scale
+        `lazy_stats`: left on the device).  rewards_per_seed[k]: the reward arrays of seed k, scaled by seed k's reward_scale;
+        returns one dict per seed."""
         if all(isinstance(r, np.ndarray) or (torch.is_tensor(r) and not r.is_cuda) for rs in rewards_per_seed for r in rs):
             out = []
-            for rewards_in in rewards_per_seed:
+            for rewards_in, h in zip(rewards_per_seed, self._seed_hparams()):
+                s = h["reward_scale"]
                 r = torch.cat([torch.as_tensor(x, dtype=torch.float32).reshape(-1) for x in rewards_in]) * s
                 out.append({"misc/train_reward_mean": r.mean().item(), "misc/train_reward_var": r.var().item() if r.numel() > 1 else float("nan")})
             return out
@@ -622,9 +681,11 @@ class Agent(nn.Module):
                 out.append({"misc/train_reward_mean": float(mean), "misc/train_reward_var": float(var)})
         return out
 
-    def try_update_target_network(self, keep_split: Optional[bool] = None):
-        soft_update_network(self.critic, self.critic_target, self.target_smoothing_tau, keep_split)
-        soft_update_network(self.actor, self.actor_target, self.target_smoothing_tau, keep_split)
+    def try_update_target_network(self, keep_split: Optional[bool] = None, hparams: Optional[torch.Tensor] = None):
+        """Polyak update of both target networks with target_smoothing_tau, or (hparams: the device table of _sync_hparams)
+        with each seed's tau read when the kernel runs."""
+        soft_update_network(self.critic, self.critic_target, self.target_smoothing_tau, keep_split, hparams)
+        soft_update_network(self.actor, self.actor_target, self.target_smoothing_tau, keep_split, hparams)
 
     # ------------------------------------------------------------------ acting
     def _rollout_plan(self, tb) -> "_RolloutPlan":

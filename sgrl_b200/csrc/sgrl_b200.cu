@@ -22,7 +22,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 6; }
+int sgrl_version(void) { return 7; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -235,7 +235,18 @@ int sgrl_gemm_pair(const float* A0, int lda0, const float* W0_hi, const float* W
 int sgrl_td3_smooth_action(const float* pi_target, const float* noise, float* next_action, float noise_clip, float max_action,
                            int64_t n, sgrl_stream_t stream) {
   SGRL_CHECK(pi_target && noise && next_action, "null pointer");
-  launch_k(td3_smooth_action_kernel, grid_for_flat(n * 4), 256, 0, ST(stream), pi_target, noise, next_action, noise_clip, max_action, n);
+  launch_k(td3_smooth_action_kernel, grid_for_flat(n * 4), 256, 0, ST(stream), pi_target, noise, next_action, noise_clip, max_action,
+           (long long)n, (const SgrlTd3Hparams*)nullptr, 1LL);
+  SGRL_LAUNCH_OK();
+  return 0;
+}
+
+int sgrl_td3_smooth_action_hp(const float* pi_target, const float* noise, float* next_action, const SgrlTd3Hparams* hp,
+                              int64_t per_seed, float max_action, int64_t n, sgrl_stream_t stream) {
+  SGRL_CHECK(pi_target && noise && next_action && hp, "null pointer");
+  SGRL_CHECK(per_seed >= 1 && n % per_seed == 0, "n must be a multiple of per_seed");
+  launch_k(td3_smooth_action_kernel, grid_for_flat(n * 4), 256, 0, ST(stream), pi_target, noise, next_action, 0.f, max_action,
+           (long long)n, hp, (long long)per_seed);
   SGRL_LAUNCH_OK();
   return 0;
 }
@@ -244,7 +255,18 @@ int sgrl_td3_smooth_action_rng(const float* pi_target, float* next_action, float
                                float max_action, int64_t n, uint64_t seed, const int32_t* draw, sgrl_stream_t stream) {
   SGRL_CHECK(pi_target && next_action && draw, "null pointer");
   launch_k(td3_smooth_action_rng_kernel, grid_for_flat(n), 256, 0, ST(stream), pi_target, next_action, noise_out, policy_noise, noise_clip,
-           max_action, (long long)n, (unsigned long long)seed, draw);
+           max_action, (long long)n, (unsigned long long)seed, draw, (const SgrlTd3Hparams*)nullptr, 1LL);
+  SGRL_LAUNCH_OK();
+  return 0;
+}
+
+int sgrl_td3_smooth_action_rng_hp(const float* pi_target, float* next_action, float* noise_out, const SgrlTd3Hparams* hp,
+                                  int64_t per_seed, float max_action, int64_t n, uint64_t seed, const int32_t* draw,
+                                  sgrl_stream_t stream) {
+  SGRL_CHECK(pi_target && next_action && draw && hp, "null pointer");
+  SGRL_CHECK(per_seed >= 1 && n % per_seed == 0, "n must be a multiple of per_seed");
+  launch_k(td3_smooth_action_rng_kernel, grid_for_flat(n), 256, 0, ST(stream), pi_target, next_action, noise_out, 0.f, 0.f, max_action,
+           (long long)n, (unsigned long long)seed, draw, hp, (long long)per_seed);
   SGRL_LAUNCH_OK();
   return 0;
 }
@@ -252,12 +274,12 @@ int sgrl_td3_smooth_action_rng(const float* pi_target, float* next_action, float
 // grid.y = seed: the kernels offset every per-seed operand by blockIdx.y (td3.cuh); one seed is the single-agent entry point
 static int critic_loss(const float* q1, const float* q2, const float* tq1, const float* tq2, const float* reward, const float* done,
                        const int32_t* tok_graph, const float* tok_weight, float* target, float* dq1, float* dq2, float* loss, float discount,
-                       float reward_scale, int T, double* reward_stats, int G, int K, cudaStream_t st) {
+                       float reward_scale, int T, double* reward_stats, int G, int K, const SgrlTd3Hparams* hp, cudaStream_t st) {
   SGRL_CHECK(q1 && q2 && tq1 && tq2 && reward && done && tok_graph && target && dq1 && dq2 && loss, "null pointer");
   SGRL_CHECK(K >= 1 && K <= MAX_NETS / 2 && T >= 1 && G >= 1, "bad seed count or batch");
   int gx = ceil_div(T, 256); if (gx > NUM_SMS) gx = NUM_SMS;
   if (det_enabled()) gx = 1;      // the loss scalar: one add
-  launch_k(td3_critic_loss_kernel, dim3(gx, K), 256, 0, st, q1, q2, tq1, tq2, reward, done, tok_graph, tok_weight, target, dq1, dq2, loss, discount, reward_scale, T, reward_stats, G);
+  launch_k(td3_critic_loss_kernel, dim3(gx, K), 256, 0, st, q1, q2, tq1, tq2, reward, done, tok_graph, tok_weight, target, dq1, dq2, loss, discount, reward_scale, T, reward_stats, G, hp);
   SGRL_LAUNCH_OK();
   return 0;
 }
@@ -276,7 +298,7 @@ int sgrl_td3_critic_loss(const float* q1, const float* q2, const float* tq1, con
                          const int32_t* tok_graph, const float* tok_weight, float* target, float* dq1, float* dq2, float* loss, float discount,
                          float reward_scale, int T, double* reward_stats, int G, sgrl_stream_t stream) {
   return critic_loss(q1, q2, tq1, tq2, reward, done, tok_graph, tok_weight, target, dq1, dq2, loss, discount, reward_scale, T, reward_stats,
-                     G, 1, ST(stream));
+                     G, 1, nullptr, ST(stream));
 }
 
 int sgrl_td3_critic_loss_seeds(const float* q, const float* tq, const float* reward, const float* done, const int32_t* tok_graph,
@@ -285,7 +307,16 @@ int sgrl_td3_critic_loss_seeds(const float* q, const float* tq, const float* rew
   SGRL_CHECK(q && tq && dq, "null pointer");
   const long long h = (long long)K * T;      // critic2 of seed k is net K + k
   return critic_loss(q, q + h, tq, tq + h, reward, done, tok_graph, tok_weight, target, dq, dq + h, loss, discount, reward_scale, T,
-                     reward_stats, G, K, ST(stream));
+                     reward_stats, G, K, nullptr, ST(stream));
+}
+
+int sgrl_td3_critic_loss_seeds_hp(const float* q, const float* tq, const float* reward, const float* done, const int32_t* tok_graph,
+                                  const float* tok_weight, float* target, float* dq, float* loss, const SgrlTd3Hparams* hp, int T,
+                                  double* reward_stats, int G, int K, sgrl_stream_t stream) {
+  SGRL_CHECK(q && tq && dq && hp, "null pointer");
+  const long long h = (long long)K * T;
+  return critic_loss(q, q + h, tq, tq + h, reward, done, tok_graph, tok_weight, target, dq, dq + h, loss, 0.f, 0.f, T,
+                     reward_stats, G, K, hp, ST(stream));
 }
 
 int sgrl_td3_actor_loss(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, sgrl_stream_t stream) {
@@ -338,18 +369,36 @@ int sgrl_adam_clip(float* p, const float* g, float* m, float* v, int64_t n, cons
   return sgrl_adam_clip_groups(p, g, m, v, n, 1, 1, sumsq, step, lr, beta1, beta2, eps, max_norm, grad_scale, p_hi, p_lo, stream);
 }
 
-int sgrl_adam_clip_groups(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
-                          const int32_t* step, double lr, double beta1, double beta2, double eps, float max_norm, float grad_scale,
-                          float* p_hi, float* p_lo, sgrl_stream_t stream) {
+// one body for sgrl_adam_clip_groups (hp == NULL: lr and max_norm for every group) and sgrl_adam_clip_groups_hp
+static int adam_clip(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
+                     const int32_t* step, double lr, const SgrlTd3Hparams* hp, int lr_of, double beta1, double beta2, double eps,
+                     float max_norm, float grad_scale, float* p_hi, float* p_lo, cudaStream_t st) {
   SGRL_CHECK(p && g && m && v && sumsq && step, "null pointer");
   SGRL_CHECK(nets >= 1 && nets <= MAX_NETS && groups >= 1 && groups <= nets && nets % groups == 0, "nets must be 1..16, a multiple of groups");
   SGRL_CHECK((p_hi == nullptr) == (p_lo == nullptr) && (!p_hi || (aligned16(p_hi) && aligned16(p_lo))), "p_hi/p_lo go together, 16-byte aligned");
   SGRL_CHECK((n_net & 3) == 0 && aligned16(p) && aligned16(g) && aligned16(m) && aligned16(v), "arenas must be 16-byte aligned, n % 4 == 0");
   const int64_t n = n_net * nets;
   AdamCfg c{lr, beta1, beta2, (float)beta1, (float)beta2, (float)(1.0 - beta1), (float)(1.0 - beta2), (float)eps, max_norm, grad_scale};
-  launch_k(adam_clip_kernel, grid_for_flat(n), 256, 0, ST(stream), p, g, m, v, (long long)n, sumsq, step, c, p_hi, p_lo, (long long)n_net, nets, groups);
+  launch_k(adam_clip_kernel, grid_for_flat(n), 256, 0, st, p, g, m, v, (long long)n, sumsq, step, c, p_hi, p_lo, (long long)n_net, nets, groups,
+           hp, lr_of);
   SGRL_LAUNCH_OK();
   return 0;
+}
+
+int sgrl_adam_clip_groups(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
+                          const int32_t* step, double lr, double beta1, double beta2, double eps, float max_norm, float grad_scale,
+                          float* p_hi, float* p_lo, sgrl_stream_t stream) {
+  return adam_clip(p, g, m, v, n_net, nets, groups, sumsq, step, lr, nullptr, 0, beta1, beta2, eps, max_norm, grad_scale, p_hi, p_lo,
+                   ST(stream));
+}
+
+int sgrl_adam_clip_groups_hp(float* p, const float* g, float* m, float* v, int64_t n_net, int nets, int groups, const float* sumsq,
+                             const int32_t* step, const SgrlTd3Hparams* hp, int lr_of, double beta1, double beta2, double eps,
+                             float grad_scale, float* p_hi, float* p_lo, sgrl_stream_t stream) {
+  SGRL_CHECK(hp != nullptr, "null pointer");
+  SGRL_CHECK(lr_of == SGRL_ACTOR || lr_of == SGRL_CRITIC, "lr_of must be SGRL_ACTOR or SGRL_CRITIC");
+  return adam_clip(p, g, m, v, n_net, nets, groups, sumsq, step, 0.0, hp, lr_of, beta1, beta2, eps, 0.f, grad_scale, p_hi, p_lo,
+                   ST(stream));
 }
 
 int sgrl_bump_step(int32_t* step, sgrl_stream_t stream) {
@@ -365,7 +414,22 @@ int sgrl_polyak(float* target, const float* source, int64_t n, float tau, float*
   SGRL_CHECK((t_hi == nullptr) == (t_lo == nullptr) && (!t_hi || (aligned16(t_hi) && aligned16(t_lo) && (n_split & 3) == 0 && n_split <= n)),
              "t_hi/t_lo go together, 16-byte aligned, n_split % 4 == 0");
   SGRL_CHECK((n & 3) == 0 && aligned16(target) && aligned16(source), "arenas must be 16-byte aligned, n % 4 == 0");
-  launch_k(polyak_kernel, grid_for_flat(n), 256, 0, ST(stream), target, source, n, tau, (float)(1.0 - (double)tau), t_hi, t_lo, n_split);
+  launch_k(polyak_kernel, grid_for_flat(n), 256, 0, ST(stream), target, source, (long long)n, tau, (float)(1.0 - (double)tau), t_hi, t_lo,
+           (long long)n_split, (const SgrlTd3Hparams*)nullptr, 1, 0LL, 0LL);
+  SGRL_LAUNCH_OK();
+  return 0;
+}
+
+int sgrl_polyak_hp(float* target, const float* source, int nets, int64_t live_net, int64_t dead_net, const SgrlTd3Hparams* hp, int K,
+                   float* t_hi, float* t_lo, sgrl_stream_t stream) {
+  SGRL_CHECK(target && source && hp, "null pointer");
+  SGRL_CHECK(K >= 1 && nets >= K && nets <= MAX_NETS && nets % K == 0, "nets must be 1..16, a multiple of K");
+  SGRL_CHECK(live_net > 0 && dead_net >= 0 && live_net % 64 == 0 && dead_net % 64 == 0, "per-net sizes must be multiples of 64 floats");
+  SGRL_CHECK((t_hi == nullptr) == (t_lo == nullptr) && (!t_hi || (aligned16(t_hi) && aligned16(t_lo))), "t_hi/t_lo go together, 16-byte aligned");
+  SGRL_CHECK(aligned16(target) && aligned16(source), "arenas must be 16-byte aligned");
+  const long long n_live = (long long)nets * live_net, n = n_live + (long long)nets * dead_net;
+  launch_k(polyak_kernel, grid_for_flat(n), 256, 0, ST(stream), target, source, n, 0.f, 0.f, t_hi, t_lo, n_live, hp, K,
+           (long long)live_net, (long long)dead_net);
   SGRL_LAUNCH_OK();
   return 0;
 }

@@ -1,15 +1,23 @@
 // K5/K6 — TD3 glue and the fused optimizer pass (src/agent.py:127-187, functional.py:7-10).
 #pragma once
+#include "../../include/sgrl_b200.h"
 #include "common.cuh"
 
 namespace sgrl {
 
+// Per-seed TD3 scalars (SgrlTd3Hparams, one row per seed) reach the kernels below as a device table that they read when they
+// run, so a captured CUDA graph applies whatever the table holds at replay.  hp == NULL: the by-value scalars (the entry points
+// without _hp), with the same arithmetic.
+
 // next_action = clamp(pi_target(s') + clamp(noise, +-c), +-max_action)        agent.py:128-133
+// hp: element i belongs to seed i / per_seed and is clipped by that seed's noise_clip
 __global__ void td3_smooth_action_kernel(const float* __restrict__ a, const float* __restrict__ noise, float* __restrict__ out,
-                                         float noise_clip, float max_action, long long n) {
+                                         float noise_clip, float max_action, long long n, const SgrlTd3Hparams* __restrict__ hp,
+                                         long long per_seed) {
   SGRL_PDL_ENTER();
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += gridDim.x * 256LL) {
-    const float nz = fminf(fmaxf(noise[i], -noise_clip), noise_clip);
+    const float c = hp ? hp[i / per_seed].noise_clip : noise_clip;
+    const float nz = fminf(fmaxf(noise[i], -c), c);
     out[i] = fminf(fmaxf(a[i] + nz, -max_action), max_action);
   }
 }
@@ -29,9 +37,12 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 // Same smoothing with the noise drawn in the kernel: eps ~ N(0, policy_noise^2) (agent.py:128 torch.randn_like * policy_noise),
 // four normals per Philox call (counter = {element / 4, 0, draw, 0}, key = seed; Box-Muller).  `draw` is a device counter the
 // caller bumps once per update (sgrl_bump_step), so a replayed CUDA graph draws fresh noise every replay.
+// hp: element i belongs to seed i / per_seed and takes that seed's policy_noise and noise_clip; the draws themselves (counter,
+// key) do not depend on the seed's row.
 __global__ void td3_smooth_action_rng_kernel(const float* __restrict__ a, float* __restrict__ out, float* __restrict__ noise_out,
                                              float policy_noise, float noise_clip, float max_action, long long n,
-                                             unsigned long long seed, const int* __restrict__ draw) {
+                                             unsigned long long seed, const int* __restrict__ draw,
+                                             const SgrlTd3Hparams* __restrict__ hp, long long per_seed) {
   SGRL_PDL_ENTER();
   const unsigned d = (unsigned)*draw;
   const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
@@ -49,9 +60,11 @@ __global__ void td3_smooth_action_rng_kernel(const float* __restrict__ a, float*
     for (int k = 0; k < 4; ++k) {
       const long long i = q * 4 + k;
       if (i >= n) break;
-      const float e = z[k] * policy_noise;
+      float sigma = policy_noise, c = noise_clip;
+      if (hp) { const SgrlTd3Hparams& h = hp[i / per_seed]; sigma = h.policy_noise; c = h.noise_clip; }
+      const float e = z[k] * sigma;
       if (noise_out) noise_out[i] = e;
-      out[i] = fminf(fmaxf(a[i] + fminf(fmaxf(e, -noise_clip), noise_clip), -max_action), max_action);
+      out[i] = fminf(fmaxf(a[i] + fminf(fmaxf(e, -c), c), -max_action), max_action);
     }
   }
 }
@@ -63,11 +76,13 @@ __global__ void __launch_bounds__(256) td3_critic_loss_kernel(
     const float* __restrict__ reward, const float* __restrict__ done, const int* __restrict__ tok_graph,
     const float* __restrict__ tok_w,
     float* __restrict__ target, float* __restrict__ dq1, float* __restrict__ dq2, float* __restrict__ loss,
-    float discount, float reward_scale, int T, double* __restrict__ rstats, int G) {
+    float discount, float reward_scale, int T, double* __restrict__ rstats, int G, const SgrlTd3Hparams* __restrict__ hp) {
   SGRL_PDL_ENTER();
   __shared__ float red[8];
-  {      // seed k = blockIdx.y (sgrl_td3_critic_loss_seeds): its own (T) outputs, (G) rewards, loss and reward statistics
+  {      // seed k = blockIdx.y (sgrl_td3_critic_loss_seeds): its own (T) outputs, (G) rewards, loss and reward statistics,
+         // and (hp) its own discount and reward scale
     const long long k = blockIdx.y;
+    if (hp) { discount = hp[k].discount; reward_scale = hp[k].reward_scale; }
     q1 += k * T; q2 += k * T; tq1 += k * T; tq2 += k * T; target += k * T; dq1 += k * T; dq2 += k * T;
     reward += k * G; done += k * G; loss += k;
     if (rstats) rstats += 2 * k;
@@ -183,6 +198,8 @@ struct AdamCfg { double lr, beta1d, beta2d; float beta1, beta2, omb1, omb2, eps,
 // grad_scale pre-multiplies g (1/world_size after a sum all-reduce).
 // Per-group clipping (sgrl_adam_clip_groups): the arena holds `nets` nets of n_net floats and sumsq one sum per net; net z is
 // clipped by the norm over its group {z' : z' % groups == z % groups}.  One net, one group: the single global norm.
+// hp (sgrl_adam_clip_groups_hp): group g takes its step size from row g's actor_lr (lr_of = SGRL_ACTOR) or critic_lr and its
+// clip threshold from row g's max_norm; NULL: c.lr and c.max_norm for every group.
 // hi/lo (nullable): the refreshed tf32 split of the parameters for the tcgen05 projections (csrc/gemm_tc.cuh).
 __device__ __forceinline__ void split_store4(float4 pv, float* hi, float* lo, long long i4) {
   float4 h, l;
@@ -205,27 +222,31 @@ __global__ void __launch_bounds__(256) split_tf32_kernel(const float* __restrict
 __global__ void __launch_bounds__(256) adam_clip_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                         float* __restrict__ v, long long n, const float* __restrict__ sumsq,
                                                         const int* __restrict__ step, AdamCfg c, float* __restrict__ hi, float* __restrict__ lo,
-                                                        long long n_net, int nets, int groups) {
+                                                        long long n_net, int nets, int groups,
+                                                        const SgrlTd3Hparams* __restrict__ hp, int lr_of) {
   SGRL_PDL_ENTER();
-  __shared__ float sh[2 + MAX_NETS];      // step size, sqrt of the second bias correction, per group: clip coef * grad_scale
+  __shared__ float sh[1 + 2 * MAX_NETS];  // sqrt of the second bias correction; per group: clip coef * grad_scale, step size
   if (threadIdx.x < groups) {
-    float s = sumsq[threadIdx.x];
-    for (int z = threadIdx.x + groups; z < nets; z += groups) s += sumsq[z];
+    const int gi = threadIdx.x;
+    double lr = c.lr;
+    float max_norm = c.max_norm;
+    if (hp) { lr = lr_of == SGRL_ACTOR ? hp[gi].actor_lr : hp[gi].critic_lr; max_norm = hp[gi].max_norm; }
+    float s = sumsq[gi];
+    for (int z = gi + groups; z < nets; z += groups) s += sumsq[z];
     const float nrm = sqrtf(s) * c.grad_scale;
     float coef = 1.f;
-    if (c.max_norm > 0.f) { coef = c.max_norm / (nrm + 1e-6f); coef = coef > 1.f ? 1.f : coef; }
-    sh[2 + threadIdx.x] = coef * c.grad_scale;
-  }
-  if (threadIdx.x == 0) {
+    if (max_norm > 0.f) { coef = max_norm / (nrm + 1e-6f); coef = coef > 1.f ? 1.f : coef; }
+    sh[1 + gi] = coef * c.grad_scale;
     const double t = (double)(*step);
-    sh[0] = (float)(c.lr / (1.0 - pow(c.beta1d, t)));
-    sh[1] = (float)sqrt(1.0 - pow(c.beta2d, t));
+    sh[1 + MAX_NETS + gi] = (float)(lr / (1.0 - pow(c.beta1d, t)));
+    if (gi == 0) sh[0] = (float)sqrt(1.0 - pow(c.beta2d, t));
   }
   __syncthreads();
-  const float step_size = sh[0], bc2s = sh[1];
+  const float bc2s = sh[0];
   const long long n4 = n >> 2;
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n4; i += gridDim.x * 256LL) {
-    const float gs = groups == 1 ? sh[2] : sh[2 + (int)((i * 4) / n_net) % groups];
+    const int gi = groups == 1 ? 0 : (int)((i * 4) / n_net) % groups;
+    const float gs = sh[1 + gi], step_size = sh[1 + MAX_NETS + gi];
     float4 pv = *reinterpret_cast<float4*>(p + i * 4);
     const float4 gv = ldg4(g + i * 4);
     float4 mv = *reinterpret_cast<float4*>(m + i * 4), vv = *reinterpret_cast<float4*>(v + i * 4);
@@ -249,11 +270,20 @@ __global__ void bump_step_kernel(int* step) {
 // Rounded exactly like the reference's three fp32 tensor ops (mul, mul, add — no FMA contraction):
 // the per-step change tau*(theta-theta_t) ~ 5e-7 is a few ulps of O(1) weights, so op order is visible.
 // hi/lo (nullable) cover the first n_split floats (the live prefix of the arena).
+// hp (sgrl_polyak_hp): the arena is [live nets | dead nets], n_split floats of live nets of live_net floats, then dead nets of
+// dead_net floats; net z (in either part) belongs to seed z % K and takes that seed's tau / one_minus_tau.  Both per-net sizes
+// are multiples of 64 floats (layout.h), so a float4 never straddles two nets.
 __global__ void __launch_bounds__(256) polyak_kernel(float* __restrict__ tgt, const float* __restrict__ src, long long n,
-                                                     float tau, float one_minus_tau, float* __restrict__ hi, float* __restrict__ lo, long long n_split) {
+                                                     float tau, float one_minus_tau, float* __restrict__ hi, float* __restrict__ lo, long long n_split,
+                                                     const SgrlTd3Hparams* __restrict__ hp, int K, long long live_net, long long dead_net) {
   SGRL_PDL_ENTER();
   const long long n4 = n >> 2;
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n4; i += gridDim.x * 256LL) {
+    if (hp) {
+      const long long e = i * 4;
+      const int k = K == 1 ? 0 : (int)((e < n_split ? e / live_net : (e - n_split) / dead_net) % K);
+      tau = hp[k].tau; one_minus_tau = hp[k].one_minus_tau;
+    }
     float4 t = *reinterpret_cast<float4*>(tgt + i * 4);
     const float4 s = ldg4(src + i * 4);
     t.x = __fadd_rn(__fmul_rn(tau, s.x), __fmul_rn(one_minus_tau, t.x));

@@ -8,12 +8,19 @@ net z reading seed z % K's batch.  The update sequence is ``Agent._update_impl``
 ``n_seeds``); clipping and Adam are per seed (one grouped launch each), Polyak and the all-reduce cover the whole arena.
 
 Each seed has its own initial weights (those of ``torch.manual_seed(seed); Agent(args)``), Adam state, target networks,
-replay data and target-policy noise; all seeds share the hyper-parameters and, at each step, the morphology.
+replay data and target-policy noise, and its own TD3 hyper-parameters (``HPARAM_KEYS``: learning rates, discount, target-policy
+noise and its clip, gradient clip, target smoothing tau, reward scale), so one seed-batched agent can run a hyper-parameter
+sweep.  The step's kernels read these from a small device table (one row per seed) when they run: ``set_hparams`` between
+updates takes effect at the next update without recapturing the step's graphs.  The seeds share the morphology of each step,
+``policy_freq``, ``max_action``, Adam's betas and eps, the batch size and the architecture.
 """
 from __future__ import annotations
 
 import contextlib
-from typing import List, Optional, Sequence
+import copy
+import math
+import numbers
+from typing import Dict, List, Optional, Sequence
 
 import torch
 
@@ -62,33 +69,52 @@ class SeedBatchedAgent(Agent):
     ``update(batches, it)`` performs one TD3 step (src/agent.py:117-183) for every seed as ONE captured CUDA graph and returns
     one loss dict per seed, with the keys ``Agent.update`` returns; ``update_packed_per_seed`` does the same for packed
     multi-morphology batches (``Agent.update_packed`` per seed).  ``agent(k)`` gives seed k as a standalone ``Agent`` (its
-    ``state_dict`` has the reference's 818 keys); ``from_agents`` builds a seed-batched agent from existing ones."""
+    ``state_dict`` has the reference's 818 keys); ``from_agents`` builds a seed-batched agent from existing ones.
 
-    def __init__(self, args, seeds: Sequence[int]):
+    hparams: None (every seed trains with args' values) or K dicts, dict k overriding args for seed k with any of ``lr`` and
+    ``HPARAM_KEYS``.  ``get_hparams(k)`` / ``set_hparams(k, **values)`` read and change seed k's values; the step reads them
+    before every update.  The Agent attributes that carry these values for a single agent (the optimizers' ``lr``,
+    ``args.discount`` and the like, ``target_smoothing_tau``, ``reward_scale``) hold seed 0's initial values and are not read."""
+
+    def __init__(self, args, seeds: Sequence[int], hparams: Optional[Sequence[Dict]] = None):
         seeds = list(seeds)
         _check_count(len(seeds))
+        base = args_hparams(args)
+        if hparams is None:
+            per_seed = [dict(base) for _ in seeds]
+        else:
+            hparams = list(hparams)
+            if len(hparams) != len(seeds):
+                raise ValueError(f"hparams: expected one dict per seed ({len(seeds)}), got {len(hparams)}")
+            per_seed = [{**base, **check_hparams(h, f"hparams[{k}]")} for k, h in enumerate(hparams)]
         agents = []
         with _rng_kept():
             for sd in seeds:
                 torch.manual_seed(sd)
                 agents.append(Agent(args))
-        self._init_from(agents)
+        self._init_from(agents, per_seed)
 
     @classmethod
     def from_agents(cls, agents: Sequence[Agent]) -> "SeedBatchedAgent":
-        """A seed-batched copy of existing agents: parameters, target networks, Adam moments and step counts.  The agents
-        must have taken the same number of optimizer steps (the seeds share one step counter)."""
+        """A seed-batched copy of existing agents: parameters, target networks, Adam moments and step counts, and each agent's
+        own hyper-parameters (its optimizers' lr, args' discount, policy noise, noise clip and gradient clip, its
+        target_smoothing_tau and reward_scale).  The agents must share policy_freq and max_action and have taken the same
+        number of optimizer steps (the seeds share one step counter)."""
         agents = list(agents)
         _check_count(len(agents))
+        for key in ("policy_freq", "max_action"):
+            values = {getattr(a.args, key) for a in agents}
+            if len(values) != 1:
+                raise ValueError(f"the agents' {key} differ ({sorted(values)}): every seed of a SeedBatchedAgent shares it")
         for name in ("actor_optimizer", "critic_optimizer"):
             steps = {int(getattr(a, name).step_count.item()) for a in agents}
             if len(steps) != 1:
                 raise ValueError(f"the agents' {name} step counts differ ({sorted(steps)}): seed-batched agents step together")
         self = cls.__new__(cls)
-        self._init_from(agents)
+        self._init_from(agents, [a._seed_hparams()[0] for a in agents])
         return self
 
-    def _init_from(self, agents: List[Agent]):
+    def _init_from(self, agents: List[Agent], per_seed: List[Dict[str, float]]):
         nn_init = super(Agent, self).__init__          # nn.Module.__init__: the modules are built here, not by Agent.__init__
         nn_init()
         a0 = agents[0]
@@ -118,16 +144,43 @@ class SeedBatchedAgent(Agent):
         self._init_runtime(args)
         self.tot_update_count = a0.tot_update_count
         self.target_smoothing_tau, self.reward_scale = a0.target_smoothing_tau, a0.reward_scale
+        self._hparams = [{key: float(h[key]) for key in HPARAM_KEYS} for h in per_seed]
         if hasattr(a0.actor, "graph"):
             self.change_morphology(a0.actor.graph)
 
-    def agent(self, k: int) -> Agent:
-        """Seed k as a standalone ``Agent`` (a copy): parameters, target networks, Adam state and update count."""
+    def _check_index(self, k: int):
         if not 0 <= k < self.n_seeds:
             raise ValueError(f"seed index {k} outside 0..{self.n_seeds - 1}")
+
+    def get_hparams(self, k: int) -> Dict[str, float]:
+        """Seed k's hyper-parameters, {HPARAM_KEYS key: value} (a copy)."""
+        self._check_index(k)
+        return dict(self._hparams[k])
+
+    def set_hparams(self, k: int, **values):
+        """Changes seed k's hyper-parameters (keywords as in the constructor's hparams dicts).  The next update uses them: the
+        step's graphs read them from the device table, which is rewritten in stream order before that update; nothing is
+        recaptured.  Raises ValueError, changing nothing, on a key or value the constructor refuses."""
+        self._check_index(k)
+        self._hparams[k].update(check_hparams(values, f"set_hparams({k})"))
+
+    def _seed_hparams(self) -> List[Dict[str, float]]:
+        return self._hparams
+
+    def try_update_target_network(self, keep_split: Optional[bool] = None, hparams=None):
+        """Polyak update of every seed's target networks with its own tau."""
+        if hparams is None:
+            hparams = self._sync_hparams(self.actor.full_arena.device)
+        super().try_update_target_network(keep_split, hparams)
+
+    def agent(self, k: int) -> Agent:
+        """Seed k as a standalone ``Agent`` (a copy): parameters, target networks, Adam state, update count and hyper-parameters
+        (in a copy of args and in the optimizers' lr)."""
+        self._check_index(k)
         dev = self.actor.full_arena.device
+        h = self._hparams[k]
         with _rng_kept():
-            a = Agent(self.args)
+            a = Agent(args_with(self.args, h))
         a.to(dev)
         for m in ("actor", "actor_target", "critic", "critic_target"):
             _copy_seed(getattr(self, m), getattr(a, m), self.n_seeds, k, False)
@@ -137,9 +190,9 @@ class SeedBatchedAgent(Agent):
             one._sync_device()
             _copy_seed_adam(mine, one, self.n_seeds, k, False)
             one.step_count.copy_(mine.step_count)
-            one.lr, one.betas, one.eps = mine.lr, mine.betas, mine.eps
+            one.lr, one.betas, one.eps = h["actor_lr" if name == "actor_optimizer" else "critic_lr"], mine.betas, mine.eps
         a.tot_update_count = self.tot_update_count
-        a.target_smoothing_tau, a.reward_scale = self.target_smoothing_tau, self.reward_scale
+        a.target_smoothing_tau, a.reward_scale = h["target_smoothing_tau"], h["reward_scale"]
         a.data_parallel, a.lazy_stats, a.use_graphs = self.data_parallel, self.lazy_stats, self.use_graphs
         if hasattr(self.actor, "graph"):
             a.change_morphology(self.actor.graph)
@@ -298,6 +351,63 @@ class SeedBatchedAgent(Agent):
                                   "update_packed_per_seed / update_packed_from_buffers_per_seed / select_actions, or agent(k) for one seed")
 
     update_packed = update_packed_from_buffers = update_from_buffer = select_action = _single
+
+
+# Per-seed hyper-parameters, as returned by get_hparams.  SeedBatchedAgent(args, seeds, hparams) and set_hparams also take
+# `lr`, which sets both learning rates (the reference's single args.lr); a more specific key given with it wins.
+HPARAM_KEYS = ("actor_lr", "critic_lr", "discount", "policy_noise", "noise_clip", "grad_clipping_value", "target_smoothing_tau",
+               "reward_scale")
+# args keys every seed shares: the delayed-update period, the action bound, the batch size and the architecture
+SHARED_KEYS = ("policy_freq", "max_action", "batch_size", "actor_type", "critic_type", "limb_obs_size", "limb_action_size", "msg_dim",
+               "max_children", "disable_fold", "td", "bu", "attention_embedding_size", "attention_heads", "attention_hidden_size",
+               "attention_layers", "dropout_rate", "condition_decoder_on_features", "transformer_norm", "traversal_types", "rel_size")
+_NON_NEGATIVE = ("lr", "actor_lr", "critic_lr", "grad_clipping_value", "policy_noise", "noise_clip")
+
+
+def check_hparams(values: Dict, where: str) -> Dict[str, float]:
+    """A dict of per-seed overrides -> {HPARAM_KEYS key: float}.  ValueError, in this order: a key every seed shares, an unknown
+    key, a value that is not a finite real number, a negative learning rate, clip, policy noise or noise clip, and a tau
+    outside [0, 1]."""
+    if not isinstance(values, dict):
+        raise ValueError(f"{where}: expected a dict of hyper-parameters, got {type(values).__name__}")
+    for key in values:
+        if key in SHARED_KEYS:
+            raise ValueError(f"{where}: {key!r} is shared by every seed of a SeedBatchedAgent; set it in args")
+    for key in values:
+        if key != "lr" and key not in HPARAM_KEYS:
+            raise ValueError(f"{where}: unknown hyper-parameter {key!r}; per-seed keys are lr, {', '.join(HPARAM_KEYS)}")
+    for key, v in values.items():
+        if isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(float(v)):
+            raise ValueError(f"{where}: {key} must be a finite real number, got {v!r}")
+    for key, v in values.items():
+        if key in _NON_NEGATIVE and v < 0:
+            raise ValueError(f"{where}: {key} must be >= 0, got {v}")
+        if key == "target_smoothing_tau" and not 0.0 <= v <= 1.0:
+            raise ValueError(f"{where}: target_smoothing_tau must lie in [0, 1], got {v}")
+    out = {}
+    if "lr" in values:
+        out["actor_lr"] = out["critic_lr"] = float(values["lr"])
+    out.update({k: float(v) for k, v in values.items() if k != "lr"})
+    return out
+
+
+def args_hparams(args) -> Dict[str, float]:
+    """The HPARAM_KEYS values an ``Agent(args)`` trains with."""
+    return dict(actor_lr=float(args.lr), critic_lr=float(args.lr), discount=float(args.discount), policy_noise=float(args.policy_noise),
+                noise_clip=float(args.noise_clip), grad_clipping_value=float(args.grad_clipping_value),
+                target_smoothing_tau=float(args.agent.target_smoothing_tau), reward_scale=float(args.agent.reward_scale))
+
+
+def args_with(args, h: Dict[str, float]):
+    """A copy of args (and of args.agent) holding the per-seed values h; args.lr only when both learning rates agree."""
+    out = copy.copy(args)
+    out.agent = copy.copy(args.agent)
+    for key in ("discount", "policy_noise", "noise_clip", "grad_clipping_value"):
+        setattr(out, key, h[key])
+    out.agent.target_smoothing_tau, out.agent.reward_scale = h["target_smoothing_tau"], h["reward_scale"]
+    if h["actor_lr"] == h["critic_lr"]:
+        out.lr = h["actor_lr"]
+    return out
 
 
 def _check_count(K: int):

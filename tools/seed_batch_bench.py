@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """K seeds of TD3 on one GPU: one seed-batched update against K single-agent updates, one process.
 
-  python tools/seed_batch_bench.py [--steps 200] [--rounds 2] [--batches 100,256] [--seeds 1,2,4,8]
+  python tools/seed_batch_bench.py [--steps 200] [--rounds 2] [--batches 100,256] [--seeds 1,2,4,8] [--sweep]
 
 Workload: 3d_humanoid_9_full at the reference configs' batch sizes (B = 100; B = 256 as in start_humanoid.sh), K seeds each
 with its own device batch (synthetic, fixed across steps).  Arms, alternated A/B/A/B:
@@ -12,6 +12,10 @@ with its own device batch (synthetic, fixed across steps).  Arms, alternated A/B
 Per arm and round: device ms per step between CUDA events around --steps steps (followed by a synchronise), the ratio
 B / A (A is K times the single-agent step), library kernels executed per step (through graph replays and outside them) and
 the card's name and power limit, read in the same run.  Prints one JSON line; writes nothing.
+
+--sweep: a hyper-parameter sweep instead of K seeds of one configuration.  Seed k trains with configuration k of
+sweep_hparams(K) (learning rate, tau, discount, target-policy noise and gradient clip all differ), in arm B through
+SeedBatchedAgent(args, seeds, hparams) and in arm A as an Agent built with those values.
 """
 from __future__ import annotations
 
@@ -58,20 +62,34 @@ def time_arms(arms, steps, rounds, it, before_window=None):
     return res
 
 
-def run_case(B, K, steps, rounds, warmup, dev):
+def sweep_hparams(K):
+    """K distinct configurations around the reference's defaults."""
+    return [dict(actor_lr=1e-4 * 2.0 ** (k % 4 - 1), critic_lr=1e-4 * 2.0 ** ((k + 1) % 4 - 1), target_smoothing_tau=0.005 * (1 + k % 3),
+                 discount=0.99 - 0.005 * (k % 2), policy_noise=0.1 + 0.05 * (k % 3), noise_clip=0.3 + 0.1 * (k % 3),
+                 grad_clipping_value=0.1 * (1 + k % 2)) for k in range(K)]
+
+
+def run_case(B, K, steps, rounds, warmup, dev, sweep=False):
     import torch
     from sgrl_b200 import graph as G, morphologies as M, synth
     from sgrl_b200.agent import Agent
     from sgrl_b200.config import default_args
-    from sgrl_b200.seed_batch import SeedBatchedAgent
+    from sgrl_b200.seed_batch import SeedBatchedAgent, args_hparams, args_with
     par = M.ALL[MORPH]
     g = G.build_graph(par, device=dev)
     seeds = list(range(K))
+    hps = sweep_hparams(K) if sweep else None
     singles = []
     for s in seeds:
         torch.manual_seed(s)
-        singles.append(Agent(default_args()))
-    sb = SeedBatchedAgent(default_args(), seeds)
+        if sweep:
+            h = {**args_hparams(default_args()), **hps[s]}
+            ag = Agent(args_with(default_args(), h))
+            ag.actor_optimizer.lr, ag.critic_optimizer.lr = h["actor_lr"], h["critic_lr"]
+            singles.append(ag)
+        else:
+            singles.append(Agent(default_args()))
+    sb = SeedBatchedAgent(default_args(), seeds, hparams=hps)
     for ag in singles + [sb]:
         ag.lazy_stats = True
         ag.change_morphology(g)
@@ -92,7 +110,7 @@ def run_case(B, K, steps, rounds, warmup, dev):
     torch.cuda.synchronize()
     res = time_arms(arms, steps, rounds, it)
     a, b = res["A_k_agents"]["device_ms_median"], res["B_seed_batched"]["device_ms_median"]
-    return {"batch": B, "seeds": K, "limb_tokens_per_seed": B * len(par), "arms": res, "ratio_B_over_A": round(b / a, 4),
+    return {"batch": B, "seeds": K, "sweep": sweep, "limb_tokens_per_seed": B * len(par), "arms": res, "ratio_B_over_A": round(b / a, 4),
             "seed_batched_faster": b < a}
 
 
@@ -103,6 +121,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=6, help="untimed steps per arm before the first round (at least 4)")
     ap.add_argument("--batches", default="100,256")
     ap.add_argument("--seeds", default="1,2,4,8")
+    ap.add_argument("--sweep", action="store_true", help="seed k trains with configuration k of sweep_hparams(K)")
     a = ap.parse_args()
     Bs = [int(x) for x in a.batches.split(",") if x]
     Ks = [int(x) for x in a.seeds.split(",") if x]
@@ -116,7 +135,7 @@ def main():
     out = {"metric": "seed_batched_td3_update", "morphology": MORPH, "steps": a.steps, "rounds": a.rounds, **card(0), "cases": []}
     for B in Bs:
         for K in Ks:
-            out["cases"].append(run_case(B, K, a.steps, a.rounds, a.warmup, dev))
+            out["cases"].append(run_case(B, K, a.steps, a.rounds, a.warmup, dev, a.sweep))
             torch.cuda.empty_cache()
     print(json.dumps(out))
 
