@@ -214,6 +214,16 @@ int sgrl_td3_actor_loss_seeds(const float* q1, const float* tok_weight, float* d
 int sgrl_td3_critic_loss_seeds_hp(const float* q, const float* tq, const float* reward, const float* done, const int32_t* tok_graph,
                                   const float* tok_weight, float* target, float* dq, float* loss, const SgrlTd3Hparams* hp, int T,
                                   double* reward_stats, int G, int K, sgrl_stream_t stream);
+/* Per-morphology TD3 statistics of a packed (seed-batched) update: for seed k (grid y) and part i (grid x),
+ * out[(k*P + i)*4 + 0..3] = critic loss, actor loss (NaN when q1 == NULL), reward mean, reward variance (unbiased; NaN
+ * for one sample) over part i's tokens [t0,t1) and graphs [g0,g1) of seed k's block.  parts: DEVICE (P,4) int32
+ * {t0,t1,g0,g1} within one seed's block; q (2K,T) [critic1 of seeds | critic2 of seeds], target (K,T), q1 (K,T) or NULL,
+ * reward (K,G); hp (K rows) supplies each seed's reward_scale.  fp64 accumulation, fixed-order reductions, no atomics.
+ * Critic loss = sum over the part's tokens of (q1-y)^2 + (q2-y)^2 over its token count, actor loss = -sum(q1) over its token
+ * count (src/agent.py:146-148, 167 restricted to the part), rewards = reward * reward_scale rounded to fp32 as the critic-loss
+ * kernel forms them.  A part that is empty or lies outside [0,T) x [0,G) gets four NaNs.  One launch of P x K CTAs. */
+int sgrl_td3_part_stats(const float* q, const float* target, const float* q1, const float* reward, const int32_t* parts,
+                        int P, int T, int G, int K, const SgrlTd3Hparams* hp, double* out, sgrl_stream_t stream);
 
 /* ---- K6: optimizer (agent.py:150-156,170-178; common/functional.py:7-10) -------------------- */
 int sgrl_sumsq(const float* g, int64_t n, float* out /*accumulates*/, sgrl_stream_t stream);

@@ -97,6 +97,7 @@ _PROTOS = {
     "sgrl_td3_critic_loss_seeds": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, C.c_float, C.c_float, c_int, c_f, c_int, c_int, c_f]),
     "sgrl_td3_actor_loss_seeds": (c_int, [c_f, c_f, c_f, c_f, c_int, c_int, c_f]),
     "sgrl_td3_critic_loss_seeds_hp": (c_int, [c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_int, c_f, c_int, c_int, c_f]),
+    "sgrl_td3_part_stats": (c_int, [c_f, c_f, c_f, c_f, c_f, c_int, c_int, c_int, c_int, c_f, c_f, c_f]),
     "sgrl_sumsq": (c_int, [c_f, c_i64, c_f, c_f]),
     "sgrl_sumsq_nets": (c_int, [c_f, c_i64, c_int, c_f, c_f]),
     "sgrl_adam_clip_groups": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_int, c_int, c_f, c_f, C.c_double, C.c_double, C.c_double, C.c_double,

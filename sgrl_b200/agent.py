@@ -176,9 +176,18 @@ class _UpdatePlan:
         # bake the pointers in).  Plans too small for the tcgen05 path leave the split stale; _run_update then marks it so.
         self.keep_split = all(m.use_tc and T >= m.SPLIT_MIN_TOKENS for m in (agent.actor, agent.critic, agent.actor_target, agent.critic_target))
         self.graphs = {}
-        self.graph_launches = {}      # (actor_step, rng) -> kernels of this library inside the captured graph
+        self.graph_launches = {}      # (actor_step, rng) [+ (True,) with the per-morphology statistics] -> kernels of this library inside the captured graph
         self.eager_runs = {}
         self.i_dev = None             # row numbers of a packed buffer gather (stage_indices), allocated on first use
+        self.part_stats = None        # (K,P,4) fp64 per-morphology statistics (sgrl_td3_part_stats), allocated on first use
+
+    def alloc_part_stats(self):
+        """The result buffer and the fork / join events of the per-morphology statistics; outside any capture, before the
+        first step that computes them."""
+        if self.part_stats is None:
+            K, P = self.agent.n_seeds, len(self.tb.parts)
+            self.part_stats = torch.full((K, P, 4), float("nan"), dtype=torch.float64, device=self.inbuf.device)
+            self.ev_ps_fork, self.ev_ps_join = torch.cuda.Event(), torch.cuda.Event()
 
     def load(self, batches, noises):
         """Stage the replay batch of every morphology of the plan (host numpy / CPU or device tensors) into the static
@@ -252,28 +261,30 @@ class _UpdatePlan:
         self.i_ev[k].record()
         return [h[g0:g1] for (_, _, g0, g1, _) in self.spans]
 
-    def replay(self, actor_step: bool, rng: bool):
-        key = (actor_step, rng)
+    def replay(self, actor_step: bool, rng: bool, per_morphology: bool = False):
+        """per_morphology: the step also computes the per-morphology statistics; such steps have graphs of their own, keyed
+        (actor_step, rng, True), so the graphs of the steps without them stay as they are, keyed (actor_step, rng)."""
+        key = (actor_step, rng, True) if per_morphology else (actor_step, rng)
         g = self.graphs.get(key)
         if g is None:
             # one eager run first (lazy one-time initialisation inside the library: function attributes, side streams,
             # tensor-map cache), then capture the second
             if self.eager_runs.get(key, 0) < 1:
                 self.eager_runs[key] = 1
-                self.agent._update_impl(self, actor_step, rng)
+                self.agent._update_impl(self, actor_step, rng, per_morphology)
                 return
             try:
                 torch.cuda.synchronize()
                 g = torch.cuda.CUDAGraph()
                 l0 = lib.sgrl_launch_count()
                 with torch.cuda.graph(g, stream=self.s_cap):
-                    self.agent._update_impl(self, actor_step, rng)
+                    self.agent._update_impl(self, actor_step, rng, per_morphology)
                 self.graph_launches[key] = lib.sgrl_launch_count() - l0
             except Exception as ex:   # keep running eagerly (still the CUDA path); say so once
                 warnings.warn(f"sgrl_b200: CUDA-graph capture of Agent.update failed ({ex}); running eagerly")
                 self.agent.use_graphs = False
                 torch.cuda.synchronize()
-                self.agent._update_impl(self, actor_step, rng)
+                self.agent._update_impl(self, actor_step, rng, per_morphology)
                 return
             self.graphs[key] = g
             self.agent.graph_replayed_launches -= self.graph_launches[key]   # the capture itself was counted by the library
@@ -475,15 +486,19 @@ class Agent(nn.Module):
         tb = self.actor._tables(B)
         return self._run_update(tb, [data_batch], it, None if noise is None else [noise])[0]
 
-    def update_packed(self, batches, it: int, noises=None, morph_count: Optional[float] = None):
+    def update_packed(self, batches, it: int, noises=None, morph_count: Optional[float] = None, per_morphology: bool = False):
         """One TD3 update on a PACKED batch of several morphologies: batches = [(graph_dict, data_batch), ...].  The loss is
         the mean over morphologies of the reference's per-morphology loss, so the gradient equals the average of the
         gradients of the separate updates the reference performs one after the other (src/trainer.py:245-250) at the same
         parameters; the limb-tokens of all morphologies go through every kernel together (SURVEY.md §8f rank 1).
         morph_count: data-parallel ranks holding different numbers of morphologies pass (total morphologies / world) so the
-        all-reduced gradient is the mean over all morphologies (modules.make_packed_tables)."""
+        all-reduced gradient is the mean over all morphologies (modules.make_packed_tables).
+        per_morphology: the loss dict also holds "per_morphology", one dict per morphology in the order of `batches` with the
+        keys a per-morphology Agent.update returns (src/agent.py:158-162, 180): that morphology's critic loss, actor loss
+        (actor steps), and the mean and unbiased variance of its scaled rewards.  Floats from one device read per call, or
+        0-dim fp64 device tensors with `lazy_stats`.  They do not depend on morph_count and are not all-reduced."""
         tb = self._packed_tables_for([(g, int(b["obs"].shape[0])) for g, b in batches], morph_count)
-        return self._run_update(tb, [b for _, b in batches], it, noises)[0]
+        return self._run_update(tb, [b for _, b in batches], it, noises, per_morphology=per_morphology)[0]
 
     def _packed_tables_for(self, specs, morph_count):
         """Packed tables of specs = [(graph_dict, batch size), ...], cached per (graphs, batch sizes, morph_count).
@@ -499,8 +514,8 @@ class Agent(nn.Module):
         return tb
 
     def update_packed_from_buffers(self, parts, batch_size: int, it: int, noises=None, morph_count: Optional[float] = None,
-                                   sequential: bool = False, allow_duplicate: bool = False):
-        """``update_packed([(g, buffer.sample(batch_size)) for g, buffer in parts], it, noises, morph_count)`` without
+                                   sequential: bool = False, allow_duplicate: bool = False, per_morphology: bool = False):
+        """``update_packed([(g, buffer.sample(batch_size)) for g, buffer in parts], it, noises, morph_count, per_morphology)`` without
         materialising the batches: parts = [(graph_dict, sgrl_b200.buffer.ReplayBuffer), ...], one device buffer per morphology
         like the reference keeps them (src/main.py:141-155, src/trainer.py:239-253).  The indices are drawn buffer by buffer in
         list order, exactly as the reference draws them (equal seeds give equal batches; a buffer holding fewer than batch_size
@@ -525,7 +540,7 @@ class Agent(nn.Module):
             gather_packed_into(buffers, rows, plan.obs, plan.act, plan.nobs, plan.rew, plan.done, idx_dev=plan.i_dev)
             return plan.load_noise(noises)
 
-        return self._run_update(tb, None, it, None, loader=load)[0]
+        return self._run_update(tb, None, it, None, loader=load, per_morphology=per_morphology)[0]
 
     def update_from_buffer(self, buffer, batch_size: int, it: int, noise: Optional[torch.Tensor] = None,
                            sequential: bool = False, allow_duplicate: bool = False):
@@ -549,8 +564,8 @@ class Agent(nn.Module):
 
         return self._run_update(tb, None, it, None, loader=load)[0]
 
-    def _run_update(self, tb, batches, it: int, noises, loader=None):
-        """The step of every seed; returns one loss dict per seed."""
+    def _run_update(self, tb, batches, it: int, noises, loader=None, per_morphology: bool = False):
+        """The step of every seed; returns one loss dict per seed (per_morphology: see update_packed)."""
         a = self.args
         dev = self.actor.full_arena.device
         if dev.type != "cuda":
@@ -567,12 +582,14 @@ class Agent(nn.Module):
             self._plans.clear()
             self._plan_sig = sig
         plan = self._plan(tb)
+        if per_morphology:
+            plan.alloc_part_stats()
         injected = loader(plan) if loader is not None else plan.load(batches, noises)
         actor_step = it % a.policy_freq == 0
         if self.use_graphs:
-            plan.replay(actor_step, not injected)
+            plan.replay(actor_step, not injected, per_morphology)
         else:
-            self._update_impl(plan, actor_step, not injected)
+            self._update_impl(plan, actor_step, not injected, per_morphology)
         if plan.keep_split:       # the step's fused Adam / Polyak kernels rewrote hi/lo from the new parameters
             self.critic.mark_split_fresh()
             if actor_step:
@@ -591,14 +608,21 @@ class Agent(nn.Module):
             if actor_step:
                 loss_dict["loss/actor_loss"] = scal[K + k]
             loss_dicts.append(loss_dict)
+        if per_morphology:
+            # plan.part_stats[k, i] = {critic loss, actor loss, reward mean, reward variance}: one read for every seed and part
+            ps = plan.part_stats.clone() if self.lazy_stats else plan.part_stats.cpu().tolist()
+            cols = ((0, "loss/critic_loss"), (2, "misc/train_reward_mean"), (3, "misc/train_reward_var")) + (((1, "loss/actor_loss"),) if actor_step else ())
+            for k, loss_dict in enumerate(loss_dicts):
+                loss_dict["per_morphology"] = [{key: ps[k][i][j] for j, key in cols} for i in range(P)]
         self.tot_update_count += 1
         self._last_target = plan.target
         return loss_dicts
 
-    def _update_impl(self, p: "_UpdatePlan", actor_step: bool, rng: bool = False):
+    def _update_impl(self, p: "_UpdatePlan", actor_step: bool, rng: bool = False, per_morphology: bool = False):
         """Enqueue one update on the current stream (+ p.s1, p.s2 and the library's side streams).  Capture-safe:
         no allocation, no host synchronisation.  The per-seed TD3 scalars are read from the table self._hp when the kernels
-        run (_run_update fills it); only max_action and policy_freq are baked in."""
+        run (_run_update fills it); only max_action and policy_freq are baked in.  per_morphology: one more launch,
+        sgrl_td3_part_stats into p.part_stats, on p.s3 (_part_stats)."""
         a = self.args
         hp = self._hp
         tb, T, st = p.tb, p.tb.T, stream()
@@ -639,6 +663,8 @@ class Agent(nn.Module):
         main.wait_event(p.ev_a)
         check(lib.sgrl_td3_critic_loss_seeds_hp(ptr(p.q), ptr(p.tq), ptr(p.rew), ptr(p.done), ptr(tb.tok_graph), ptr(tb.tok_weight),
                                                 ptr(p.target), ptr(p.dq), ptr(p.scal), ptr(hp), T, ptr(p.rstats), tb.G, K, st))
+        if per_morphology and not actor_step:
+            self._part_stats(p, None)
         self.critic_optimizer.zero_grad()
         self._backward_allreduce(self.critic, tb, p.stash_c, p.dq, 2 * K, p.ws, world)
         self.critic_optimizer.step(world_size=world, keep_split=p.keep_split, hparams=hp)
@@ -648,11 +674,30 @@ class Agent(nn.Module):
             # critic1 of every seed = the first K nets of the critic arena
             self.critic.forward_raw(tb, p.obs, p.pi, keep=True, nb=K, in_nets=K, trusted_split=True, out=p.q1, stash=p.stash_c)
             check(lib.sgrl_td3_actor_loss_seeds(ptr(p.q1), ptr(tb.tok_weight), ptr(p.dq1), ptr(p.scal[K:]), T, K, st))
+            if per_morphology:
+                self._part_stats(p, p.q1)
             self.critic.backward_raw(tb, p.stash_c, p.dq1, K, None, True, trusted_split=True, ws=p.ws, dact=p.dact)   # only d/d(action)
             self.actor_optimizer.zero_grad()
             self._backward_allreduce(self.actor, tb, p.stash_a, p.dact, K, p.ws, world)
             self.actor_optimizer.step(world_size=world, keep_split=p.keep_split, hparams=hp)
             self.try_update_target_network(keep_split=p.keep_split, hparams=hp)
+        if per_morphology:
+            main.wait_event(p.ev_ps_join)
+
+    def _part_stats(self, p: "_UpdatePlan", q1):
+        """Per-morphology statistics of the step (sgrl_td3_part_stats) off the critical chain: forked from the current stream to
+        p.s3, whose critic forward the current stream has already joined, and joined again at the end of the step.  It reads
+        p.q, p.target, p.rew and q1 (p.q1 on actor steps, else None), which nothing later in the step writes."""
+        main = torch.cuda.current_stream()
+        check(lib.sgrl_stream_fence(stream()))       # eager runs only (no-op under capture): see csrc/net.cuh stream_fence
+        p.ev_ps_fork.record(main)
+        with torch.cuda.stream(p.s3):
+            p.s3.wait_event(p.ev_ps_fork)
+            tb = p.tb
+            check(lib.sgrl_td3_part_stats(ptr(p.q), ptr(p.target), ptr(q1), ptr(p.rew), ptr(tb.part_table), len(tb.parts), tb.T, tb.G,
+                                          self.n_seeds, ptr(self._hp), ptr(p.part_stats), stream()), "sgrl_td3_part_stats")
+            check(lib.sgrl_stream_fence(stream()))
+            p.ev_ps_join.record(p.s3)
 
     train_step = update   # BASELINE.json calls the TD3 step "train()"; the reference name is update (agent.py:117)
 

@@ -22,7 +22,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 7; }
+int sgrl_version(void) { return 8; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -325,6 +325,17 @@ int sgrl_td3_actor_loss(const float* q1, const float* tok_weight, float* dq1, fl
 
 int sgrl_td3_actor_loss_seeds(const float* q1, const float* tok_weight, float* dq1, float* loss, int T, int K, sgrl_stream_t stream) {
   return actor_loss(q1, tok_weight, dq1, loss, T, K, ST(stream));
+}
+
+int sgrl_td3_part_stats(const float* q, const float* target, const float* q1, const float* reward, const int32_t* parts, int P, int T,
+                        int G, int K, const SgrlTd3Hparams* hp, double* out, sgrl_stream_t stream) {
+  SGRL_CHECK(q && target && reward && parts && hp && out, "null pointer");
+  SGRL_CHECK(P >= 1 && P <= 64, "P must be 1..64");
+  SGRL_CHECK(K >= 1 && K <= MAX_NETS / 2, "K must be 1..8");
+  SGRL_CHECK(T >= 1 && G >= 1, "empty batch");
+  launch_k(td3_part_stats_kernel, dim3(P, K), 256, 0, ST(stream), q, target, q1, reward, parts, T, G, K, hp, out);
+  SGRL_LAUNCH_OK();
+  return 0;
 }
 
 int sgrl_sumsq(const float* g, int64_t n, float* out, sgrl_stream_t stream) { return sgrl_sumsq_nets(g, n, 1, out, stream); }

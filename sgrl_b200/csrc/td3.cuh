@@ -142,6 +142,64 @@ __global__ void __launch_bounds__(256) td3_actor_loss_kernel(const float* __rest
   }
 }
 
+// Per-morphology statistics of a packed update (src/agent.py:146-148, 158-162, 167 restricted to one morphology): CTA (i, k) =
+// (part, seed) reduces part i's tokens [t0,t1) and graphs [g0,g1) of seed k's block into out[(k*P + i)*4 + 0..3] = {critic loss,
+// actor loss (NaN without q1), reward mean, unbiased reward variance (NaN for one sample)}.  fp64 throughout; every thread sums
+// a fixed stride and the block combines warps in index order, so the result does not depend on timing.  A part outside the
+// block (or empty) gives four NaNs.
+__device__ __forceinline__ double block_sum_fixed(double v, double* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();                                    // red may still be read by the previous call
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double s = 0.0;
+#pragma unroll
+  for (int w = 0; w < 8; ++w) s += red[w];
+  return s;
+}
+
+__global__ void __launch_bounds__(256) td3_part_stats_kernel(const float* __restrict__ q, const float* __restrict__ target,
+                                                             const float* __restrict__ q1, const float* __restrict__ reward,
+                                                             const int* __restrict__ parts, int T, int G, int K,
+                                                             const SgrlTd3Hparams* __restrict__ hp, double* __restrict__ out) {
+  SGRL_PDL_ENTER();
+  __shared__ double red[8];
+  const int i = blockIdx.x, k = blockIdx.y;
+  const int t0 = parts[4 * i], t1 = parts[4 * i + 1], g0 = parts[4 * i + 2], g1 = parts[4 * i + 3];
+  out += ((long long)k * gridDim.x + i) * 4;
+  if (t0 < 0 || t1 > T || t0 >= t1 || g0 < 0 || g1 > G || g0 >= g1) {
+    if (threadIdx.x < 4) out[threadIdx.x] = __longlong_as_double(0x7ff8000000000000LL);
+    return;
+  }
+  const float* c1 = q + (long long)k * T;             // critic1 of seed k is net k, critic2 net K + k
+  const float* c2 = q + (long long)(K + k) * T;
+  const float* y = target + (long long)k * T;
+  const float* r = reward + (long long)k * G;
+  const float scale = hp[k].reward_scale;
+  double sc = 0.0, sa = 0.0, sr = 0.0;
+  for (int t = t0 + threadIdx.x; t < t1; t += 256) {
+    const double yt = (double)y[t], e1 = (double)c1[t] - yt, e2 = (double)c2[t] - yt;
+    sc += e1 * e1 + e2 * e2;
+    if (q1) sa += (double)q1[(long long)k * T + t];
+  }
+  for (int g = g0 + threadIdx.x; g < g1; g += 256) sr += (double)(r[g] * scale);
+  sc = block_sum_fixed(sc, red);
+  sa = block_sum_fixed(sa, red);
+  sr = block_sum_fixed(sr, red);
+  const double nt = (double)(t1 - t0), ng = (double)(g1 - g0), mean = sr / ng;
+  double sd = 0.0;                                    // second pass: squared deviations from the mean
+  for (int g = g0 + threadIdx.x; g < g1; g += 256) { const double d = (double)(r[g] * scale) - mean; sd += d * d; }
+  sd = block_sum_fixed(sd, red);
+  if (threadIdx.x == 0) {
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    out[0] = sc / nt;
+    out[1] = q1 ? -sa / nt : nan;
+    out[2] = mean;
+    out[3] = g1 - g0 > 1 ? sd / (ng - 1.0) : nan;
+  }
+}
+
 // sum of squares of a flat gradient buffer                                                  clip_grad_norm_, agent.py:152-155
 // Deterministic (no atomics): every block leaves its partial sum in a scratch slot, a second launch adds the partials in
 // index order.  The norm feeds the clip coefficient of every data-parallel replica: with an atomic reduction the ranks

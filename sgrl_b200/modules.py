@@ -55,11 +55,12 @@ def _check_args(args):
 class GraphTables:
     """Device-side tables of one morphology (or of a packed mix of morphologies)."""
 
-    def __init__(self, cu_limbs, rank3, tok_graph, relation, rel_off, T, G, tok_weight=None, parts=None):
+    def __init__(self, cu_limbs, rank3, tok_graph, relation, rel_off, T, G, tok_weight=None, parts=None, part_table=None):
         self.cu_limbs, self.rank3, self.tok_graph = cu_limbs, rank3, tok_graph
         self.relation, self.rel_off, self.T, self.G = relation, rel_off, T, G
         self.tok_weight = tok_weight          # (T) loss weight per token, packed mixed-morphology batches only
         self.parts = parts or [(0, T, 0, G, T // max(G, 1))]     # per morphology: (token0, token1, graph0, graph1, limbs)
+        self.part_table = part_table          # (P,4) int32 {token0, token1, graph0, graph1} of self.parts, packed batches only
         self.nmax = max(p[4] for p in self.parts)                 # largest graph: sizes the attention kernel's staging
 
 
@@ -89,7 +90,8 @@ def make_packed_tables(parts, device, morph_count: Optional[float] = None) -> Gr
     batch is the mean over morphologies of the reference's per-morphology loss (the reference steps the morphologies one
     after the other, src/trainer.py:245-250; SURVEY.md §8f rank 1).  morph_count (default: len(parts)) replaces
     #morphologies in the weight: a data-parallel rank that holds n_r of n morphologies passes n / world, so that the
-    all-reduced sum / world is the mean over ALL n morphologies whatever the split (bench.py --set, N > 1)."""
+    all-reduced sum / world is the mean over ALL n morphologies whatever the split (bench.py --set, N > 1).
+    `part_table` holds each morphology's token and graph span for the per-morphology statistics (sgrl_td3_part_stats)."""
     cu, rank3, tokg, rel, reloff, w, spans = [0], [], [], [], [], [], []
     t0 = g0 = ro = 0
     m = len(parts)
@@ -108,7 +110,8 @@ def make_packed_tables(parts, device, morph_count: Optional[float] = None) -> Gr
     i32 = lambda x: torch.as_tensor(x, dtype=torch.int32).to(device).contiguous()
     return GraphTables(i32(cu), torch.cat(rank3).to(device).contiguous(), torch.cat(tokg).to(torch.int32).to(device).contiguous(),
                        torch.cat(rel).to(device).contiguous(), i32(reloff), t0, g0,
-                       tok_weight=torch.cat(w).to(device).contiguous() if (m > 1 or mw != 1.0) else None, parts=spans)
+                       tok_weight=torch.cat(w).to(device).contiguous() if (m > 1 or mw != 1.0) else None, parts=spans,
+                       part_table=i32([s[:4] for s in spans]))
 
 
 _VERSION_OF = operator.attrgetter("_version")

@@ -245,12 +245,14 @@ class SeedBatchedAgent(Agent):
 
         return self._run_update(tb, None, it, None, loader=load)
 
-    def update_packed_per_seed(self, batches_per_seed, it: int, noises=None, morph_count: Optional[float] = None):
+    def update_packed_per_seed(self, batches_per_seed, it: int, noises=None, morph_count: Optional[float] = None,
+                               per_morphology: bool = False):
         """``Agent.update_packed`` of every seed in ONE captured step: batches_per_seed[k] is what seed k's own agent would pass
         to update_packed, [(graph_dict, data_batch), ...].  The seeds share the morphologies (the same parents in the same
         order) and the batch size of each; seed 0's graph dicts build the packed tables.  noises: None or K lists of one
         (B_i, 3 N_i) tensor per morphology.  Returns K loss dicts; seed k's loss is the mean over its morphologies, as in
-        update_packed.  morph_count: as in ``Agent.update_packed`` (data parallelism)."""
+        update_packed.  morph_count and per_morphology: as in ``Agent.update_packed`` (data parallelism; seed k's
+        "per_morphology" list holds seed k's own values, its rewards scaled by its own reward_scale)."""
         graphs = self._check_seed_morphologies(batches_per_seed, "batches_per_seed")
         specs = [(g, int(b["obs"].shape[0])) for g, b in batches_per_seed[0]]
         for k, parts in enumerate(batches_per_seed):
@@ -260,16 +262,17 @@ class SeedBatchedAgent(Agent):
                                      f"every seed needs the same batch size per morphology")
         flat_noises = self._seed_noises(noises, len(graphs))
         tb = self._packed_tables_for(specs, morph_count)
-        return self._run_update(tb, [b for parts in batches_per_seed for _, b in parts], it, flat_noises)
+        return self._run_update(tb, [b for parts in batches_per_seed for _, b in parts], it, flat_noises, per_morphology=per_morphology)
 
     def update_packed_from_buffers_per_seed(self, parts_per_seed, batch_size: int, it: int, noises=None,
-                                            morph_count: Optional[float] = None, sequential: bool = False, allow_duplicate: bool = False):
+                                            morph_count: Optional[float] = None, sequential: bool = False, allow_duplicate: bool = False,
+                                            per_morphology: bool = False):
         """``update_packed_per_seed([[(g, buf.sample(batch_size)) for g, buf in parts] for parts in parts_per_seed], ...)``
         without materialising the batches: parts_per_seed[k] = [(graph_dict, ReplayBuffer), ...] is seed k's device buffer of
         each morphology.  The indices are drawn with ``buf.draw_indices`` seed after seed, buffer after buffer (the draws of K
         agents calling ``update_packed_from_buffers`` in seed order), sent as ONE H2D copy, and ONE gather launch
         (``gather_seeds_into``) writes every seed's rows into its block of the step's static inputs.  Per step: one copy and
-        one library launch outside the graph.  The plan is update_packed_per_seed's."""
+        one library launch outside the graph.  The plan is update_packed_per_seed's, and so is per_morphology."""
         from .buffer import check_seed_buffers, gather_seeds_into
         graphs = self._check_seed_morphologies(parts_per_seed, "parts_per_seed")
         flat_noises = self._seed_noises(noises, len(graphs))
@@ -298,7 +301,7 @@ class SeedBatchedAgent(Agent):
                               plan.rew, plan.done, idx_dev=plan.i_dev)
             return plan.load_noise(flat_noises)
 
-        return self._run_update(tb, None, it, None, loader=load)
+        return self._run_update(tb, None, it, None, loader=load, per_morphology=per_morphology)
 
     def _check_seed_morphologies(self, parts_per_seed, what: str):
         """One list of (graph_dict, data) per seed, 1..MAX_PACKED_PARTS of them, the same morphologies in the same order for

@@ -37,11 +37,13 @@ MORPH = "3d_humanoid_9_full"
 def time_arms(arms, steps, rounds, it, before_window=None):
     """The alternated A/B timing of the seed benchmarks: arms = {name: (fn, agents)}, fn() one step of the arm (reading it[0],
     which is bumped after every step).  Per arm and round: device ms per step between CUDA events around `steps` steps followed
-    by a synchronise, and the library kernels executed per step (through graph replays and outside them).  before_window(name),
-    if given, runs untimed before each window.  Returns {name: {"device_ms", "kernels_per_step", "device_ms_median"}}."""
+    by a synchronise, wall ms per step on the host clock around the same window (synchronise included), and the library
+    kernels executed per step (through graph replays and outside them).  before_window(name), if given, runs untimed before
+    each window.  Returns {name: {"device_ms", "wall_ms", "kernels_per_step", "device_ms_median", "wall_ms_median"}}."""
+    import time
     import torch
     from sgrl_b200._lib import lib
-    res = {k: {"device_ms": [], "kernels_per_step": []} for k in arms}
+    res = {k: {"device_ms": [], "wall_ms": [], "kernels_per_step": []} for k in arms}
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for _ in range(rounds):
         for name, (fn, ags) in arms.items():
@@ -49,16 +51,20 @@ def time_arms(arms, steps, rounds, it, before_window=None):
                 before_window(name)
             torch.cuda.synchronize()
             l0 = lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags)
+            w0 = time.perf_counter()
             ev0.record()
             for _ in range(steps):
                 fn(); it[0] += 1
             ev1.record()
             torch.cuda.synchronize()
+            w1 = time.perf_counter()
             r = res[name]
             r["device_ms"].append(round(ev0.elapsed_time(ev1) / steps, 4))
+            r["wall_ms"].append(round((w1 - w0) * 1e3 / steps, 4))
             r["kernels_per_step"].append((lib.sgrl_launch_count() + sum(a.graph_replayed_launches for a in ags) - l0) / steps)
     for r in res.values():
         r["device_ms_median"] = statistics.median(r["device_ms"])
+        r["wall_ms_median"] = statistics.median(r["wall_ms"])
     return res
 
 
