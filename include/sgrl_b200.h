@@ -7,8 +7,8 @@
  * the stub a reference maintainer would add.
  *
  * Conventions: every pointer is a DEVICE pointer to contiguous row-major fp32 (int32 for
- * indices) owned by the caller (two exceptions: the HOST descriptor arrays of
- * sgrl_replay_gather_packed and sgrl_replay_gather_seeds); the library allocates nothing, never synchronises and never
+ * indices) owned by the caller (exceptions: the HOST descriptor arrays of
+ * sgrl_replay_gather_packed, sgrl_replay_gather_seeds and sgrl_seed_copy); the library allocates nothing, never synchronises and never
  * throws.  Every call enqueues work on the given cudaStream_t (pass
  * torch.cuda.current_stream().cuda_stream) and returns 0, or a negative code with a
  * thread-local message in sgrl_last_error().  Calls are re-entrant per stream.
@@ -305,6 +305,18 @@ int sgrl_replay_gather_packed(const SgrlReplayPart* parts, int n_parts, const in
  * seed k's rows start at k x the per-seed totals: the block of seed k in a seed-batched update's inputs. */
 int sgrl_replay_gather_seeds(const SgrlReplayPart* parts, int n_parts, int n_seeds, const int64_t* idx, float* obs, float* action,
                              float* next_obs, float* reward, float* done, sgrl_stream_t stream);
+
+/* ---- population-based training (SeedBatchedAgent.exploit) ------------------------------------ */
+/* One per-seed state array of a seed-batched agent: nets of n_net floats, net z at base + z * n_net.  Seed k of K owns the
+ * nets k + j*K for j < nets_per_seed (1: actors; 2: twin critics [critic1 of seeds | critic2 of seeds]). */
+typedef struct { float* base; int64_t n_net; int32_t nets_per_seed, pad_; } SgrlSeedPlane;
+/* For every pair p, copy seed src[p]'s nets onto seed dst[p]'s nets in every plane.  One launch.
+ * planes, dst and src are HOST arrays, read while the call enqueues.  Limits: 1..32 planes, 1..7 pairs.
+ * Refused with nothing enqueued: a seed index outside [0, K); dst[p] == src[p]; a repeated dst; a seed that is both a dst
+ * and a src in one call; n_net not a multiple of 4; a base that is not 16-byte aligned.  Also refused: NULL arrays or bases,
+ * K outside 1..8, n_net <= 0, nets_per_seed outside 1..2. */
+int sgrl_seed_copy(const SgrlSeedPlane* planes, int n_planes, int K, const int32_t* dst, const int32_t* src, int n_pairs,
+                   sgrl_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -53,6 +53,10 @@ class ReplayPart(C.Structure):
     ]
 
 
+class SeedPlane(C.Structure):
+    _fields_ = [("base", c_f), ("n_net", c_i64), ("nets_per_seed", C.c_int32), ("pad_", C.c_int32)]
+
+
 # One row of the per-seed TD3 table (SgrlTd3Hparams): the layout of the C struct, 48 bytes
 TD3_HPARAMS = np.dtype([("actor_lr", "<f8"), ("critic_lr", "<f8"), ("discount", "<f4"), ("reward_scale", "<f4"),
                         ("policy_noise", "<f4"), ("noise_clip", "<f4"), ("tau", "<f4"), ("one_minus_tau", "<f4"),
@@ -114,6 +118,7 @@ _PROTOS = {
     "sgrl_replay_scatter": (c_int, [c_f, c_i64, c_i64, c_f, c_f, c_int, c_f]),
     "sgrl_replay_gather_packed": (c_int, [C.POINTER(ReplayPart), c_int, c_f, c_f, c_f, c_f, c_f, c_f, c_f]),
     "sgrl_replay_gather_seeds": (c_int, [C.POINTER(ReplayPart), c_int, c_int, c_f, c_f, c_f, c_f, c_f, c_f, c_f]),
+    "sgrl_seed_copy": (c_int, [C.POINTER(SeedPlane), c_int, c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32), c_int, c_f]),
 }
 EXPORTS = tuple(_PROTOS)
 

@@ -3,6 +3,7 @@
 
 #include "net.cuh"
 #include "replay.cuh"
+#include "seed_copy.cuh"
 #include "td3.cuh"
 
 namespace sgrl {
@@ -22,7 +23,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 8; }
+int sgrl_version(void) { return 9; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -513,6 +514,36 @@ int sgrl_replay_gather_seeds(const SgrlReplayPart* parts, int n_parts, int n_see
       }
     }
   return replay_gather_parts<SGRL_REPLAY_MAX_SEED_PARTS>(parts, n_parts, idx, obs, action, next_obs, reward, done, ST(stream));
+}
+
+int sgrl_seed_copy(const SgrlSeedPlane* planes, int n_planes, int K, const int32_t* dst, const int32_t* src, int n_pairs,
+                   sgrl_stream_t stream) {
+  SGRL_CHECK(planes && dst && src, "null pointer");
+  SGRL_CHECK(n_planes >= 1 && n_planes <= SGRL_SEED_COPY_MAX_PLANES, "n_planes must be 1..32");
+  SGRL_CHECK(n_pairs >= 1 && n_pairs <= SGRL_SEED_COPY_MAX_PAIRS, "n_pairs must be 1..7");
+  SGRL_CHECK(K >= 1 && K <= MAX_NETS / 2, "K must be 1..8");
+  SeedCopyArgs a;
+  memset(&a, 0, sizeof(a));
+  int nps[SGRL_SEED_COPY_MAX_PLANES];
+  for (int i = 0; i < n_planes; ++i) {
+    const SgrlSeedPlane& q = planes[i];
+    SGRL_CHECK(q.base != nullptr, "null plane base");
+    SGRL_CHECK(aligned16(q.base), "plane base must be 16-byte aligned");
+    SGRL_CHECK(q.n_net > 0 && (q.n_net & 3) == 0, "n_net must be a positive multiple of 4");
+    SGRL_CHECK(q.nets_per_seed >= 1 && q.nets_per_seed <= 2, "nets_per_seed must be 1..2");
+    a.base[i] = q.base; a.n4[i] = q.n_net / 4; nps[i] = q.nets_per_seed;
+  }
+  for (int p = 0; p < n_pairs; ++p) {
+    SGRL_CHECK(dst[p] >= 0 && dst[p] < K && src[p] >= 0 && src[p] < K, "seed index outside [0, K)");
+    SGRL_CHECK(dst[p] != src[p], "dst == src");
+    for (int q = 0; q < n_pairs; ++q) {
+      SGRL_CHECK(q == p || dst[q] != dst[p], "repeated dst");
+      SGRL_CHECK(dst[p] != src[q], "a seed is both a dst and a src");
+    }
+    a.dst[p] = dst[p]; a.src[p] = src[p];
+  }
+  a.n_planes = n_planes; a.K = K;
+  return seed_copy(a, nps, n_pairs, ST(stream));
 }
 
 int sgrl_replay_scatter(float* rows, int64_t row_floats, int64_t capacity, const int64_t* dst, const float* staged, int n, sgrl_stream_t stream) {

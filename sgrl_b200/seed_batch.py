@@ -18,13 +18,14 @@ from __future__ import annotations
 
 import contextlib
 import copy
+import ctypes as C
 import math
 import numbers
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
 
-from ._lib import ACTOR, CRITIC
+from ._lib import ACTOR, CRITIC, SeedPlane, SgrlError, check, lib, ptr, stream
 from .agent import Agent, FusedAdam
 from .buffer import MAX_SEEDS
 from .modules import SetNetModule
@@ -74,7 +75,8 @@ class SeedBatchedAgent(Agent):
     hparams: None (every seed trains with args' values) or K dicts, dict k overriding args for seed k with any of ``lr`` and
     ``HPARAM_KEYS``.  ``get_hparams(k)`` / ``set_hparams(k, **values)`` read and change seed k's values; the step reads them
     before every update.  The Agent attributes that carry these values for a single agent (the optimizers' ``lr``,
-    ``args.discount`` and the like, ``target_smoothing_tau``, ``reward_scale``) hold seed 0's initial values and are not read."""
+    ``args.discount`` and the like, ``target_smoothing_tau``, ``reward_scale``) hold seed 0's initial values and are not read.
+    ``exploit({dst: src})`` copies whole seeds onto others in place (population-based training), without recapturing."""
 
     def __init__(self, args, seeds: Sequence[int], hparams: Optional[Sequence[Dict]] = None):
         seeds = list(seeds)
@@ -197,6 +199,85 @@ class SeedBatchedAgent(Agent):
         if hasattr(self.actor, "graph"):
             a.change_morphology(self.actor.graph)
         return a
+
+    # ------------------------------------------------------------------ population-based training
+    def exploit(self, pairs: Dict[int, int]):
+        """The exploit step of population-based training: for every dst: src of `pairs`, seed dst becomes a bit-for-bit copy of
+        seed src's training state: the online actor and twin critics (live and dead parameters), the target networks, both
+        optimizers' Adam moments, the tf32 weight splits where allocated, and the hyper-parameters (get_hparams(dst) ==
+        get_hparams(src) afterwards).  Explore with set_hparams after it.
+
+        One ``sgrl_seed_copy`` launch on the current stream, in stream order between two updates, and no host synchronisation.
+        The copies land in the arenas the plans and their captured graphs already point at, so nothing is reallocated or
+        recaptured: the next update replays the graphs it would have replayed anyway, and the changed hyper-parameter rows
+        reach the device table before it like any set_hparams change.
+        Left as they are: the replay buffers (the caller owns them), the Adam step count and tot_update_count (shared by every
+        seed) and each seed's target-policy noise stream (dst keeps drawing its own noise).  The gradient arenas, the
+        optimizers' per-net norms and the plans' buffers are not copied: every step overwrites them before reading them.
+        Data parallelism: every rank must call exploit with the same mapping (there is no collective), or the replicas
+        diverge.
+
+        ValueError, before anything changes, for: `pairs` not a dict, an index that is not an int, an index outside 0..K-1,
+        dst == src, a repeated dst, a seed that is both a dst and a src.  An empty dict does nothing.  Off CUDA: SgrlError,
+        after these checks, as for every module call without a GPU."""
+        mapping = self._check_pairs(pairs)
+        if not mapping:
+            return
+        if self.actor.full_arena.device.type != "cuda":
+            raise SgrlError("SeedBatchedAgent.exploit needs the modules on a CUDA device (no CPU fallback)")
+        planes = self._seed_planes()
+        desc = (SeedPlane * len(planes))(*(SeedPlane(ptr(t), n_net, per, 0) for t, n_net, per in planes))
+        n = len(mapping)
+        dst = (C.c_int32 * n)(*(d for d, _ in mapping))
+        src = (C.c_int32 * n)(*(s for _, s in mapping))
+        # The raw writes bump no version counter, so a tf32 split flagged fresh stays flagged fresh.  That is right: a fresh
+        # split is an elementwise function of the live parameters, and dst's hi / lo planes are copied with them.  A stale
+        # split stays flagged stale and is re-derived before its next use, as it would have been.
+        check(lib.sgrl_seed_copy(desc, len(planes), self.n_seeds, dst, src, n, stream()), "sgrl_seed_copy")
+        for d, s in mapping:
+            self._hparams[d] = dict(self._hparams[s])
+
+    def _check_pairs(self, pairs) -> List[Tuple[int, int]]:
+        """exploit's {dst: src} -> [(dst, src)], with the refusals of sgrl_seed_copy as ValueError."""
+        if not isinstance(pairs, dict):
+            raise ValueError(f"exploit: expected a {{dst: src}} dict of seed indices, got {type(pairs).__name__}")
+        out = []
+        for d, s in pairs.items():
+            for x in (d, s):
+                if isinstance(x, bool) or not isinstance(x, numbers.Integral):
+                    raise ValueError(f"exploit: seed indices must be ints, got {x!r}")
+                self._check_index(int(x))
+            if int(d) == int(s):
+                raise ValueError(f"exploit: seed {int(d)} would be copied onto itself")
+            out.append((int(d), int(s)))
+        dsts = [d for d, _ in out]
+        if len(set(dsts)) != len(dsts):
+            raise ValueError(f"exploit: a dst seed appears twice in {sorted(dsts)}")
+        both = set(dsts) & {s for _, s in out}
+        if both:
+            raise ValueError(f"exploit: seeds {sorted(both)} would both receive and give a copy in one call")
+        return out
+
+    def _seed_planes(self) -> List[Tuple[torch.Tensor, int, int]]:
+        """Every per-seed state array of the agent, each once, as the planes of sgrl_seed_copy: (tensor, n_net, nets_per_seed),
+        net z of the tensor at z * n_net floats, seed k's nets k + j*K for j < nets_per_seed.  Per module its live and its dead
+        parameters (the arena is [live nets | dead nets]) and, where allocated, the tf32 split hi and lo of the live ones; per
+        optimizer its Adam exp_avg and exp_avg_sq."""
+        K = self.n_seeds
+        for opt in (self.actor_optimizer, self.critic_optimizer):
+            opt._sync_device()              # a moved module: the moments follow it before their pointers are taken
+        planes = []
+        for m in (self.actor, self.actor_target, self.critic, self.critic_target):
+            per, L, D = m._nb // K, m._live, m._dead
+            planes.append((m.live_arena, L, per))
+            if D:
+                planes.append((m.full_arena[m._nb * L:], D, per))
+            if m._split is not None:
+                planes += [(m._split[0], L, per), (m._split[1], L, per)]
+        for opt in (self.actor_optimizer, self.critic_optimizer):
+            m = opt.module
+            planes += [(opt.exp_avg, m._live, m._nb // K), (opt.exp_avg_sq, m._live, m._nb // K)]
+        return planes
 
     # ------------------------------------------------------------------ TD3 step
     def update(self, batches, it: int, noises=None):
