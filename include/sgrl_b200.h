@@ -132,7 +132,8 @@ int sgrl_attention_bwd(const float* qkv, const float* vgp, const float* gd, cons
                        const float* relation, int G, int max_limbs, float* dqkv, float* dvgp, float* drel_w /*nullable, accumulates*/,
                        sgrl_stream_t stream);
 /* K3: C[M,N] = epi(alpha * A B^T): every nn.Linear call site (SURVEY.md Appendix G).
- * trans_a/trans_b as in csrc/gemm_simt.cuh; bias/rowdiv nullable; relu 0/1; use_tc as above. */
+ * trans_a/trans_b as in csrc/gemm_simt.cuh; bias/rowdiv nullable; relu 0/1; use_tc as above.
+ * splitk > 1 lets K be split with atomic adds into C: it requires accumulate = 1 and no bias (refused otherwise). */
 int sgrl_gemm(const float* A, int lda, int trans_a, const float* B, int ldb, int trans_b, float* C, int ldc,
               int M, int N, int K, float alpha, const float* bias, const float* rowdiv, int relu, int accumulate,
               int splitk, int use_tc, sgrl_stream_t stream);
@@ -158,6 +159,51 @@ int sgrl_gemm_gd(const float* A, int lda, const float* W_hi, const float* W_lo, 
 int sgrl_gemm_pair(const float* A0, int lda0, const float* W0_hi, const float* W0_lo, const float* b0, float* C0, int ldc0, int M0, int N0,
                    int K0, const float* A1, int lda1, const float* W1_hi, const float* W1_lo, const float* b1, float* C1, int ldc1, int M1,
                    int N1, int K1, int relu, sgrl_stream_t stream);
+/* The whole GEMM contract of the library's projections in one descriptor (kernel tests: every variant, epilogue and
+ * instance layout that csrc/net.cuh launches can be reached and checked from here).  One problem, per instance z < nb
+ * (z-stride 0 = the operand is shared by every instance; every pointer but A, B and C is nullable):
+ *   v = alpha * sum_k A(m,k) B(n,k) (+ bias[n]) -> relu -> / rowdiv[m] -> * colscale (n < colscale_n) -> mask[m][n] > 0 ? v : 0
+ *       -> + res1[m][n] + res2[m][n] -> C[m][n] = v, or C[m][n] += v (accumulate)
+ *   rowsum[m] += alpha * sum_k A(m,k); gd: columns 30, 31 of row m = 3t+r replaced by gd[t][r][0..1] (N = 32);
+ *   gram_z (M,96) set: row m of A is the packed Gram triangle of Z_m (K = 544, B pre-split), gram_f[m] = ||G_m||_F + 1,
+ *   gram_g (M,544) = the generated rows.  A(m,k), B(n,k) as in sgrl_gemm.  splitk > 1 lets the tcgen05 model split K
+ *   with atomics (requires accumulate = 1 and no bias).  B_hi/B_lo (both or neither): B pre-split, tcgen05 only. */
+typedef struct {
+  const float* A; int64_t zs_a; int32_t lda, trans_a;
+  const float* B; const float* B_hi; const float* B_lo; int64_t zs_b; int32_t ldb, trans_b;
+  float* C; int64_t zs_c; int32_t ldc, M, N, K;
+  float alpha; int32_t relu;
+  const float* bias; int64_t zs_bias;
+  const float* rowdiv; int64_t zs_rowdiv;
+  float colscale; int32_t colscale_n;
+  const float* mask; int64_t zs_mask;
+  const float* res1; int64_t zs_res1;
+  const float* res2; int64_t zs_res2;
+  int32_t ldmask, ldres1, ldres2, accumulate;
+  float* rowsum; int64_t zs_rowsum;
+  const float* gd; int64_t zs_gd;
+  const float* gram_z; int64_t zs_gram_z;   /* zs_gram_z also strides gram_f and gram_g */
+  float* gram_f; float* gram_g;
+  int32_t splitk, nb;
+} SgrlGemmProblem;
+/* n = 1..4 problems; n > 1 runs them like the networks' grouped projections (one launch when their kernel variants agree).
+ * use_tc: 0 fp32 SIMT (n = 1, no rowsum / gd / gram), 1 tcgen05 3xTF32, 2 tcgen05 BF16-input.  sm2_ok / lat: the hints the
+ * networks give the tile model (inference pass / critical chain).  Overrides of the tcgen05 planner, -1 = its model (every
+ * field -1: exactly the plan sgrl_gemm and the networks get): bn 64 | 128; split = atomic split-K factor (needs splitk > 1);
+ * csk 0 | 2 | 3 cluster split-K ranks; sm2, persist, tma_store, group 0 | 1.  An override the shape or epilogue cannot take
+ * is refused with nothing enqueued. */
+typedef struct {
+  SgrlGemmProblem pr[4];
+  int32_t n, use_tc, sm2_ok, lat;
+  int32_t bn, split, csk, sm2, persist, tma_store, group, pad_;
+} SgrlGemmDesc;
+/* What was launched, per problem.  path: 0 SIMT tile kernel, 1 skinny kernel, 2 tcgen05.  split: atomic split-K factor
+ * (sk_x: folded into blockIdx.x); cluster: cluster split-K ranks (1 = none); tma_c: TMA-store epilogue; epi: the epilogue
+ * class the tcgen05 tile kernel selects (0 plain, 1 /rowdiv (+colscale), 2 relu mask, 3 residuals, 4 accumulate, 5 split-K
+ * atomics, 6 generic, 7 [X P^T | gd]), -1 where that choice is not made (SIMT, TMA-store and persistent epilogues). */
+typedef struct { int32_t path, bn, amn, bmn, bpre, sm2, gram, persist, split, sk_x, cluster, tma_c, epi; } SgrlGemmPlan;
+typedef struct { SgrlGemmPlan pr[4]; int32_t launches, pad_; } SgrlGemmPlanInfo;
+int sgrl_gemm_desc(const SgrlGemmDesc* d, SgrlGemmPlanInfo* info /* nullable */, sgrl_stream_t stream);
 /* hi = tf32_rna(w), lo = tf32_rna(w - hi): the operand split of the 3xTF32 tensor-core projections, done once per
  * optimizer step for weights instead of once per tile load */
 int sgrl_split_tf32(const float* w, float* hi, float* lo, int64_t n, sgrl_stream_t stream);

@@ -57,6 +57,39 @@ class SeedPlane(C.Structure):
     _fields_ = [("base", c_f), ("n_net", c_i64), ("nets_per_seed", C.c_int32), ("pad_", C.c_int32)]
 
 
+class GemmProblem(C.Structure):
+    _fields_ = [
+        ("A", c_f), ("zs_a", c_i64), ("lda", C.c_int32), ("trans_a", C.c_int32),
+        ("B", c_f), ("B_hi", c_f), ("B_lo", c_f), ("zs_b", c_i64), ("ldb", C.c_int32), ("trans_b", C.c_int32),
+        ("C", c_f), ("zs_c", c_i64), ("ldc", C.c_int32), ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32),
+        ("alpha", C.c_float), ("relu", C.c_int32),
+        ("bias", c_f), ("zs_bias", c_i64), ("rowdiv", c_f), ("zs_rowdiv", c_i64),
+        ("colscale", C.c_float), ("colscale_n", C.c_int32),
+        ("mask", c_f), ("zs_mask", c_i64), ("res1", c_f), ("zs_res1", c_i64), ("res2", c_f), ("zs_res2", c_i64),
+        ("ldmask", C.c_int32), ("ldres1", C.c_int32), ("ldres2", C.c_int32), ("accumulate", C.c_int32),
+        ("rowsum", c_f), ("zs_rowsum", c_i64), ("gd", c_f), ("zs_gd", c_i64),
+        ("gram_z", c_f), ("zs_gram_z", c_i64), ("gram_f", c_f), ("gram_g", c_f),
+        ("splitk", C.c_int32), ("nb", C.c_int32),
+    ]
+
+
+class GemmDesc(C.Structure):
+    _fields_ = [("pr", GemmProblem * 4), ("n", C.c_int32), ("use_tc", C.c_int32), ("sm2_ok", C.c_int32), ("lat", C.c_int32),
+                ("bn", C.c_int32), ("split", C.c_int32), ("csk", C.c_int32), ("sm2", C.c_int32), ("persist", C.c_int32),
+                ("tma_store", C.c_int32), ("group", C.c_int32), ("pad_", C.c_int32)]
+
+
+GEMM_PLAN_FIELDS = ("path", "bn", "amn", "bmn", "bpre", "sm2", "gram", "persist", "split", "sk_x", "cluster", "tma_c", "epi")
+
+
+class GemmPlan(C.Structure):
+    _fields_ = [(f, C.c_int32) for f in GEMM_PLAN_FIELDS]
+
+
+class GemmPlanInfo(C.Structure):
+    _fields_ = [("pr", GemmPlan * 4), ("launches", C.c_int32), ("pad_", C.c_int32)]
+
+
 # One row of the per-seed TD3 table (SgrlTd3Hparams): the layout of the C struct, 48 bytes
 TD3_HPARAMS = np.dtype([("actor_lr", "<f8"), ("critic_lr", "<f8"), ("discount", "<f4"), ("reward_scale", "<f4"),
                         ("policy_noise", "<f4"), ("noise_clip", "<f4"), ("tau", "<f4"), ("one_minus_tau", "<f4"),
@@ -91,6 +124,7 @@ _PROTOS = {
     "sgrl_gemm_gd": (c_int, [c_f, c_int, c_f, c_f, c_int, c_f, c_f, c_int, c_int, c_f]),
     "sgrl_gemm_pair": (c_int, [c_f, c_int, c_f, c_f, c_f, c_f, c_int, c_int, c_int, c_int, c_f, c_int, c_f, c_f, c_f, c_f, c_int, c_int,
                                c_int, c_int, c_int, c_f]),
+    "sgrl_gemm_desc": (c_int, [C.POINTER(GemmDesc), C.POINTER(GemmPlanInfo), c_f]),
     "sgrl_split_tf32": (c_int, [c_f, c_f, c_f, c_i64, c_f]),
     "sgrl_td3_smooth_action": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, c_i64, c_f]),
     "sgrl_td3_smooth_action_rng": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, C.c_float, c_i64, C.c_uint64, c_f, c_f]),

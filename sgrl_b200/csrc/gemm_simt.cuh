@@ -27,7 +27,7 @@ struct GemmP {
   const float* res1; long long zsR1; int ldr1;      // + res1[m][n]
   const float* res2; long long zsR2; int ldr2;      // + res2[m][n]
   int accumulate;                           // C += v instead of C = v
-  int splitk;                               // >1: split K over blockIdx.y, atomicAdd (implies accumulate)
+  int splitk;                               // >1: K may be split, partial sums atomically added into C (needs accumulate, no bias)
   int nb;                                   // instances (blockIdx.z)
   int vecA, vecB;                           // set by the launcher: operand rows may be fetched as float4
   const float* Bhi; const float* Blo;       // tcgen05 path only, optional: B pre-split into tf32 hi/lo parts (same layout/strides as B)
@@ -278,6 +278,7 @@ inline int gemm_simt(const GemmP& p_in, cudaStream_t st) {
   SGRL_CHECK(p.splitk >= 1, "gemm: splitk");
   SGRL_CHECK(p.splitk == 1 || (!p.relu && !p.rowdiv && !p.mask && !p.res1 && !p.res2 && p.colscale_n == 0),
              "gemm: split-K only with a linear epilogue");
+  SGRL_CHECK(p.splitk == 1 || (p.accumulate && !p.bias), "gemm: split-K needs accumulate = 1 and no bias");   // as the tcgen05 path
   if (gemm_skinny_eligible(p)) return gemm_skinny(p, st);
   const int tiles = ceil_div(p.M, GB_M) * ceil_div(p.N, GB_N);
   dim3 grid(tiles, p.splitk, p.nb);

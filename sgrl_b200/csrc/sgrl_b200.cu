@@ -23,7 +23,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 9; }
+int sgrl_version(void) { return 10; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -176,6 +176,7 @@ int sgrl_gemm(const float* A, int lda, int trans_a, const float* B, int ldb, int
   GemmP g = gemm_defaults();
   g.A = A; g.lda = lda; g.transA = trans_a; g.B = B; g.ldb = ldb; g.transB = trans_b; g.C = C; g.ldc = ldc;
   g.M = M; g.N = N; g.K = K; g.alpha = alpha; g.bias = bias; g.rowdiv = rowdiv; g.relu = relu; g.accumulate = accumulate;
+  SGRL_CHECK(splitk <= 1 || (accumulate && !bias), "splitk > 1 needs accumulate = 1 and no bias");
   g.splitk = (splitk < 1 || det_enabled()) ? 1 : splitk;
   if (use_tc) {
     SGRL_CHECK(gemm_tc_eligible(g), "shape/epilogue not eligible for the tcgen05 path");
@@ -192,10 +193,67 @@ int sgrl_gemm_presplit(const float* A, int lda, int trans_a, const float* B_hi, 
   GemmP g = gemm_defaults();
   g.A = A; g.lda = lda; g.transA = trans_a; g.B = B_hi; g.Bhi = B_hi; g.Blo = B_lo; g.ldb = ldb; g.transB = trans_b; g.C = C; g.ldc = ldc;
   g.M = M; g.N = N; g.K = K; g.alpha = alpha; g.bias = bias; g.rowdiv = rowdiv; g.relu = relu; g.accumulate = accumulate;
+  SGRL_CHECK(splitk <= 1 || (accumulate && !bias), "splitk > 1 needs accumulate = 1 and no bias");
   g.splitk = (splitk < 1 || det_enabled()) ? 1 : splitk;
   SGRL_CHECK(gemm_tc_eligible(g), "shape/epilogue not eligible for the tcgen05 path");
   return gemm_tc(g, ST(stream));
 }
+
+int sgrl_gemm_desc(const SgrlGemmDesc* d, SgrlGemmPlanInfo* info, sgrl_stream_t stream) {
+  SGRL_CHECK(d != nullptr, "null descriptor");
+  SGRL_CHECK(d->n >= 1 && d->n <= TC_MAXG, "gemm_desc: 1..4 problems");
+  SGRL_CHECK(d->use_tc >= 0 && d->use_tc <= 2, "gemm_desc: use_tc must be 0, 1 or 2");
+  GemmP g[TC_MAXG];
+  for (int i = 0; i < d->n; ++i) {
+    const SgrlGemmProblem& s = d->pr[i];
+    SGRL_CHECK((s.A || s.gram_z) && s.B && s.C, "gemm_desc: null A, B or C");
+    SGRL_CHECK(s.M >= 0 && s.N >= 0 && s.K >= 1 && s.nb >= 1 && s.nb <= 64, "gemm_desc: M, N >= 0, K >= 1, nb 1..64");
+    SGRL_CHECK(s.splitk >= 1 && s.splitk <= 64, "gemm_desc: splitk 1..64");
+    SGRL_CHECK(s.splitk == 1 || (s.accumulate && !s.bias), "gemm_desc: splitk > 1 needs accumulate = 1 and no bias");
+    SGRL_CHECK((s.B_hi == nullptr) == (s.B_lo == nullptr), "gemm_desc: B_hi and B_lo go together");
+    SGRL_CHECK(!s.gram_z || !s.A, "gemm_desc: A and gram_z exclude each other");
+    SGRL_CHECK(s.gram_z || (!s.gram_f && !s.gram_g), "gemm_desc: gram_f / gram_g need gram_z");
+    GemmP& p = g[i];
+    p = gemm_defaults();
+    p.A = s.A; p.zsA = s.zs_a; p.lda = s.lda; p.transA = s.trans_a != 0;
+    p.B = s.B_hi ? s.B_hi : s.B; p.Bhi = s.B_hi; p.Blo = s.B_lo; p.zsB = s.zs_b; p.ldb = s.ldb; p.transB = s.trans_b != 0;
+    p.C = s.C; p.zsC = s.zs_c; p.ldc = s.ldc; p.M = s.M; p.N = s.N; p.K = s.K; p.nb = s.nb;
+    p.alpha = s.alpha; p.relu = s.relu != 0; p.bias = s.bias; p.zsBias = s.zs_bias; p.rowdiv = s.rowdiv; p.zsRow = s.zs_rowdiv;
+    p.colscale = s.colscale; p.colscale_n = s.colscale_n;
+    p.mask = s.mask; p.zsMask = s.zs_mask; p.ldmask = s.ldmask;
+    p.res1 = s.res1; p.zsR1 = s.zs_res1; p.ldr1 = s.ldres1; p.res2 = s.res2; p.zsR2 = s.zs_res2; p.ldr2 = s.ldres2;
+    p.accumulate = s.accumulate != 0; p.splitk = det_enabled() ? 1 : s.splitk;
+    p.rowsum = s.rowsum; p.zsRowsum = s.zs_rowsum; p.gdcols = s.gd; p.zsGd = s.zs_gd;
+    p.gramZ = s.gram_z; p.zsGramZ = s.zs_gram_z; p.gramF = s.gram_f; p.gramG = s.gram_g;
+    p.sm2_ok = d->sm2_ok != 0; p.lat = d->lat != 0; p.prec = d->use_tc == 2 ? 1 : 0;
+  }
+  TcPlanInfo rep[TC_MAXG];
+  memset(rep, 0, sizeof(rep));
+  int launches = 1;
+  if (d->use_tc == 0) {
+    const GemmP& p = g[0];
+    SGRL_CHECK(d->n == 1, "gemm_desc: the SIMT kernels take one problem");
+    SGRL_CHECK(!p.Bhi && !p.rowsum && !p.gdcols && !p.gramZ, "gemm_desc: B_hi/B_lo, rowsum, gd and gram_z need the tcgen05 path");
+    SGRL_CHECK(d->bn == -1 && d->split == -1 && d->csk == -1 && d->sm2 == -1 && d->persist == -1 && d->tma_store == -1 && d->group == -1,
+               "gemm_desc: planner overrides need the tcgen05 path");
+    rep[0] = TcPlanInfo{gemm_skinny_eligible(p) ? 1 : 0, GB_N, p.transA, p.transB, 0, 0, 0, 0, p.splitk, 0, 1, 0, -1};
+    SGRL_TRY(gemm_simt(p, ST(stream)));
+  } else {
+    for (int i = 0; i < d->n; ++i)
+      SGRL_CHECK(g[i].M == 0 || g[i].N == 0 || gemm_tc_eligible(g[i]), "gemm_desc: shape/operands not eligible for the tcgen05 path");
+    TcForce f;
+    f.bn = d->bn; f.split = d->split; f.csk = d->csk; f.sm2 = d->sm2; f.persist = d->persist; f.tma_store = d->tma_store; f.group = d->group;
+    if (d->n == 1) SGRL_TRY(gemm_tc_ex(g[0], f, rep, ST(stream)));
+    else SGRL_TRY(gemm_tc_group_ex(g, d->n, f, rep, &launches, ST(stream)));
+  }
+  if (info) {
+    memset(info, 0, sizeof(*info));
+    for (int i = 0; i < d->n; ++i) memcpy(&info->pr[i], &rep[i], sizeof(SgrlGemmPlan));
+    info->launches = launches;
+  }
+  return 0;
+}
+static_assert(sizeof(SgrlGemmPlan) == sizeof(TcPlanInfo), "SgrlGemmPlan mirrors TcPlanInfo");
 
 int sgrl_gemm_gram(const float* Z, const float* W_hi, const float* W_lo, const float* bias, float* C, int ldc, float* F, float* G,
                    int T, int N, int relu, sgrl_stream_t stream) {

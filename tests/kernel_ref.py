@@ -1,5 +1,5 @@
-"""fp64 references of the attention core (K2) and the invariant features (K1) in the packed token layout of the C ABI
-(include/sgrl_b200.h: sgrl_attention_fwd/bwd, sgrl_inv_feature_fwd/bwd).
+"""fp64 references of the attention core (K2), the invariant features (K1) and the projections (K3) in the layouts of the C ABI
+(include/sgrl_b200.h: sgrl_attention_fwd/bwd, sgrl_inv_feature_fwd/bwd, sgrl_gemm_desc).
 
 Plain torch, no CUDA needed; every function computes in float64 on the device its inputs live on.  They restate
 subequivariant_attentions.py:90-151 of the reference for packed variable-size graphs (token t = limb t - cu_limbs[g] of
@@ -116,3 +116,96 @@ def inv_feature_bwd_ref(dGp, dF, Z):
         loss = (dGp.double().reshape(-1, GP_K)[:, slots] * G[:, ri, ci]).sum() + (dF.double().reshape(-1) * F).sum()
         (dz,) = torch.autograd.grad(loss, z)
     return dz
+
+
+def bf16_round(x):
+    """fp32 values rounded to bf16 with round-to-nearest-even (what the BF16-input mode feeds the tensor core), as fp64."""
+    return x.float().to(torch.bfloat16).double()
+
+
+def _mat(buf, off, rows, cols, ld, trans=False):
+    """(rows, cols) matrix view of a flat buffer at element offset off: X[r][c] = buf[off + r*ld + c], or buf[off + c*ld + r]
+    when trans."""
+    return buf.as_strided((rows, cols), (1, ld) if trans else (ld, 1), off)
+
+
+def gemm_ref(pr, bf16=False):
+    """One SgrlGemmProblem of sgrl_gemm_desc in fp64.  pr: dict with the descriptor's fields, each pointer a flat tensor (or
+    None) holding all nb instances at z * zs.  For every instance z:
+
+        v = alpha * A B^T + bias -> relu -> / rowdiv -> * colscale (n < colscale_n) -> mask > 0 ? v : 0 -> + res1 + res2
+        C = v, or C += v (accumulate);  columns 30, 31 of row m = 3t+r are gd[t][r][0..1] instead (gd)
+        rowsum += alpha * sum_k A;  gram_z: row m of A = packed triangle of G_m = Z_m^T Z_m, gram_f = ||G_m||_F + 1, gram_g = rows
+
+    (the order of gemm_simt_kernel's epilogue).  bf16: A and B rounded to bf16 (RN-even) before the product (B from B_hi when
+    given: the kernel rounds the weights' hi part); rowsum sums the unrounded A.  Returns {name: (value, bound, written)}
+    for C, rowsum, gram_f, gram_g: fp64 copies of the whole buffers with the computed entries replaced, a bound on each
+    entry's magnitude built from the operands' absolute values (the scale of its rounding error) and the mask of the
+    entries the call writes.  Everything else in a buffer must come back bit-identical."""
+    M, N, K, nb = pr["M"], pr["N"], pr["K"], pr["nb"]
+    d = {k: (v.detach().double().reshape(-1) if torch.is_tensor(v) else v) for k, v in pr.items()}
+    out = {}
+    for name in ("C", "rowsum", "gram_f", "gram_g"):
+        if d.get(name) is not None:
+            out[name] = (d[name].clone(), torch.zeros_like(d[name]), torch.zeros_like(d[name], dtype=torch.bool))
+    Bsrc = d["B_hi"] if bf16 and d.get("B_hi") is not None else d["B"]
+    alpha = float(pr.get("alpha", 1.0))
+    with torch.no_grad():
+        for z in range(nb):
+            if d.get("gram_z") is not None:
+                Z = _mat(d["gram_z"], z * d["zs_gram_z"], M, 96, 96).reshape(M, 3, 32)
+                G, A = gram_packed(Z)
+                F = (torch.linalg.matrix_norm(G) + 1.0)[:, None]
+                for name, val, mag in (("gram_f", F, F), ("gram_g", A, gram_packed(Z.abs())[1])):
+                    if name in out:
+                        w = val.shape[1]
+                        _mat(out[name][0], z * d["zs_gram_z"], M, w, w).copy_(val)
+                        _mat(out[name][1], z * d["zs_gram_z"], M, w, w).copy_(mag)
+                        _mat(out[name][2], z * d["zs_gram_z"], M, w, w).fill_(True)
+            else:
+                A = _mat(d["A"], z * d["zs_a"], M, K, d["lda"], bool(pr["trans_a"]))
+            B = _mat(Bsrc, z * d["zs_b"], N, K, d["ldb"], bool(pr["trans_b"]))
+            if "rowsum" in out:
+                rs, rb, rw = out["rowsum"]
+                o = z * d["zs_rowsum"]
+                rb[o:o + M] = rs[o:o + M].abs() + abs(alpha) * A.abs().sum(1)
+                rs[o:o + M] += alpha * A.sum(1)
+                rw[o:o + M] = True
+            Aq, Bq = (bf16_round(A), bf16_round(B)) if bf16 else (A, B)
+            v = alpha * (Aq @ Bq.T)
+            mag = abs(alpha) * (Aq.abs() @ Bq.abs().T)
+            if d.get("bias") is not None:
+                b = d["bias"][z * d["zs_bias"]: z * d["zs_bias"] + N]
+                v = v + b
+                mag = mag + b.abs()
+            if pr.get("relu"):
+                v = v.clamp_min(0.0)
+            if d.get("rowdiv") is not None:
+                r = d["rowdiv"][z * d["zs_rowdiv"]: z * d["zs_rowdiv"] + M, None]
+                v = v / r
+                mag = mag / r.abs()
+            cn = min(int(pr.get("colscale_n", 0)), N)
+            if cn > 0:
+                cs = float(pr.get("colscale", 1.0))
+                v[:, :cn] *= cs
+                mag[:, :cn] *= abs(cs)
+            if d.get("mask") is not None:
+                v = torch.where(_mat(d["mask"], z * d["zs_mask"], M, N, d["ldmask"]) > 0, v, torch.zeros_like(v))
+            for res, zs, ld in (("res1", "zs_res1", "ldres1"), ("res2", "zs_res2", "ldres2")):
+                if d.get(res) is not None:
+                    t = _mat(d[res], z * d[zs], M, N, d[ld])
+                    v = v + t
+                    mag = mag + t.abs()
+            c, cb, cw = out["C"]
+            dst = _mat(c, z * d["zs_c"], M, N, d["ldc"])
+            if pr.get("accumulate"):
+                mag = mag + dst.abs()
+                v = dst + v
+            if d.get("gd") is not None:
+                gd = d["gd"][z * d["zs_gd"]: z * d["zs_gd"] + 2 * M].reshape(M, 2)
+                v[:, 30:32] = gd if not pr.get("accumulate") else dst[:, 30:32] + gd
+                mag[:, 30:32] = v[:, 30:32].abs()
+            dst.copy_(v)
+            _mat(cb, z * d["zs_c"], M, N, d["ldc"]).copy_(mag)
+            _mat(cw, z * d["zs_c"], M, N, d["ldc"]).fill_(True)
+    return out

@@ -110,3 +110,60 @@ def test_modules_build_on_cpu_with_reference_state_dict_keys():
             a(torch.zeros(1, 82))
     with pytest.raises(NotImplementedError):
         SEPolicy(41, 3, 32, 100, 1.0, None, False, False, False, ref_loader.default_args(attention_heads=4))
+
+
+def _desc(**over):
+    """A one-problem sgrl_gemm_desc descriptor on fake (never dereferenced) 16-byte aligned addresses: 2304 x 256 x 64, pre-split
+    B, tcgen05 path, every planner override at -1 (the model)."""
+    from sgrl_b200 import _lib
+    d = _lib.GemmDesc()
+    p = d.pr[0]
+    p.A, p.lda, p.B, p.B_hi, p.B_lo, p.ldb, p.C, p.ldc = 1 << 20, 64, 2 << 20, 3 << 20, 4 << 20, 64, 5 << 20, 256
+    p.M, p.N, p.K, p.alpha, p.colscale, p.splitk, p.nb = 2304, 256, 64, 1.0, 1.0, 1, 1
+    d.n, d.use_tc = 1, 1
+    for f in ("bn", "split", "csk", "sm2", "persist", "tma_store", "group"):
+        setattr(d, f, -1)
+    for k, v in over.items():
+        setattr(d if hasattr(d, k) else p, k, v)
+    return d
+
+
+@pytest.mark.parametrize("over,msg", [
+    (dict(bias=6 << 20, splitk=4, accumulate=1), b"no bias"),                    # the atomic split-K epilogue carries no bias
+    (dict(splitk=4, accumulate=0), b"accumulate = 1"),                           # partial sums are added into C
+    (dict(csk=3), b"without k-blocks"),                                          # K = 64: 2 k-blocks for 3 ranks
+    (dict(csk=1), b"csk override"),
+    (dict(bn=96), b"bn override"),
+    (dict(split=4), b"split override needs splitk > 1"),
+    (dict(persist=1, rowsum=6 << 20), b"persistent kernels cannot"),
+    (dict(tma_store=1, accumulate=1), b"TMA-store epilogue cannot"),
+    (dict(sm2=1, trans_a=1, lda=2304), b"two-CTAs-per-SM variant cannot"),
+    (dict(sm2=1, persist=1), b"exclude each other"),
+    (dict(group=1), b"several problems"),
+    (dict(use_tc=0, bn=64), b"need the tcgen05 path"),
+    (dict(use_tc=0, rowsum=6 << 20), b"need the tcgen05 path"),
+    (dict(n=5), b"1..4 problems"),
+    (dict(B_lo=0), b"go together"),
+    (dict(M=64, N=128, K=255), b"not eligible"),                                 # M N K < 2^21: launch-bound sizes stay on SIMT
+])
+def test_gemm_desc_refuses_invalid_descriptors(over, msg):
+    """sgrl_gemm_desc refuses a descriptor its kernels cannot run, or an override the problem cannot take, before anything is
+    enqueued (fake addresses: a call that got as far as a launch would fault, so a refusal is the only way to pass here)."""
+    from sgrl_b200 import _lib
+    lib = _lib.lib
+    rc = lib.sgrl_gemm_desc(ctypes.byref(_desc(**over)), None, None)
+    assert rc < 0 and msg in lib.sgrl_last_error(), lib.sgrl_last_error()
+
+
+def test_gemm_refuses_bias_or_store_with_split_k():
+    """splitk > 1 lets K be split with atomic adds into C: sgrl_gemm and sgrl_gemm_presplit refuse it with a bias or without
+    accumulate, on both paths (the tcgen05 split epilogue used to drop the bias while the SIMT kernel added it)."""
+    from sgrl_b200 import _lib
+    lib, f = _lib.lib, 1 << 20
+    for use_tc in (0, 1):
+        assert lib.sgrl_gemm(f, 64, 1, f, 64, 1, f, 64, 30, 128, 2304, 1.0, f, None, 0, 1, 8, use_tc, None) < 0
+        assert b"no bias" in lib.sgrl_last_error()
+        assert lib.sgrl_gemm(f, 64, 1, f, 64, 1, f, 64, 30, 128, 2304, 1.0, None, None, 0, 0, 8, use_tc, None) < 0
+        assert b"accumulate = 1" in lib.sgrl_last_error()
+    assert lib.sgrl_gemm_presplit(f, 64, 1, f, f, 64, 1, f, 64, 30, 128, 2304, 1.0, f, None, 0, 1, 8, None) < 0
+    assert b"no bias" in lib.sgrl_last_error()

@@ -157,3 +157,110 @@ def test_attention_bwd_ref_finite_difference():
             e = torch.zeros_like(rw)
             e[hh, c] = h
             assert abs((L(w=rw + e) - L(w=rw - e)) / (2 * h) - dw[hh, c]) < 1e-7
+
+
+def _gemm_problem(gen, M, N, K, nb, trans_a, trans_b, accumulate, epi):
+    """Random SgrlGemmProblem of small size with every instance in its own slice of each flat buffer (z-strides padded)."""
+    def buf(n):
+        return torch.randn(n, generator=gen, dtype=torch.float64)
+    lda, ldb, ldc = (M if trans_a else K) + 3, (N if trans_b else K) + 2, N + 5
+    pr = dict(M=M, N=N, K=K, nb=nb, trans_a=trans_a, trans_b=trans_b, lda=lda, ldb=ldb, ldc=ldc, alpha=-0.75,
+              accumulate=accumulate, relu="relu" in epi, colscale=1.5, colscale_n=3 if "colscale" in epi else 0,
+              zs_a=(K if trans_a else M) * lda + 7, zs_b=(K if trans_b else N) * ldb + 1, zs_c=M * ldc + 2)
+    pr["A"], pr["B"], pr["C"] = buf(nb * pr["zs_a"]), buf(nb * pr["zs_b"]), buf(nb * pr["zs_c"])
+    pr["B_hi"] = None
+    if "bias" in epi:
+        pr["bias"], pr["zs_bias"] = buf(nb * (N + 1)), N + 1
+    if "rowdiv" in epi:
+        pr["rowdiv"], pr["zs_rowdiv"] = buf(nb * (M + 2)).abs() + 0.5, M + 2
+    for k, ld in (("mask", "ldmask"), ("res1", "ldres1"), ("res2", "ldres2")):
+        if k in epi:
+            pr[ld] = N + 1
+            pr[k], pr["zs_" + k] = buf(nb * M * (N + 1)), M * (N + 1)
+    if "rowsum" in epi:
+        pr["rowsum"], pr["zs_rowsum"] = buf(nb * (M + 3)), M + 3
+    return pr
+
+
+def _gemm_loop(pr):
+    """gemm_simt_kernel's product and epilogue restated element by element (plain Python floats), and the fused row sum."""
+    C, rs = pr["C"].clone(), (pr["rowsum"].clone() if pr.get("rowsum") is not None else None)
+    M, N, K = pr["M"], pr["N"], pr["K"]
+    for z in range(pr["nb"]):
+        def A(m, k):
+            return pr["A"][z * pr["zs_a"] + (k * pr["lda"] + m if pr["trans_a"] else m * pr["lda"] + k)].item()
+
+        def B(n, k):
+            return pr["B"][z * pr["zs_b"] + (k * pr["ldb"] + n if pr["trans_b"] else n * pr["ldb"] + k)].item()
+        for m in range(M):
+            if rs is not None:
+                rs[z * pr["zs_rowsum"] + m] += pr["alpha"] * sum(A(m, k) for k in range(K))
+            for n in range(N):
+                v = pr["alpha"] * sum(A(m, k) * B(n, k) for k in range(K))
+                if pr.get("bias") is not None:
+                    v += pr["bias"][z * pr["zs_bias"] + n].item()
+                if pr["relu"]:
+                    v = max(v, 0.0)
+                if pr.get("rowdiv") is not None:
+                    v = v / pr["rowdiv"][z * pr["zs_rowdiv"] + m].item()
+                if n < pr["colscale_n"]:
+                    v *= pr["colscale"]
+                if pr.get("mask") is not None:
+                    v = v if pr["mask"][z * pr["zs_mask"] + m * pr["ldmask"] + n].item() > 0 else 0.0
+                for r in ("res1", "res2"):
+                    if pr.get(r) is not None:
+                        v += pr[r][z * pr["zs_" + r] + m * pr["ld" + r] + n].item()
+                c = z * pr["zs_c"] + m * pr["ldc"] + n
+                C[c] = C[c] + v if pr["accumulate"] else v
+    return C, rs
+
+
+@pytest.mark.parametrize("trans_a,trans_b", [(0, 0), (0, 1), (1, 1), (1, 0)])
+@pytest.mark.parametrize("epi", [(), ("bias", "relu"), ("bias", "relu", "rowdiv", "colscale"), ("mask", "res1", "res2"),
+                                 ("bias", "rowdiv", "colscale", "mask", "res1", "rowsum")])
+@pytest.mark.parametrize("accumulate", [0, 1])
+def test_gemm_ref_matches_simt_epilogue_loop(trans_a, trans_b, epi, accumulate):
+    """gemm_ref (the reference of the K3 kernel tests) against a plain loop over gemm_simt_kernel's epilogue order, two
+    instances with their own slices of every operand, leading dimensions past N and K."""
+    gen = torch.Generator().manual_seed(len(epi) * 8 + trans_a * 4 + trans_b * 2 + accumulate)
+    pr = _gemm_problem(gen, 5, 6, 7, 2, trans_a, trans_b, accumulate, epi)
+    out = R.gemm_ref(pr)
+    C, rs = _gemm_loop(pr)
+    assert rel(out["C"][0], C) < TOL
+    written = out["C"][2]
+    assert torch.equal(out["C"][0][~written], pr["C"][~written])          # nothing outside the instances' M x N blocks
+    assert int(written.sum()) == 2 * 5 * 6
+    assert bool((out["C"][1][written] > 0).all())
+    if rs is not None:
+        assert rel(out["rowsum"][0], rs) < TOL and int(out["rowsum"][2].sum()) == 2 * 5
+
+
+def test_gemm_ref_bf16_rounds_operands_nearest_even():
+    a = torch.tensor([1.0 + 2.0 ** -8, 1.0 + 3 * 2.0 ** -8, 1.0 + 2.0 ** -9], dtype=torch.float64)
+    assert R.bf16_round(a).tolist() == [1.0, 1.0 + 2.0 ** -6, 1.0]       # ties to even, below half down
+
+
+def test_gemm_ref_gram_rows_follow_pack_indices():
+    """With gram_z, row m of A is the packed upper triangle of G_m = Z_m^T Z_m in the slots of packing.pack_indices() (the
+    16 padding slots zero), gram_f = ||G_m||_F + 1 and gram_g the rows, per instance at z * zs_gram_z."""
+    from sgrl_b200.packing import GP_K, pack_indices
+    gen = torch.Generator().manual_seed(5)
+    M, N, nb, zs = 3, 4, 2, 3 * GP_K + 8
+    Z = torch.randn(nb * zs, generator=gen, dtype=torch.float64)
+    W = torch.randn(N * GP_K, generator=gen, dtype=torch.float64)
+    pr = dict(M=M, N=N, K=GP_K, nb=nb, trans_a=0, trans_b=0, ldb=GP_K, ldc=N, zs_b=0, zs_c=M * N, alpha=1.0, accumulate=0,
+              A=None, B=W, B_hi=None, C=torch.zeros(nb * M * N, dtype=torch.float64), gram_z=Z, zs_gram_z=zs,
+              gram_f=torch.zeros(nb * zs, dtype=torch.float64), gram_g=torch.zeros(nb * zs, dtype=torch.float64))
+    out = R.gemm_ref(pr)
+    slots, ri, ci = pack_indices()
+    for z in range(nb):
+        for m in range(M):
+            Zm = Z[z * zs + m * 96: z * zs + (m + 1) * 96].reshape(3, 32)
+            G = Zm.T @ Zm
+            row = torch.zeros(GP_K, dtype=torch.float64)
+            for s, i, j in zip(slots, ri, ci):
+                row[s] = G[i, j]
+            assert rel(out["gram_g"][0][z * zs + m * GP_K: z * zs + (m + 1) * GP_K], row) < TOL
+            assert abs(out["gram_f"][0][z * zs + m].item() - (G.norm().item() + 1.0)) < 1e-12 * G.norm().item()
+            assert rel(out["C"][0][z * M * N + m * N: z * M * N + (m + 1) * N], W.reshape(N, GP_K) @ row) < TOL
+    assert len(set(slots)) == 528
