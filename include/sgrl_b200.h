@@ -8,7 +8,7 @@
  *
  * Conventions: every pointer is a DEVICE pointer to contiguous row-major fp32 (int32 for
  * indices) owned by the caller (exceptions: the HOST descriptor arrays of
- * sgrl_replay_gather_packed, sgrl_replay_gather_seeds and sgrl_seed_copy); the library allocates nothing, never synchronises and never
+ * sgrl_replay_gather_packed, sgrl_replay_gather_seeds, sgrl_seed_copy, sgrl_input_grad and sgrl_fold_sym / sgrl_unfold_sym); the library allocates nothing, never synchronises and never
  * throws.  Every call enqueues work on the given cudaStream_t (pass
  * torch.cuda.current_stream().cuda_stream) and returns 0, or a negative code with a
  * thread-local message in sgrl_last_error().  Calls are re-entrant per stream.
@@ -204,6 +204,73 @@ typedef struct {
 typedef struct { int32_t path, bn, amn, bmn, bpre, sm2, gram, persist, split, sk_x, cluster, tma_c, epi; } SgrlGemmPlan;
 typedef struct { SgrlGemmPlan pr[4]; int32_t launches, pad_; } SgrlGemmPlanInfo;
 int sgrl_gemm_desc(const SgrlGemmDesc* d, SgrlGemmPlanInfo* info /* nullable */, sgrl_stream_t stream);
+/* ---- the kernels around the projections (csrc/misc.cuh) and the triangle fold (csrc/feature.cuh), one entry point each ----
+ * Each launches exactly what the network passes launch: the same host launcher picks the grid (its caps, the deterministic-mode
+ * override) and, for the LayerNorms, the float4 / scalar access of every operand from its pointer, leading dimension and z-stride.
+ * nb = 1..16 instances on the grid, instance z of an operand at pointer + z * its z-stride (zs_s: forward stash, zs_w: backward
+ * workspace, zs_p: parameters, zs_g: gradients, as in csrc/net.cuh).  grid (nullable, 3 ints) receives the grid launched.  T >= 0
+ * tokens.  Outputs marked "+=" accumulate; everything else is overwritten.  Refused with nothing enqueued: NULL required pointers,
+ * nb outside 1..16, T < 0, and each operand a kernel reads or writes as float4 (float2: dog) that is not 16-byte (8-byte) aligned
+ * together with its leading dimension and z-stride.
+ *  sgrl_embed_fwd: the input stage (SEActor.py:237-251): obs (T,41) of block z % in_nets (zs_obs), act (T,3) of critics (ng = 20;
+ *    NULL for actors, ng = 17), rank3 (T,3) rows 0..14 of the positional tables E0 (15,42), E1 (15,42), E2 (15,44); Wg (128,8),
+ *    We (128,ng), be (128).  V0 (T,24), GD (T,6), SH[:, :ng] (row stride ldsh) copies of obs / act; VG (T,3,128) and H (row stride ldh).
+ *  sgrl_input_grad: d obs (T,41) (zs_dobs) as sgrl_set_backward_dobs gathers it; dz (3L), dog (L), P (L) are HOST arrays of device
+ *    pointers, L = 1..8; dzh2, gph, dout, out, w3 for actors (ng = 17) only.  Deterministic.
+ *  sgrl_pos_embed_bwd: dE0, dE1, dE2 += scatter of dH (T,128, row stride ldh) over rank3.
+ *  sgrl_layernorm_fwd: x = a + b (b nullable), y = LN(x) gamma + beta (row stride ldy; y2 nullable, a second copy), stats (T,2) =
+ *    mean, rstd; x (nullable) is stored with row stride 128.
+ *  sgrl_layernorm_bwd: dx = LN backward of dy1 + dy2 (dy2 nullable); dgamma, dbeta (both or neither) +=; with rd_* (all or none)
+ *    also rd_out = dx / rd_F and rd_dF[t] += -<dx, rd_y> / rd_F (rd_y, rd_F in the stash, rd_dF, rd_out in the workspace).
+ *  sgrl_matapply_fwd / _bwd: R = Z (3x32) M (32x32) per token; backward dZ = dR M^T, dT = Z^T dR / F, dF[t] += -<Z^T dR, M> / F.
+ *  sgrl_matapply_l5_fwd / _bwd: the same fused with linear5 and the residuals: Vn = Vg + dV + (Z M) W5^T (W5 (128,32)), R = Z M
+ *    kept unless NULL; backward from dVn with dR = dVn W5.
+ *  sgrl_actor_out_fwd / _bwd: w = R (3,32) wd, out_i = max_action tanh(sum_r V0[r][5+i] w_r), W3 = w; backward dR and dwd +=.
+ *  sgrl_rowdiv_bwd: backward of y = t / F (* colscale on the first cs_n <= N columns): dy = g cs / F with g = src (or dy in place),
+ *    dF[t] += -<g, y> / F.
+ *  sgrl_colsum: out[n] += alpha * sum_m X[m][n] (zs_x, zs_o).
+ *  sgrl_block_copy: dst = (add ? dst : 0) + src (+ src2) on an (M, N) block.
+ *  sgrl_fold_sym / sgrl_unfold_sym: n = 1..17 folds W'[o][p(i,j)] = W[o][32i+j] + W[o][32j+i] of the (rows[m],1024) matrix at
+ *    params + src[m] into wf + dst[m] (row stride 544; with_split: tf32 hi / lo planes at + plane, + 2 plane), and the gradient
+ *    grads + src[m] += unfold of gf + dst[m].  src, dst, rows are HOST arrays. */
+int sgrl_embed_fwd(const float* obs, int64_t zs_obs, const float* act, int64_t zs_act, const int32_t* rank3, const float* Wg, const float* We,
+                   const float* be, const float* E0, const float* E1, const float* E2, int64_t zs_p, float* V0, float* GD, float* SH, int ldsh,
+                   float* VG, float* H, int ldh, int64_t zs_s, int T, int ng, int nb, int in_nets, int32_t* grid, sgrl_stream_t stream);
+int sgrl_input_grad(const float* dvg0, const float* dh0, const float* dzh, const float* dzh2, const float* dsh, int ldsh,
+                    const float* const* dz, const float* const* dog, const float* const* P, const float* Wg, const float* We, const float* gg,
+                    const float* gph, int ng, const float* dout, int64_t zs_do, const float* out, const float* w3, float max_action,
+                    float* dobs, int64_t zs_dobs, const int32_t* cu_limbs, int G, int T, int L, int64_t zs_w, int64_t zs_s, int64_t zs_p, int nb,
+                    int32_t* grid, sgrl_stream_t stream);
+int sgrl_pos_embed_bwd(const float* dH, int ldh, int64_t zs_w, const int32_t* rank3, float* dE0, float* dE1, float* dE2, int64_t zs_g, int T, int nb,
+                       int32_t* grid, sgrl_stream_t stream);
+int sgrl_layernorm_fwd(const float* a, int lda, const float* b, int ldb, const float* gamma, const float* beta, int64_t zs_p, float* x, float* y,
+                       int ldy, float* y2, int ldy2, float* stats, int64_t zs_s, int T, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_layernorm_bwd(const float* dy1, int ld1, const float* dy2, int ld2, const float* x, int ldx, const float* stats, int64_t zs_s,
+                       const float* gamma, int64_t zs_p, float* dx, int lddx, int64_t zs_w, float* dgamma, float* dbeta, int64_t zs_g,
+                       const float* rd_y, int rd_ldy, const float* rd_F, float* rd_dF, float* rd_out, int rd_ldout, int T, int nb,
+                       int32_t* grid, sgrl_stream_t stream);
+int sgrl_matapply_fwd(const float* Z, const float* M, float* R, int64_t zs_s, int T, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_matapply_bwd(const float* dR, const float* Z, const float* M, const float* F, int64_t zs_s, float* dZ, float* dT, float* dF, int64_t zs_w,
+                      int T, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_matapply_l5_fwd(const float* Z, const float* M, const float* W5, int64_t zs_p, const float* Vg, const float* dV, float* R, float* Vn,
+                         int64_t zs_s, int T, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_matapply_l5_bwd(const float* dVn, const float* W5, int64_t zs_p, const float* Z, const float* M, const float* F, int64_t zs_s, float* dZ,
+                         float* dT, float* dF, int64_t zs_w, int T, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_actor_out_fwd(const float* R, const float* V0, const float* wd, int64_t zs_p, float* W3, float* out, int64_t zs_s, float max_action, int T,
+                       int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_actor_out_bwd(const float* dout, int64_t zs_do, const float* out, const float* R, const float* V0, int64_t zs_s, const float* wd,
+                       int64_t zs_p, float* dR, int64_t zs_w, float* dwd, int64_t zs_g, float max_action, int T, int nb, int32_t* grid,
+                       sgrl_stream_t stream);
+int sgrl_rowdiv_bwd(float* dy, int lddy, int64_t zs_w, const float* y, int ldy, const float* F, int64_t zs_s, float* dF, int N, float colscale,
+                    int cs_n, const float* src, int ldsrc, int64_t zs_src, int T, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_colsum(const float* X, int ldx, int64_t zs_x, float* out, int64_t zs_o, int M, int N, float alpha, int nb, int32_t* grid,
+                sgrl_stream_t stream);
+int sgrl_block_copy(float* dst, int ldd, int64_t zs_d, const float* src, int lds, int64_t zs_src, const float* src2, int lds2, int64_t zs_src2,
+                    int M, int N, int add, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_fold_sym(const float* params, int64_t zs_p, float* wf, int64_t zs_s, int64_t plane, int with_split, const int64_t* src, const int64_t* dst,
+                  const int32_t* rows, int n, int nb, int32_t* grid, sgrl_stream_t stream);
+int sgrl_unfold_sym(const float* gf, int64_t zs_w, float* grads, int64_t zs_g, const int64_t* src, const int64_t* dst, const int32_t* rows, int n,
+                    int nb, int32_t* grid, sgrl_stream_t stream);
 /* hi = tf32_rna(w), lo = tf32_rna(w - hi): the operand split of the 3xTF32 tensor-core projections, done once per
  * optimizer step for weights instead of once per tile load */
 int sgrl_split_tf32(const float* w, float* hi, float* lo, int64_t n, sgrl_stream_t stream);

@@ -32,6 +32,8 @@ lib = C.CDLL(LIB_PATH)
 c_f = C.c_void_p      # device pointers travel as integers
 c_i64 = C.c_int64
 c_int = C.c_int
+c_grid = C.POINTER(C.c_int32)     # int32_t grid[3] (nullable): the grid a single-kernel entry point launched
+c_ptrs = C.POINTER(c_f)           # HOST array of device pointers
 
 
 class NetCall(C.Structure):
@@ -125,6 +127,27 @@ _PROTOS = {
     "sgrl_gemm_pair": (c_int, [c_f, c_int, c_f, c_f, c_f, c_f, c_int, c_int, c_int, c_int, c_f, c_int, c_f, c_f, c_f, c_f, c_int, c_int,
                                c_int, c_int, c_int, c_f]),
     "sgrl_gemm_desc": (c_int, [C.POINTER(GemmDesc), C.POINTER(GemmPlanInfo), c_f]),
+    "sgrl_embed_fwd": (c_int, [c_f, c_i64, c_f, c_i64, c_f, c_f, c_f, c_f, c_f, c_f, c_f, c_i64, c_f, c_f, c_f, c_int, c_f, c_f, c_int, c_i64,
+                               c_int, c_int, c_int, c_int, c_grid, c_f]),
+    "sgrl_input_grad": (c_int, [c_f, c_f, c_f, c_f, c_f, c_int, c_ptrs, c_ptrs, c_ptrs, c_f, c_f, c_f, c_f, c_int, c_f, c_i64, c_f, c_f,
+                                C.c_float, c_f, c_i64, c_f, c_int, c_int, c_int, c_i64, c_i64, c_i64, c_int, c_grid, c_f]),
+    "sgrl_pos_embed_bwd": (c_int, [c_f, c_int, c_i64, c_f, c_f, c_f, c_f, c_i64, c_int, c_int, c_grid, c_f]),
+    "sgrl_layernorm_fwd": (c_int, [c_f, c_int, c_f, c_int, c_f, c_f, c_i64, c_f, c_f, c_int, c_f, c_int, c_f, c_i64, c_int, c_int, c_grid, c_f]),
+    "sgrl_layernorm_bwd": (c_int, [c_f, c_int, c_f, c_int, c_f, c_int, c_f, c_i64, c_f, c_i64, c_f, c_int, c_i64, c_f, c_f, c_i64,
+                                   c_f, c_int, c_f, c_f, c_f, c_int, c_int, c_int, c_grid, c_f]),
+    "sgrl_matapply_fwd": (c_int, [c_f, c_f, c_f, c_i64, c_int, c_int, c_grid, c_f]),
+    "sgrl_matapply_bwd": (c_int, [c_f, c_f, c_f, c_f, c_i64, c_f, c_f, c_f, c_i64, c_int, c_int, c_grid, c_f]),
+    "sgrl_matapply_l5_fwd": (c_int, [c_f, c_f, c_f, c_i64, c_f, c_f, c_f, c_f, c_i64, c_int, c_int, c_grid, c_f]),
+    "sgrl_matapply_l5_bwd": (c_int, [c_f, c_f, c_i64, c_f, c_f, c_f, c_i64, c_f, c_f, c_f, c_i64, c_int, c_int, c_grid, c_f]),
+    "sgrl_actor_out_fwd": (c_int, [c_f, c_f, c_f, c_i64, c_f, c_f, c_i64, C.c_float, c_int, c_int, c_grid, c_f]),
+    "sgrl_actor_out_bwd": (c_int, [c_f, c_i64, c_f, c_f, c_f, c_i64, c_f, c_i64, c_f, c_i64, c_f, c_i64, C.c_float, c_int, c_int, c_grid, c_f]),
+    "sgrl_rowdiv_bwd": (c_int, [c_f, c_int, c_i64, c_f, c_int, c_f, c_i64, c_f, c_int, C.c_float, c_int, c_f, c_int, c_i64, c_int, c_int,
+                                c_grid, c_f]),
+    "sgrl_colsum": (c_int, [c_f, c_int, c_i64, c_f, c_i64, c_int, c_int, C.c_float, c_int, c_grid, c_f]),
+    "sgrl_block_copy": (c_int, [c_f, c_int, c_i64, c_f, c_int, c_i64, c_f, c_int, c_i64, c_int, c_int, c_int, c_int, c_grid, c_f]),
+    "sgrl_fold_sym": (c_int, [c_f, c_i64, c_f, c_i64, c_i64, c_int, C.POINTER(c_i64), C.POINTER(c_i64), C.POINTER(C.c_int32), c_int, c_int,
+                              c_grid, c_f]),
+    "sgrl_unfold_sym": (c_int, [c_f, c_i64, c_f, c_i64, C.POINTER(c_i64), C.POINTER(c_i64), C.POINTER(C.c_int32), c_int, c_int, c_grid, c_f]),
     "sgrl_split_tf32": (c_int, [c_f, c_f, c_f, c_i64, c_f]),
     "sgrl_td3_smooth_action": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, c_i64, c_f]),
     "sgrl_td3_smooth_action_rng": (c_int, [c_f, c_f, c_f, C.c_float, C.c_float, C.c_float, c_i64, C.c_uint64, c_f, c_f]),

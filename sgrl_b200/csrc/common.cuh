@@ -73,6 +73,12 @@ inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
   cfg.attrs = at; cfg.numAttrs = (pdl_enabled() && pdl_stream_ok(st)) ? 1 : 0;
   cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
+// after a launch_k of the host launchers (misc.cuh, feature.cuh): count it, report its grid (grid nullable) and its launch error
+inline int launched(dim3 g, int* grid) {
+  if (grid) { grid[0] = (int)g.x; grid[1] = (int)g.y; grid[2] = (int)g.z; }
+  SGRL_LAUNCH_OK();
+  return 0;
+}
 
 // ---- optional per-kernel-class device timing (bench.py roofline pass): CUDA events around
 // the launches of one class on the launching stream, collected after a synchronize.

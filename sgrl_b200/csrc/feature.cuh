@@ -451,4 +451,18 @@ __global__ void __launch_bounds__(256) unfold_sym_kernel(const float* __restrict
   }
 }
 
+// host launchers of the two (network passes and sgrl_fold_sym / sgrl_unfold_sym; grid nullable, as misc.cuh's)
+inline int fold_sym_launch(const float* params, long long zsP, float* wf, long long zsS, long long plane, int with_split, const FoldDesc& d, int nb,
+                           cudaStream_t st, int* grid = nullptr) {
+  const dim3 g(48, d.n, nb);
+  launch_k(fold_sym_kernel, g, 256, 0, st, params, zsP, wf, zsS, plane, with_split, d);
+  return launched(g, grid);
+}
+inline int unfold_sym_launch(const float* gf, long long zsW, float* grads, long long zsG, const FoldDesc& d, int nb, cudaStream_t st,
+                             int* grid = nullptr) {
+  const dim3 g(64, d.n, nb);
+  launch_k(unfold_sym_kernel, g, 256, 0, st, gf, zsW, grads, zsG, d);
+  return launched(g, grid);
+}
+
 }  // namespace sgrl

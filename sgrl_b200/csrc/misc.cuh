@@ -648,4 +648,130 @@ __global__ void __launch_bounds__(256) block_copy_kernel(float* __restrict__ dst
 
 inline int grid_for_warps(int T) { int g = ceil_div(T, 8); return g > 8 * NUM_SMS ? 8 * NUM_SMS : (g < 1 ? 1 : g); }
 
+// =====================================================================================
+// Host launchers: the grid of each kernel above (its caps, the deterministic-mode override) and the vector flags of the
+// LayerNorms, in one place for the network passes (net.cuh) and the single-kernel entry points (sgrl_b200.cu).  Arguments
+// are the kernel's own; nb net instances on the grid's y (z for colsum); grid (nullable) receives the grid launched.
+// =====================================================================================
+
+inline int embed_fwd_launch(const float* obs, long long zsObs, const float* act, long long zsAct, const int* rank3, const float* Wg,
+                            const float* We, const float* be, const float* E0, const float* E1, const float* E2, long long zsP, float* V0,
+                            float* GD, float* SH, int ldsh, float* VG, float* H, int ldh, long long zsS, int T, int ng, int nb, int in_nets,
+                            cudaStream_t st, int* grid = nullptr) {
+  int gx = ceil_div(T, E_TOK); if (gx > 4 * NUM_SMS) gx = 4 * NUM_SMS; if (gx < 1) gx = 1;     // above 4 736 tokens CTAs walk groups
+  const dim3 g(gx, nb);
+  launch_k(embed_fwd_kernel, g, 128, 0, st, obs, zsObs, act, zsAct, rank3, Wg, We, be, E0, E1, E2, zsP, V0, GD, SH, ldsh, VG, H, ldh, zsS, T, ng,
+           in_nets);
+  return launched(g, grid);
+}
+
+inline int input_grad_launch(const InGradP& p, int nb, cudaStream_t st, int* grid = nullptr) {
+  int gx = grid_for_warps(p.T); if (gx > 2 * NUM_SMS) gx = 2 * NUM_SMS;
+  const dim3 g(gx, nb);
+  launch_k(input_grad_kernel, g, 256, 0, st, p);
+  return launched(g, grid);
+}
+
+inline int pos_embed_bwd_launch(const float* dH, int ldh, long long zsW, const int* rank3, float* dE0, float* dE1, float* dE2, long long zsG,
+                                int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  int gx = ceil_div(T, 64); if (gx > NUM_SMS) gx = NUM_SMS; if (gx < 1) gx = 1;
+  if (det_enabled()) gx = 1;
+  const dim3 g(gx, nb);
+  launch_k(pos_embed_bwd_kernel, g, 128, 0, st, dH, ldh, zsW, rank3, dE0, dE1, dE2, zsG, T);
+  return launched(g, grid);
+}
+
+inline int layernorm_fwd_launch(const float* a, int lda, const float* b, int ldb, const float* gamma, const float* beta, long long zsP, float* x,
+                                float* y, int ldy, float* y2, int ldy2, float* stats, long long zsS, int T, int nb, cudaStream_t st,
+                                int* grid = nullptr) {
+  const int vf = host_vec_ok(a, lda, zsS) | (host_vec_ok(b, ldb, zsS) << 1) | (host_vec_ok(y, ldy, zsS) << 2) | (host_vec_ok(y2, ldy2, zsS) << 3);
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(layernorm_fwd_kernel, g, 256, 0, st, a, lda, b, ldb, gamma, beta, zsP, x, y, ldy, y2, ldy2, stats, zsS, T, vf);
+  return launched(g, grid);
+}
+
+// dgamma == nullptr: data-only backward (dbeta ignored)
+inline int layernorm_bwd_launch(const float* dy1, int ld1, const float* dy2, int ld2, const float* x, int ldx, const float* stats, long long zsS,
+                                const float* gamma, long long zsP, float* dx, int lddx, long long zsW, float* dgamma, float* dbeta, long long zsG,
+                                LnRowdiv rd, int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  int gx = grid_for_warps(T); if (gx > 2 * NUM_SMS) gx = 2 * NUM_SMS;
+  if (dgamma && det_enabled()) gx = 1;      // dgamma / dbeta: one add per address
+  const int vf = host_vec_ok(dy1, ld1, zsW) | (host_vec_ok(dy2, ld2, zsW) << 1) | (host_vec_ok(x, ldx, zsS) << 2) | (host_vec_ok(dx, lddx, zsW) << 3) |
+                 ((rd.y && host_vec_ok(rd.y, rd.ldy, zsS)) << 4) | ((rd.out && host_vec_ok(rd.out, rd.ldout, zsW)) << 5);
+  const dim3 g(gx, nb);
+  launch_k(layernorm_bwd_kernel, g, 256, 0, st, dy1, ld1, dy2, ld2, x, ldx, stats, zsS, gamma, zsP, dx, lddx, zsW, dgamma, dbeta, zsG, T,
+           vf, rd);
+  return launched(g, grid);
+}
+
+inline int matapply_fwd_launch(const float* Z, const float* M, float* R, long long zsS, int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(matapply_fwd_kernel, g, 256, 0, st, Z, M, R, zsS, T);
+  return launched(g, grid);
+}
+
+inline int matapply_bwd_launch(const float* dR, const float* Z, const float* M, const float* Fn, long long zsS, float* dZ, float* dT, float* dF,
+                               long long zsW, int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(matapply_bwd_kernel, g, 256, 0, st, dR, Z, M, Fn, zsS, dZ, dT, dF, zsW, T);
+  return launched(g, grid);
+}
+
+inline int matapply_l5_fwd_launch(const float* Z, const float* M, const float* W5, long long zsP, const float* Vg, const float* dV, float* R,
+                                  float* Vn, long long zsS, int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(matapply_l5_fwd_kernel, g, 256, 0, st, Z, M, W5, zsP, Vg, dV, R, Vn, zsS, T);
+  return launched(g, grid);
+}
+
+inline int matapply_l5_bwd_launch(const float* dVn, const float* W5, long long zsP, const float* Z, const float* M, const float* Fn, long long zsS,
+                                  float* dZ, float* dT, float* dF, long long zsW, int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(matapply_l5_bwd_kernel, g, 256, 0, st, dVn, W5, zsP, Z, M, Fn, zsS, dZ, dT, dF, zsW, T);
+  return launched(g, grid);
+}
+
+inline int actor_out_fwd_launch(const float* R, const float* V0, const float* wd, long long zsP, float* W3, float* out, long long zsS,
+                                float max_action, int T, int nb, cudaStream_t st, int* grid = nullptr) {
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(actor_out_fwd_kernel, g, 256, 0, st, R, V0, wd, zsP, W3, out, zsS, max_action, T);
+  return launched(g, grid);
+}
+
+// wgrad: dwd is a parameter gradient (one CTA in deterministic mode), else scratch whose sums are discarded
+inline int actor_out_bwd_launch(const float* dOut, long long zsDo, const float* out, const float* R, const float* V0, long long zsS, const float* wd,
+                                long long zsP, float* dR, long long zsW, float* dwd, long long zsG, bool wgrad, float max_action, int T, int nb,
+                                cudaStream_t st, int* grid = nullptr) {
+  int gx = grid_for_warps(T); if (gx > 2 * NUM_SMS) gx = 2 * NUM_SMS;
+  if (wgrad && det_enabled()) gx = 1;
+  const dim3 g(gx, nb);
+  launch_k(actor_out_bwd_kernel, g, 256, 0, st, dOut, zsDo, out, R, V0, zsS, wd, zsP, dR, zsW, dwd, zsG, max_action, T);
+  return launched(g, grid);
+}
+
+inline int rowdiv_bwd_launch(float* dy, int lddy, long long zsW, const float* y, int ldy, const float* Fn, long long zsS, float* dF, int N,
+                             float colscale, int cs_n, int T, const float* src, int ldsrc, long long zsSrc, int nb, cudaStream_t st,
+                             int* grid = nullptr) {
+  const dim3 g(grid_for_warps(T), nb);
+  launch_k(rowdiv_bwd_kernel, g, 256, 0, st, dy, lddy, zsW, y, ldy, Fn, zsS, dF, N, colscale, cs_n, T, src, ldsrc, zsSrc);
+  return launched(g, grid);
+}
+
+inline int colsum_launch(const float* X, int ldx, long long zsX, float* out, long long zsO, int M, int N, float alpha, int nb, cudaStream_t st,
+                         int* grid = nullptr) {
+  int gy = ceil_div(M, 64); if (gy > 32) gy = 32; if (gy < 1) gy = 1;
+  if (det_enabled()) gy = 1;
+  const dim3 g(ceil_div(N, 32), gy, nb);
+  launch_k(colsum_kernel, g, 256, 0, st, X, ldx, zsX, out, zsO, M, N, alpha);
+  return launched(g, grid);
+}
+
+inline int block_copy_launch(float* dst, int ldd, long long zsD, const float* src, int lds, long long zsSrc, const float* src2, int lds2,
+                             long long zsSrc2, int M, int N, int add, int nb, cudaStream_t st, int* grid = nullptr) {
+  int gx = ceil_div((long long)M * N, 256); if (gx > 4 * NUM_SMS) gx = 4 * NUM_SMS; if (gx < 1) gx = 1;
+  const dim3 g(gx, nb);
+  launch_k(block_copy_kernel, g, 256, 0, st, dst, ldd, zsD, src, lds, zsSrc, src2, lds2, zsSrc2, M, N, add);
+  return launched(g, grid);
+}
+
 }  // namespace sgrl

@@ -148,10 +148,7 @@ inline int run_gemm(const NetCtx& c, const GemmP& g, cudaStream_t st = nullptr) 
   SGRL_TRY(gemm_simt(g, st));
   if (g.rowsum) {      // the SIMT kernel has no fused row sum: rowsum[m] += alpha * sum_k A(m,k) as a column sum of dY (A = dY^T)
     SGRL_CHECK(g.transA, "rowsum: only for weight-gradient GEMMs (A = dY^T)");
-    int gy = ceil_div(g.K, 64); if (gy > 32) gy = 32; if (gy < 1) gy = 1;
-    if (det_enabled()) gy = 1;
-    launch_k(colsum_kernel, dim3(ceil_div(g.M, 32), gy, g.nb), 256, 0, st, g.A, g.lda, g.zsA, g.rowsum, g.zsRowsum, g.K, g.M, g.alpha);
-    SGRL_LAUNCH_OK();
+    SGRL_TRY(colsum_launch(g.A, g.lda, g.zsA, g.rowsum, g.zsRowsum, g.K, g.M, g.alpha, g.nb, st));
   }
   return 0;
 }
@@ -270,55 +267,30 @@ inline GemmP wgrad_fold(const NetCtx& c, const float* dY, int lddy, const float*
   return g;
 }
 inline int fold_weights(const NetCtx& c, cudaStream_t st) {
-  const FoldDesc d = fold_desc(c);
-  launch_k(fold_sym_kernel, dim3(48, d.n, c.nb), 256, 0, st, c.params, c.zsP, c.stash + c.st.wf, c.zsS, c.st.wf_plane, c.phi ? 1 : 0, d);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return fold_sym_launch(c.params, c.zsP, c.stash + c.st.wf, c.zsS, c.st.wf_plane, c.phi ? 1 : 0, fold_desc(c), c.nb, st);
 }
 
-inline int colsum(const NetCtx& c, const float* X, int ldx, long long g_off, int M, int N, float alpha, cudaStream_t st) {
-  int gy = ceil_div(M, 64); if (gy > 32) gy = 32; if (gy < 1) gy = 1;
-  if (det_enabled()) gy = 1;
-  launch_k(colsum_kernel, dim3(ceil_div(N, 32), gy, c.nb), 256, 0, st, X, ldx, c.zsW, c.Gr(g_off), c.zsG, M, N, alpha);
-  SGRL_LAUNCH_OK();
-  return 0;
-}
 inline int block_copy(const NetCtx& c, float* dst, int ldd, long long zsD, const float* src, int lds, long long zsSrc, int M, int N, int add,
                       const float* src2 = nullptr, int lds2 = 0, long long zsSrc2 = 0, cudaStream_t st = nullptr) {
   if (!st) st = c.stream;
-  int gx = ceil_div((long long)M * N, 256); if (gx > 4 * NUM_SMS) gx = 4 * NUM_SMS; if (gx < 1) gx = 1;
-  launch_k(block_copy_kernel, dim3(gx, c.nb), 256, 0, st, dst, ldd, zsD, src, lds, zsSrc, src2, lds2, zsSrc2, M, N, add);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return block_copy_launch(dst, ldd, zsD, src, lds, zsSrc, src2, lds2, zsSrc2, M, N, add, c.nb, st);
 }
 inline int layernorm_fwd(const NetCtx& c, const float* a, int lda, const float* b, int ldb, long long g_off, long long b_off,
                          float* x, float* y, int ldy, float* stats, cudaStream_t st = nullptr) {
   if (!st) st = c.stream;
-  const int vf = host_vec_ok(a, lda, c.zsS) | (host_vec_ok(b, ldb, c.zsS) << 1) | (host_vec_ok(y, ldy, c.zsS) << 2);
-  launch_k(layernorm_fwd_kernel, dim3(grid_for_warps(c.T), c.nb), 256, 0, st, a, lda, b, ldb, c.P(g_off), c.P(b_off), c.zsP, x, y, ldy,
-                                                                              nullptr, 0, stats, c.zsS, c.T, vf);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return layernorm_fwd_launch(a, lda, b, ldb, c.P(g_off), c.P(b_off), c.zsP, x, y, ldy, nullptr, 0, stats, c.zsS, c.T, c.nb, st);
 }
 inline int layernorm_bwd(const NetCtx& c, const float* dy1, int ld1, const float* dy2, int ld2, const float* x, int ldx,
                          const float* stats, long long g_off, long long b_off, float* dx, int lddx, bool wg, cudaStream_t st = nullptr,
                          LnRowdiv rd = LnRowdiv{nullptr, nullptr, nullptr, nullptr, 0, 0}) {
   if (!st) st = c.stream;
-  int gx = grid_for_warps(c.T); if (gx > 2 * NUM_SMS) gx = 2 * NUM_SMS;
-  if (wg && det_enabled()) gx = 1;      // dgamma / dbeta: one add per address
-  const int vf = host_vec_ok(dy1, ld1, c.zsW) | (host_vec_ok(dy2, ld2, c.zsW) << 1) | (host_vec_ok(x, ldx, c.zsS) << 2) | (host_vec_ok(dx, lddx, c.zsW) << 3) |
-                 ((rd.y && host_vec_ok(rd.y, rd.ldy, c.zsS)) << 4) | ((rd.out && host_vec_ok(rd.out, rd.ldout, c.zsW)) << 5);
-  launch_k(layernorm_bwd_kernel, dim3(gx, c.nb), 256, 0, st, dy1, ld1, dy2, ld2, x, ldx, stats, c.zsS, c.P(g_off), c.zsP, dx, lddx, c.zsW,
-                                                             wg ? c.Gr(g_off) : nullptr, wg ? c.Gr(b_off) : nullptr, c.zsG, c.T, vf, rd);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return layernorm_bwd_launch(dy1, ld1, dy2, ld2, x, ldx, stats, c.zsS, c.P(g_off), c.zsP, dx, lddx, c.zsW, wg ? c.Gr(g_off) : nullptr,
+                              wg ? c.Gr(b_off) : nullptr, c.zsG, rd, c.T, c.nb, st);
 }
 inline int rowdiv_bwd(const NetCtx& c, float* dy, int lddy, const float* y, int ldy, const float* Fn, float* dF, int N, float cs, int cs_n,
                       cudaStream_t st = nullptr, const float* src = nullptr, int ldsrc = 0, long long zsSrc = 0) {
   if (!st) st = c.stream;
-  launch_k(rowdiv_bwd_kernel, dim3(grid_for_warps(c.T), c.nb), 256, 0, st, dy, lddy, c.zsW, y, ldy, Fn, c.zsS, dF, N, cs, cs_n, c.T, src, ldsrc, zsSrc);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return rowdiv_bwd_launch(dy, lddy, c.zsW, y, ldy, Fn, c.zsS, dF, N, cs, cs_n, c.T, src, ldsrc, zsSrc, c.nb, st);
 }
 // the dF accumulators (||G||_F gradients, T floats each) of EVERY frame in one launch at the start of the backward
 // (they were 2 * nb memset nodes per layer on the data-gradient chain)
@@ -338,9 +310,7 @@ inline int zero_df_frames(const NetCtx& c) {
 }
 
 inline int unfold_grads(const NetCtx& c, const FoldDesc& d, cudaStream_t st) {
-  launch_k(unfold_sym_kernel, dim3(64, d.n, c.nb), 256, 0, st, c.ws + c.wl.gf, c.zsW, c.grads, c.zsG, d);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return unfold_sym_launch(c.ws + c.wl.gf, c.zsW, c.grads, c.zsG, d, c.nb, st);
 }
 
 constexpr float QSCALE = 0.08838834764831845f;   // (2*head_dim)^-0.5 = 128^-0.5, subequivariant_attentions.py:88
@@ -366,13 +336,9 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
   static const int fold_side = getenv("SGRL_FOLD_SIDE") ? atoi(getenv("SGRL_FOLD_SIDE")) : 1;
   bool fold_pending = false;
   if (fused && fold_side) { SGRL_TRY(side_fork(c, &sb, 0)); SGRL_TRY(fold_weights(c, sb)); fold_pending = true; }
-  {
-    int gx = ceil_div(T, E_TOK); if (gx > 4 * NUM_SMS) gx = 4 * NUM_SMS;
-    launch_k(embed_fwd_kernel, dim3(gx, c.nb), 128, 0, st, obs, zsObs, c.kind == CRITIC ? act : nullptr, zsAct, c.rank3,
-        c.P(Y.gp[G_GENC_W]), c.P(Y.gp[G_ENC_W]), c.P(Y.gp[G_ENC_B]), c.P(Y.gp[G_POS0]), c.P(Y.gp[G_POS1]), c.P(Y.gp[G_POS2]), c.zsP,
-        c.S(T_V0), c.S(T_GD), c.S(T_SH), KS, c.SL(0, S_VGIN), c.SL(0, S_UA) + 128, 256, zS, T, ng, c.in_nets);
-    SGRL_LAUNCH_OK();
-  }
+  SGRL_TRY(embed_fwd_launch(obs, zsObs, c.kind == CRITIC ? act : nullptr, zsAct, c.rank3, c.P(Y.gp[G_GENC_W]), c.P(Y.gp[G_ENC_W]),
+                            c.P(Y.gp[G_ENC_B]), c.P(Y.gp[G_POS0]), c.P(Y.gp[G_POS1]), c.P(Y.gp[G_POS2]), c.zsP, c.S(T_V0), c.S(T_GD), c.S(T_SH),
+                            KS, c.SL(0, S_VGIN), c.SL(0, S_UA) + 128, 256, zS, T, ng, c.nb, c.in_nets, st));
   if (fused && !fold_pending) SGRL_TRY(fold_weights(c, st));
   for (int l = 0; l < c.L; ++l) {
     const long long* lp = Y.lp[l];
@@ -441,9 +407,8 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
       SGRL_TRY(side_fork(c, &sb, 0));
       SGRL_TRY(layernorm_fwd(c, ub + 128, 256, c.SL(l, S_FF), 128, lp[L_N2_W], lp[L_N2_B], c.SL(l, S_X2), h_next, ld_hn, c.SL(l, S_ST2), sb));
       if (last) SGRL_TRY(layernorm_fwd(c, c.S(T_HL), 128, nullptr, 0, Y.gp[G_NORM_W], Y.gp[G_NORM_B], nullptr, c.S(T_SH) + ng, KS, c.S(T_STF), sb));
-      launch_k(matapply_l5_fwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, c.SL(l, S_Z3), c.SL(l, S_MM), c.P(lp[L_L5_W]), c.zsP, Vg, c.SL(l, S_DV),
-               c.keep ? c.SL(l, S_R) : nullptr, Vg_next, zS, T);
-      SGRL_LAUNCH_OK();
+      SGRL_TRY(matapply_l5_fwd_launch(c.SL(l, S_Z3), c.SL(l, S_MM), c.P(lp[L_L5_W]), c.zsP, Vg, c.SL(l, S_DV), c.keep ? c.SL(l, S_R) : nullptr,
+                                      Vg_next, zS, T, c.nb, st));
       SGRL_TRY(side_join(c, 0));
       continue;
     }
@@ -496,9 +461,8 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
     g.rowdiv = c.SL(l, S_F2); g.zsRow = zS;
     SGRL_TRY(run_gemm(c, g));
     // Vg' = Vg + dV + linear5(Z3 . M): matrix apply, the K = 32 projection and both residuals in one launch (misc.cuh)
-    launch_k(matapply_l5_fwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, c.SL(l, S_Z3), c.SL(l, S_MM), c.P(lp[L_L5_W]), c.zsP, Vg, c.SL(l, S_DV),
-             c.keep ? c.SL(l, S_R) : nullptr, Vg_next, zS, T);
-    SGRL_LAUNCH_OK();
+    SGRL_TRY(matapply_l5_fwd_launch(c.SL(l, S_Z3), c.SL(l, S_MM), c.P(lp[L_L5_W]), c.zsP, Vg, c.SL(l, S_DV), c.keep ? c.SL(l, S_R) : nullptr,
+                                    Vg_next, zS, T, c.nb, st));
     SGRL_TRY(side_join(c));
   }
   // final LayerNorm -> right part of SH = [s0 | h]
@@ -532,11 +496,8 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
     g = lin(c, c.S(T_M1), 256, zS, Y.gp[G_H2M_W], Y.gp[G_H2M_B], c.S(T_MH), 1024, zS, T, 1024, 256);
     g.rowdiv = c.S(T_FH); g.zsRow = zS;
     SGRL_TRY(run_gemm(c, g));
-    launch_k(matapply_fwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, c.S(T_ZH2), c.S(T_MH), c.S(T_RH), zS, T);
-    SGRL_LAUNCH_OK();
-    launch_k(actor_out_fwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, c.S(T_RH), c.S(T_V0), c.P(Y.gp[G_DG_W]), c.zsP, c.S(T_W3), c.S(T_OUT), zS,
-                                                                        c.max_action, T);
-    SGRL_LAUNCH_OK();
+    SGRL_TRY(matapply_fwd_launch(c.S(T_ZH2), c.S(T_MH), c.S(T_RH), zS, T, c.nb, st));
+    SGRL_TRY(actor_out_fwd_launch(c.S(T_RH), c.S(T_V0), c.P(Y.gp[G_DG_W]), c.zsP, c.S(T_W3), c.S(T_OUT), zS, c.max_action, T, c.nb, st));
   }
   const int od = c.kind == ACTOR ? 3 : 1;
   if (out) SGRL_TRY(block_copy(c, out, od, zsOut, c.S(T_OUT), od, zS, T, od, 0));
@@ -573,10 +534,7 @@ inline int input_grad(const NetCtx& c, const float* dOut, long long zsDo, float*
   p.dobs = dobs; p.zsDobs = zsDobs;
   p.cu_limbs = c.gr.cu_limbs; p.G = c.gr.G; p.T = c.T; p.L = c.L;
   p.zsW = c.zsW; p.zsS = c.zsS; p.zsP = c.zsP;
-  int gx = grid_for_warps(c.T); if (gx > 2 * NUM_SMS) gx = 2 * NUM_SMS;
-  launch_k(input_grad_kernel, dim3(gx, c.nb), 256, 0, c.stream, p);
-  SGRL_LAUNCH_OK();
-  return 0;
+  return input_grad_launch(p, c.nb, c.stream);
 }
 
 inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, int need_wgrad, float* dact, long long zsDact,
@@ -628,13 +586,9 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     g = dgrad(c, W(W_DQ), 1, Y.gp[G_DNG_W], 256, W(W_DUH), 256, T, 1, 256);
     SGRL_TRY(run_gemm(c, g));
   } else {
-    launch_k(actor_out_bwd_kernel, dim3((wg && det_enabled()) ? 1 : grid_for_warps(T) > 2 * NUM_SMS ? 2 * NUM_SMS : grid_for_warps(T), c.nb), 256, 0, st, dOut, zsDo, c.S(T_OUT),
-             c.S(T_RH), c.S(T_V0), zS, c.P(Y.gp[G_DG_W]), c.zsP, W(W_DR), zW, wg ? c.Gr(Y.gp[G_DG_W]) : W(W_DQ) /*discarded*/, wg ? c.zsG : zW,
-             c.max_action, T);
-    SGRL_LAUNCH_OK();
-    launch_k(matapply_bwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, W(W_DR), c.S(T_ZH2), c.S(T_MH), c.S(T_FH), zS, W(W_DZ3), W(W_DT4), dFh,
-             zW, T);
-    SGRL_LAUNCH_OK();
+    SGRL_TRY(actor_out_bwd_launch(dOut, zsDo, c.S(T_OUT), c.S(T_RH), c.S(T_V0), zS, c.P(Y.gp[G_DG_W]), c.zsP, W(W_DR), zW,
+                                  wg ? c.Gr(Y.gp[G_DG_W]) : W(W_DQ) /*discarded*/, wg ? c.zsG : zW, wg, c.max_action, T, c.nb, st));
+    SGRL_TRY(matapply_bwd_launch(W(W_DR), c.S(T_ZH2), c.S(T_MH), c.S(T_FH), zS, W(W_DZ3), W(W_DT4), dFh, zW, T, c.nb, st));
     SGRL_TRY(side_w(W(W_DT4), 1024, c.S(T_M1), 256, zS, Y.gp[G_H2M_W], 256, T, 1024, 256, Y.gp[G_H2M_B]));
     g = dgrad(c, W(W_DT4), 1024, Y.gp[G_H2M_W], 256, W(W_DA), 256, T, 1024, 256);
     g.mask = c.S(T_M1); g.zsMask = zS; g.ldmask = 256;
@@ -710,9 +664,8 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     // ---- main: Vg' = Vg + dV + linear5([g_proj3(dV)|gd] . M)
     SGRL_TRY(side_w(Wn(W_DVG), 128, c.SL(l, S_R), 32, zS, lp[L_L5_W], 32, T3, 128, 32));
     // dR = dVg' W5 and the matrix-apply backward in one launch (misc.cuh)
-    launch_k(matapply_l5_bwd_kernel, dim3(grid_for_warps(T), c.nb), 256, 0, st, Wn(W_DVG), c.P(lp[L_L5_W]), c.zsP, c.SL(l, S_Z3), c.SL(l, S_MM),
-             c.SL(l, S_F2), zS, W(W_DZ3), W(W_DT4), W(W_DF2), zW, T);
-    SGRL_LAUNCH_OK();
+    SGRL_TRY(matapply_l5_bwd_launch(Wn(W_DVG), c.P(lp[L_L5_W]), c.zsP, c.SL(l, S_Z3), c.SL(l, S_MM), c.SL(l, S_F2), zS, W(W_DZ3), W(W_DT4),
+                                    W(W_DF2), zW, T, c.nb, st));
     SGRL_TRY(side_w(W(W_DT4), 1024, T31, 512, zS, lp[L_L4_W], 256, T, 1024, 256, lp[L_L4_B]));
     g = dgrad(c, W(W_DT4), 1024, lp[L_L4_W], 256, W(W_DT31), 512, T, 1024, 256);
     g.mask = T31; g.zsMask = zS; g.ldmask = 512;
@@ -787,10 +740,7 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
   if (wg) {
     SGRL_TRY(side_w(W(W_DVG), 128, c.S(T_V0), 8, zS, Y.gp[G_GENC_W], GN, T3, 128, GN, -1, SQRT_D));
     SGRL_TRY(side_w(W(W_DH), 128, c.S(T_SH), KS, zS, Y.gp[G_ENC_W], ng, T, 128, ng, Y.gp[G_ENC_B], SQRT_D));
-    int gx = ceil_div(T, 64); if (gx > NUM_SMS) gx = NUM_SMS; if (gx < 1) gx = 1;
-    if (det_enabled()) gx = 1;
-    launch_k(pos_embed_bwd_kernel, dim3(gx, c.nb), 128, 0, st, W(W_DH), 128, zW, c.rank3, c.Gr(Y.gp[G_POS0]), c.Gr(Y.gp[G_POS1]), c.Gr(Y.gp[G_POS2]), c.zsG, T);
-    SGRL_LAUNCH_OK();
+    SGRL_TRY(pos_embed_bwd_launch(W(W_DH), 128, zW, c.rank3, c.Gr(Y.gp[G_POS0]), c.Gr(Y.gp[G_POS1]), c.Gr(Y.gp[G_POS2]), c.zsG, T, c.nb, st));
   }
   if (dact) {   // + sqrt(128) * dh0 . encoder.weight[:, 17:20]
     SGRL_CHECK(c.kind == CRITIC, "d/d(action) only exists for critics");

@@ -23,7 +23,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 10; }
+int sgrl_version(void) { return 11; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -167,6 +167,198 @@ int sgrl_attention_bwd(const float* qkv, const float* vgp, const float* gd, cons
   SGRL_CHECK((drel_w == nullptr) || relation, "drel_w needs relation");
   AttnGraphs gr{cu_limbs, rel_off, relation, G, 0, max_limbs};
   return attention_bwd(qkv, vgp, gd, p, 0, d_o, d_og, dqkv, dvgp, 0, drel_w, 0, gr, 1, ST(stream));
+}
+
+// ---- the small kernels around the GEMMs (misc.cuh) and the triangle fold (feature.cuh), one entry point per launcher.  Every
+// refusal happens before anything is enqueued; a 16-byte check guards each operand a kernel accesses as float4 (float2 for d og)
+// unconditionally.
+static bool al16(const void* p, long long ld = 0, long long zs = 0) { return aligned16(p) && (ld & 3) == 0 && (zs & 3) == 0; }
+#define SGRL_NETS(nb) SGRL_CHECK((nb) >= 1 && (nb) <= MAX_NETS, "nb must be 1..16")
+#define SGRL_TOKENS(T) SGRL_CHECK((T) >= 0, "T must be >= 0")
+
+int sgrl_embed_fwd(const float* obs, int64_t zs_obs, const float* act, int64_t zs_act, const int32_t* rank3, const float* Wg, const float* We,
+                   const float* be, const float* E0, const float* E1, const float* E2, int64_t zs_p, float* V0, float* GD, float* SH, int ldsh,
+                   float* VG, float* H, int ldh, int64_t zs_s, int T, int ng, int nb, int in_nets, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(obs && rank3 && Wg && We && be && E0 && E1 && E2 && V0 && GD && SH && VG && H, "null pointer");
+  SGRL_CHECK(ng == 17 || ng == 20, "ng must be 17 (actor) or 20 (critic)");
+  SGRL_CHECK((act != nullptr) == (ng == 20), "act is read by critics (ng = 20) only");
+  SGRL_NETS(nb);
+  SGRL_CHECK(in_nets >= 1 && in_nets <= nb, "in_nets must be 1..nb");
+  SGRL_TOKENS(T);
+  SGRL_CHECK(ldsh >= ng && ldh >= D, "ldsh < ng or ldh < 128");
+  return embed_fwd_launch(obs, zs_obs, act, zs_act, rank3, Wg, We, be, E0, E1, E2, zs_p, V0, GD, SH, ldsh, VG, H, ldh, zs_s, T, ng, nb, in_nets,
+                          ST(stream), grid);
+}
+
+int sgrl_input_grad(const float* dvg0, const float* dh0, const float* dzh, const float* dzh2, const float* dsh, int ldsh,
+                    const float* const* dz, const float* const* dog, const float* const* P, const float* Wg, const float* We, const float* gg,
+                    const float* gph, int ng, const float* dout, int64_t zs_do, const float* out, const float* w3, float max_action,
+                    float* dobs, int64_t zs_dobs, const int32_t* cu_limbs, int G, int T, int L, int64_t zs_w, int64_t zs_s, int64_t zs_p, int nb,
+                    int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dvg0 && dh0 && dzh && dsh && dz && dog && P && Wg && We && gg && dobs && cu_limbs, "null pointer");
+  SGRL_CHECK(ng == 17 || ng == 20, "ng must be 17 (actor) or 20 (critic)");
+  SGRL_CHECK(L >= 1 && L <= MAX_LAYERS, "L must be 1..8");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  SGRL_CHECK(G >= 1, "G must be >= 1");
+  SGRL_CHECK(ldsh >= 17, "ldsh < 17");
+  const bool actor = dzh2 != nullptr;
+  SGRL_CHECK(actor == (ng == 17), "dzh2 (the head's dZ3) is the actor's (ng = 17) and only the actor's");
+  SGRL_CHECK(!actor || (gph && dout && out && w3), "the actor variant needs gph, dout, out and w3");
+  InGradP p{};
+  for (int l = 0; l < L; ++l) {
+    SGRL_CHECK(dz[3 * l] && dz[3 * l + 1] && dz[3 * l + 2] && dog[l] && P[l], "null pointer in dz / dog / P");
+    SGRL_CHECK((reinterpret_cast<uintptr_t>(dog[l]) & 7u) == 0 && (zs_w & 1) == 0, "dog must be 8-byte aligned with an even zs_w (float2 loads)");
+    p.dz[3 * l] = dz[3 * l]; p.dz[3 * l + 1] = dz[3 * l + 1]; p.dz[3 * l + 2] = dz[3 * l + 2]; p.dog[l] = dog[l]; p.P[l] = P[l];
+  }
+  p.dvg0 = dvg0; p.dh0 = dh0; p.dzh = dzh; p.dzh2 = dzh2; p.dsh = dsh; p.ldsh = ldsh;
+  p.Wg = Wg; p.We = We; p.gg = gg; p.gph = actor ? gph : nullptr; p.ng = ng;
+  if (actor) { p.dout = dout; p.zsDo = zs_do; p.out = out; p.w3 = w3; }
+  p.max_action = max_action; p.dobs = dobs; p.zsDobs = zs_dobs;
+  p.cu_limbs = cu_limbs; p.G = G; p.T = T; p.L = L; p.zsW = zs_w; p.zsS = zs_s; p.zsP = zs_p;
+  return input_grad_launch(p, nb, ST(stream), grid);
+}
+
+int sgrl_pos_embed_bwd(const float* dH, int ldh, int64_t zs_w, const int32_t* rank3, float* dE0, float* dE1, float* dE2, int64_t zs_g, int T, int nb,
+                       int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dH && rank3 && dE0 && dE1 && dE2, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  SGRL_CHECK(ldh >= D, "ldh < 128");
+  return pos_embed_bwd_launch(dH, ldh, zs_w, rank3, dE0, dE1, dE2, zs_g, T, nb, ST(stream), grid);
+}
+
+int sgrl_layernorm_fwd(const float* a, int lda, const float* b, int ldb, const float* gamma, const float* beta, int64_t zs_p, float* x, float* y,
+                       int ldy, float* y2, int ldy2, float* stats, int64_t zs_s, int T, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(a && gamma && beta && y && stats, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  SGRL_CHECK(lda >= D && (!b || ldb >= D) && ldy >= D && (!y2 || ldy2 >= D), "a leading dimension < 128");
+  SGRL_CHECK(al16(gamma, 0, zs_p) && al16(beta), "gamma, beta and zs_p must be 16-byte aligned (float4 loads)");
+  SGRL_CHECK(!x || al16(x, 0, zs_s), "x and zs_s must be 16-byte aligned (float4 stores)");
+  return layernorm_fwd_launch(a, lda, b, ldb, gamma, beta, zs_p, x, y, ldy, y2, ldy2, stats, zs_s, T, nb, ST(stream), grid);
+}
+
+int sgrl_layernorm_bwd(const float* dy1, int ld1, const float* dy2, int ld2, const float* x, int ldx, const float* stats, int64_t zs_s,
+                       const float* gamma, int64_t zs_p, float* dx, int lddx, int64_t zs_w, float* dgamma, float* dbeta, int64_t zs_g,
+                       const float* rd_y, int rd_ldy, const float* rd_F, float* rd_dF, float* rd_out, int rd_ldout, int T, int nb,
+                       int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dy1 && x && stats && gamma && dx, "null pointer");
+  SGRL_CHECK((dgamma == nullptr) == (dbeta == nullptr), "dgamma and dbeta go together");
+  const int nrd = (rd_y != nullptr) + (rd_F != nullptr) + (rd_dF != nullptr) + (rd_out != nullptr);
+  SGRL_CHECK(nrd == 0 || nrd == 4, "rd_y, rd_F, rd_dF and rd_out go together");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  SGRL_CHECK(ld1 >= D && (!dy2 || ld2 >= D) && ldx >= D && lddx >= D && (!nrd || (rd_ldy >= D && rd_ldout >= D)), "a leading dimension < 128");
+  SGRL_CHECK(al16(gamma, 0, zs_p), "gamma and zs_p must be 16-byte aligned (float4 loads)");
+  return layernorm_bwd_launch(dy1, ld1, dy2, ld2, x, ldx, stats, zs_s, gamma, zs_p, dx, lddx, zs_w, dgamma, dbeta, zs_g,
+                              LnRowdiv{rd_y, rd_F, rd_dF, rd_out, rd_ldy, rd_ldout}, T, nb, ST(stream), grid);
+}
+
+int sgrl_matapply_fwd(const float* Z, const float* M, float* R, int64_t zs_s, int T, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(Z && M && R, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  return matapply_fwd_launch(Z, M, R, zs_s, T, nb, ST(stream), grid);
+}
+
+int sgrl_matapply_bwd(const float* dR, const float* Z, const float* M, const float* F, int64_t zs_s, float* dZ, float* dT, float* dF, int64_t zs_w,
+                      int T, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dR && Z && M && F && dZ && dT && dF, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  return matapply_bwd_launch(dR, Z, M, F, zs_s, dZ, dT, dF, zs_w, T, nb, ST(stream), grid);
+}
+
+int sgrl_matapply_l5_fwd(const float* Z, const float* M, const float* W5, int64_t zs_p, const float* Vg, const float* dV, float* R, float* Vn,
+                         int64_t zs_s, int T, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(Z && M && W5 && Vg && dV && Vn, "null pointer");      // R == NULL: inference pass
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  return matapply_l5_fwd_launch(Z, M, W5, zs_p, Vg, dV, R, Vn, zs_s, T, nb, ST(stream), grid);
+}
+
+int sgrl_matapply_l5_bwd(const float* dVn, const float* W5, int64_t zs_p, const float* Z, const float* M, const float* F, int64_t zs_s, float* dZ,
+                         float* dT, float* dF, int64_t zs_w, int T, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dVn && W5 && Z && M && F && dZ && dT && dF, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  SGRL_CHECK(al16(dVn, 0, zs_w), "dVn and zs_w must be 16-byte aligned (float4 loads)");
+  return matapply_l5_bwd_launch(dVn, W5, zs_p, Z, M, F, zs_s, dZ, dT, dF, zs_w, T, nb, ST(stream), grid);
+}
+
+int sgrl_actor_out_fwd(const float* R, const float* V0, const float* wd, int64_t zs_p, float* W3, float* out, int64_t zs_s, float max_action, int T,
+                       int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(R && V0 && wd && W3 && out, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  return actor_out_fwd_launch(R, V0, wd, zs_p, W3, out, zs_s, max_action, T, nb, ST(stream), grid);
+}
+
+int sgrl_actor_out_bwd(const float* dout, int64_t zs_do, const float* out, const float* R, const float* V0, int64_t zs_s, const float* wd,
+                       int64_t zs_p, float* dR, int64_t zs_w, float* dwd, int64_t zs_g, float max_action, int T, int nb, int32_t* grid,
+                       sgrl_stream_t stream) {
+  SGRL_CHECK(dout && out && R && V0 && wd && dR && dwd, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  return actor_out_bwd_launch(dout, zs_do, out, R, V0, zs_s, wd, zs_p, dR, zs_w, dwd, zs_g, true, max_action, T, nb, ST(stream), grid);
+}
+
+int sgrl_rowdiv_bwd(float* dy, int lddy, int64_t zs_w, const float* y, int ldy, const float* F, int64_t zs_s, float* dF, int N, float colscale,
+                    int cs_n, const float* src, int ldsrc, int64_t zs_src, int T, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dy && y && F && dF, "null pointer");      // src == NULL: dy is read in place
+  SGRL_NETS(nb);
+  SGRL_TOKENS(T);
+  SGRL_CHECK(N >= 1 && lddy >= N && ldy >= N && (!src || ldsrc >= N), "N must be >= 1 and no leading dimension < N");
+  SGRL_CHECK(cs_n >= 0 && cs_n <= N, "cs_n must be 0..N");
+  return rowdiv_bwd_launch(dy, lddy, zs_w, y, ldy, F, zs_s, dF, N, colscale, cs_n, T, src, ldsrc, zs_src, nb, ST(stream), grid);
+}
+
+int sgrl_colsum(const float* X, int ldx, int64_t zs_x, float* out, int64_t zs_o, int M, int N, float alpha, int nb, int32_t* grid,
+                sgrl_stream_t stream) {
+  SGRL_CHECK(X && out, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_CHECK(M >= 0 && N >= 1 && ldx >= N, "M must be >= 0, N >= 1 and ldx >= N");
+  return colsum_launch(X, ldx, zs_x, out, zs_o, M, N, alpha, nb, ST(stream), grid);
+}
+
+int sgrl_block_copy(float* dst, int ldd, int64_t zs_d, const float* src, int lds, int64_t zs_src, const float* src2, int lds2, int64_t zs_src2,
+                    int M, int N, int add, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(dst && src, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_CHECK(M >= 0 && N >= 1 && ldd >= N && lds >= N && (!src2 || lds2 >= N), "M must be >= 0, N >= 1 and no leading dimension < N");
+  return block_copy_launch(dst, ldd, zs_d, src, lds, zs_src, src2, lds2, zs_src2, M, N, add ? 1 : 0, nb, ST(stream), grid);
+}
+
+static int fold_desc_of(const int64_t* src, const int64_t* dst, const int32_t* rows, int n, FoldDesc& d) {
+  SGRL_CHECK(src && dst && rows, "null pointer");
+  SGRL_CHECK(n >= 1 && n <= 2 * MAX_LAYERS + 1, "n must be 1..17");
+  d.n = n;
+  for (int i = 0; i < n; ++i) {
+    SGRL_CHECK(src[i] >= 0 && dst[i] >= 0 && rows[i] >= 1, "offsets must be >= 0, rows >= 1");
+    SGRL_CHECK((dst[i] & 3) == 0, "folded matrices must start 16-byte aligned (the tcgen05 GEMMs read them by TMA)");
+    d.src[i] = src[i]; d.dst[i] = dst[i]; d.rows[i] = rows[i];
+  }
+  return 0;
+}
+
+int sgrl_fold_sym(const float* params, int64_t zs_p, float* wf, int64_t zs_s, int64_t plane, int with_split, const int64_t* src, const int64_t* dst,
+                  const int32_t* rows, int n, int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(params && wf, "null pointer");
+  SGRL_NETS(nb);
+  SGRL_CHECK(al16(wf, 0, zs_s) && (!with_split || (plane & 3) == 0), "the fold planes (wf, zs_s, plane) must be 16-byte aligned (TMA operands)");
+  FoldDesc d;
+  SGRL_TRY(fold_desc_of(src, dst, rows, n, d));
+  return fold_sym_launch(params, zs_p, wf, zs_s, plane, with_split ? 1 : 0, d, nb, ST(stream), grid);
+}
+
+int sgrl_unfold_sym(const float* gf, int64_t zs_w, float* grads, int64_t zs_g, const int64_t* src, const int64_t* dst, const int32_t* rows, int n,
+                    int nb, int32_t* grid, sgrl_stream_t stream) {
+  SGRL_CHECK(gf && grads, "null pointer");
+  SGRL_NETS(nb);
+  FoldDesc d;
+  SGRL_TRY(fold_desc_of(src, dst, rows, n, d));
+  return unfold_sym_launch(gf, zs_w, grads, zs_g, d, nb, ST(stream), grid);
 }
 
 int sgrl_gemm(const float* A, int lda, int trans_a, const float* B, int ldb, int trans_b, float* C, int ldc, int M, int N, int K,

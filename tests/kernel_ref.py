@@ -209,3 +209,245 @@ def gemm_ref(pr, bf16=False):
             _mat(cb, z * d["zs_c"], M, N, d["ldc"]).copy_(mag)
             _mat(cw, z * d["zs_c"], M, N, d["ldc"]).fill_(True)
     return out
+
+
+# ======================================================================================================================
+# The kernels around the projections (csrc/misc.cuh) and the triangle fold (csrc/feature.cuh), in the layouts of their entry
+# points (sgrl_embed_fwd .. sgrl_unfold_sym) for ONE net instance: every operand a dense tensor of that net (the tests slice the
+# instances out of their strided buffers).  Each takes the fp32 values the kernel reads and returns {output: (value, scale)} in
+# float64, scale = the sum of the absolute values of the terms that form each element (the reference on absolute values where
+# the map is linear; stated per kernel where it is not): the size of the rounding error an fp32 kernel can make there.
+# ======================================================================================================================
+S128 = 128.0 ** 0.5
+LN_EPS = 1e-5
+
+
+def _d(t):
+    return None if t is None else t.detach().double()
+
+
+def v0_of(obs):
+    """V0 (T,3,8) with V0[r][j] = obs[3j + r] (SEActor.py:239-245)."""
+    return obs[:, :24].reshape(-1, 8, 3).transpose(1, 2)
+
+
+def pos_rows(E0, E1, E2, rank3):
+    """ConcatPositionalEmbedding of each token: [E0[rank3[t,0]] | E1[rank3[t,1]] | E2[rank3[t,2]]] (T,128)."""
+    r = rank3.long()
+    return torch.cat([E0[r[:, 0]], E1[r[:, 1]], E2[r[:, 2]]], 1)
+
+
+def embed_fwd_ref(obs, act, rank3, Wg, We, be, E0, E1, E2):
+    """sgrl_embed_fwd: obs (T,41), act (T,3) for critics (We (128,20)) or None (We (128,17)).  V0 (T,24), GD (T,6), SH (T,ng),
+    VG (T,3,128), H (T,128)."""
+    obs, act, Wg, We, be = _d(obs), _d(act), _d(Wg), _d(We), _d(be)
+    E0, E1, E2 = _d(E0), _d(E1), _d(E2)
+    V0 = v0_of(obs)
+    s0 = obs[:, 24:] if act is None else torch.cat([obs[:, 24:], act], 1)
+    pos = pos_rows(E0, E1, E2, rank3)
+    out = {"V0": (V0.reshape(-1, 24), None), "GD": (V0[:, :, 1:3].reshape(-1, 6), None), "SH": (s0, None),
+           "VG": (S128 * V0 @ Wg.T, S128 * V0.abs() @ Wg.abs().T),
+           "H": (S128 * (s0 @ We.T + be) + pos, S128 * (s0.abs() @ We.abs().T + be.abs()) + pos.abs())}
+    return out
+
+
+def _graph_gather(cu_limbs):
+    """[(token indices (ng, n))] of the packed batch, one entry per graph size."""
+    return [tok for _, (_, tok) in _graphs_by_size(cu_limbs).items()]
+
+
+def _ingrad_loss(x, a, cu_limbs, L):
+    """sum of <upstream, linear map of obs x> over every term input_grad_kernel gathers (csrc/misc.cuh), with the upstream
+    gradients and coefficients in `a` (absolute values for the scale)."""
+    V0 = v0_of(x)                                   # (T,3,8)
+    s0 = x[:, 24:41]
+    gd = V0[:, :, 1:3]                              # (T,3,2)
+    loss = (a["dvg0"] * (S128 * V0 @ a["Wg"].T)).sum()                                 # Vg0 = sqrt(128) V0 Wg^T
+    loss = loss + (a["dh0"] * (S128 * s0 @ a["We"][:, :17].T)).sum()                   # h0 = sqrt(128) We s0 (+ be + pos)
+    for dz, W in ((a["dzh"], a["gg"]), (a["dzh2"], a["gph"])):                         # head invariants [V0 P[:, :8]^T | gd]
+        if dz is not None:
+            loss = loss + (dz[:, :, :30] * (V0 @ W[:, :8].T)).sum() + (dz[:, :, 30:32] * gd).sum()
+    loss = loss + (a["dsh"][:, :17] * s0).sum()                                        # [s0 | h] -> linear1_ng
+    for s in range(3 * L):                                                             # gd columns of every layer's Z1, Z2, Z3
+        loss = loss + (a["dz"][s][:, :, 30:32] * gd).sum()
+    for tok in _graph_gather(cu_limbs):                                                # gd in channels 126, 127 of the values
+        tok = tok.to(x.device)
+        n = tok.shape[1]
+        g = gd[tok]                                                                    # (ng, n, 3, 2): key j
+        for l in range(L):
+            P = a["P"][l][tok][..., :n]                                                # (ng, n, 2, n): query i, head h, key j
+            og = torch.einsum("gihj,gjrk->girhk", P, g)
+            d = a["dog"][l][tok].view(*tok.shape, 3, 2, 128)[..., 126:128]             # (ng, n, 3, 2, 2)
+            loss = loss + (d * og).sum()
+    if a["dy"] is not None:                                                            # out_i = max_action tanh(sum_r V0[r][5+i] w_r)
+        p = torch.einsum("tri,tr->ti", V0[:, :, 5:8], a["w3"])
+        loss = loss + (a["dy"] * p).sum()
+    return loss
+
+
+def input_grad_ref(dvg0, dh0, dzh, dzh2, dsh, dz, dog, P, Wg, We, gg, gph, dout, out, w3, max_action, cu_limbs, L):
+    """sgrl_input_grad for one net: d obs (T,41) = the gradient of _ingrad_loss.  dz: 3L tensors (T,3,32), dog: L (T,768),
+    P: L (T,2,16); actor: dzh2 (T,3,32), gph (30,136), dout, out, w3 (T,3) (dy = dout max_action (1 - (out/max_action)^2), from
+    the stored out as the kernel forms it), critic: all None.  Returns {"dobs": (value, scale)}."""
+    T = dvg0.shape[0]
+    a = {"dvg0": _d(dvg0).reshape(T, 3, 128), "dh0": _d(dh0).reshape(T, 128), "dzh": _d(dzh).reshape(T, 3, 32),
+         "dzh2": None if dzh2 is None else _d(dzh2).reshape(T, 3, 32), "dsh": _d(dsh), "Wg": _d(Wg), "We": _d(We), "gg": _d(gg),
+         "gph": _d(gph), "dz": [_d(t).reshape(T, 3, 32) for t in dz[:3 * L]], "dog": [_d(t).reshape(T, 768) for t in dog[:L]],
+         "P": [_d(t).reshape(T, 2, 16) for t in P[:L]], "dy": None, "w3": _d(w3)}
+    if dzh2 is not None:
+        o = _d(out) / float(max_action)
+        a["dy"] = _d(dout) * float(max_action) * (1.0 - o * o)
+        a["dy_abs"] = _d(dout).abs() * float(max_action) * (1.0 + o * o)
+    res = []
+    for absval in (False, True):
+        b = a
+        if absval:
+            b = {k: (None if v is None else [t.abs() for t in v] if isinstance(v, list) else v.abs()) for k, v in a.items()}
+            if a["dy"] is not None:
+                b["dy"] = a["dy_abs"]
+        x = torch.zeros(T, 41, dtype=torch.float64, device=dvg0.device, requires_grad=True)
+        with torch.enable_grad():
+            (g,) = torch.autograd.grad(_ingrad_loss(x, b, cu_limbs, L), x)
+        res.append(g)
+    return {"dobs": tuple(res)}
+
+
+def pos_embed_bwd_ref(dH, rank3):
+    """sgrl_pos_embed_bwd: the gradients (15,42), (15,42), (15,44) of the three positional tables from dH (T,128)."""
+    dH, r = _d(dH), rank3.long()
+    out = {}
+    for i, (c0, c1) in enumerate(((0, 42), (42, 84), (84, 128))):
+        for name, src in (("v", dH), ("s", dH.abs())):
+            t = torch.zeros(15, c1 - c0, dtype=torch.float64, device=dH.device).index_add_(0, r[:, i], src[:, c0:c1])
+            out.setdefault(f"dE{i}", []).append(t)
+    return {k: tuple(v) for k, v in out.items()}
+
+
+def layernorm_fwd_ref(a, b, gamma, beta):
+    """sgrl_layernorm_fwd: x = a + b (b None: x = a), y = (x - mean) rstd gamma + beta, rstd = (var + 1e-5)^-1/2, stats (T,2).
+    Scales: x |a| + |b|; y |gamma| rstd (|x| + mean(|x|)) + |beta| (the rounding of x and of the mean, amplified by rstd); mean
+    mean(|x|); rstd rstd (1 + mean(|x|) rstd) (the deviations' rounding relative to the standard deviation)."""
+    a, b, g, be = _d(a), _d(b), _d(gamma), _d(beta)
+    x = a if b is None else a + b
+    xs = a.abs() if b is None else a.abs() + b.abs()
+    mean = x.mean(1, keepdim=True)
+    var = ((x - mean) ** 2).mean(1, keepdim=True)
+    rstd = (var + LN_EPS).rsqrt()
+    y = (x - mean) * rstd * g + be
+    ax = x.abs().mean(1, keepdim=True)
+    return {"x": (x, xs), "y": (y, g.abs() * rstd * (x.abs() + ax) + be.abs()),
+            "mean": (mean[:, 0], ax[:, 0]), "rstd": (rstd[:, 0], (rstd * (1.0 + ax * rstd))[:, 0])}
+
+
+def layernorm_bwd_ref(dy1, dy2, x, stats, gamma, rd_y=None, rd_F=None):
+    """sgrl_layernorm_bwd from the stored stats (mean, rstd): with dy = dy1 + dy2 and xh = (x - mean) rstd,
+    dx = rstd (g dy - mean(g dy) - xh mean(g dy xh)), dgamma = sum_t dy xh, dbeta = sum_t dy; the tail (rd_y, rd_F given):
+    out = dx / F, dF = -<dx, y> / F.  Scales: the same expressions on absolute values."""
+    dy = _d(dy1) if dy2 is None else _d(dy1) + _d(dy2)
+    dys = _d(dy1).abs() if dy2 is None else _d(dy1).abs() + _d(dy2).abs()
+    st, g = _d(stats), _d(gamma)
+    mean, rstd = st[:, :1], st[:, 1:2]
+    xh = (_d(x) - mean) * rstd
+    gd = g * dy
+    s1, s2 = gd.mean(1, keepdim=True), (gd * xh).mean(1, keepdim=True)
+    dx = rstd * (gd - s1 - xh * s2)
+    gds = g.abs() * dys
+    dxs = rstd * (gds + gds.mean(1, keepdim=True) + xh.abs() * (gds * xh.abs()).mean(1, keepdim=True))
+    out = {"dx": (dx, dxs), "dgamma": ((dy * xh).sum(0), (dys * xh.abs()).sum(0)), "dbeta": (dy.sum(0), dys.sum(0))}
+    if rd_y is not None:
+        F, y = _d(rd_F).reshape(-1, 1), _d(rd_y)
+        out["rd_out"] = (dx / F, dxs / F.abs())
+        out["rd_dF"] = (-(dx * y).sum(1) / F[:, 0], (dxs * y.abs()).sum(1) / F[:, 0].abs())
+    return out
+
+
+def matapply_fwd_ref(Z, M):
+    """sgrl_matapply_fwd: R = Z (3x32) M (32x32) per token; Z (T,3,32), M (T,32,32)."""
+    Z, M = _d(Z).reshape(-1, 3, 32), _d(M).reshape(-1, 32, 32)
+    return {"R": (Z @ M, Z.abs() @ M.abs())}
+
+
+def _matapply_bwd(dR, dRs, Z, M, F):
+    dM, dMs = Z.transpose(1, 2) @ dR, Z.abs().transpose(1, 2) @ dRs
+    F = F.reshape(-1, 1, 1)
+    return {"dZ": (dR @ M.transpose(1, 2), dRs @ M.abs().transpose(1, 2)), "dT": (dM / F, dMs / F.abs()),
+            "dF": (-(dM * M).sum((1, 2)) / F[:, 0, 0], (dMs * M.abs()).sum((1, 2)) / F[:, 0, 0].abs())}
+
+
+def matapply_bwd_ref(dR, Z, M, F):
+    """sgrl_matapply_bwd with M = Tm / F: dZ = dR M^T, dT = Z^T dR / F, dF = -<Z^T dR, M> / F."""
+    dR = _d(dR).reshape(-1, 3, 32)
+    return _matapply_bwd(dR, dR.abs(), _d(Z).reshape(-1, 3, 32), _d(M).reshape(-1, 32, 32), _d(F))
+
+
+def matapply_l5_fwd_ref(Z, M, W5, Vg, dV):
+    """sgrl_matapply_l5_fwd: R = Z M, Vn = Vg + dV + R W5^T; W5 (128,32), Vg, dV (T,3,128)."""
+    r = matapply_fwd_ref(Z, M)["R"]
+    W5, Vg, dV = _d(W5), _d(Vg).reshape(-1, 3, 128), _d(dV).reshape(-1, 3, 128)
+    return {"R": r, "Vn": (Vg + dV + r[0] @ W5.T, Vg.abs() + dV.abs() + r[1] @ W5.abs().T)}
+
+
+def matapply_l5_bwd_ref(dVn, W5, Z, M, F):
+    """sgrl_matapply_l5_bwd: dR = dVn W5, then matapply_bwd_ref's math."""
+    dVn, W5 = _d(dVn).reshape(-1, 3, 128), _d(W5)
+    return _matapply_bwd(dVn @ W5, dVn.abs() @ W5.abs(), _d(Z).reshape(-1, 3, 32), _d(M).reshape(-1, 32, 32), _d(F))
+
+
+def actor_out_fwd_ref(R, V0, wd, max_action):
+    """sgrl_actor_out_fwd: w_r = sum_c R[r][c] wd[c] (W3), p_i = sum_r V0[r][5+i] w_r, out = max_action tanh(p).  Scale of out:
+    max_action ((1 - tanh^2) scale(p) + |tanh p|) (the argument's rounding through the slope, and tanhf's own)."""
+    R, V0, wd = _d(R).reshape(-1, 3, 32), _d(V0).reshape(-1, 3, 8), _d(wd).reshape(32)
+    w, ws = R @ wd, R.abs() @ wd.abs()
+    ax = V0[:, :, 5:8]
+    p = torch.einsum("tri,tr->ti", ax, w)
+    ps = torch.einsum("tri,tr->ti", ax.abs(), ws)
+    a = torch.tanh(p)
+    return {"W3": (w, ws), "out": (max_action * a, max_action * ((1 - a * a) * ps + a.abs())), "p": (p, ps)}
+
+
+def actor_out_bwd_ref(dout, out, R, V0, wd, max_action):
+    """sgrl_actor_out_bwd from the stored out: a = out / max_action, dp = dout max_action (1 - a^2), dw_r = sum_i dp_i V0[r][5+i],
+    dR = dw wd^T, dwd = sum_t sum_r dw_r R[r]."""
+    a = _d(out) / float(max_action)
+    do = _d(dout)
+    dp, dps = do * float(max_action) * (1 - a * a), do.abs() * float(max_action) * (1 + a * a)
+    R, V0, wd = _d(R).reshape(-1, 3, 32), _d(V0).reshape(-1, 3, 8), _d(wd).reshape(32)
+    ax = V0[:, :, 5:8]
+    dw, dws = torch.einsum("tri,ti->tr", ax, dp), torch.einsum("tri,ti->tr", ax.abs(), dps)
+    return {"dR": (dw[..., None] * wd, dws[..., None] * wd.abs()),
+            "dwd": ((dw[..., None] * R).sum((0, 1)), (dws[..., None] * R.abs()).sum((0, 1)))}
+
+
+def rowdiv_bwd_ref(g, y, F, colscale, cs_n):
+    """sgrl_rowdiv_bwd: with y = t / F (* colscale on columns < cs_n) and upstream g (T,N): dt = g cs / F, dF = -<g, y> / F."""
+    g, y, F = _d(g), _d(y), _d(F).reshape(-1, 1)
+    cs = torch.ones(g.shape[1], dtype=torch.float64, device=g.device)
+    cs[:cs_n] = float(colscale)
+    return {"dt": (g * cs / F, g.abs() * cs.abs() / F.abs()),
+            "dF": (-(g * y).sum(1) / F[:, 0], (g.abs() * y.abs()).sum(1) / F[:, 0].abs())}
+
+
+def colsum_ref(X, alpha):
+    """sgrl_colsum: alpha * sum_m X[m][n] (added to the output)."""
+    X = _d(X)
+    return {"out": (float(alpha) * X.sum(0), abs(float(alpha)) * X.abs().sum(0))}
+
+
+def fold_ref(W):
+    """sgrl_fold_sym of one (rows,1024) weight in fp32, as the kernel adds: W'[o][p(i,j)] = W[o][32i+j] + W[o][32j+i] (i < j),
+    W[o][33i] (i = j), in the slots of packing.pack_indices(); the 16 padding slots 0."""
+    slots, ri, ci = pack_indices()
+    ri, ci = torch.tensor(ri, device=W.device), torch.tensor(ci, device=W.device)
+    Wf = W.new_zeros(W.shape[0], GP_K)
+    Wf[:, slots] = torch.where(ri == ci, W[:, ri * 32 + ci], W[:, ri * 32 + ci] + W[:, ci * 32 + ri])
+    return Wf
+
+
+def unfold_ref(gf):
+    """sgrl_unfold_sym's term for one (rows,544) folded gradient: dW[o][32a+b] = gf[o][p(min(a,b), max(a,b))] (rows,1024)."""
+    slots, ri, ci = pack_indices()
+    dW = gf.new_zeros(gf.shape[0], 32, 32)
+    ri, ci, sl = (torch.tensor(v, device=gf.device) for v in (ri, ci, slots))
+    dW[:, ri, ci] = gf[:, sl]
+    dW[:, ci, ri] = gf[:, sl]
+    return dW.reshape(-1, 1024)

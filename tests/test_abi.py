@@ -167,3 +167,111 @@ def test_gemm_refuses_bias_or_store_with_split_k():
         assert b"accumulate = 1" in lib.sgrl_last_error()
     assert lib.sgrl_gemm_presplit(f, 64, 1, f, f, 64, 1, f, 64, 30, 128, 2304, 1.0, f, None, 0, 1, 8, None) < 0
     assert b"no bias" in lib.sgrl_last_error()
+
+
+_F = 1 << 20          # fake, never dereferenced, 16-byte aligned device addresses
+_ARGS = {             # a valid call of each single-kernel entry point (ABI 11), argument by argument, grid and stream at the end
+    "sgrl_embed_fwd": dict(obs=_F, zs_obs=0, act=None, zs_act=0, rank3=_F, Wg=_F, We=_F, be=_F, E0=_F, E1=_F, E2=_F, zs_p=0, V0=_F, GD=_F,
+                           SH=_F, ldsh=145, VG=_F, H=_F, ldh=256, zs_s=0, T=100, ng=17, nb=2, in_nets=1),
+    "sgrl_input_grad": dict(dvg0=_F, dh0=_F, dzh=_F, dzh2=_F, dsh=_F, ldsh=145, dz="dz", dog="dog", P="P", Wg=_F, We=_F, gg=_F, gph=_F, ng=17,
+                            dout=_F, zs_do=0, out=_F, w3=_F, max_action=1.0, dobs=_F, zs_dobs=0, cu_limbs=_F, G=10, T=100, L=3, zs_w=0,
+                            zs_s=0, zs_p=0, nb=1),
+    "sgrl_pos_embed_bwd": dict(dH=_F, ldh=128, zs_w=0, rank3=_F, dE0=_F, dE1=_F, dE2=_F, zs_g=0, T=100, nb=1),
+    "sgrl_layernorm_fwd": dict(a=_F, lda=256, b=None, ldb=0, gamma=_F, beta=_F, zs_p=0, x=_F, y=_F, ldy=145, y2=None, ldy2=0, stats=_F,
+                               zs_s=0, T=100, nb=1),
+    "sgrl_layernorm_bwd": dict(dy1=_F, ld1=128, dy2=None, ld2=0, x=_F, ldx=128, stats=_F, zs_s=0, gamma=_F, zs_p=0, dx=_F, lddx=128, zs_w=0,
+                               dgamma=_F, dbeta=_F, zs_g=0, rd_y=None, rd_ldy=0, rd_F=None, rd_dF=None, rd_out=None, rd_ldout=0, T=100,
+                               nb=1),
+    "sgrl_matapply_fwd": dict(Z=_F, M=_F, R=_F, zs_s=0, T=100, nb=1),
+    "sgrl_matapply_bwd": dict(dR=_F, Z=_F, M=_F, F=_F, zs_s=0, dZ=_F, dT=_F, dF=_F, zs_w=0, T=100, nb=1),
+    "sgrl_matapply_l5_fwd": dict(Z=_F, M=_F, W5=_F, zs_p=0, Vg=_F, dV=_F, R=None, Vn=_F, zs_s=0, T=100, nb=1),
+    "sgrl_matapply_l5_bwd": dict(dVn=_F, W5=_F, zs_p=0, Z=_F, M=_F, F=_F, zs_s=0, dZ=_F, dT=_F, dF=_F, zs_w=0, T=100, nb=1),
+    "sgrl_actor_out_fwd": dict(R=_F, V0=_F, wd=_F, zs_p=0, W3=_F, out=_F, zs_s=0, max_action=1.0, T=100, nb=1),
+    "sgrl_actor_out_bwd": dict(dout=_F, zs_do=0, out=_F, R=_F, V0=_F, zs_s=0, wd=_F, zs_p=0, dR=_F, zs_w=0, dwd=_F, zs_g=0, max_action=1.0,
+                               T=100, nb=1),
+    "sgrl_rowdiv_bwd": dict(dy=_F, lddy=768, zs_w=0, y=_F, ldy=768, F=_F, zs_s=0, dF=_F, N=768, colscale=0.5, cs_n=256, src=None, ldsrc=0,
+                            zs_src=0, T=100, nb=1),
+    "sgrl_colsum": dict(X=_F, ldx=128, zs_x=0, out=_F, zs_o=0, M=100, N=128, alpha=1.0, nb=1),
+    "sgrl_block_copy": dict(dst=_F, ldd=3, zs_d=0, src=_F, lds=3, zs_src=0, src2=None, lds2=0, zs_src2=0, M=100, N=3, add=0, nb=1),
+    "sgrl_fold_sym": dict(params=_F, zs_p=0, wf=_F, zs_s=0, plane=1024, with_split=1, src="src", dst="dst", rows="rows", n=7, nb=1),
+    "sgrl_unfold_sym": dict(gf=_F, zs_w=0, grads=_F, zs_g=0, src="src", dst="dst", rows="rows", n=7, nb=1),
+}
+
+
+def _call(name, **over):
+    from sgrl_b200 import _lib
+    a = dict(_ARGS[name], **over)
+    host = {"dz": (ctypes.c_void_p * 24)(*([_F] * 24)), "dog": (ctypes.c_void_p * 8)(*([_F] * 8)), "P": (ctypes.c_void_p * 8)(*([_F] * 8)),
+            "src": (ctypes.c_int64 * 17)(*([0] * 17)), "dst": (ctypes.c_int64 * 17)(*([544 * 256 * i for i in range(17)])),
+            "rows": (ctypes.c_int32 * 17)(*([256] * 17))}
+    vals = [host[v] if isinstance(v, str) else v for v in a.values()]
+    return getattr(_lib.lib, name)(*vals, None, None)
+
+
+@pytest.mark.parametrize("name,over,msg", [
+    ("sgrl_embed_fwd", dict(obs=None), b"null pointer"),
+    ("sgrl_embed_fwd", dict(ng=18), b"ng must be 17"),
+    ("sgrl_embed_fwd", dict(act=_F), b"act is read by critics"),                    # actor layout with an action
+    ("sgrl_embed_fwd", dict(ng=20), b"act is read by critics"),                     # critic without one
+    ("sgrl_embed_fwd", dict(nb=17), b"nb must be 1..16"),
+    ("sgrl_embed_fwd", dict(nb=0), b"nb must be 1..16"),
+    ("sgrl_embed_fwd", dict(in_nets=3), b"in_nets must be 1..nb"),
+    ("sgrl_embed_fwd", dict(in_nets=0), b"in_nets must be 1..nb"),
+    ("sgrl_embed_fwd", dict(T=-1), b"T must be >= 0"),
+    ("sgrl_input_grad", dict(dobs=None), b"null pointer"),
+    ("sgrl_input_grad", dict(L=0), b"L must be 1..8"),
+    ("sgrl_input_grad", dict(L=9), b"L must be 1..8"),
+    ("sgrl_input_grad", dict(ng=20), b"dzh2"),                                      # actor head with the critic's ng
+    ("sgrl_input_grad", dict(dzh2=None), b"dzh2"),                                  # critic head with the actor's ng
+    ("sgrl_input_grad", dict(ng=19, dzh2=None), b"ng must be 17"),
+    ("sgrl_input_grad", dict(w3=None), b"needs gph, dout, out and w3"),
+    ("sgrl_input_grad", dict(dog=None), b"null pointer"),
+    ("sgrl_input_grad", dict(zs_w=3), b"8-byte aligned"),                           # float2 loads of d og
+    ("sgrl_input_grad", dict(nb=17), b"nb must be 1..16"),
+    ("sgrl_input_grad", dict(T=-5), b"T must be >= 0"),
+    ("sgrl_pos_embed_bwd", dict(rank3=None), b"null pointer"),
+    ("sgrl_pos_embed_bwd", dict(nb=0), b"nb must be 1..16"),
+    ("sgrl_layernorm_fwd", dict(stats=None), b"null pointer"),
+    ("sgrl_layernorm_fwd", dict(gamma=_F + 4), b"gamma, beta and zs_p"),
+    ("sgrl_layernorm_fwd", dict(beta=_F + 8), b"gamma, beta and zs_p"),
+    ("sgrl_layernorm_fwd", dict(zs_p=6), b"gamma, beta and zs_p"),
+    ("sgrl_layernorm_fwd", dict(x=_F + 4), b"x and zs_s"),
+    ("sgrl_layernorm_fwd", dict(zs_s=2), b"x and zs_s"),
+    ("sgrl_layernorm_fwd", dict(T=-1), b"T must be >= 0"),
+    ("sgrl_layernorm_bwd", dict(dx=None), b"null pointer"),
+    ("sgrl_layernorm_bwd", dict(dbeta=None), b"dgamma and dbeta go together"),
+    ("sgrl_layernorm_bwd", dict(rd_y=_F, rd_ldy=128), b"go together"),
+    ("sgrl_layernorm_bwd", dict(gamma=_F + 12), b"gamma and zs_p"),
+    ("sgrl_layernorm_bwd", dict(nb=17), b"nb must be 1..16"),
+    ("sgrl_matapply_fwd", dict(R=None), b"null pointer"),
+    ("sgrl_matapply_bwd", dict(dF=None), b"null pointer"),
+    ("sgrl_matapply_l5_fwd", dict(Vn=None), b"null pointer"),
+    ("sgrl_matapply_l5_bwd", dict(dVn=_F + 4), b"dVn and zs_w"),
+    ("sgrl_matapply_l5_bwd", dict(zs_w=2), b"dVn and zs_w"),
+    ("sgrl_actor_out_fwd", dict(nb=17), b"nb must be 1..16"),
+    ("sgrl_actor_out_bwd", dict(dwd=None), b"null pointer"),
+    ("sgrl_rowdiv_bwd", dict(cs_n=769), b"cs_n must be 0..N"),
+    ("sgrl_rowdiv_bwd", dict(T=-1), b"T must be >= 0"),
+    ("sgrl_colsum", dict(N=0), b"N >= 1"),
+    ("sgrl_block_copy", dict(src=None), b"null pointer"),
+    ("sgrl_fold_sym", dict(n=18), b"n must be 1..17"),
+    ("sgrl_fold_sym", dict(n=0), b"n must be 1..17"),
+    ("sgrl_fold_sym", dict(wf=_F + 4), b"fold planes"),
+    ("sgrl_fold_sym", dict(plane=1022), b"fold planes"),
+    ("sgrl_fold_sym", dict(zs_s=5), b"fold planes"),
+    ("sgrl_unfold_sym", dict(rows=None), b"null pointer"),
+    ("sgrl_unfold_sym", dict(nb=17), b"nb must be 1..16"),
+])
+def test_single_kernel_entry_points_refuse_bad_arguments(name, over, msg):
+    """Every single-kernel entry point refuses a call its kernel cannot run, before anything is enqueued (fake addresses: a call
+    that got as far as a launch would fault, so a refusal is the only way to pass here)."""
+    from sgrl_b200 import _lib
+    rc = _call(name, **over)
+    assert rc < 0 and msg in _lib.lib.sgrl_last_error(), _lib.lib.sgrl_last_error()
+
+
+def test_single_kernel_entry_points_are_abi_11():
+    from sgrl_b200 import _lib
+    assert _lib.lib.sgrl_version() == 11
+    for name, args in _ARGS.items():
+        assert len(getattr(_lib.lib, name).argtypes) == len(args) + 2, name

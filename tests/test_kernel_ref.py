@@ -264,3 +264,224 @@ def test_gemm_ref_gram_rows_follow_pack_indices():
             assert abs(out["gram_f"][0][z * zs + m].item() - (G.norm().item() + 1.0)) < 1e-12 * G.norm().item()
             assert rel(out["C"][0][z * M * N + m * N: z * M * N + (m + 1) * N], W.reshape(N, GP_K) @ row) < TOL
     assert len(set(slots)) == 528
+
+
+# ---- the kernels around the projections (csrc/misc.cuh) and the triangle fold -------------------------------------------------
+def _embed_inputs(name, B, kind):
+    """Oracle parameters (fp64), the network input x (B,N,41|44), the graph and the packed per-token operands of the embedding."""
+    par = M.ALL[name]
+    N = len(par)
+    g = G.build_graph(par)
+    p = {k: v.double() for k, v in O.synth_params(kind, 5).items()}
+    b = synth.make_batch(B, N, seed=4)
+    obs = b["obs"].view(B * N, 41).double()
+    act = b["action"].view(B * N, 3).double() if kind == "critic" else None
+    rank3 = torch.stack(g["traversals"], 1).repeat(B, 1).int()                 # (T,3): token t = limb t % N
+    return p, g, obs, act, rank3, N
+
+
+@pytest.mark.parametrize("name,B", CASES)
+@pytest.mark.parametrize("kind", ["actor", "critic"])
+def test_embed_fwd_ref_reproduces_oracle(name, B, kind):
+    """embed_fwd_ref's V0, GD, SH, VG and H against the input stage of transformer_model (trace V0, GD, SH, 0.VGIN) and
+    pos_embedding: h0 = (We s0 + be) sqrt(128) + pos."""
+    p, g, obs, act, rank3, N = _embed_inputs(name, B, kind)
+    T = B * N
+    x = obs.view(B, N, 41) if act is None else torch.cat([obs.view(B, N, 41), act.view(B, N, 3)], 2)
+    tr = {}
+    with torch.no_grad():
+        O.transformer_model(p, x, dict(g, relation=g["relation"].double()), trace=tr)
+    E = [p[f"pos_encoder.embeddings.{i}.weight"] for i in range(3)]
+    r = R.embed_fwd_ref(obs, act, rank3, p["g_encoder.weight"], p["encoder.weight"], p["encoder.bias"], *E)
+    assert rel(r["V0"][0], _tok(tr["V0"], T)) < TOL and rel(r["GD"][0], _tok(tr["GD"], T)) < TOL
+    ng = 17 if kind == "actor" else 20
+    assert rel(r["SH"][0], _tok(tr["SH"], T)[:, :ng]) < TOL
+    assert rel(r["VG"][0].reshape(T, -1), _tok(tr["0.VGIN"], T)) < TOL
+    s0 = x.reshape(T, -1)[:, 24:]
+    h0 = (s0 @ p["encoder.weight"].T + p["encoder.bias"]) * 128 ** 0.5 + O.pos_embedding(p, g["traversals"]).repeat(B, 1)
+    assert rel(r["H"][0], h0) < TOL
+    for k in ("VG", "H"):
+        assert bool((r[k][1] >= r[k][0].abs()).all())
+
+
+@pytest.mark.parametrize("a_mean,a_std", [(0.0, 1.0), (1e3, 1e-2), (5.0, 0.0)])
+@pytest.mark.parametrize("resid", [False, True])
+def test_layernorm_fwd_ref_matches_torch(a_mean, a_std, resid):
+    gen = torch.Generator().manual_seed(int(a_mean) + resid)
+    T = 6
+    a = a_mean + a_std * torch.randn(T, 128, generator=gen, dtype=torch.float64)
+    b = 0.1 * a_std * torch.randn(T, 128, generator=gen, dtype=torch.float64) if resid else None
+    gamma, beta = torch.randn(128, generator=gen, dtype=torch.float64), torch.randn(128, generator=gen, dtype=torch.float64)
+    r = R.layernorm_fwd_ref(a, b, gamma, beta)
+    x = a if b is None else a + b
+    y = torch.nn.functional.layer_norm(x, (128,), gamma, beta, eps=1e-5)
+    assert bool(((r["y"][0] - y).abs() <= 1e-13 * r["y"][1]).all())        # torch's fp64 rounding, within the stated scale
+    assert rel(r["x"][0], x) < TOL
+    assert rel(r["mean"][0], x.mean(1)) < TOL
+    assert bool(((r["rstd"][0] - 1 / (x.var(1, unbiased=False) + 1e-5).sqrt()).abs() <= 1e-13 * r["rstd"][1]).all())
+
+
+@pytest.mark.parametrize("tail", [False, True])
+@pytest.mark.parametrize("second", [False, True])
+def test_layernorm_bwd_ref_matches_autograd(tail, second):
+    """dx, dgamma, dbeta against autograd of <dy1 + dy2, LN(a + f)>; with the tail f = t / F also d t (rd_out) and d F (rd_dF)."""
+    gen = torch.Generator().manual_seed(tail * 2 + second)
+    T = 5
+    a = torch.randn(T, 128, generator=gen, dtype=torch.float64)
+    t = torch.randn(T, 128, generator=gen, dtype=torch.float64).requires_grad_(True)
+    Fn = (torch.rand(T, generator=gen, dtype=torch.float64) * 3 + 0.5).requires_grad_(True)
+    gamma = torch.randn(128, generator=gen, dtype=torch.float64).requires_grad_(True)
+    beta = torch.randn(128, generator=gen, dtype=torch.float64).requires_grad_(True)
+    dy1 = torch.randn(T, 128, generator=gen, dtype=torch.float64)
+    dy2 = torch.randn(T, 128, generator=gen, dtype=torch.float64) if second else None
+    ain = a.clone().requires_grad_(True)
+    f = t / Fn[:, None]
+    x = ain + f if tail else ain
+    y = torch.nn.functional.layer_norm(x, (128,), gamma, beta, eps=1e-5)
+    dy = dy1 if dy2 is None else dy1 + dy2
+    (y * dy).sum().backward()
+    fw = R.layernorm_fwd_ref(x.detach(), None, gamma.detach(), beta.detach())
+    stats = torch.stack([fw["mean"][0], fw["rstd"][0]], 1)
+    r = R.layernorm_bwd_ref(dy1, dy2, x.detach(), stats, gamma, f.detach() if tail else None, Fn.detach() if tail else None)
+    assert rel(r["dx"][0], ain.grad) < 1e-12
+    assert rel(r["dgamma"][0], gamma.grad) < 1e-12 and rel(r["dbeta"][0], beta.grad) < 1e-12
+    if tail:
+        assert rel(r["rd_out"][0], t.grad) < 1e-12 and rel(r["rd_dF"][0], Fn.grad) < 1e-12
+
+
+def test_matapply_refs_match_autograd():
+    """matapply_bwd_ref with M = Tm / F and matapply_l5_bwd_ref (dR = dVn W5) against autograd of the forward references."""
+    gen = torch.Generator().manual_seed(11)
+    T = 4
+    Z = torch.randn(T, 3, 32, generator=gen, dtype=torch.float64).requires_grad_(True)
+    Tm = torch.randn(T, 32, 32, generator=gen, dtype=torch.float64).requires_grad_(True)
+    Fn = (torch.rand(T, generator=gen, dtype=torch.float64) * 2 + 0.1).requires_grad_(True)
+    W5 = torch.randn(128, 32, generator=gen, dtype=torch.float64).requires_grad_(True)
+    Vg, dV = torch.randn(T, 3, 128, generator=gen, dtype=torch.float64), torch.randn(T, 3, 128, generator=gen, dtype=torch.float64)
+    Mm = Tm / Fn[:, None, None]
+    dR = torch.randn(T, 3, 32, generator=gen, dtype=torch.float64)
+    R0 = Z @ Mm
+    assert rel(R.matapply_fwd_ref(Z, Mm)["R"][0], R0) < TOL
+    (R0 * dR).sum().backward()
+    r = R.matapply_bwd_ref(dR, Z, Mm.detach(), Fn)
+    assert rel(r["dZ"][0], Z.grad) < 1e-12 and rel(r["dT"][0], Tm.grad) < 1e-12 and rel(r["dF"][0], Fn.grad) < 1e-12
+    Z.grad = Tm.grad = Fn.grad = None
+    Mm = Tm / Fn[:, None, None]
+    f5 = R.matapply_l5_fwd_ref(Z, Mm, W5, Vg, dV)
+    Vn = Vg + dV + (Z @ Mm) @ W5.T
+    assert rel(f5["Vn"][0], Vn) < TOL and rel(f5["R"][0], Z @ Mm) < TOL
+    dVn = torch.randn(T, 3, 128, generator=gen, dtype=torch.float64)
+    (Vn * dVn).sum().backward()
+    r = R.matapply_l5_bwd_ref(dVn, W5, Z, Mm.detach(), Fn)
+    assert rel(r["dZ"][0], Z.grad) < 1e-12 and rel(r["dT"][0], Tm.grad) < 1e-12 and rel(r["dF"][0], Fn.grad) < 1e-12
+
+
+@pytest.mark.parametrize("max_action", [0.4, 2.5])
+def test_actor_out_refs_match_oracle_and_autograd(max_action):
+    """actor_out_fwd_ref against the oracle's actor head (transformer_model's output axes . w, then SEPolicy's tanh), and
+    actor_out_bwd_ref (from the stored out) against autograd of <dout, out> w.r.t. R and wd."""
+    gen = torch.Generator().manual_seed(int(max_action * 10))
+    T = 6
+    Rh = torch.randn(T, 3, 32, generator=gen, dtype=torch.float64).requires_grad_(True)
+    V0 = torch.randn(T, 3, 8, generator=gen, dtype=torch.float64)
+    wd = torch.randn(1, 32, generator=gen, dtype=torch.float64).requires_grad_(True)
+    w = torch.nn.functional.linear(Rh, wd).squeeze(-1)                         # set_oracle.transformer_model :275-285
+    out = max_action * torch.tanh(torch.einsum("bri,br->bi", V0[..., 5:8], w))
+    f = R.actor_out_fwd_ref(Rh, V0, wd, max_action)
+    assert rel(f["out"][0], out) < TOL and rel(f["W3"][0], w) < TOL
+    dout = torch.randn(T, 3, generator=gen, dtype=torch.float64)
+    (out * dout).sum().backward()
+    b = R.actor_out_bwd_ref(dout, out.detach(), Rh, V0, wd, max_action)
+    assert rel(b["dR"][0], Rh.grad) < 1e-12 and rel(b["dwd"][0], wd.grad[0]) < 1e-12
+
+
+def test_rowdiv_and_pos_embed_bwd_refs_match_autograd():
+    gen = torch.Generator().manual_seed(3)
+    T, N = 5, 40
+    t = torch.randn(T, N, generator=gen, dtype=torch.float64).requires_grad_(True)
+    Fn = (torch.rand(T, generator=gen, dtype=torch.float64) * 5 + 0.05).requires_grad_(True)
+    cs = torch.ones(N, dtype=torch.float64)
+    cs[:7] = 0.3
+    y = t / Fn[:, None] * cs
+    g = torch.randn(T, N, generator=gen, dtype=torch.float64)
+    (y * g).sum().backward()
+    r = R.rowdiv_bwd_ref(g, y.detach(), Fn, 0.3, 7)
+    assert rel(r["dt"][0], t.grad) < 1e-12 and rel(r["dF"][0], Fn.grad) < 1e-12
+
+    par = M.ALL["3d_humanoid_9_full"]
+    gr = G.build_graph(par)
+    p = {k: v.double().requires_grad_(True) for k, v in O.synth_params("actor", 2).items() if k.startswith("pos_encoder")}
+    B = 3
+    pos = O.pos_embedding(p, gr["traversals"]).repeat(B, 1)
+    dH = torch.randn(B * len(par), 128, generator=gen, dtype=torch.float64)
+    (pos * dH).sum().backward()
+    r = R.pos_embed_bwd_ref(dH, torch.stack(gr["traversals"], 1).repeat(B, 1))
+    for i in range(3):
+        assert rel(r[f"dE{i}"][0], p[f"pos_encoder.embeddings.{i}.weight"].grad) < 1e-12
+    assert rel(R.colsum_ref(dH, -0.5)["out"][0], -0.5 * dH.sum(0)) < TOL
+
+
+@pytest.mark.parametrize("actor", [True, False])
+def test_input_grad_ref_matches_per_token_formulas(actor):
+    """input_grad_ref (autograd of the summed linear terms) against the per-token formulas of input_grad_kernel's comment
+    (csrc/misc.cuh) written out element by element, on ragged graphs of 2, 5 and 16 limbs and L = 2."""
+    gen = torch.Generator().manual_seed(int(actor))
+    sizes, L, ng, ma = [2, 5, 16], 2, (17 if actor else 20), 2.5
+    cu = torch.tensor([0] + list(torch.tensor(sizes).cumsum(0)), dtype=torch.int32)
+    T = int(cu[-1])
+    rn = lambda *s: torch.randn(*s, generator=gen, dtype=torch.float64)
+    dvg0, dh0, dzh, dsh = rn(T, 3, 128), rn(T, 128), rn(T, 3, 32), rn(T, ng + 128)
+    dzh2 = rn(T, 3, 32) if actor else None
+    dz = [rn(T, 3, 32) for _ in range(3 * L)]
+    dog = [rn(T, 768) for _ in range(L)]
+    P = [rn(T, 2, 16).abs() for _ in range(L)]
+    Wg, We, gg = rn(128, 8), rn(128, ng), rn(30, 136)
+    gph = rn(30, 136) if actor else None
+    dout, w3 = rn(T, 3), rn(T, 3)
+    out = ma * torch.tanh(rn(T, 3))
+    got = R.input_grad_ref(dvg0, dh0, dzh, dzh2, dsh, dz, dog, P, Wg, We, gg, gph, dout if actor else None,
+                           out if actor else None, w3, ma, cu, L)["dobs"][0]
+    s = 128 ** 0.5
+    want = torch.zeros(T, 41, dtype=torch.float64)
+    for t in range(T):
+        g = int(torch.searchsorted(cu, torch.tensor(t, dtype=torch.int32), right=True)) - 1
+        t0, n = int(cu[g]), int(cu[g + 1] - cu[g])
+        dV0 = s * dvg0[t] @ Wg                                             # (3,8)
+        for dzx, W in ((dzh, gg), (dzh2, gph)):
+            if dzx is not None:
+                dV0 += dzx[t, :, :30] @ W[:, :8]
+                dV0[:, 1:3] += dzx[t, :, 30:32]
+        for d in dz:
+            dV0[:, 1:3] += d[t, :, 30:32]
+        for l in range(L):
+            for i in range(n):
+                for h in range(2):
+                    dV0[:, 1:3] += P[l][t0 + i, h, t - t0] * dog[l][t0 + i].view(3, 2, 128)[:, h, 126:128]
+        if actor:
+            a = out[t] / ma
+            dy = dout[t] * ma * (1 - a * a)
+            dV0[:, 5:8] += w3[t][:, None] * dy[None, :]
+        for r in range(3):
+            for j in range(8):
+                want[t, 3 * j + r] = dV0[r, j]
+        want[t, 24:] = s * dh0[t] @ We[:, :17] + dsh[t, :17]
+    assert rel(got, want) < 1e-12
+
+
+def test_fold_and_unfold_refs_follow_pack_indices():
+    """fold_ref's W' contracts the packed triangle of a symmetric G like vec(G) contracts W, and unfold_ref of dW' is the gradient
+    of that contraction w.r.t. W (the algebra of tests/test_fold_math.py, in the layout of sgrl_fold_sym / sgrl_unfold_sym)."""
+    from sgrl_b200.packing import pack_indices
+    gen = torch.Generator().manual_seed(9)
+    slots, ri, ci = pack_indices()
+    W = torch.randn(5, 1024, generator=gen, dtype=torch.float64).requires_grad_(True)
+    Z = torch.randn(4, 3, 32, generator=gen, dtype=torch.float64)
+    Gf, Gp = R.gram_packed(Z)
+    Wf = R.fold_ref(W.detach())
+    pad = sorted(set(range(544)) - set(slots))
+    assert torch.all(Wf[:, pad] == 0)
+    y = Gf.reshape(4, 1024) @ W.T
+    assert rel(Gp @ Wf.T, y.detach()) < 1e-13
+    dy = torch.randn(4, 5, generator=gen, dtype=torch.float64)
+    (y * dy).sum().backward()
+    assert rel(R.unfold_ref(dy.T @ Gp), W.grad) < 1e-13
