@@ -187,15 +187,15 @@ typedef struct {
   int32_t splitk, nb;
 } SgrlGemmProblem;
 /* n = 1..4 problems; n > 1 runs them like the networks' grouped projections (one launch when their kernel variants agree).
- * use_tc: 0 fp32 SIMT (n = 1, no rowsum / gd / gram), 1 tcgen05 3xTF32, 2 tcgen05 BF16-input.  sm2_ok / lat: the hints the
- * networks give the tile model (inference pass / critical chain).  Overrides of the tcgen05 planner, -1 = its model (every
+ * use_tc: 0 fp32 SIMT (n = 1, no rowsum / gd / gram), 1 tcgen05 3xTF32, 2 tcgen05 BF16-input.  sm2_ok: the hint the
+ * networks give the tile model (inference pass).  Overrides of the tcgen05 planner, -1 = its model (every
  * field -1: exactly the plan sgrl_gemm and the networks get): bn 64 | 128; split = atomic split-K factor (needs splitk > 1);
  * csk 0 | 2 | 3 cluster split-K ranks; sm2, persist, tma_store, group 0 | 1.  An override the shape or epilogue cannot take
  * is refused with nothing enqueued. */
 typedef struct {
   SgrlGemmProblem pr[4];
-  int32_t n, use_tc, sm2_ok, lat;
-  int32_t bn, split, csk, sm2, persist, tma_store, group, pad_;
+  int32_t n, use_tc, sm2_ok;
+  int32_t bn, split, csk, sm2, persist, tma_store, group;
 } SgrlGemmDesc;
 /* What was launched, per problem.  path: 0 SIMT tile kernel, 1 skinny kernel, 2 tcgen05.  split: atomic split-K factor
  * (sk_x: folded into blockIdx.x); cluster: cluster split-K ranks (1 = none); tma_c: TMA-store epilogue; epi: the epilogue
@@ -373,7 +373,7 @@ int sgrl_polyak_hp(float* target, const float* source, int nets, int64_t live_ne
 /* Call before recording an event on `stream` that another stream will wait on when the last work on `stream` was a
  * kernel of this library and the stream is not being captured: enqueues an empty non-programmatic launch (see
  * csrc/net.cuh, stream_fence: events recorded right after a programmatic-launch kernel did not reliably order the
- * waiting stream in eager execution).  No-op during stream capture or with SGRL_PDL=0. */
+ * waiting stream in eager execution).  No-op during stream capture. */
 int sgrl_stream_fence(sgrl_stream_t stream);
 
 /* Deterministic mode: enable = 1 / 0 switches it, -1 only queries; returns the previous state (default: environment

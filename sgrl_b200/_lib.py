@@ -76,9 +76,9 @@ class GemmProblem(C.Structure):
 
 
 class GemmDesc(C.Structure):
-    _fields_ = [("pr", GemmProblem * 4), ("n", C.c_int32), ("use_tc", C.c_int32), ("sm2_ok", C.c_int32), ("lat", C.c_int32),
+    _fields_ = [("pr", GemmProblem * 4), ("n", C.c_int32), ("use_tc", C.c_int32), ("sm2_ok", C.c_int32),
                 ("bn", C.c_int32), ("split", C.c_int32), ("csk", C.c_int32), ("sm2", C.c_int32), ("persist", C.c_int32),
-                ("tma_store", C.c_int32), ("group", C.c_int32), ("pad_", C.c_int32)]
+                ("tma_store", C.c_int32), ("group", C.c_int32)]
 
 
 GEMM_PLAN_FIELDS = ("path", "bn", "amn", "bmn", "bpre", "sm2", "gram", "persist", "split", "sk_x", "cluster", "tma_c", "epi")

@@ -495,8 +495,7 @@ inline int attention_fwd(const float* QKV, const float* VGP, const float* GD, fl
     attr_done = true;
   }
   const int nr = attn_rows(gr);
-  static const int v2 = getenv("SGRL_ATTN_V2") ? atoi(getenv("SGRL_ATTN_V2")) : 1;
-  if (v2 && gr.G >= 4 * NUM_SMS) {      // few graphs: one graph's latency is what counts and the first version's is shorter (18.4 vs 19.5 us at 256 graphs)
+  if (gr.G >= 4 * NUM_SMS) {      // few graphs: one graph's latency is what counts and the first version's is shorter (18.4 vs 19.5 us at 256 graphs)
     static int occ12 = 0, occ16 = 0;
     if (!occ12) {
       SGRL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ12, attention_fwd_v2_kernel<12>, A_FWD_THREADS, attn_fwd_v2_smem(12)));

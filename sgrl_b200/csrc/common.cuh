@@ -29,12 +29,8 @@ constexpr int MAX_NETS = 16;
 // with SGRL_PDL_ENTER(): "my dependents may start launching" + "wait until the kernel before me has completed and its
 // memory is visible".  A kernel's CTAs therefore get scheduled (and the tcgen05 GEMM runs its barrier/TMEM/tensor-map
 // prologue) while its predecessor is still draining, instead of paying the ~3 us kernel-to-kernel launch gap after it.
-// Nothing is read or written before the wait, so stream order semantics are unchanged.  SGRL_PDL=0 disables.
-extern int g_pdl;
-inline bool pdl_enabled() {
-  if (g_pdl < 0) { const char* e = getenv("SGRL_PDL"); g_pdl = e ? atoi(e) : 1; }
-  return g_pdl != 0;
-}
+// Nothing is read or written before the wait, so stream order semantics are unchanged.  The tcgen05 GEMM alone releases its
+// dependents later, once its accumulators are complete (gemm_tc_kernel).
 // ---- deterministic mode (SGRL_DETERMINISTIC=1 or sgrl_deterministic(1)): run-to-run bit-identical gradients.  The default
 // backward sums in an order that depends on timing in three places: split-K weight-gradient GEMMs (fp32 atomics), small
 // cross-CTA reductions (LayerNorm / positional / decoder / relative-bias weight gradients, the loss scalars) and the dF
@@ -50,18 +46,6 @@ inline bool det_enabled() {
 #define SGRL_PDL_TRIGGER() asm volatile("griddepcontrol.launch_dependents;" ::: "memory")
 #define SGRL_PDL_WAIT() asm volatile("griddepcontrol.wait;" ::: "memory")
 #define SGRL_PDL_ENTER() do { SGRL_PDL_TRIGGER(); SGRL_PDL_WAIT(); } while (0)
-// SGRL_PDL_LATE: 0 = every kernel releases its dependents at entry; 1 (default) = the tcgen05 GEMM releases them when its
-// accumulators are complete.  Measured on the B=256 update (profiles/r05c..e_pdl_late.txt): 5.36 / 5.11 ms; two further variants
-// that existed for the experiment — the small kernels never releasing early, and the GEMM never releasing explicitly either —
-// measured 5.15 / 5.13 ms and were removed again.
-inline int pdl_late_mode() { static const int m = getenv("SGRL_PDL_LATE") ? atoi(getenv("SGRL_PDL_LATE")) : 1; return m; }
-// streams on which kernels are launched WITHOUT the programmatic attribute (experiment knob SGRL_PDL_SIDE=0: the side lanes)
-extern cudaStream_t g_nopdl_streams[32];
-extern int g_nopdl_count;
-inline bool pdl_stream_ok(cudaStream_t st) {
-  for (int i = 0; i < g_nopdl_count; ++i) if (g_nopdl_streams[i] == st) return false;
-  return true;
-}
 template <typename... KArgs, typename... Args>
 inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg;
@@ -70,7 +54,7 @@ inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = (pdl_enabled() && pdl_stream_ok(st)) ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
   cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 // after a launch_k of the host launchers (misc.cuh, feature.cuh): count it, report its grid (grid nullable) and its launch error

@@ -32,9 +32,7 @@ struct GemmP {
   int vecA, vecB;                           // set by the launcher: operand rows may be fetched as float4
   const float* Bhi; const float* Blo;       // tcgen05 path only, optional: B pre-split into tf32 hi/lo parts (same layout/strides as B)
   int vecE;                                 // set by the tcgen05 launcher: C/mask/res rows allow float4 access
-  int pdl_late;                             // tcgen05 path: griddepcontrol.launch_dependents when the accumulators are complete instead of at entry (SGRL_PDL_LATE)
   int csk;                                  // tcgen05 path, set by the launcher: K is split over a (1, splitk, 1) cluster, rank 0 reduces through DSMEM
-  int lat;                                  // tcgen05 path: launch sits on the step's critical chain (target-network forwards, data gradients): tile model may use its own wave
   int sm2_ok;                               // tcgen05 path: the single-accumulator two-CTAs-per-SM variant may be used (inference passes only)
   long long* dbg;                           // optional (tools/gemm_trace.py): SM-clock timestamps of one CTA's pipeline phases
   int dbg_cta;                              // which CTA (blockIdx.x) writes them (SGRL_TRACE_CTA, default 0)

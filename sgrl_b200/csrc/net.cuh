@@ -44,20 +44,20 @@ inline WsLayout make_ws(int n_layers, long long T) {
 
 // ---- side streams: weight-gradient work (dW GEMMs, bias column sums) forks off the data-gradient chain ----------
 // fork = record an event on the main stream, make a side stream wait for it, launch there; join = main waits for
-// every side stream.  Under CUDA-graph capture this becomes plain fork/join edges of the graph.  SGRL_SIDE=0 disables.
+// every side stream.  Under CUDA-graph capture this becomes plain fork/join edges of the graph.
 // Measured on B200 (CUDA 12.9 / driver 580, tests/test_backward_gpu.py, humanoid B=100): with programmatic dependent launch
 // on, a cross-stream dependency built from cudaEventRecord (timing-disabled event) right after a kernel launched with the
 // programmatic attribute + cudaStreamWaitEvent does NOT reliably order the waiting stream after that kernel in EAGER
 // execution — a forked weight-gradient GEMM occasionally read a dY the data-gradient chain was still writing (errors of
-// 1e-4..6e-2 in a few layer-1 gradients, 3 runs out of 4; SGRL_PDL=0 or SGRL_SIDE=0 cured it).  A plain, non-programmatic
+// 1e-4..6e-2 in a few layer-1 gradients, 3 runs out of 4; without PDL or without side streams it did not happen).  A plain, non-programmatic
 // launch between the kernel and the event restores the ordering (0 failures in 4), so outside stream capture every fork /
 // join event is preceded by this empty kernel.  Inside a captured graph the same record/wait pairs become explicit full
-// dependency edges and no fence is needed (Agent.update's hot path is the replayed graph).  SGRL_FORK_FENCE=0 disables.
+// dependency edges and no fence is needed (Agent.update's hot path is the replayed graph).
 __global__ void fence_kernel() {}
 inline int stream_fence(cudaStream_t st) {
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   SGRL_CUDA(cudaStreamIsCapturing(st, &cs));
-  if (cs == cudaStreamCaptureStatusNone && pdl_enabled()) fence_kernel<<<1, 1, 0, st>>>();
+  if (cs == cudaStreamCaptureStatusNone) fence_kernel<<<1, 1, 0, st>>>();
   return 0;
 }
 struct SideSet {
@@ -68,17 +68,14 @@ struct SideSet {
 struct Side {
   static constexpr int NSETS = 8;          // one set per distinct main stream seen (main, the agent's two forward streams, a capture stream, ...)
   SideSet set[NSETS];
-  bool made = false; int enabled = -1; int nowners = 0; int fork_fence = 0;
+  bool made = false; int nowners = 0;
   int dev = -1;                            // device the lanes were created on: one process drives one GPU (DESIGN.md §6)
   int init() {
-    if (enabled < 0) { const char* e = getenv("SGRL_SIDE"); enabled = e ? atoi(e) : 1; }
-    if (enabled) {
-      int cur = -1;
-      SGRL_CUDA(cudaGetDevice(&cur));
-      if (!made) dev = cur;
-      SGRL_CHECK(cur == dev, "the library's side streams belong to another CUDA device: one process per GPU (set the device before the first call)");
-    }
-    if (!made && enabled) {              // everything is created up front: nothing but event record/wait happens later (capture-safe)
+    int cur = -1;
+    SGRL_CUDA(cudaGetDevice(&cur));
+    if (!made) dev = cur;
+    SGRL_CHECK(cur == dev, "the library's side streams belong to another CUDA device: one process per GPU (set the device before the first call)");
+    if (!made) {                         // everything is created up front: nothing but event record/wait happens later (capture-safe)
       for (int k = 0; k < NSETS; ++k) {
         for (int i = 0; i < SideSet::N; ++i) {
           SGRL_CUDA(cudaStreamCreateWithFlags(&set[k].s[i], cudaStreamNonBlocking));
@@ -88,11 +85,6 @@ struct Side {
         SGRL_CUDA(cudaEventCreateWithFlags(&set[k].fork_ev, cudaEventDisableTiming));
         set[k].rr = 0; set[k].owner = nullptr;
       }
-      { const char* e = getenv("SGRL_PDL_SIDE");
-        if (e && atoi(e) == 0)
-          for (int k = 0; k < NSETS && g_nopdl_count + SideSet::N <= 32; ++k)
-            for (int i = 0; i < SideSet::N; ++i) g_nopdl_streams[g_nopdl_count++] = set[k].s[i]; }
-      { const char* e = getenv("SGRL_FORK_FENCE"); fork_fence = e ? atoi(e) : 1; }
       made = true;
     }
     return 0;
@@ -108,8 +100,8 @@ struct Side {
   }
 };
 extern Side g_side;
-// no forks: side streams switched off, the bench's per-class timing pass, or deterministic mode (program order on one stream)
-inline bool side_off(const Side& sd) { return !sd.enabled || g_prof.on || det_enabled(); }
+// no forks: the bench's per-class timing pass, or deterministic mode (program order on one stream)
+inline bool side_off() { return g_prof.on || det_enabled(); }
 
 struct NetCtx {
   int kind, L, nb, T;
@@ -123,7 +115,6 @@ struct NetCtx {
   WsLayout wl; float* ws; long long zsW;
   AttnGraphs gr; const int* rank3;
   float max_action;
-  int bwd = 0;                            // set by net_backward (tile-model hint: data-gradient chain)
   int use_tc;                             // 0: fp32 SIMT; 1: eligible GEMMs on the tcgen05 kernel (3xTF32, fp32 parity); 2: tcgen05 in BF16-input mode
   cudaStream_t stream;
 
@@ -141,7 +132,6 @@ inline int run_gemm(const NetCtx& c, const GemmP& g, cudaStream_t st = nullptr) 
   if (c.use_tc && gemm_tc_eligible(g)) {
     GemmP gi = g;
     gi.sm2_ok = c.keep ? 0 : 1;
-    gi.lat = (!c.keep || c.bwd) ? 1 : 0;
     gi.prec = c.use_tc == 2 ? 1 : 0;      // use_tc 2: BF16-input mode (reported separately, never the default)
     return gemm_tc(gi, st);
   }
@@ -157,29 +147,29 @@ inline int run_gemm(const NetCtx& c, const GemmP& g, cudaStream_t st = nullptr) 
 // projection fills the machine by itself, as one launch each on the same stream (the two-CTAs-per-SM variant stays available).
 inline int run_group(const NetCtx& c, const GemmP* gs, int n, cudaStream_t st = nullptr) {
   if (!st) st = c.stream;
-  static const long long group_maxt = getenv("SGRL_GROUP_MAXT") ? atoll(getenv("SGRL_GROUP_MAXT")) : 32768;
-  bool all_tc = c.use_tc && n > 1 && (long long)c.T * c.nb <= group_maxt;
+  constexpr long long GROUP_MAXT = 32768;      // tokens x nets
+  bool all_tc = c.use_tc && n > 1 && (long long)c.T * c.nb <= GROUP_MAXT;
   for (int i = 0; i < n && all_tc; ++i) all_tc = gemm_tc_eligible(gs[i]);
   if (all_tc) {
     GemmP gp[TC_MAXG];
-    for (int i = 0; i < n; ++i) { gp[i] = gs[i]; gp[i].prec = c.use_tc == 2 ? 1 : 0; gp[i].lat = (!c.keep || c.bwd) ? 1 : 0; }
+    for (int i = 0; i < n; ++i) { gp[i] = gs[i]; gp[i].prec = c.use_tc == 2 ? 1 : 0; }
     return gemm_tc_group(gp, n, st);
   }
   for (int i = 0; i < n; ++i) SGRL_TRY(run_gemm(c, gs[i], st));
   return 0;
 }
 // stream for the next piece of weight-gradient work: a side stream that has been made to wait for everything
-// enqueued on the main stream so far (or the main stream itself when side streams are off / profiling is on)
+// enqueued on the main stream so far (or the main stream itself when side streams are off: side_off)
 // `from`: the stream whose work so far the forked stream must wait for (default: the main stream)
 inline int side_fork(const NetCtx& c, cudaStream_t* out, int lane = -1, cudaStream_t from = nullptr) {
   Side& sd = g_side;
-  if (side_off(sd)) { *out = c.stream; return 0; }
+  if (side_off()) { *out = c.stream; return 0; }
   SideSet& ss = sd.of(c.stream);
   int i = lane;
   if (i < 0) { i = 1 + ss.rr; ss.rr = (ss.rr + 1) % (SideSet::N - 1); }
   if (!from) from = c.stream;
   if (from == ss.s[i]) { *out = from; return 0; }      // same queue: already ordered
-  if (sd.fork_fence) SGRL_TRY(stream_fence(from));
+  SGRL_TRY(stream_fence(from));
   SGRL_CUDA(cudaEventRecord(ss.fork_ev, from));
   SGRL_CUDA(cudaStreamWaitEvent(ss.s[i], ss.fork_ev, 0));
   ss.used[i] = true;
@@ -189,11 +179,11 @@ inline int side_fork(const NetCtx& c, cudaStream_t* out, int lane = -1, cudaStre
 // lane < 0: every lane; else only that lane
 inline int side_join(const NetCtx& c, int lane = -1) {
   Side& sd = g_side;
-  if (side_off(sd)) return 0;
+  if (side_off()) return 0;
   SideSet& ss = sd.of(c.stream);
   for (int i = 0; i < SideSet::N; ++i) {
     if (!ss.used[i] || (lane >= 0 && i != lane)) continue;
-    if (sd.fork_fence) SGRL_TRY(stream_fence(ss.s[i]));
+    SGRL_TRY(stream_fence(ss.s[i]));
     SGRL_CUDA(cudaEventRecord(ss.join_ev[i], ss.s[i]));
     SGRL_CUDA(cudaStreamWaitEvent(c.stream, ss.join_ev[i], 0));
     ss.used[i] = false;
@@ -329,17 +319,13 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
   SGRL_TRY(g_side.init());
   cudaStream_t sb;                 // side stream of the independent branch of the moment (== st when side streams are off)
   // fused schedule: needs the pre-split weights (tcgen05 path) and enough rows for the N = 32 projections to be worth a tile
-  static const int fused_env = getenv("SGRL_FUSED") ? atoi(getenv("SGRL_FUSED")) : 1;
-  const bool fused = fused_env && c.use_tc && c.phi != nullptr && (long long)T3 * 32 * 128 >= (1 << 21);
+  const bool fused = c.use_tc && c.phi != nullptr && (long long)T3 * 32 * 128 >= (1 << 21);
   // triangle-folded vec(G) consumers of every layer: on the branch lane next to the embedding and the first projection, joined
-  // before the first Gram-generating GEMM reads them (SGRL_FOLD_SIDE=0: on the main chain)
-  static const int fold_side = getenv("SGRL_FOLD_SIDE") ? atoi(getenv("SGRL_FOLD_SIDE")) : 1;
-  bool fold_pending = false;
-  if (fused && fold_side) { SGRL_TRY(side_fork(c, &sb, 0)); SGRL_TRY(fold_weights(c, sb)); fold_pending = true; }
+  // before the first Gram-generating GEMM reads them
+  if (fused) { SGRL_TRY(side_fork(c, &sb, 0)); SGRL_TRY(fold_weights(c, sb)); }
   SGRL_TRY(embed_fwd_launch(obs, zsObs, c.kind == CRITIC ? act : nullptr, zsAct, c.rank3, c.P(Y.gp[G_GENC_W]), c.P(Y.gp[G_ENC_W]),
                             c.P(Y.gp[G_ENC_B]), c.P(Y.gp[G_POS0]), c.P(Y.gp[G_POS1]), c.P(Y.gp[G_POS2]), c.zsP, c.S(T_V0), c.S(T_GD), c.S(T_SH),
                             KS, c.SL(0, S_VGIN), c.SL(0, S_UA) + 128, 256, zS, T, ng, c.nb, c.in_nets, st));
-  if (fused && !fold_pending) SGRL_TRY(fold_weights(c, st));
   for (int l = 0; l < c.L; ++l) {
     const long long* lp = Y.lp[l];
     float* Vg = c.SL(l, S_VGIN);
@@ -366,7 +352,7 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
       GemmP gz = lin(c, Vg, 128, zS, lp[L_GPROJ], -1, c.SL(l, S_Z1), 32, zS, T3, 32, 128);
       gz.gdcols = c.S(T_GD); gz.zsGd = zS;
       SGRL_TRY(run_gemm(c, gz));
-      if (fold_pending) { SGRL_TRY(side_join(c, 0)); fold_pending = false; }
+      if (l == 0) SGRL_TRY(side_join(c, 0));
       GemmP g1 = lin_fold(c, nullptr, fold_offset(c.L, l, 0), lp[L_G1_B], c.SL(l, S_A1), 256, T, 256); g1.relu = 1;
       g1.gramZ = c.SL(l, S_Z1); g1.zsGramZ = zS; g1.gramF = c.SL(l, S_F1); g1.gramG = c.keep ? c.SL(l, S_G1) : nullptr;
       SGRL_TRY(run_gemm(c, g1));
@@ -472,10 +458,8 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
   fh.P1 = c.P(Y.gp[G_GG_W]); fh.P2 = c.kind == ACTOR ? c.P(Y.gp[G_GPH_W]) : nullptr; fh.zsP = c.zsP;
   fh.Z = c.S(T_ZH); fh.Z2 = c.kind == ACTOR ? c.S(T_ZH2) : nullptr; fh.G = c.S(T_GH); fh.Fn = c.S(T_FH); fh.zsAct = zS; fh.T = T; fh.nb = c.nb;
   // the scalar branch u[:, 128:] = linear2_ng(relu(linear1_ng([s0 | h]))) only needs the final norm: on the branch lane, next to
-  // the invariant branch K1 -> linear1_g -> linear2_g (3 instead of 5 dependent launches; SGRL_HEAD_SIDE=0: one after the other)
-  static const int head_side = getenv("SGRL_HEAD_SIDE") ? atoi(getenv("SGRL_HEAD_SIDE")) : 1;
-  sb = st;
-  if (head_side) SGRL_TRY(side_fork(c, &sb, 0));
+  // the invariant branch K1 -> linear1_g -> linear2_g (3 instead of 5 dependent launches)
+  SGRL_TRY(side_fork(c, &sb, 0));
   GemmP g = lin(c, c.S(T_SH), KS, zS, Y.gp[G_H1NG_W], Y.gp[G_H1NG_B], c.S(T_BH), 128, zS, T, 128, KS); g.relu = 1;
   SGRL_TRY(run_gemm(c, g, sb));
   g = lin(c, c.S(T_BH), 128, zS, Y.gp[G_H2NG_W], Y.gp[G_H2NG_B], c.S(T_UH) + 128, 256, zS, T, 128, 128);
@@ -485,7 +469,7 @@ inline int net_forward(const NetCtx& c, const float* obs, long long zsObs, const
   SGRL_TRY(run_gemm(c, g));
   g = lin(c, c.S(T_AH), 128, zS, Y.gp[G_H2G_W], Y.gp[G_H2G_B], c.S(T_UH), 256, zS, T, 128, 128);
   SGRL_TRY(run_gemm(c, g));
-  if (head_side) SGRL_TRY(side_join(c, 0));
+  SGRL_TRY(side_join(c, 0));
   if (c.kind == CRITIC) {
     g = lin(c, c.S(T_UH), 256, zS, Y.gp[G_DNG_W], Y.gp[G_DNG_B], c.S(T_OUT), 1, zS, T, 1, 256);
     g.rowdiv = c.S(T_FH); g.zsRow = zS;
@@ -537,9 +521,8 @@ inline int input_grad(const NetCtx& c, const float* dOut, long long zsDo, float*
   return input_grad_launch(p, c.nb, c.stream);
 }
 
-inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, int need_wgrad, float* dact, long long zsDact,
+inline int net_backward(const NetCtx& c, const float* dOut, long long zsDo, int need_wgrad, float* dact, long long zsDact,
                         float* dobs = nullptr, long long zsDobs = 0) {
-  NetCtx c = c_in; c.bwd = 1;
   const int T = c.T, T3 = 3 * c.T, ng = c.ng(), KS = c.ks();
   const NetLayout& Y = c.lay;
   cudaStream_t st = c.stream;
@@ -598,10 +581,9 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     SGRL_TRY(run_gemm(c, g));
   }
   // ---- branch lane (hb): the scalar branch u[:, 128:] = linear2_ng(relu(linear1_ng([s0 | h]))) and the final LayerNorm, next to
-  // the invariant branch below (both start from dUH; SGRL_HEAD_SIDE=0: one after the other on the main stream)
-  static const int head_side = getenv("SGRL_HEAD_SIDE") ? atoi(getenv("SGRL_HEAD_SIDE")) : 1;
-  cudaStream_t hb = st;
-  if (head_side) SGRL_TRY(side_fork(c, &hb, 0));
+  // the invariant branch below (both start from dUH)
+  cudaStream_t hb;
+  SGRL_TRY(side_fork(c, &hb, 0));
   SGRL_TRY(side_w(W(W_DUH) + 128, 256, c.S(T_BH), 128, zS, Y.gp[G_H2NG_W], 128, T, 128, 128, Y.gp[G_H2NG_B]));
   g = dgrad(c, W(W_DUH) + 128, 256, Y.gp[G_H2NG_W], 128, W(W_DA3), 128, T, 128, 128);
   g.mask = c.S(T_BH); g.zsMask = zS; g.ldmask = 128;
@@ -634,7 +616,7 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     SGRL_TRY(side_w(W(W_DZ3), 32, c.S(T_V0), 8, zS, Y.gp[G_GPH_W], D + GN, T3, NPJ, GN));
     SGRL_TRY(side_w(W(W_DZ3), 32, c.S(T_VGF), 128, zS, Y.gp[G_GPH_W] + GN, D + GN, T3, NPJ, 128));
   }
-  if (head_side) SGRL_TRY(side_join(c, 0));
+  SGRL_TRY(side_join(c, 0));
 
   // ---------------------------------------------------------------- encoder layers (frame l reads frame l+1)
   for (int l = c.L - 1; l >= 0; --l) {
@@ -650,13 +632,11 @@ inline int net_backward(const NetCtx& c_in, const float* dOut, long long zsDo, i
     // incoming dh: the final norm's output for the last layer; below it, dx1 + du[:, 128:] of the layer above, summed here
     // instead of by a copy kernel at the end of that layer
     // ... with the backward of f = linear2(..)/F2 on the same rows: dFF = dx / F2, dF2 -= <dx, f> / F2 (dx itself stays: LN1's residual)
-    static const int ln_rd = getenv("SGRL_LN_ROWDIV") ? atoi(getenv("SGRL_LN_ROWDIV")) : 1;
-    const LnRowdiv rd = ln_rd ? LnRowdiv{c.SL(l, S_FF), c.SL(l, S_F2), W(W_DF2), W(W_DFF), 128, 128} : LnRowdiv{nullptr, nullptr, nullptr, nullptr, 0, 0};
+    const LnRowdiv rd{c.SL(l, S_FF), c.SL(l, S_F2), W(W_DF2), W(W_DFF), 128, 128};
     if (l == c.L - 1)
       SGRL_TRY(layernorm_bwd(c, Wn(W_DH), 128, nullptr, 0, c.SL(l, S_X2), 128, c.SL(l, S_ST2), lp[L_N2_W], lp[L_N2_B], W(W_DX), 128, wg, sb, rd));
     else
       SGRL_TRY(layernorm_bwd(c, Wn(W_DH1), 128, Wn(W_DUA) + 128, 256, c.SL(l, S_X2), 128, c.SL(l, S_ST2), lp[L_N2_W], lp[L_N2_B], W(W_DX), 128, wg, sb, rd));
-    if (!ln_rd) SGRL_TRY(rowdiv_bwd(c, W(W_DFF), 128, c.SL(l, S_FF), 128, c.SL(l, S_F2), W(W_DF2), 128, 1.f, 0, sb, W(W_DX), 128, zW));    // reads dx (kept: LN1's residual), writes dFF
     SGRL_TRY(side_w(W(W_DFF), 128, T31 + 256, 512, zS, lp[L_L2_W], 256, T, 128, 256, lp[L_L2_B], 1.f, sb));
     g = dgrad(c, W(W_DFF), 128, lp[L_L2_W], 256, W(W_DT31) + 256, 512, T, 128, 256);
     g.mask = T31 + 256; g.zsMask = zS; g.ldmask = 512;

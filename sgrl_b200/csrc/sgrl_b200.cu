@@ -11,10 +11,7 @@ thread_local char g_err[512] = "";
 long long g_launches = 0;
 Prof g_prof;
 long long* g_gemm_trace = nullptr;
-int g_pdl = -1;
 int g_det = -1;
-cudaStream_t g_nopdl_streams[32];
-int g_nopdl_count = 0;
 Side g_side;
 }
 using namespace sgrl;
@@ -23,7 +20,7 @@ using namespace sgrl;
 
 extern "C" {
 
-int sgrl_version(void) { return 11; }
+int sgrl_version(void) { return 12; }
 const char* sgrl_last_error(void) { return g_err; }
 
 long long sgrl_launch_count(void) { return g_launches; }
@@ -417,7 +414,7 @@ int sgrl_gemm_desc(const SgrlGemmDesc* d, SgrlGemmPlanInfo* info, sgrl_stream_t 
     p.accumulate = s.accumulate != 0; p.splitk = det_enabled() ? 1 : s.splitk;
     p.rowsum = s.rowsum; p.zsRowsum = s.zs_rowsum; p.gdcols = s.gd; p.zsGd = s.zs_gd;
     p.gramZ = s.gram_z; p.zsGramZ = s.zs_gram_z; p.gramF = s.gram_f; p.gramG = s.gram_g;
-    p.sm2_ok = d->sm2_ok != 0; p.lat = d->lat != 0; p.prec = d->use_tc == 2 ? 1 : 0;
+    p.sm2_ok = d->sm2_ok != 0; p.prec = d->use_tc == 2 ? 1 : 0;
   }
   TcPlanInfo rep[TC_MAXG];
   memset(rep, 0, sizeof(rep));
@@ -446,6 +443,7 @@ int sgrl_gemm_desc(const SgrlGemmDesc* d, SgrlGemmPlanInfo* info, sgrl_stream_t 
   return 0;
 }
 static_assert(sizeof(SgrlGemmPlan) == sizeof(TcPlanInfo), "SgrlGemmPlan mirrors TcPlanInfo");
+static_assert(sizeof(SgrlGemmDesc) == 4 * sizeof(SgrlGemmProblem) + 40, "SgrlGemmDesc: the layout _lib.GemmDesc mirrors");
 
 int sgrl_gemm_gram(const float* Z, const float* W_hi, const float* W_lo, const float* bias, float* C, int ldc, float* F, float* G,
                    int T, int N, int relu, sgrl_stream_t stream) {

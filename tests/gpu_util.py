@@ -19,6 +19,26 @@ def make_modules(seed=parity.WEIGHT_SEED, use_tc=1):
     return actor, critic, pa, pc
 
 
+def gemm_desc(persist, **pr):
+    """One problem through sgrl_gemm_desc on the tcgen05 3xTF32 path, the planner's model everywhere but the persist override
+    (0 | 1).  pr: SgrlGemmProblem fields (tensors for pointers; alpha, colscale, splitk, nb default to 1).  Returns the plan the
+    library reports for the problem."""
+    import ctypes
+    from sgrl_b200._lib import GEMM_PLAN_FIELDS, GemmDesc, GemmPlanInfo, lib, ptr, stream, check
+    d = GemmDesc()
+    d.n, d.use_tc, d.persist = 1, 1, persist
+    for f in ("bn", "split", "csk", "sm2", "tma_store", "group"):
+        setattr(d, f, -1)
+    p = d.pr[0]
+    p.alpha, p.colscale, p.splitk, p.nb = 1.0, 1.0, 1, 1
+    for k, v in pr.items():
+        setattr(p, k, ptr(v) if torch.is_tensor(v) or v is None else v)
+    info = GemmPlanInfo()
+    check(lib.sgrl_gemm_desc(ctypes.byref(d), ctypes.byref(info), stream()), "sgrl_gemm_desc")
+    torch.cuda.synchronize()
+    return {f: getattr(info.pr[0], f) for f in GEMM_PLAN_FIELDS}
+
+
 def to_cuda(d):
     return {k: (v.cuda() if torch.is_tensor(v) else [t.cuda() for t in v] if isinstance(v, list) and v and torch.is_tensor(v[0]) else v) for k, v in d.items()}
 

@@ -270,8 +270,10 @@ def test_single_kernel_entry_points_refuse_bad_arguments(name, over, msg):
     assert rc < 0 and msg in _lib.lib.sgrl_last_error(), _lib.lib.sgrl_last_error()
 
 
-def test_single_kernel_entry_points_are_abi_11():
+def test_single_kernel_entry_points_are_abi_12():
     from sgrl_b200 import _lib
-    assert _lib.lib.sgrl_version() == 11
+    assert _lib.lib.sgrl_version() == 12
     for name, args in _ARGS.items():
         assert len(getattr(_lib.lib, name).argtypes) == len(args) + 2, name
+    # SgrlGemmDesc: four problems and ten int32 fields (n, use_tc, sm2_ok and the seven planner overrides); the library asserts the same size
+    assert ctypes.sizeof(_lib.GemmDesc) == 4 * ctypes.sizeof(_lib.GemmProblem) + 40

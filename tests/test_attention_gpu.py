@@ -10,7 +10,6 @@ tests/kernel_ref.py, in every launch regime the update and the rollout reach:
 Errors are taken per graph (the worst graph of the batch, not the batch norm: one wrong graph out of thousands moves a
 batch norm by little), outputs are NaN-prefilled with pad rows past T that must stay untouched, and each regime case
 asserts from a torch.profiler trace which kernel ran, so that a change of the 592 threshold cannot make it vacuous."""
-import os
 
 import pytest
 import torch
@@ -21,7 +20,6 @@ import kernel_ref as R
 pytestmark = pytest.mark.gpu
 
 PAD = 5                  # sentinel rows past T in every output buffer
-V2_OFF = os.environ.get("SGRL_ATTN_V2", "1").strip() == "0"
 V2_MIN = 4 * 148         # the graph count from which the forward runs the second version
 TOL_GRAPH = 1e-5         # worst graph, relative (o, og, dqkv, dvgp)
 TOL_P = 1e-6             # probabilities, absolute
@@ -182,11 +180,6 @@ def assert_kernel(names, want):
     assert names and all(want in n for n in names), f"expected {want}, the trace shows {names}"
 
 
-def skip_if_v2_off(G):
-    if G >= V2_MIN and V2_OFF:
-        pytest.skip("SGRL_ATTN_V2=0 in the environment: the second forward version is switched off")
-
-
 # ---------------------------------------------------------------------------------------------------------------- regimes
 REGIMES = [1, 148, 149, 591, 592, 2400, 6000]
 
@@ -195,7 +188,6 @@ REGIMES = [1, 148, 149, 591, 592, 2400, 6000]
 @pytest.mark.parametrize("G", REGIMES)
 def test_regime_forward_backward(G, wide):
     """Ragged graphs with a per-graph relation table: forward (P stored) and backward on the kernel's own P."""
-    skip_if_v2_off(G)
     must = (16, 13, 15, 14) if wide else (12, 2, 11)
     sizes = ragged_sizes(G, 1, 16 if wide else 12, seed=G * 2 + wide, must=must)
     c = make_case(sizes, seed=G + 17 * wide)
@@ -212,7 +204,6 @@ def test_regime_forward_backward(G, wide):
 @pytest.mark.parametrize("n", list(range(1, 17)))
 def test_uniform_limb_count(n, G):
     """Each n = 1..16 as a uniform batch (n = 1: the softmax of one key is 1; n = 16: a full tile), both versions."""
-    skip_if_v2_off(G)
     c = make_case([n] * G, seed=100 + n)
     names = []
     o, og, p = run_fwd(c, kernels=names)
@@ -226,7 +217,6 @@ def test_uniform_limb_count(n, G):
 @pytest.mark.parametrize("bias", [None, "ragged", "null"])
 @pytest.mark.parametrize("G", [300, 2400])
 def test_relation_bias_variants(bias, G):
-    skip_if_v2_off(G)
     c = make_case(ragged_sizes(G, 2, 16, seed=5, must=(16,)), seed=6, bias=bias)
     o, og, p = run_fwd(c)
     check_fwd(c, o, og, p)
@@ -238,7 +228,6 @@ def test_max_limbs_hint():
     """The hint sizes the staging and picks NR: exact, 0 (unknown -> 16) and larger than needed all compute the same.
     12-limb graphs with hint 12 run NR = 12 and with hint 13 NR = 16; 9-limb graphs with hint 9 vs 0 likewise.  The
     accumulator rows only change which registers hold the sums, not their arithmetic: the results are bit-identical."""
-    skip_if_v2_off(V2_MIN)
     for n, hints in ((12, (12, 13, 0, 16)), (9, (9, 0, 14))):
         c = make_case(ragged_sizes(700, 1, n, seed=n, must=(n,)), seed=n, bias=None)
         outs = []
@@ -262,7 +251,6 @@ def test_v1_v2_same_arithmetic(bias):
     """v1 and v2 accumulate in the same order: graphs 0..590 launched as 591 graphs (v1) and with one more graph (v2)
     give bit-identical o, og and p without a bias.  With the bias, `wr . rr + br` is a short expression whose fp
     contraction into FMAs may differ between the two kernels: there the outputs agree to a few ulp of fp32."""
-    skip_if_v2_off(V2_MIN)
     sizes = ragged_sizes(V2_MIN, 1, 16, seed=11, must=(16, 13))
     full = make_case(sizes, seed=12, bias=bias)
     part = dict(full, G=V2_MIN - 1, T=int(full["cu"][V2_MIN - 1]), sizes=sizes[:-1], cu=full["cu"][:V2_MIN],
@@ -283,7 +271,6 @@ def test_v1_v2_same_arithmetic(bias):
 @pytest.mark.parametrize("G", [300, 2400])
 def test_inference_pass_without_p(G):
     """p = NULL (the rollout's inference pass): the same o and og, bit for bit, as the launch that stores P."""
-    skip_if_v2_off(G)
     c = make_case(ragged_sizes(G, 2, 16, seed=21, must=(16,)), seed=22)
     o, og, _ = run_fwd(c)
     names = []
@@ -296,8 +283,6 @@ def test_inference_pass_without_p(G):
 def test_large_logits():
     """Scores of order +-100: the max subtraction keeps every output finite and P within 1e-4 of fp64 per element."""
     for G in (300, 2400):
-        if G >= V2_MIN and V2_OFF:
-            continue
         c = make_case(ragged_sizes(G, 1, 16, seed=31, must=(16,)), seed=32, score_scale=100.0)
         o, og, p = run_fwd(c)
         _, _, rp = ref_fwd(c)

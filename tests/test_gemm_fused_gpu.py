@@ -58,10 +58,12 @@ def test_gram_gemm(T, N, keep):
 
 
 @pytest.mark.parametrize("T,N", [(40000, 256), (38001, 128), (60000, 256)])
-def test_gram_gemm_persistent(monkeypatch, T, N):
+def test_gram_gemm_persistent(T, N):
     """Persistent GRAM projection of inference passes (csrc/gemm_tc_persist.cuh: all N <= 256 columns in one tile, every packed Gram
-    row generated once) against fp64 and against the per-tile kernel; row tail, sub-matrix ldc, F = ||G|| + 1."""
-    from sgrl_b200._lib import lib, ptr, stream, check
+    row generated once) against fp64 and against the per-tile kernel, each selected by the persist override of sgrl_gemm_desc;
+    row tail, sub-matrix ldc, F = ||G|| + 1."""
+    from gpu_util import gemm_desc
+    from sgrl_b200.packing import GP_K
     g = torch.Generator(device="cuda").manual_seed(T + N)
     Z = torch.randn(T, 3, 32, device="cuda", generator=g)
     Z[:, :, 30] = torch.tensor([0.0, 0.0, -9.81], device="cuda")
@@ -69,12 +71,12 @@ def test_gram_gemm_persistent(monkeypatch, T, N):
     b = torch.randn(N, device="cuda", generator=g)
     hi, lo = split(fold(W).contiguous())
     out = []
-    for mode in ("2", "0"):
-        monkeypatch.setenv("SGRL_TC_PERSIST", mode)
+    for persist in (1, 0):
         Cm = torch.full((T, N + 4), 7.0, device="cuda")
         F = torch.zeros(T, device="cuda")
-        check(lib.sgrl_gemm_gram(ptr(Z), ptr(hi), ptr(lo), ptr(b), ptr(Cm), N + 4, ptr(F), None, T, N, 1, stream()), "gram")
-        torch.cuda.synchronize()
+        plan = gemm_desc(persist, A=None, gram_z=Z, gram_f=F, B=hi, B_hi=hi, B_lo=lo, ldb=GP_K, C=Cm, ldc=N + 4, M=T, N=N, K=GP_K,
+                         bias=b, relu=1)
+        assert plan["path"] == 2 and plan["gram"] == 1 and plan["persist"] == persist, plan
         out.append((Cm, F))
     Zd = Z.double()
     G = Zd.transpose(1, 2) @ Zd

@@ -101,12 +101,12 @@ def test_presplit_weights(M, N, K, tb):
 
 @pytest.mark.parametrize("M,N,K,rowdiv,relu", [(40000, 768, 256, 1, 0), (38017, 252, 128, 0, 0), (40000, 128, 256, 0, 1), (37990, 1024, 384, 1, 1),
                                                (150000, 512, 256, 0, 1)])
-def test_persistent_projection_kernel(monkeypatch, M, N, K, rowdiv, relu):
+def test_persistent_projection_kernel(M, N, K, rowdiv, relu):
     """Persistent inference variant (csrc/gemm_tc_persist.cuh: tile loop per SM, two accumulator buffers, TMA tensor stores) against
     fp64: row / column tails, the /F + column-scale and relu epilogues, sub-matrix ldc with untouched neighbours, more tiles than
-    two rounds of the 148 SMs.  SGRL_TC_PERSIST=2 selects it for a caller that did not flag an inference pass."""
+    two rounds of the 148 SMs; and against the per-tile kernel, each selected by the persist override of sgrl_gemm_desc."""
     from sgrl_b200._lib import lib, ptr, stream, check
-    monkeypatch.setenv("SGRL_TC_PERSIST", "2")
+    from gpu_util import gemm_desc
     g = torch.Generator(device="cuda").manual_seed(M + N + K)
     X = torch.randn(M, K, device="cuda", generator=g)
     W = torch.randn(N, K, device="cuda", generator=g) / K ** 0.5
@@ -114,10 +114,15 @@ def test_persistent_projection_kernel(monkeypatch, M, N, K, rowdiv, relu):
     check(lib.sgrl_split_tf32(ptr(W), ptr(hi), ptr(lo), W.numel(), stream()))
     b = torch.randn(N, device="cuda", generator=g)
     F = torch.rand(M, device="cuda", generator=g) * 500 + 100
-    Y = torch.full((M, N + 4), 7.0, device="cuda")
+
+    def run(persist):
+        Y = torch.full((M, N + 4), 7.0, device="cuda")
+        plan = gemm_desc(persist, A=X, lda=K, B=hi, B_hi=hi, B_lo=lo, ldb=K, C=Y, ldc=N + 4, M=M, N=N, K=K, bias=b,
+                         rowdiv=F if rowdiv else None, relu=relu)
+        assert plan["path"] == 2 and plan["persist"] == persist, plan
+        return Y
     n0 = lib.sgrl_launch_count()
-    check(lib.sgrl_gemm_presplit(ptr(X), K, 0, ptr(hi), ptr(lo), K, 0, ptr(Y), N + 4, M, N, K, 1.0, ptr(b), ptr(F) if rowdiv else None, relu, 0, 1, stream()))
-    torch.cuda.synchronize()
+    Y = run(1)
     assert lib.sgrl_launch_count() == n0 + 1
     ref = X.double() @ W.double().T + b.double()
     if relu:
@@ -126,10 +131,7 @@ def test_persistent_projection_kernel(monkeypatch, M, N, K, rowdiv, relu):
         ref = ref / F.double()[:, None]
     assert rel(Y[:, :N], ref) < TOL[1]
     assert torch.all(Y[:, N:] == 7.0)
-    monkeypatch.setenv("SGRL_TC_PERSIST", "0")
-    Y2 = torch.full((M, N + 4), 7.0, device="cuda")
-    check(lib.sgrl_gemm_presplit(ptr(X), K, 0, ptr(hi), ptr(lo), K, 0, ptr(Y2), N + 4, M, N, K, 1.0, ptr(b), ptr(F) if rowdiv else None, relu, 0, 1, stream()))
-    torch.cuda.synchronize()
+    Y2 = run(0)
     assert rel(Y2[:, :N], ref) < TOL[1] and rel(Y[:, :N], Y2[:, :N]) < 1e-5
 
 

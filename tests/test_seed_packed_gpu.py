@@ -322,7 +322,8 @@ def test_draws_are_those_of_agents_in_seed_order(allow_duplicate):
 
 def test_one_plan_one_launch_and_launches_do_not_grow():
     """Both methods share one plan; a replayed step makes one library launch outside the graph (the gather); below
-    SGRL_GROUP_MAXT the captured graphs hold as many library launches for K = 4 as for K = 1."""
+    the grouped-projection size (32 768 tokens x nets, run_group in csrc/net.cuh) the captured graphs hold as many library
+    launches for K = 4 as for K = 1."""
     from sgrl_b200.seed_batch import SeedBatchedAgent
     B, plans = 32, {}
     with warnings.catch_warnings():

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Device time of one pre-split tcgen05 projection (K-major operands), CUDA events over `reps` back-to-back launches.
-usage: gemm_time.py M N K [rowdiv] [reps]   (variant / tile knobs come from the SGRL_TC_* environment)"""
+usage: gemm_time.py M N K [rowdiv] [reps]   (the plan the library's tile model picks for the shape)"""
 import os
 import sys
 
